@@ -24,6 +24,11 @@ configuration alone; `--no-subrecords` keeps the line to the main workload.
 `--impl reference` times that CPU path alone with all host threads (the reference itself needs
 ROS + PCL and cannot be built in this image).
 
+`--steps` is the number of timed steps of every measurement in the run (sub-records and config 5 too).
+`--dump-outputs DIR` writes what the device-resident path returned in its last timed step of the main
+configuration (see dump_outputs) as DIR/<name>.npy; the inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
+
 Multi-GPU: scans are independent, so every rank processes its own batch (weak scaling) with no
 data-path collective; torch.distributed is only the barrier and the max-over-ranks of the time.
 """
@@ -62,7 +67,13 @@ def parse():
     ap.add_argument("--scans", type=int, default=0, help="scans per GPU per step (default: the config's batch)")
     ap.add_argument("--cpu-sample", type=int, default=1536, help="scans of the CPU baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.in_process or args.config == 5):
+        ap.error("--dump-outputs writes the device-resident path of configs 1-4")
+    return args
 
 
 def default_scans(cfg):
@@ -272,9 +283,34 @@ def descriptor_parity(dg, d_o):
             "rows_beyond_1e-5": int((rows > 1e-5).sum()), "max_rel_err": float(rows.max()) if len(rows) else 0.0}
 
 
-def measure(job, cfg, B, steps, warmup, cpu_sample=0, packed=False):
+DUMP_MAX_BYTES = 64 << 20
+DUMP_DESCRIPTOR_ROWS = 4096  # 32 MB of descriptors; a batch of 10k scans has ~37k keypoints (290 MB)
+
+
+def dump_outputs(out_dir, node, ko, K, p_kp, p_d):
+    """What a caller of processBatchDevice receives, copied to the host: keypoint_offsets (B+1,) as
+    float64, keypoints (K,4) float32, and the (n,1980) float32 descriptors of `descriptor_rows`: every
+    keypoint, or a sample of DUMP_DESCRIPTOR_ROWS of them drawn with a fixed seed when there are more."""
+    from feature_extraction_b200.node import DESC_LEN
+    arrays = {"keypoint_offsets": ko.astype(np.float64), "keypoints": node.download(p_kp, (K, 4))}
+    if p_d:
+        rows = np.arange(K)
+        if K > DUMP_DESCRIPTOR_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(K, DUMP_DESCRIPTOR_ROWS, replace=False))
+        arrays["descriptors"] = node.download(p_d, (K, DESC_LEN))[rows]
+        arrays["descriptor_rows"] = rows.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed %d; use fewer --scans" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(job, cfg, B, steps, warmup, cpu_sample=0, packed=False, dump_dir=None):
     """One configuration on every rank (each its own B scans): device-resident value, per-stage times and
-    roofline, e2e through the host entry point, optional 1-thread CPU baseline (rank 0 of a 1-GPU job)."""
+    roofline, e2e through the host entry point, optional 1-thread CPU baseline (rank 0 of a 1-GPU job).
+    With `dump_dir`, rank 0 writes the results of its last timed device-resident step there."""
     torch = job.torch
     from feature_extraction_b200 import FeatureExtractionNode, PinnedBuffer, synth
     A = synth.default_azimuth_steps(cfg)
@@ -304,6 +340,8 @@ def measure(job, cfg, B, steps, warmup, cpu_sample=0, packed=False):
     wall_ms = (time.perf_counter() - t0) * 1e3
     ms_step = job.max_over_ranks(ev_ms / steps)
     value = job.world * B / (ms_step * 1e-3)
+    if dump_dir and job.rank == 0:
+        dump_outputs(dump_dir, dev_node, ko, K, p_kp, p_d)  # before the stage-timing steps overwrite the results
     stats = dev_node.batchStats()
     # Per-kernel durations for the roofline: the same steps repeated right here with the stages serialised
     # (fe_enable_stage_timing) and every stage bracketed by CUDA events on the launching stream.
@@ -647,7 +685,7 @@ def main():
     sampler.start()
 
     if cfg == 5:
-        sw = measure_sweep(job, args.sweep_scans, max(1, min(args.steps, 3)), max(1, min(args.warmup, 1)))
+        sw = measure_sweep(job, args.sweep_scans, args.steps, max(1, min(args.warmup, 1)))
         clocks = sampler.stop()
         if job.rank == 0:
             out = {"metric": "scans/sec", "value": sw["value"], "unit": "scans/s", "n_gpus": job.world, "steps": sw["steps"], "warmup": sw["warmup"],
@@ -663,7 +701,7 @@ def main():
 
     B = args.scans or default_scans(cfg)
     want_cpu = 0 if args.no_cpu_baseline else args.cpu_sample
-    m = measure(job, cfg, B, args.steps, args.warmup, cpu_sample=want_cpu, packed=True)
+    m = measure(job, cfg, B, args.steps, args.warmup, cpu_sample=want_cpu, packed=True, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if (args.config or args.no_subrecords) else None
     out = {"metric": "scans/sec", "value": m["value"], "unit": "scans/s", "n_gpus": job.world, "steps": args.steps, "warmup": args.warmup,
            "ms_per_step": m["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic"}
@@ -677,9 +715,9 @@ def main():
     # ---- the other BASELINE.json configurations, in the same run (sub-records) ----
     if not args.config and not args.no_subrecords:
         subs = {}
-        for c, st, wu, cs in ((1, 200, 20, 96), (3, 5, 3, 96), (4, 5, 3, 96)):
+        for c, wu, cs in ((1, 20, 96), (3, 3, 96), (4, 3, 96)):
             try:
-                r = measure(job, c, default_scans(c), min(st, max(args.steps, 1) * 10), wu, cpu_sample=(0 if args.no_cpu_baseline else cs))
+                r = measure(job, c, default_scans(c), args.steps, wu, cpu_sample=(0 if args.no_cpu_baseline else cs))
                 for k in ("kernels",):  # keep the line readable: stage times only
                     r[k] = {nm: {"ms": v["ms"], "frac": v["frac"]} for nm, v in r[k].items()}
                 subs[str(c)] = r
@@ -687,7 +725,7 @@ def main():
                 subs[str(c)] = {"error": repr(e)[:300]}
         out["configs"] = subs
         try:
-            out["config5"] = measure_sweep(job, args.sweep_scans, 2, 1)
+            out["config5"] = measure_sweep(job, args.sweep_scans, args.steps, 1)
         except Exception as e:
             out["config5"] = {"error": repr(e)[:300]}
         clocks = sampler.stop()

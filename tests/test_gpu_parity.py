@@ -439,3 +439,21 @@ def test_lean_chain_runs_a_deferring_scan_again_with_the_fallback_kernels(ob, sy
         ko, kp, d = nd.processBatch(sc0, one, rp[0:1])
         assert bits_equal(kp, w0["keypoints"]) and bits_equal(d, w0["descriptors"])
     nd.close()
+
+
+def test_bench_dump_outputs_are_the_oracles_results(ob, synth, tmp_path):
+    """bench.py --dump-outputs: the device-resident results of the last timed step of the main configuration,
+    float32/float64 .npy files, equal to the oracle's on the batch the bench generates (rank 0: scans 0..B-1)."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--config", "4", "--scans", "6", "--steps", "2", "--warmup", "1",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    got = {n: np.load(tmp_path / (n + ".npy")) for n in ("keypoint_offsets", "keypoints", "descriptors", "descriptor_rows")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    pts, offs, rp = synth.generate(4, 6)
+    ko_o, kp_o, d_o, _ = ob.process_batch(_params(ob, 4), pts, offs, rp, mode=1, n_threads=4)
+    assert len(kp_o) > 0 and np.array_equal(got["keypoint_offsets"], ko_o) and bits_equal(got["keypoints"], kp_o)
+    assert np.array_equal(got["descriptor_rows"], np.arange(len(kp_o))) and bits_equal(got["descriptors"], d_o)

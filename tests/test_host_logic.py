@@ -191,6 +191,48 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert "workload" in d["config"]
 
 
+def test_bench_rejects_zero_steps_and_dumps_outside_the_device_path():
+    import subprocess
+    import sys
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "x"], ["--config", "5", "--dump-outputs", "x"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120)
+        assert out.returncode == 2 and "error:" in out.stderr, (extra, out.stderr[-2000:])
+
+
+def test_bench_dump_outputs_samples_descriptor_rows_with_a_fixed_seed(tmp_path):
+    """bench.py's dump_outputs on more keypoints than DUMP_DESCRIPTOR_ROWS: float32/float64 files within
+    DUMP_MAX_BYTES, every keypoint, and the same seeded sample of descriptor rows on every call."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+
+    class Node:  # FeatureExtractionNode.download over host arrays keyed by "device pointer"
+        def __init__(self, arrays):
+            self.arrays = arrays
+
+        def download(self, ptr, shape, dtype=np.float32):
+            return self.arrays[ptr].reshape(shape).copy()
+
+    rng = np.random.default_rng(5)
+    K = bench.DUMP_DESCRIPTOR_ROWS + 1000
+    kp = rng.standard_normal((K, 4)).astype(np.float32)
+    desc = rng.standard_normal((K, 1980)).astype(np.float32)
+    ko = np.array([0, 7, 7, K], np.int64)
+    got = []
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), Node({1: kp, 2: desc}), ko, K, 1, 2)
+        got.append({n: np.load(tmp_path / run / (n + ".npy")) for n in ("keypoint_offsets", "keypoints", "descriptors", "descriptor_rows")})
+    a, b = got
+    assert sum(x.nbytes for x in a.values()) <= bench.DUMP_MAX_BYTES
+    assert all(x.dtype in (np.float32, np.float64) for x in a.values())
+    assert np.array_equal(a["keypoint_offsets"], ko) and np.array_equal(a["keypoints"], kp)
+    rows = a["descriptor_rows"].astype(np.int64)
+    assert len(rows) == bench.DUMP_DESCRIPTOR_ROWS and np.all(np.diff(rows) > 0) and rows[-1] < K
+    assert np.array_equal(a["descriptors"], desc[rows])
+    assert all(np.array_equal(a[n], b[n]) for n in a)
+
+
 def test_header_is_plain_c_and_links_from_c(tmp_path):
     """The boundary is a C ABI: include/fe_b200.h must compile as C99 and a C program must link
     against the library (no C++ types or name mangling in the exported interface)."""
