@@ -24,11 +24,36 @@ namespace {
 // graph and replayed (fe_process_batch, sub-batches of at most GRAPH_MAX_SCANS scans).
 constexpr int GRAPH_MAX_SCANS = 16;
 static_assert(GRAPH_MAX_SCANS <= 32, "k_kp_offsets_gather_small gives every scan a warp of one 1024-thread block");
+
+// What one enqueue of the pipeline computes (enqueue_pipeline).  The slot keeps the sub-batch in flight, so that
+// lean_rerun_if_deferred can run it again and the stats hooks can read its shape.
+struct SubBatch {
+  const float4* pts = nullptr;  // device input: a slot's d_pts or the caller's array (fe_process_batch_device)
+  int nscans = 0;
+  int64_t npts = 0;
+  int nch = 0;                  // K1 chunks of the staged scans
+  int k1flags = 0;
+  bool desc = false, wantKc = false;
+  RawLayout lay = {nullptr, 0, 0, 0, 0};
+  bool lean = false;            // first instantiation of every stage only (see enqueue_subbatch)
+};
+
+// A captured graph replays the launches of one SubBatch: the record plus whatever else the host code of
+// enqueue_pipeline branches on.  npts is left out: it enters through `by` and through nch (no chunks, no points);
+// every setting of the context that changes the launches bumps `epoch`.
 struct GraphKey {
-  int nscans, nch, by, k1flags, stride, xo, yo, zo;
-  int desc, wantKc, bnd, epoch, lean;
-  const void* pts;  // device-resident input (fe_process_batch_device): the pointer is part of the captured launches
-  bool operator==(const GraphKey& o) const { return memcmp(this, &o, sizeof(GraphKey)) == 0; }
+  SubBatch sb;
+  int by;        // density_blocks_per_scan: K4c's grid
+  bool bigScan;  // a scan of more than 65,535 points: launch_surface_grid adds the radix kernel
+  bool bnd;
+  int epoch;
+  bool operator==(const GraphKey& o) const {
+    const SubBatch &a = sb, &b = o.sb;
+    return a.pts == b.pts && a.nscans == b.nscans && a.nch == b.nch && a.k1flags == b.k1flags && a.desc == b.desc &&
+           a.wantKc == b.wantKc && a.lay.raw == b.lay.raw && a.lay.stride == b.lay.stride && a.lay.xo == b.lay.xo &&
+           a.lay.yo == b.lay.yo && a.lay.zo == b.lay.zo && a.lean == b.lean && by == o.by && bigScan == o.bigScan &&
+           bnd == o.bnd && epoch == o.epoch;
+  }
 };
 struct GraphEntry {
   GraphKey key;
@@ -38,11 +63,7 @@ struct GraphEntry {
 
 struct Slot {
   cudaStream_t stream = nullptr;
-  // lean chain (see process_batch_host): what finalize_subbatch needs to run the sub-batch again with every fallback kernel
-  bool lean = false;
-  const float4* rrPts = nullptr;
-  int rrNch = 0, rrK1flags = 0, rrStride = 0, rrXo = 0, rrYo = 0, rrZo = 0;
-  bool rrDesc = false, rrWantKc = false, rrRaw = false;
+  SubBatch sb;  // the sub-batch in flight (or the last one)
   std::vector<GraphEntry> graphs;
   int64_t capPts = 0;
   int capScans = 0, capChunks = 0;
@@ -85,16 +106,8 @@ struct Slot {
   int* h_kpOff = nullptr;
   int* h_perScan = nullptr;
   cudaEvent_t evDone = nullptr, evT0 = nullptr, evT1 = nullptr;
-  // K4a depends on K1 only: it runs on a side stream next to K2/K3 (fork after K1, join before K4b)
-  cudaStream_t stream2 = nullptr;
-  cudaEvent_t evFork = nullptr, evJoin = nullptr;
-  bool sideK4a = false;  // the pipeline in flight uses the side stream
-  int lastNch = 0;
   int64_t maxScanPts = 0;  // largest scan of the staged sub-batch
-  // bookkeeping of the sub-batch in flight
-  int nscans = 0;
-  int64_t npts = 0;
-  int firstScan = 0;
+  int firstScan = 0;       // where the sub-batch in flight goes in the call's results
   bool busy = false;
   // stage timing
   std::vector<cudaEvent_t> ev;
@@ -158,6 +171,22 @@ namespace {
 int fail(fe_ctx* ctx, int code, const std::string& msg) {
   if (ctx) ctx->err = msg;
   return code;
+}
+
+// wait for whatever the two slots have in flight
+int sync_slots(fe_ctx* ctx) {
+  for (Slot& s : ctx->slot) if (s.stream) CK(cudaStreamSynchronize(s.stream));
+  return FE_OK;
+}
+
+// scans [pts, ...) of a batch call: K1 runs every stage, K4 whenever the parameters ask for descriptors
+SubBatch batch_subbatch(const fe_ctx* ctx, const float4* pts, int nscans) {
+  SubBatch sb;
+  sb.pts = pts;
+  sb.nscans = nscans;
+  sb.desc = ctx->params.estimate_descriptors != 0;
+  sb.k1flags = F_ELEV | F_ROT | F_CROP | F_RING | (sb.desc ? F_SURF : 0);
+  return sb;
 }
 
 // ---- parameter derivation (host, float/double exactly as PCL narrows them) ------------------
@@ -286,8 +315,6 @@ void free_slot(Slot& s) {
   if (s.evDone) cudaEventDestroy(s.evDone);
   if (s.evT0) cudaEventDestroy(s.evT0);
   if (s.evT1) cudaEventDestroy(s.evT1);
-  for (cudaEvent_t e : {s.evFork, s.evJoin}) if (e) cudaEventDestroy(e);
-  if (s.stream2) cudaStreamDestroy(s.stream2);
   if (s.stream) cudaStreamDestroy(s.stream);
   s = Slot();
 }
@@ -305,9 +332,6 @@ int ensure_slot(fe_ctx* ctx, Slot& s, bool ownPoints) {
   s.capKf = (int)L.max_ring_clusters_per_call;
   s.capKc = 0;
   CK(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-  CK(cudaStreamCreateWithFlags(&s.stream2, cudaStreamNonBlocking));
-  CK(cudaEventCreateWithFlags(&s.evFork, cudaEventDisableTiming));
-  CK(cudaEventCreateWithFlags(&s.evJoin, cudaEventDisableTiming));
   CK(cudaEventCreateWithFlags(&s.evDone, cudaEventDisableTiming));
   CK(cudaEventCreate(&s.evT0));
   CK(cudaEventCreate(&s.evT1));
@@ -363,10 +387,8 @@ std::string err_bits(int e) {
   return m;
 }
 
-// Host-side staging of the small per-scan arrays of a sub-batch.  offs are absolute offsets of
-// the caller's array; the device sees offsets relative to the first point of the sub-batch.
-// the device copies of the staged arrays (from the pinned mirrors: the same addresses every call, so the copies can
-// live inside a captured graph)
+// the device copies of the arrays stage_scans left in the pinned mirrors (the same addresses every call, so the
+// copies can live inside a captured graph)
 int stage_scans_copy(fe_ctx* ctx, Slot& s, int nscans, bool deferRot) {
   CK(cudaMemcpyAsync(s.d_scan_off, s.h_scan_off, (nscans + 1) * sizeof(long long), cudaMemcpyHostToDevice, s.stream));
   CK(cudaMemcpyAsync(s.d_chunk_off, s.h_chunk_off, (nscans + 1) * sizeof(int), cudaMemcpyHostToDevice, s.stream));
@@ -378,8 +400,10 @@ int stage_scans_copy(fe_ctx* ctx, Slot& s, int nscans, bool deferRot) {
   return FE_OK;
 }
 
+// Host-side staging of the small per-scan arrays of a sub-batch into the pinned mirrors.  offs are absolute offsets
+// of the caller's array; the device sees offsets relative to the first point of the sub-batch.
 int stage_scans(fe_ctx* ctx, Slot& s, const int64_t* offs, const double* rp, int nscans, int64_t* nptsOut, int* nchOut,
-                bool deferRot = false, bool copy = true) {
+                bool deferRot = false) {
   // the pinned mirrors hold capScans(+1) entries: check before the first write
   if (nscans > s.capScans) return fail(ctx, FE_ERR_CAPACITY, "sub-batch exceeds max_scans_per_call");
   const int64_t o0 = offs[0];
@@ -406,18 +430,18 @@ int stage_scans(fe_ctx* ctx, Slot& s, const int64_t* offs, const double* rp, int
   *nptsOut = offs[nscans] - o0;
   *nchOut = nch;
   if (nch > s.capChunks) return fail(ctx, FE_ERR_CAPACITY, "sub-batch exceeds the chunk capacity");
-  if (copy) return stage_scans_copy(ctx, s, nscans, deferRot);
   return FE_OK;
 }
 
-int ensure_rowstart(fe_ctx* ctx, Slot& s, int nscans) {
-  const int64_t need = (int64_t)std::max(nscans, s.capScans) * (ctx->dp.sg_ny + 1);
+// P: the parameters whose descriptor grid the surface index of the launches will use
+int ensure_rowstart(fe_ctx* ctx, Slot& s, const DevParams& P, int nscans) {
+  const int64_t need = (int64_t)std::max(nscans, s.capScans) * (P.sg_ny + 1);
   if (need > s.capRowStart) {
     if (s.d_rowStart) { CK(cudaStreamSynchronize(s.stream)); CK(cudaFree(s.d_rowStart)); s.d_rowStart = nullptr; }
     CK(dalloc(&s.d_rowStart, (size_t)need));
     s.capRowStart = need;
   }
-  const int64_t ncells = (int64_t)ctx->dp.sg_nx * ctx->dp.sg_ny;
+  const int64_t ncells = (int64_t)P.sg_nx * P.sg_ny;
   if (ncells <= SURF_MAX_CELLS) {
     const int64_t needT = (int64_t)std::max(nscans, s.capScans) * grid_hdr_bytes((int)ncells);
     if (needT > s.capGridHdr) {
@@ -429,8 +453,8 @@ int ensure_rowstart(fe_ctx* ctx, Slot& s, int nscans) {
   return FE_OK;
 }
 
-SurfIndex surf_index(const fe_ctx* ctx, const Slot& s) {
-  const int64_t ncells = (int64_t)ctx->dp.sg_nx * ctx->dp.sg_ny;
+SurfIndex surf_index(const DevParams& P, const Slot& s) {
+  const int64_t ncells = (int64_t)P.sg_nx * P.sg_ny;
   SurfIndex X;
   X.sortedKey = s.d_sortedKey;
   X.rowStart = s.d_rowStart;
@@ -482,8 +506,6 @@ int set_kernel_attrs(fe_ctx* ctx) {
 // K4d: three instantiations split the keypoints by neighbour count (smaller footprint = more blocks / SM)
 void launch_desc_hist(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int gridKp, bool records, bool lean = false) {
   const int descStride = records ? FE_RECORD_FLOATS : FE_DESC_LEN, descOff = records ? 5 : 0;
-#define FE_DESC_ARGS s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_kpNbr, s.d_sorted, surf_index(ctx, s), s.d_scan_off, P, \
-                     s.d_rho, ctx->d_lut, ctx->d_axes, ctx->axesCap, s.d_keyA, s.d_kpNbrOff, s.d_kpRank, FE_DESC_LIST, s.d_desc, descStride, descOff, s.d_ctr, warpCap
   // the blocks stride over the keypoints with equal shares: grids of exactly one resident wave
   static const int perSm = []() {  // initialised once, also when fe_multi's threads get here together
     int v = 0;
@@ -510,20 +532,21 @@ void launch_desc_hist(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int 
         s.d_keyA, s.d_kpNbrOff, s.d_kpRank, s.d_desc, descStride, descOff, s.d_ctr);
     ctx->launches++;
   }
-#define FE_DESC_LIST nullptr, nullptr
-  k_desc_hist<256, DCAP, DW_CAP, false, true><<<std::min(gridKp, ctx->numSms * std::max(perSm, 1)), 256, desc_smem_bytes(DCAP, 256), s.stream>>>(FE_DESC_ARGS);
-#undef FE_DESC_LIST
-  ctx->launches++;
+  // glist / nlist: the keypoints the previous instantiation listed for this one (null: every keypoint)
+  auto hist = [&](auto kernel, int grid, int nt, size_t smem, const int* glist, const int* nlist) {
+    kernel<<<grid, nt, smem, s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_kpNbr, s.d_sorted, surf_index(P, s),
+                                         s.d_scan_off, P, s.d_rho, ctx->d_lut, ctx->d_axes, ctx->axesCap, s.d_keyA, s.d_kpNbrOff,
+                                         s.d_kpRank, glist, nlist, s.d_desc, descStride, descOff, s.d_ctr, warpCap);
+    ctx->launches++;
+  };
+  hist(k_desc_hist<256, DCAP, DW_CAP, false, true>, std::min(gridKp, ctx->numSms * std::max(perSm, 1)), 256,
+       desc_smem_bytes(DCAP, 256), nullptr, nullptr);
   if (!lean) {  // lean: keypoints listed for the two larger instantiations make the caller run the sub-batch again
-#define FE_DESC_LIST s.d_kpListM, &s.d_ctr->n_list_m
-  k_desc_hist<512, DCAP_M, DCAP, false, false><<<std::min(gridKp, ctx->numSms * 2), 512, desc_smem_bytes(DCAP_M, 512), s.stream>>>(FE_DESC_ARGS);
-#undef FE_DESC_LIST
-#define FE_DESC_LIST s.d_kpListL, &s.d_ctr->n_list_l
-  k_desc_hist<512, DCAP_L, DCAP_M, true, false><<<std::min(gridKp, ctx->numSms), 512, desc_smem_bytes(DCAP_L, 512), s.stream>>>(FE_DESC_ARGS);
-#undef FE_DESC_LIST
-  ctx->launches += 2;
+    hist(k_desc_hist<512, DCAP_M, DCAP, false, false>, std::min(gridKp, ctx->numSms * 2), 512, desc_smem_bytes(DCAP_M, 512),
+         s.d_kpListM, &s.d_ctr->n_list_m);
+    hist(k_desc_hist<512, DCAP_L, DCAP_M, true, false>, std::min(gridKp, ctx->numSms), 512, desc_smem_bytes(DCAP_L, 512),
+         s.d_kpListL, &s.d_ctr->n_list_l);
   }
-#undef FE_DESC_ARGS
   if (records) {
     k_record_frame<<<ctx->numSms * 2, 256, 0, s.stream>>>(s.d_kpOut, s.d_kpOff, nscans, s.d_desc, descStride, FE_DESC_LEN);
     ctx->launches++;
@@ -541,7 +564,7 @@ void launch_desc_mark(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int 
   }();
   gridKp = std::min(gridKp, ctx->numSms * std::max(perSm, 1));
   k_desc_mark<<<gridKp, 256, MARK_LCAP * sizeof(unsigned), s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_sorted,
-                                                                       surf_index(ctx, s), s.d_scan_off, P, s.d_rho, s.d_kpNbr,
+                                                                       surf_index(P, s), s.d_scan_off, P, s.d_rho, s.d_kpNbr,
                                                                        s.d_keyA, nbrCap, s.d_kpNbrOff, s.d_ctr);
   k_kp_rank<<<(int)((s.capKp + 255) / 256), 256, 0, s.stream>>>(s.d_kpScan, s.d_kpOff, nscans, s.d_kpNbr, s.d_kpRank, s.d_kpListM, s.d_kpListL, s.d_ctr);
   ctx->launches += 2;
@@ -549,22 +572,22 @@ void launch_desc_mark(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int 
 
 // K4a: counting sort by cell in shared memory for scans that fit (<= 65,535 surface points, grid <=
 // SURF_MAX_CELLS cells), radix sort through global memory for the deferred rest.
-void launch_surface_grid(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, cudaStream_t q) {
+void launch_surface_grid(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P) {
   const int ncells = P.sg_nx * P.sg_ny;
   if (ncells <= SURF_MAX_CELLS) {
-    k_surface_grid_cells<NT_SURF><<<nscans, NT_SURF, surf_cells_smem_bytes(ncells), q>>>(
+    k_surface_grid_cells<NT_SURF><<<nscans, NT_SURF, surf_cells_smem_bytes(ncells), s.stream>>>(
         s.d_surf, s.d_surfCnt, s.d_scan_off, s.d_chunk_off, P, s.d_kpOut, s.d_kpOff, s.d_sorted, s.d_rho,
         s.d_surfN, s.d_ctr, s.d_ovfSurf, s.d_gridHdr, grid_hdr_bytes(ncells), s.d_tabOk);
     ctx->launches++;
     // the radix kernel only takes scans the counting sort defers: more than 65,535 surface points or more halo
     // cells than counters — impossible when every scan is small and the grid has no more cells than counters
     if (s.maxScanPts <= 65535 && ncells <= GRID_TAB_CAP) return;
-    k_surface_grid<<<std::min(nscans, ctx->numSms * 2), NT2, 0, q>>>(s.d_surf, s.d_surfCnt, s.d_scan_off, s.d_chunk_off, P, s.d_keyA,
+    k_surface_grid<<<std::min(nscans, ctx->numSms * 2), NT2, 0, s.stream>>>(s.d_surf, s.d_surfCnt, s.d_scan_off, s.d_chunk_off, P, s.d_keyA,
                                                                    s.d_keyB, s.d_valA, s.d_valB, s.d_sorted, s.d_sortedKey,
                                                                    s.d_rowStart, s.d_surfN, s.d_ctr, s.d_ovfSurf, &s.d_ctr->ovf_surf,
                                                                    s.d_tabOk, s.d_rho);
   } else {
-    k_surface_grid<<<nscans, NT2, 0, q>>>(s.d_surf, s.d_surfCnt, s.d_scan_off, s.d_chunk_off, P, s.d_keyA, s.d_keyB, s.d_valA,
+    k_surface_grid<<<nscans, NT2, 0, s.stream>>>(s.d_surf, s.d_surfCnt, s.d_scan_off, s.d_chunk_off, P, s.d_keyA, s.d_keyB, s.d_valA,
                                                  s.d_valB, s.d_sorted, s.d_sortedKey, s.d_rowStart, s.d_surfN, s.d_ctr, nullptr, nullptr,
                                                  s.d_tabOk, s.d_rho);
   }
@@ -579,14 +602,12 @@ int density_blocks_per_scan(int nscans, int64_t npts) {
 void launch_density(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int64_t npts) {
   if (nscans <= 0) return;
   const int by = density_blocks_per_scan(nscans, npts);
-  k_density<<<dim3((unsigned)nscans, (unsigned)by), 256, 0, s.stream>>>(s.d_sorted, surf_index(ctx, s), s.d_scan_off, P, s.d_surfN, s.d_rho, s.d_ctr->dens_work);
+  k_density<<<dim3((unsigned)nscans, (unsigned)by), 256, 0, s.stream>>>(s.d_sorted, surf_index(P, s), s.d_scan_off, P, s.d_surfN, s.d_rho, s.d_ctr->dens_work);
   ctx->launches++;
 }
 
 // K2 + K3 for `nscans` scans: the 2-blocks-per-SM instantiation first, then the large one over
 // whatever scans it deferred (an immediate exit when there are none).
-void mark(fe_ctx* ctx, Slot& s, const char* name);
-
 void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool wantKc, bool merge, bool marks = false, bool lean = false) {
   // Every stage is a chain of instantiations: the fast one takes all scans and defers those that do
   // not fit its shared memory to a list; the large shared-memory one takes that list; what does not
@@ -602,22 +623,36 @@ void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool w
   int* kcB = wantKc ? s.d_kcBase : nullptr;
   int* kcC = wantKc ? s.d_kcCnt : nullptr;
   const int sr = singleRing ? 1 : 0;
-#define FE_K2_ARGS s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, \
-                   s.capKc, kcB, kcC, s.d_ctr
+  // inList / inN: the scans the previous instantiation deferred to this one (null: every scan); outList / outN: where
+  // this one defers what it cannot take (null: the last of the chain); slabs: per-entry arrays in global memory
+  auto k2 = [&](auto kernel, int grid, int nt, size_t smem, const int* inList, const int* inN, int* outList, int* outN,
+                unsigned char* slabs) {
+    kernel<<<grid, nt, smem, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_kfPool,
+                                         s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr, inList, inN, outList,
+                                         outN, slabs);
+    ctx->launches++;
+  };
+  auto k3 = [&](auto kernel, int grid, int nt, size_t smem, const int* inList, const int* inN, int* outList, int* outN,
+                unsigned char* slabs) {
+    kernel<<<grid, nt, smem, s.stream>>>(s.d_kfPool, s.d_kfBase, s.d_kfCnt, P, s.d_kpPool, (int)s.capKp, s.d_kpBase, s.d_kpCnt,
+                                         s.d_ctr, inList, inN, outList, outN, slabs);
+    ctx->launches++;
+  };
   // K2: the run-based kernel takes every scan; what it cannot handle (a ring with more than RW runs — unordered
   // input — or more ring entries than the scan's scratch slot) goes down the chain of grid-based instantiations.
   if (ctx->gridClustering) {
-    k_cluster_rings<ECAP, NTF, 4, false><<<nscans, NTF, kClusterSmem, s.stream>>>(FE_K2_ARGS, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr);
-    ctx->launches++;
+    k2(k_cluster_rings<ECAP, NTF, 4, false>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr);
   } else {
-#define FE_RR_ARGS s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_ringPts, s.d_ringBase, s.d_kfPool, s.capKf, \
-                   s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr, s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR
+    auto rr = [&](auto kernel, int nt, size_t smem) {
+      kernel<<<nscans, nt, smem, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_ringPts,
+                                             s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
+                                             s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR);
+      ctx->launches++;
+    };
     if (nscans <= GRAPH_MAX_SCANS)  // a handful of scans: a warp for each of a scan's 16 rings at once (latency, not throughput)
-      k_ring_runs<NW_RR_SMALL><<<nscans, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>), s.stream>>>(FE_RR_ARGS);
+      rr(k_ring_runs<NW_RR_SMALL>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>));
     else
-      k_ring_runs<NW_RR><<<nscans, NT_RR, sizeof(RingRunsSmT<RW>), s.stream>>>(FE_RR_ARGS);
-#undef FE_RR_ARGS
-    ctx->launches++;
+      rr(k_ring_runs<NW_RR>, NT_RR, sizeof(RingRunsSmT<RW>));
     if (!lean) {
       k_ring_runs_wide<<<std::min(nscans * 4, ctx->numSms * 7), NT_RR, NW_RR * sizeof(RunBufT<RW2>), s.stream>>>(
           s.d_scan_off, P, s.d_ringPts, s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
@@ -628,22 +663,16 @@ void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool w
   // lean: the fallback instantiations are left out; whatever the first kernel deferred shows in the counters and the
   // caller runs the sub-batch again with the whole chain
   if (!lean) {
-    k_cluster_rings<ECAP_L, NTL, 1, false><<<gridL, NTL, kClusterSmemL2, s.stream>>>(FE_K2_ARGS, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr);
-    k_cluster_rings<ECAP_G, NT2, 1, true><<<gridG, NT2, smemG, s.stream>>>(FE_K2_ARGS, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs);
-    ctx->launches += 2;
+    k2(k_cluster_rings<ECAP_L, NTL, 1, false>, gridL, NTL, kClusterSmemL2, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr);
+    k2(k_cluster_rings<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs);
   }
-#undef FE_K2_ARGS
   if (marks) mark(ctx, s, "K2 ring clusters");
   if (merge) {
-#define FE_K3_ARGS s.d_kfPool, s.d_kfBase, s.d_kfCnt, P, s.d_kpPool, (int)s.capKp, s.d_kpBase, s.d_kpCnt, s.d_ctr
-    k_merge_keypoints<ECAP_M, NTM, 8, false><<<nscans, NTM, kClusterSmemM, s.stream>>>(FE_K3_ARGS, nullptr, nullptr, s.d_ovfMerge, ovfM, nullptr);
-    ctx->launches++;
+    k3(k_merge_keypoints<ECAP_M, NTM, 8, false>, nscans, NTM, kClusterSmemM, nullptr, nullptr, s.d_ovfMerge, ovfM, nullptr);
     if (!lean) {
-      k_merge_keypoints<ECAP_L, NT2, 1, false><<<gridL, NT2, kClusterSmemL, s.stream>>>(FE_K3_ARGS, s.d_ovfMerge, ovfM, s.d_ovfMerge2, ovfM2, nullptr);
-      k_merge_keypoints<ECAP_G, NT2, 1, true><<<gridG, NT2, smemG, s.stream>>>(FE_K3_ARGS, s.d_ovfMerge2, ovfM2, nullptr, nullptr, s.d_slabs);
-      ctx->launches += 2;
+      k3(k_merge_keypoints<ECAP_L, NT2, 1, false>, gridL, NT2, kClusterSmemL, s.d_ovfMerge, ovfM, s.d_ovfMerge2, ovfM2, nullptr);
+      k3(k_merge_keypoints<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfMerge2, ovfM2, nullptr, nullptr, s.d_slabs);
     }
-#undef FE_K3_ARGS
   }
 }
 
@@ -669,16 +698,17 @@ int ensure_bnd(fe_ctx* ctx, Slot& s) {
   return FE_OK;
 }
 
-// Enqueue the kernels of one sub-batch whose points are at d_pts.  k1flags selects what K1 does;
-// `fromStage`: 0 = K1 first; 1 = crop/cropMeta/cropCnt already filled by the caller.
-int enqueue_pipeline(fe_ctx* ctx, Slot& s, const float4* d_pts, int nscans, int64_t npts, int nch,
-                     int k1flags, bool doDesc, bool singleRing, bool wantKc, RawLayout lay = RawLayout{nullptr, 0, 0, 0, 0},
-                     const double* lateRp = nullptr, bool recordDone = true, bool lean = false) {
-  DevParams& P = ctx->dp;
+// Enqueue the kernels of the slot's sub-batch s.sb, K1 to K4d, and the copies of its counters, keypoint offsets and
+// boundary counts to the pinned mirrors; its scan offsets must be on the device already (stage_scans_copy).  With
+// `lateRp` the levelling matrices are computed here, interleaved with K1.  recordDone: record the slot's evDone.
+int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone) {
+  const DevParams& P = ctx->dp;
+  const SubBatch& sb = s.sb;
+  const int nscans = sb.nscans;
   s.nev = 0;
   mark(ctx, s, "begin");
   CK(cudaMemsetAsync(s.d_ctr, 0, sizeof(DevCounters), s.stream));
-  if (nch > 0 && k1flags >= 0) {
+  if (sb.nch > 0) {
     // With `lateRp` the levelling matrices (two sincos and a quaternion product per scan on the host,
     // ~0.4 ms for 10 k scans) are not staged yet: they are computed range by range — an eighth, an
     // eighth, a quarter, a half of the scans — and K1 is launched per range, so that all but the first
@@ -697,12 +727,12 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const float4* d_pts, int nscans, int6
       }
       const int ca = s.h_chunk_off[a], cb = s.h_chunk_off[b];
       if (cb <= ca) continue;
-      if (lay.raw)
-        k_level_crop_ring<true, true><<<cb - ca, 256, 0, s.stream>>>(d_pts, s.d_chunkTab, s.d_rot, P, k1flags,
-                                                               s.d_surf, s.d_surfCnt, s.d_crop, s.d_cropMeta, s.d_cropCnt, nullptr, lay, ca);
+      if (sb.lay.raw)
+        k_level_crop_ring<true, true><<<cb - ca, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.k1flags,
+                                                               s.d_surf, s.d_surfCnt, s.d_crop, s.d_cropMeta, s.d_cropCnt, nullptr, sb.lay, ca);
       else
-        k_level_crop_ring<false, true><<<cb - ca, 256, 0, s.stream>>>(d_pts, s.d_chunkTab, s.d_rot, P, k1flags,
-                                                                s.d_surf, s.d_surfCnt, s.d_crop, s.d_cropMeta, s.d_cropCnt, nullptr, lay, ca);
+        k_level_crop_ring<false, true><<<cb - ca, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.k1flags,
+                                                                s.d_surf, s.d_surfCnt, s.d_crop, s.d_cropMeta, s.d_cropCnt, nullptr, sb.lay, ca);
       ctx->launches++;
       if (lateRp && part + 1 < nparts) mark(ctx, s, "K1 level+crop+ring");
     }
@@ -713,16 +743,15 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const float4* d_pts, int nscans, int6
     int st = ensure_bnd(ctx, s);
     if (st) return st;
     CK(cudaMemsetAsync(s.d_bnd, 0, (size_t)nscans * 4 * sizeof(unsigned long long), s.stream));
-    k_boundary_rings<<<nscans, 256, 0, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, singleRing ? 1 : 0,
+    k_boundary_rings<<<nscans, 256, 0, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, 0,
                                                    boundary_spec(ctx), s.d_bnd);
     ctx->launches++;
   }
-  s.sideK4a = false;
-  if (doDesc) {
-    int st = ensure_rowstart(ctx, s, nscans);
+  if (sb.desc) {
+    int st = ensure_rowstart(ctx, s, P, nscans);
     if (st) return st;
   }
-  launch_clustering(ctx, s, nscans, singleRing, wantKc, true, true, lean);
+  launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean);
   mark(ctx, s, "K3 merge keypoints");
   if (bnd) {
     k_boundary_merge<<<nscans, 128, 0, s.stream>>>(s.d_kfPool, s.d_kfBase, s.d_kfCnt, P, boundary_spec(ctx), s.d_bnd);
@@ -738,27 +767,27 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const float4* d_pts, int nscans, int6
     ctx->launches += 2;
   }
   mark(ctx, s, "keypoint CSR");
-  if (doDesc) {
+  if (sb.desc) {
     // K4a runs after the keypoints are known: it only keeps the surface points a keypoint can reach
-    launch_surface_grid(ctx, s, nscans, P, s.stream);
+    launch_surface_grid(ctx, s, nscans, P);
     mark(ctx, s, "K4a surface grid");
     const int gridKp = ctx->numSms * 8;
     launch_desc_mark(ctx, s, nscans, P, gridKp);
     mark(ctx, s, "K4b mark neighbours");
     if (bnd) {  // before K4c turns the marks in rho into densities
-      k_boundary_support<<<ctx->numSms * 4, 256, 0, s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_sorted, surf_index(ctx, s),
+      k_boundary_support<<<ctx->numSms * 4, 256, 0, s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_sorted, surf_index(P, s),
                                                          s.d_scan_off, P, boundary_spec(ctx), s.d_bnd);
-      if (npts > 0)
-        k_boundary_density<<<nscans, 256, 0, s.stream>>>(s.d_sorted, surf_index(ctx, s), s.d_scan_off, P, s.d_surfN, s.d_rho,
+      if (sb.npts > 0)
+        k_boundary_density<<<nscans, 256, 0, s.stream>>>(s.d_sorted, surf_index(P, s), s.d_scan_off, P, s.d_surfN, s.d_rho,
                                                          boundary_spec(ctx), s.d_bnd);
       ctx->launches += 2;
     }
-    launch_density(ctx, s, nscans, P, npts);
+    launch_density(ctx, s, nscans, P, sb.npts);
     mark(ctx, s, "K4c density");
-    launch_desc_hist(ctx, s, nscans, P, gridKp, ctx->recordOutput, lean);
+    launch_desc_hist(ctx, s, nscans, P, gridKp, ctx->recordOutput, sb.lean);
     mark(ctx, s, "K4d shape context");
   }
-  if (wantKc && ctx->cloudOutputs && nscans > 0) {
+  if (sb.wantKc && ctx->cloudOutputs && nscans > 0) {
     // ~cloud (src:137-139) and ~keypoint_cloud (src:133-135): per-scan counts, offsets and the ordered gather all
     // on the device; the host only learns the offsets (finalize_subbatch then copies the dense arrays out)
     const int gb = (nscans + 255) / 256;
@@ -792,80 +821,66 @@ void collect_times(fe_ctx* ctx, Slot& s) {
   }
 }
 
-int grow_results(fe_ctx* ctx, int64_t needKp, bool desc) {
-  if (needKp > ctx->capResKp) {
-    for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
-    const int64_t cap = std::max<int64_t>(needKp * 3 / 2, 4096);
-    fe_point_t* nk = nullptr;
-    CK(halloc(&nk, (size_t)cap));
-    if (ctx->h_kp) { memcpy(nk, ctx->h_kp, (size_t)ctx->capResKp * sizeof(fe_point_t)); cudaFreeHost(ctx->h_kp); }
-    ctx->h_kp = nk;
-    ctx->capResKp = cap;
-  }
-  if (desc && ctx->capResKp > ctx->capResDesc) {
-    for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
-    float* nd = nullptr;
-    CK(halloc(&nd, (size_t)ctx->capResKp * FE_RECORD_FLOATS));
-    if (ctx->h_desc) { memcpy(nd, ctx->h_desc, (size_t)ctx->capResDesc * FE_RECORD_FLOATS * sizeof(float)); cudaFreeHost(ctx->h_desc); }
-    ctx->h_desc = nd;
-    ctx->capResDesc = ctx->capResKp;
-  }
-  return FE_OK;
-}
-
-int grow_pinned_points(fe_ctx* ctx, fe_point_t** buf, int64_t* cap, int64_t used, int64_t need) {
+// Grow the pinned result buffer *buf of *cap records of `rec` elements to hold `need` records (half as many again, at
+// least minCap), keeping its first `keep` records.  A sub-batch in flight may still be copying into the old buffer:
+// both slots are drained first.
+template <class T>
+int grow_pinned(fe_ctx* ctx, T** buf, int64_t* cap, int64_t need, int64_t minCap, int64_t keep, size_t rec = 1) {
   if (need <= *cap) return FE_OK;
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
-  const int64_t ncap = std::max<int64_t>(need * 3 / 2, 1 << 16);
-  fe_point_t* nb = nullptr;
-  CK(halloc(&nb, (size_t)ncap));
-  if (*buf) { memcpy(nb, *buf, (size_t)used * sizeof(fe_point_t)); cudaFreeHost(*buf); }
+  int st = sync_slots(ctx);
+  if (st) return st;
+  const int64_t ncap = std::max<int64_t>(need * 3 / 2, minCap);
+  T* nb = nullptr;
+  CK(halloc(&nb, (size_t)ncap * rec));
+  if (*buf) { memcpy(nb, *buf, (size_t)keep * rec * sizeof(T)); cudaFreeHost(*buf); }
   *buf = nb;
   *cap = ncap;
   return FE_OK;
 }
 
-// wait for the sub-batch in `s`, check its error word, append its keypoints to the results
-// The sub-batch ran the lean chain (first instantiation of every stage only, see enqueue_small).  Anything one of
+// The sub-batch ran the lean chain (first instantiation of every stage only, see enqueue_subbatch).  Anything one of
 // them deferred to a fallback kernel is in the counters: run the sub-batch again, eagerly, with the whole chain (its
 // points and staged offsets are still where they were), and keep the lean chain off for a while — inputs that defer
 // once (unordered clouds, very large descriptor radii) usually keep doing so.  Call after the slot's evDone.
 int lean_rerun_if_deferred(fe_ctx* ctx, Slot& s) {
-  if (!s.lean) return FE_OK;
-  s.lean = false;
+  if (!s.sb.lean) return FE_OK;
+  s.sb.lean = false;
   const DevCounters& c = *s.h_ctr;
   if (c.err || !(c.ovf_runs | c.ovf_rings | c.ovf_rings2 | c.ovf_merge | c.ovf_merge2 | c.n_list_m | c.n_list_l)) return FE_OK;
   ctx->leanHold = 256;
   ctx->leanReruns++;
-  RawLayout lay = {s.rrRaw ? (const unsigned char*)s.rrPts : nullptr, s.rrStride, s.rrXo, s.rrYo, s.rrZo};
-  int st = enqueue_pipeline(ctx, s, s.rrPts, s.nscans, s.npts, s.rrNch, s.rrK1flags, s.rrDesc, false, s.rrWantKc, lay);
+  int st = enqueue_pipeline(ctx, s, nullptr, true);
   if (st) return st;
   CK(cudaEventSynchronize(s.evDone));
   return FE_OK;
 }
 
-// A sub-batch of at most GRAPH_MAX_SCANS scans whose offsets stage_scans(copy = false) left in the pinned mirrors:
-// the chain is captured into a CUDA graph per shape (second sighting) and replayed from then on.  Lean chain: a
-// handful of scans almost never needs a fallback instantiation, and seven kernels that only find that out cost more
-// than a tenth of a single scan's latency; they are left out and lean_rerun_if_deferred repairs the rare miss.
-// Records the slot's evDone.
-int enqueue_small(fe_ctx* ctx, Slot& s, const float4* d_pts, bool ptsInKey, int ns, int64_t npts, int nch, int k1flags, bool desc,
-                  bool wantKc, RawLayout lay) {
+// Enqueue `sb`, whose offsets stage_scans left in the slot's pinned mirrors, and record the slot's evDone; `upload`:
+// `bytes` of host points to copy to the slot's d_pts first (none: the points are on the device).  A large sub-batch
+// runs eagerly.  One of at most GRAPH_MAX_SCANS scans is captured into a CUDA graph per GraphKey (on its second
+// sighting) and replayed from then on.  Lean chain: a handful of scans almost never needs a fallback instantiation,
+// and seven kernels that only find that out cost more than a tenth of a single scan's latency; they are left out and
+// lean_rerun_if_deferred repairs the rare miss.
+int enqueue_subbatch(fe_ctx* ctx, Slot& s, const SubBatch& sb, const double* lateRp, const void* upload = nullptr,
+                     size_t bytes = 0) {
+  s.sb = sb;
+  s.sb.lean = false;
   int st;
+  if (lateRp || !ctx->useGraphs || ctx->stageTiming || sb.nscans > GRAPH_MAX_SCANS) {
+    // offsets and chunk table ahead of the points: with the points first, 10k scans through fe_process_batch took
+    // 49 instead of 43 ms on a B200 (1,000 W)
+    st = stage_scans_copy(ctx, s, sb.nscans, lateRp != nullptr);
+    if (st) return st;
+    if (bytes) CK(cudaMemcpyAsync(s.d_pts, upload, bytes, cudaMemcpyHostToDevice, s.stream));
+    return enqueue_pipeline(ctx, s, lateRp, true);
+  }
+  if (bytes) CK(cudaMemcpyAsync(s.d_pts, upload, bytes, cudaMemcpyHostToDevice, s.stream));
   // every allocation the pipeline may need happens before a capture starts
-  if (desc) { st = ensure_rowstart(ctx, s, ns); if (st) return st; }
+  if (sb.desc) { st = ensure_rowstart(ctx, s, ctx->dp, sb.nscans); if (st) return st; }
   if (ctx->bndEps > 0.0) { st = ensure_bnd(ctx, s); if (st) return st; }
-  GraphKey key;
-  memset(&key, 0, sizeof key);
-  key.nscans = ns; key.nch = nch; key.by = density_blocks_per_scan(ns, npts); key.k1flags = k1flags | ((s.maxScanPts > 65535) ? (1 << 16) : 0);
-  key.stride = lay.raw ? lay.stride : 0; key.xo = lay.xo; key.yo = lay.yo; key.zo = lay.zo;
-  key.desc = desc; key.wantKc = wantKc; key.bnd = ctx->bndEps > 0.0; key.epoch = ctx->epoch;
-  key.pts = ptsInKey ? (const void*)d_pts : nullptr;
-  const bool lean = ctx->leanHold == 0;
+  s.sb.lean = ctx->leanHold == 0;
   if (ctx->leanHold > 0) ctx->leanHold--;
-  key.lean = lean;
-  s.lean = lean; s.rrPts = d_pts; s.rrNch = nch; s.rrK1flags = k1flags; s.rrDesc = desc; s.rrWantKc = wantKc;
-  s.rrRaw = lay.raw != nullptr; s.rrStride = lay.stride; s.rrXo = lay.xo; s.rrYo = lay.yo; s.rrZo = lay.zo;
+  const GraphKey key = {s.sb, density_blocks_per_scan(sb.nscans, sb.npts), s.maxScanPts > 65535, ctx->bndEps > 0.0, ctx->epoch};
   GraphEntry* ge = nullptr;
   for (GraphEntry& g : s.graphs) if (g.key == key) { ge = &g; break; }
   if (ge && ge->exec) {  // replay
@@ -873,9 +888,9 @@ int enqueue_small(fe_ctx* ctx, Slot& s, const float4* d_pts, bool ptsInKey, int 
     ctx->launches += ge->launches;
     ctx->graphReplays++;
   } else if (!ge) {      // first sighting of the shape: eager, so that every lazily initialised piece exists
-    st = stage_scans_copy(ctx, s, ns, false);
+    st = stage_scans_copy(ctx, s, sb.nscans, false);
     if (st) return st;
-    st = enqueue_pipeline(ctx, s, d_pts, ns, npts, nch, k1flags, desc, false, wantKc, lay, nullptr, false, lean);
+    st = enqueue_pipeline(ctx, s, nullptr, false);
     if (st) return st;
     if (s.graphs.size() >= 16) {  // drop the oldest shape
       if (s.graphs[0].exec) cudaGraphExecDestroy(s.graphs[0].exec);
@@ -886,8 +901,8 @@ int enqueue_small(fe_ctx* ctx, Slot& s, const float4* d_pts, bool ptsInKey, int 
   } else {               // second sighting: capture, instantiate, launch
     const int64_t l0 = ctx->launches;
     CK(cudaStreamBeginCapture(s.stream, cudaStreamCaptureModeThreadLocal));
-    st = stage_scans_copy(ctx, s, ns, false);
-    if (st == FE_OK) st = enqueue_pipeline(ctx, s, d_pts, ns, npts, nch, k1flags, desc, false, wantKc, lay, nullptr, false, lean);
+    st = stage_scans_copy(ctx, s, sb.nscans, false);
+    if (st == FE_OK) st = enqueue_pipeline(ctx, s, nullptr, false);
     cudaGraph_t graph = nullptr;
     const cudaError_t ce = cudaStreamEndCapture(s.stream, &graph);
     if (st) { if (graph) cudaGraphDestroy(graph); return st; }
@@ -905,31 +920,47 @@ int enqueue_small(fe_ctx* ctx, Slot& s, const float4* d_pts, bool ptsInKey, int 
   return FE_OK;
 }
 
-int finalize_subbatch(fe_ctx* ctx, Slot& s, int64_t& kpRun, bool desc) {
-  if (!s.busy) return FE_OK;
+// Wait for the sub-batch in `s`, run it again in full if its lean chain deferred anything, check its error word, and
+// write its keypoint offsets (plus kpBase) and boundary counts at scan s.firstScan of the call's results.
+int complete_subbatch(fe_ctx* ctx, Slot& s, int64_t kpBase) {
   CK(cudaEventSynchronize(s.evDone));
-  s.busy = false;
-  { int st = lean_rerun_if_deferred(ctx, s); if (st) return st; }
-  if (s.h_ctr->err) return fail(ctx, FE_ERR_CAPACITY, err_bits(s.h_ctr->err));
-  const int K = s.h_kpOff[s.nscans];
-  int st = grow_results(ctx, kpRun + K, desc);
+  int st = lean_rerun_if_deferred(ctx, s);
   if (st) return st;
-  for (int i = 0; i <= s.nscans; i++) ctx->kpOffsets[s.firstScan + i] = kpRun + s.h_kpOff[i];
+  if (s.h_ctr->err) return fail(ctx, FE_ERR_CAPACITY, err_bits(s.h_ctr->err));
+  const int ns = s.sb.nscans;
+  for (int i = 0; i <= ns; i++) ctx->kpOffsets[s.firstScan + i] = kpBase + s.h_kpOff[i];
   if (ctx->bndEps > 0.0 && s.h_bnd)
-    for (int i = 0; i < s.nscans * 4; i++) ctx->bndCounts[(size_t)s.firstScan * 4 + i] = (int64_t)s.h_bnd[i];
+    for (int i = 0; i < ns * 4; i++) ctx->bndCounts[(size_t)s.firstScan * 4 + i] = (int64_t)s.h_bnd[i];
+  return FE_OK;
+}
+
+// complete the sub-batch in `s` (if any) and append its results to the host call's pinned result buffers
+int finalize_subbatch(fe_ctx* ctx, Slot& s, int64_t& kpRun) {
+  if (!s.busy) return FE_OK;
+  s.busy = false;
+  int st = complete_subbatch(ctx, s, kpRun);
+  if (st) return st;
+  const int ns = s.sb.nscans;
+  const int K = s.h_kpOff[ns];
+  st = grow_pinned(ctx, &ctx->h_kp, &ctx->capResKp, kpRun + K, 4096, kpRun);
+  if (st) return st;
+  if (s.sb.desc) {
+    st = grow_pinned(ctx, &ctx->h_desc, &ctx->capResDesc, kpRun + K, 4096, kpRun, FE_RECORD_FLOATS);
+    if (st) return st;
+  }
   if (K > 0) {
     CK(cudaMemcpyAsync(ctx->h_kp + kpRun, s.d_kpOut, (size_t)K * sizeof(float4), cudaMemcpyDeviceToHost, s.stream));
     const size_t dl = ctx->recordOutput ? FE_RECORD_FLOATS : FE_DESC_LEN;
-    if (desc) CK(cudaMemcpyAsync(ctx->h_desc + kpRun * dl, s.d_desc, (size_t)K * dl * sizeof(float), cudaMemcpyDeviceToHost, s.stream));
+    if (s.sb.desc) CK(cudaMemcpyAsync(ctx->h_desc + kpRun * dl, s.d_desc, (size_t)K * dl * sizeof(float), cudaMemcpyDeviceToHost, s.stream));
   }
   kpRun += K;
   if (ctx->cloudOutputs && s.h_cloudOff) {  // the two optional clouds, gathered on the device by enqueue_pipeline
-    const int64_t tc = s.h_cloudOff[s.nscans], tk = s.h_kcOff[s.nscans];
-    st = grow_pinned_points(ctx, &ctx->h_cloud, &ctx->capCloud, ctx->cloudRun, ctx->cloudRun + tc);
+    const int64_t tc = s.h_cloudOff[ns], tk = s.h_kcOff[ns];
+    st = grow_pinned(ctx, &ctx->h_cloud, &ctx->capCloud, ctx->cloudRun + tc, 1 << 16, ctx->cloudRun);
     if (st) return st;
-    st = grow_pinned_points(ctx, &ctx->h_kc, &ctx->capKcRes, ctx->kcRun, ctx->kcRun + tk);
+    st = grow_pinned(ctx, &ctx->h_kc, &ctx->capKcRes, ctx->kcRun + tk, 1 << 16, ctx->kcRun);
     if (st) return st;
-    for (int i = 0; i <= s.nscans; i++) {
+    for (int i = 0; i <= ns; i++) {
       ctx->cloudOff[s.firstScan + i] = ctx->cloudRun + s.h_cloudOff[i];
       ctx->kcOff[s.firstScan + i] = ctx->kcRun + s.h_kcOff[i];
     }
@@ -976,7 +1007,6 @@ struct SlotDrain {
     for (int k = 0; k < 2; k++) {
       Slot& s = ctx->slot[k];
       if (s.stream) cudaStreamSynchronize(s.stream);
-      if (s.stream2) cudaStreamSynchronize(s.stream2);
       s.busy = false;
     }
   }
@@ -1081,7 +1111,7 @@ int fe_create(int device, const fe_params_t* params, const fe_limits_t* limits, 
 int fe_set_params(fe_ctx_t* ctx, const fe_params_t* params) {
   if (!ctx || !params) return FE_ERR_INVALID;
   cudaSetDevice(ctx->device);
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) cudaStreamSynchronize(ctx->slot[k].stream);
+  sync_slots(ctx);
   ctx->epoch++;
   return derive_params(ctx, *params);
 }
@@ -1108,7 +1138,7 @@ int fe_enable_cloud_outputs(fe_ctx_t* ctx, int32_t enable) {
 
 int fe_enable_stage_timing(fe_ctx_t* ctx, int32_t enable) {
   if (!ctx) return FE_ERR_INVALID;
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
+  if (int st = sync_slots(ctx)) return st;
   ctx->stageTiming = enable != 0;
   ctx->epoch++;
   return FE_OK;
@@ -1116,7 +1146,7 @@ int fe_enable_stage_timing(fe_ctx_t* ctx, int32_t enable) {
 
 int fe_enable_record_output(fe_ctx_t* ctx, int32_t enable) {
   if (!ctx) return FE_ERR_INVALID;
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
+  if (int st = sync_slots(ctx)) return st;
   ctx->recordOutput = enable != 0;
   ctx->epoch++;
   return FE_OK;
@@ -1124,7 +1154,7 @@ int fe_enable_record_output(fe_ctx_t* ctx, int32_t enable) {
 
 int fe_set_angle_libm(fe_ctx_t* ctx, int32_t mode) {
   if (!ctx || (mode != FE_LIBM_FDLIBM && mode != FE_LIBM_CORRECTLY_ROUNDED)) return FE_ERR_INVALID;
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
+  if (int st = sync_slots(ctx)) return st;
   ctx->angleLibm = mode;
   ctx->dp.angle_libm = mode;
   ctx->epoch++;
@@ -1133,7 +1163,7 @@ int fe_set_angle_libm(fe_ctx_t* ctx, int32_t mode) {
 
 int fe_enable_boundary_report(fe_ctx_t* ctx, double eps_m) {
   if (!ctx || !(eps_m == eps_m)) return FE_ERR_INVALID;
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
+  if (int st = sync_slots(ctx)) return st;
   ctx->bndEps = eps_m > 0.0 ? eps_m : 0.0;
   ctx->bndCounts.clear();
   ctx->epoch++;
@@ -1209,7 +1239,7 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
     int st = ensure_slot(ctx, s, true);
     if (st) return st;
     // previous sub-batch of this slot must have been finalised (its device buffers are reused)
-    st = finalize_subbatch(ctx, s, kpRun, desc);
+    st = finalize_subbatch(ctx, s, kpRun);
     if (st) return st;
     // greedy sub-batch
     int last = first;
@@ -1222,40 +1252,29 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
       npts += n;
       last++;
     }
-    const int ns = last - first;
-    int64_t np2; int nch;
-    const bool graphable = ctx->useGraphs && !ctx->stageTiming && ns <= GRAPH_MAX_SCANS;
-    st = stage_scans(ctx, s, scan_offsets + first, roll_pitch + 2 * first, ns, &np2, &nch, false, !graphable);
+    SubBatch sb = batch_subbatch(ctx, s.d_pts, last - first);
+    sb.wantKc = ctx->cloudOutputs;
+    sb.lay = RawLayout{isFloat4 ? nullptr : (const unsigned char*)s.d_pts, stride, xo, yo, zo};
+    st = stage_scans(ctx, s, scan_offsets + first, roll_pitch + 2 * first, sb.nscans, &sb.npts, &sb.nch);
     if (st) return st;
-    if (npts > 0)
-      CK(cudaMemcpyAsync(s.d_pts, points + scan_offsets[first] * (int64_t)stride, (size_t)npts * (size_t)stride, cudaMemcpyHostToDevice, s.stream));
-    const bool wantKc = ctx->cloudOutputs;
-    if (wantKc) { st = ensure_kc(ctx, s); if (st) return st; }
-    RawLayout lay = {isFloat4 ? nullptr : (const unsigned char*)s.d_pts, stride, xo, yo, zo};
-    const int k1flags = F_ELEV | F_ROT | F_CROP | F_RING | (desc ? F_SURF : 0);
-    if (!graphable) {
-      s.lean = false;
-      st = enqueue_pipeline(ctx, s, s.d_pts, ns, npts, nch, k1flags, desc, false, wantKc, lay);
-      if (st) return st;
-    } else {
-      st = enqueue_small(ctx, s, s.d_pts, false, ns, npts, nch, k1flags, desc, wantKc, lay);
-      if (st) return st;
-    }
-    s.busy = true; s.nscans = ns; s.npts = npts; s.firstScan = first;
+    if (sb.wantKc) { st = ensure_kc(ctx, s); if (st) return st; }
+    st = enqueue_subbatch(ctx, s, sb, nullptr, points + scan_offsets[first] * (int64_t)stride, (size_t)npts * (size_t)stride);
+    if (st) return st;
+    s.busy = true; s.firstScan = first;
     nsub++;
     // the other slot's sub-batch was enqueued earlier: finalise it while this one runs
     Slot& o = ctx->slot[cur ^ 1];
-    if (o.busy) { st = finalize_subbatch(ctx, o, kpRun, desc); if (st) return st; }
+    if (o.busy) { st = finalize_subbatch(ctx, o, kpRun); if (st) return st; }
     first = last;
     cur ^= 1;
   }
   // drain in submission order
   for (int k = 0; k < 2; k++) {
     Slot& s = ctx->slot[cur ^ k];  // cur now points at the older one
-    int st = finalize_subbatch(ctx, s, kpRun, desc);
+    int st = finalize_subbatch(ctx, s, kpRun);
     if (st) return st;
   }
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
+  if (int st = sync_slots(ctx)) return st;
   if (nsub == 1) collect_times(ctx, ctx->slot[0]);
   out->n_scans = n_scans;
   out->n_keypoints = kpRun;
@@ -1325,33 +1344,20 @@ int fe_process_batch_device(fe_ctx_t* ctx, const fe_point_t* d_points, const int
   int st = ensure_slot(ctx, s, false);
   if (st) return st;
   ctx->kpOffsets.assign((size_t)n_scans + 1, 0);
-  int64_t npts = 0; int nch = 0;
   if (n_scans > 0) {
-    const bool late = n_scans >= 2048;
-    const bool small = ctx->useGraphs && !ctx->stageTiming && n_scans <= GRAPH_MAX_SCANS;
-    const int k1flags = F_ELEV | F_ROT | F_CROP | F_RING | (desc ? F_SURF : 0);
-    const float4* d_pts = (const float4*)d_points + scan_offsets[0];
-    st = stage_scans(ctx, s, scan_offsets, roll_pitch, n_scans, &npts, &nch, late, !small);
+    // 2048 scans and more: the levelling matrices are computed while K1 runs (enqueue_pipeline)
+    const double* lateRp = n_scans >= 2048 ? roll_pitch : nullptr;
+    // the input's address is part of the graph key: a replay reads the same address
+    SubBatch sb = batch_subbatch(ctx, (const float4*)d_points + scan_offsets[0], n_scans);
+    st = stage_scans(ctx, s, scan_offsets, roll_pitch, n_scans, &sb.npts, &sb.nch, lateRp != nullptr);
     if (st) return st;
-    s.nscans = n_scans; s.npts = npts;
-    if (small) {  // a handful of scans: lean chain, replayed from a graph captured for this shape and input pointer
-      st = enqueue_small(ctx, s, d_pts, true, n_scans, npts, nch, k1flags, desc, false, RawLayout{nullptr, 0, 0, 0, 0});
-    } else {
-      s.lean = false;
-      st = enqueue_pipeline(ctx, s, d_pts, n_scans, npts, nch, k1flags, desc, false, false, RawLayout{nullptr, 0, 0, 0, 0},
-                            late ? roll_pitch : nullptr);
-    }
+    st = enqueue_subbatch(ctx, s, sb, lateRp);
     if (st) return st;
-    CK(cudaEventSynchronize(s.evDone));
-    st = lean_rerun_if_deferred(ctx, s);
-    if (st) return st;
-    if (s.h_ctr->err) return fail(ctx, FE_ERR_CAPACITY, err_bits(s.h_ctr->err));
-    for (int i = 0; i <= n_scans; i++) ctx->kpOffsets[i] = s.h_kpOff[i];
     ctx->bndCounts.assign(ctx->bndEps > 0.0 ? (size_t)n_scans * 4 : 0, 0);
-    if (ctx->bndEps > 0.0 && s.h_bnd)
-      for (int i = 0; i < n_scans * 4; i++) ctx->bndCounts[i] = (int64_t)s.h_bnd[i];
+    s.firstScan = 0;
+    st = complete_subbatch(ctx, s, 0);
+    if (st) return st;
     collect_times(ctx, s);
-    s.nscans = n_scans; s.npts = npts; s.lastNch = nch;
   }
   out->n_scans = n_scans;
   out->n_keypoints = ctx->kpOffsets[n_scans];
@@ -1387,18 +1393,18 @@ int fe_get_batch_stats(fe_ctx_t* ctx, int64_t out[10]) {
   Slot& s = ctx->slot[0];
   CK(cudaStreamSynchronize(s.stream));
   for (int i = 0; i < 10; i++) out[i] = 0;
-  out[0] = s.npts;
-  std::vector<int> a((size_t)std::max(s.lastNch, 1)), b((size_t)std::max(s.lastNch, 1));
-  if (s.lastNch > 0) {
-    CK(cudaMemcpy(a.data(), s.d_surfCnt, (size_t)s.lastNch * sizeof(int), cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(b.data(), s.d_cropCnt, (size_t)s.lastNch * sizeof(int), cudaMemcpyDeviceToHost));
-    for (int i = 0; i < s.lastNch; i++) { out[1] += a[i]; out[2] += b[i]; }
+  out[0] = s.sb.npts;
+  std::vector<int> a((size_t)std::max(s.sb.nch, 1)), b((size_t)std::max(s.sb.nch, 1));
+  if (s.sb.nch > 0) {
+    CK(cudaMemcpy(a.data(), s.d_surfCnt, (size_t)s.sb.nch * sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(b.data(), s.d_cropCnt, (size_t)s.sb.nch * sizeof(int), cudaMemcpyDeviceToHost));
+    for (int i = 0; i < s.sb.nch; i++) { out[1] += a[i]; out[2] += b[i]; }
   }
-  if (s.nscans > 0) {
-    std::vector<int> kf((size_t)s.nscans * 16);
+  if (s.sb.nscans > 0) {
+    std::vector<int> kf((size_t)s.sb.nscans * 16);
     CK(cudaMemcpy(kf.data(), s.d_kfCnt, kf.size() * sizeof(int), cudaMemcpyDeviceToHost));
     for (int v : kf) out[3] += v;
-    const int K = s.h_kpOff[s.nscans];
+    const int K = s.h_kpOff[s.sb.nscans];
     out[4] = K;
     if (K > 0 && ctx->params.estimate_descriptors) {
       std::vector<int> nb((size_t)K);
@@ -1422,59 +1428,53 @@ int fe_download(fe_ctx_t* ctx, void* host_dst, const void* device_src, int64_t b
 
 // ---- one entry point per reference function ----------------------------------------------------------
 
-static int stage_k1(fe_ctx* ctx, fe_point_t* cloud, int64_t n, double roll, double pitch, int flags) {
-  // K1 with full_out: every point transformed in place (no compaction)
-  Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, true);
-  if (st) return st;
-  if (n == 0) return FE_OK;
-  if (!s.d_full) CK(dalloc(&s.d_full, (size_t)s.capPts));
+// Upload a one-scan cloud and run K1 on it with `flags` and the parameters P, levelled by rp = {roll, pitch} (null:
+// the identity).  K1 compacts its survivors into the chunk pieces; with fullOut it also writes every point, transformed
+// in place, to s.d_full, which is copied to fullOut before this returns.
+static int scan_k1(fe_ctx* ctx, Slot& s, const DevParams& P, const fe_point_t* in, int64_t n, int flags,
+                   const double* rp = nullptr, fe_point_t* fullOut = nullptr) {
+  if (fullOut && !s.d_full) CK(dalloc(&s.d_full, (size_t)s.capPts));
   int64_t offs[2] = {0, n};
-  double rp[2] = {roll, pitch};
   int64_t npts; int nch;
-  st = stage_scans(ctx, s, offs, rp, 1, &npts, &nch);
+  int st = stage_scans(ctx, s, offs, rp, 1, &npts, &nch);
+  if (st == FE_OK) st = stage_scans_copy(ctx, s, 1, false);
   if (st) return st;
-  CK(cudaMemcpyAsync(s.d_pts, cloud, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, s.stream));
-  k_level_crop_ring<false, false><<<nch, 256, 0, s.stream>>>(s.d_pts, s.d_chunkTab, s.d_rot, ctx->dp, flags, s.d_surf,
-                                               s.d_surfCnt, s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_full, RawLayout{nullptr, 0, 0, 0, 0}, 0);
-  ctx->launches++;
+  if (n > 0) CK(cudaMemcpyAsync(s.d_pts, in, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, s.stream));
+  if (nch > 0) {
+    k_level_crop_ring<false, false><<<nch, 256, 0, s.stream>>>(s.d_pts, s.d_chunkTab, s.d_rot, P, flags, s.d_surf, s.d_surfCnt,
+                                                               s.d_crop, s.d_cropMeta, s.d_cropCnt, fullOut ? s.d_full : nullptr,
+                                                               RawLayout{nullptr, 0, 0, 0, 0}, 0);
+    ctx->launches++;
+  }
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(cloud, s.d_full, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, s.stream));
-  CK(cudaStreamSynchronize(s.stream));
+  if (fullOut) {
+    CK(cudaMemcpyAsync(fullOut, s.d_full, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, s.stream));
+    CK(cudaStreamSynchronize(s.stream));
+  }
   return FE_OK;
 }
 
 int fe_get_elevation_angles(fe_ctx_t* ctx, fe_point_t* cloud, int64_t n) {
   if (!ctx || (n > 0 && !cloud) || n < 0) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
-  return stage_k1(ctx, cloud, n, 0.0, 0.0, F_ELEV);
+  int st = ensure_slot(ctx, ctx->slot[0], true);
+  if (st || n == 0) return st;
+  const double rp[2] = {0.0, 0.0};
+  return scan_k1(ctx, ctx->slot[0], ctx->dp, cloud, n, F_ELEV, rp, cloud);
 }
 
 int fe_rotate_cloud(fe_ctx_t* ctx, fe_point_t* cloud, int64_t n, double roll, double pitch) {
   if (!ctx || (n > 0 && !cloud) || n < 0) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
-  return stage_k1(ctx, cloud, n, roll, pitch, F_ROT);
+  int st = ensure_slot(ctx, ctx->slot[0], true);
+  if (st || n == 0) return st;
+  const double rp[2] = {roll, pitch};
+  return scan_k1(ctx, ctx->slot[0], ctx->dp, cloud, n, F_ROT, rp, cloud);
 }
 
 int fe_rotation_matrix(double roll, double pitch, float m[9]) {
   if (!m) return FE_ERR_INVALID;
   leveling_matrix(roll, pitch, m);
-  return FE_OK;
-}
-
-// upload a one-scan cloud and run K1 with the given flags (compacting into the chunk pieces)
-static int stage_upload_k1(fe_ctx* ctx, Slot& s, const fe_point_t* in, int64_t n, int flags, int* nchOut) {
-  int64_t offs[2] = {0, n};
-  int64_t npts;
-  int st = stage_scans(ctx, s, offs, nullptr, 1, &npts, nchOut);
-  if (st) return st;
-  if (n > 0) CK(cudaMemcpyAsync(s.d_pts, in, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, s.stream));
-  if (*nchOut > 0) {
-    k_level_crop_ring<false, false><<<*nchOut, 256, 0, s.stream>>>(s.d_pts, s.d_chunkTab, s.d_rot, ctx->dp, flags, s.d_surf,
-                                                     s.d_surfCnt, s.d_crop, s.d_cropMeta, s.d_cropCnt, nullptr, RawLayout{nullptr, 0, 0, 0, 0}, 0);
-    ctx->launches++;
-  }
-  CK(cudaGetLastError());
   return FE_OK;
 }
 
@@ -1496,8 +1496,7 @@ int fe_filter_cloud(fe_ctx_t* ctx, const fe_point_t* in, int64_t n, fe_point_t* 
   if (st) return st;
   st = ensure_kc(ctx, s);
   if (st) return st;
-  int nch;
-  st = stage_upload_k1(ctx, s, in, n, F_CROP, &nch);
+  st = scan_k1(ctx, s, ctx->dp, in, n, F_CROP);
   if (st) return st;
   std::vector<int64_t> off;
   std::vector<fe_point_t> pts;
@@ -1557,8 +1556,7 @@ static int stage_keypoints(fe_ctx* ctx, const fe_point_t* cloud, int64_t n, bool
   if (st) return st;
   st = ensure_kc(ctx, s);
   if (st) return st;
-  int nch;
-  st = stage_upload_k1(ctx, s, cloud, n, singleRing ? 0 : F_RING, &nch);
+  st = scan_k1(ctx, s, ctx->dp, cloud, n, singleRing ? 0 : F_RING);
   if (st) return st;
   CK(cudaMemsetAsync(s.d_ctr, 0, sizeof(DevCounters), s.stream));
   launch_clustering(ctx, s, 1, singleRing, true, merge);
@@ -1618,20 +1616,12 @@ int fe_estimate_descriptors(fe_ctx_t* ctx, const fe_point_t* cloud_full, int64_t
     for (int d = 0; d < 3; d++) { lo[d] = std::min(lo[d], v[d]); hi[d] = std::max(hi[d], v[d]); }
   }
   if (!(lo[0] <= hi[0])) { for (int d = 0; d < 3; d++) { lo[d] = 0.f; hi[d] = 0.f; } }
-  DevParams saved = ctx->dp;
-  surface_grid(ctx->dp, ctx->params.descriptor_radius, lo[0], hi[0], lo[1], hi[1], lo[2], hi[2]);
   DevParams P = ctx->dp;
-  auto restore = [&](int code) { ctx->dp = saved; return code; };
-  int nch = 0;
-  st = stage_upload_k1(ctx, s, cloud_full, n, F_SURF, &nch);
-  if (st) return restore(st);
-  if (n == 0) {  // one empty scan
-    int64_t offs[2] = {0, 0}; int64_t np0;
-    st = stage_scans(ctx, s, offs, nullptr, 1, &np0, &nch);
-    if (st) return restore(st);
-  }
-  st = ensure_rowstart(ctx, s, 1);
-  if (st) return restore(st);
+  surface_grid(P, ctx->params.descriptor_radius, lo[0], hi[0], lo[1], hi[1], lo[2], hi[2]);
+  st = scan_k1(ctx, s, P, cloud_full, n, F_SURF);  // n == 0: one empty scan
+  if (st) return st;
+  st = ensure_rowstart(ctx, s, P, 1);
+  if (st) return st;
   cudaStream_t q = s.stream;
   std::vector<int> kpOff = {0, (int)k};
   std::vector<int> kpScan((size_t)k, 0);
@@ -1639,12 +1629,11 @@ int fe_estimate_descriptors(fe_ctx_t* ctx, const fe_point_t* cloud_full, int64_t
       cudaMemcpyAsync(s.d_kpOff, kpOff.data(), 2 * sizeof(int), cudaMemcpyHostToDevice, q) != cudaSuccess ||
       cudaMemcpyAsync(s.d_kpScan, kpScan.data(), (size_t)k * sizeof(int), cudaMemcpyHostToDevice, q) != cudaSuccess ||
       cudaMemcpyAsync(s.d_kpOut, keypoints, (size_t)k * sizeof(float4), cudaMemcpyHostToDevice, q) != cudaSuccess)
-    return restore(fail(ctx, FE_ERR_CUDA, "staging of the descriptor inputs failed"));
-  launch_surface_grid(ctx, s, 1, P, s.stream);
+    return fail(ctx, FE_ERR_CUDA, "staging of the descriptor inputs failed");
+  launch_surface_grid(ctx, s, 1, P);
   launch_desc_mark(ctx, s, 1, P, ctx->numSms * 4);
   launch_density(ctx, s, 1, P, n);
   launch_desc_hist(ctx, s, 1, P, ctx->numSms * 4, false);
-  ctx->dp = saved;
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(s.h_ctr, s.d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, q));
   CK(cudaMemcpyAsync(descriptors, s.d_desc, (size_t)k * FE_DESC_LEN * sizeof(float), cudaMemcpyDeviceToHost, q));
@@ -1828,8 +1817,8 @@ int fe_debug_density_work(fe_ctx_t* ctx, int64_t out[3]) {
   out[0] = (int64_t)s.h_ctr->dens_work[0];
   out[1] = (int64_t)s.h_ctr->dens_work[1];
   out[2] = 0;
-  if (s.nscans > 0 && ctx->params.estimate_descriptors) {
-    std::vector<int> sn((size_t)s.nscans);
+  if (s.sb.nscans > 0 && ctx->params.estimate_descriptors) {
+    std::vector<int> sn((size_t)s.sb.nscans);
     CK(cudaMemcpy(sn.data(), s.d_surfN, sn.size() * sizeof(int), cudaMemcpyDeviceToHost));
     for (int v : sn) out[2] += v;
   }
@@ -1859,7 +1848,7 @@ int fe_debug_h2d_probe(fe_ctx_t* ctx, const void* host, int64_t bytes, float* ms
 // that tests can cross-check the two algorithms against each other and against the oracle
 int fe_debug_force_grid_clustering(fe_ctx_t* ctx, int32_t enable) {
   if (!ctx) return FE_ERR_INVALID;
-  for (int k = 0; k < 2; k++) if (ctx->slot[k].stream) CK(cudaStreamSynchronize(ctx->slot[k].stream));
+  if (int st = sync_slots(ctx)) return st;
   ctx->gridClustering = enable != 0;
   ctx->epoch++;
   return FE_OK;

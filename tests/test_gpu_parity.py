@@ -255,8 +255,8 @@ def test_record_output_equals_concatenate_fields_on_the_host(ob, synth, nodes):
 
 
 def test_stage_timing_mode_serialises_without_changing_results(ob, synth, nodes):
-    """fe_enable_stage_timing: the surface-grid kernel leaves its side stream, every stage gets a
-    CUDA-event pair; results stay bit-identical and fe_get_stage_times reports the stages."""
+    """fe_enable_stage_timing: small calls run eagerly instead of from a captured graph, every stage
+    gets a CUDA-event pair; results stay bit-identical and fe_get_stage_times reports the stages."""
     import torch
     nd = nodes(2)
     pts, offs, rp = synth.generate(2, 48, scan_index_base=4100)
