@@ -25,6 +25,7 @@ EXPORTS = [
     "fe_filter_cloud", "fe_extract_clusters", "fe_get_cylinder_segments", "fe_estimate_keypoints",
     "fe_estimate_descriptors", "fe_pack_point_descriptors",
     "fe_set_angle_libm", "fe_enable_boundary_report", "fe_get_boundary_report",
+    "fe_enable_boundary_report_all", "fe_get_boundary_report_all",
     "fe_multi_enable_cloud_outputs", "fe_multi_get_cloud_outputs",
 ]
 
@@ -135,6 +136,8 @@ def lib():
         L.fe_set_angle_libm.argtypes = [C.c_void_p, C.c_int32]
         L.fe_enable_boundary_report.argtypes = [C.c_void_p, C.c_double]
         L.fe_get_boundary_report.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_int32)]
+        L.fe_enable_boundary_report_all.argtypes = [C.c_void_p, C.c_double]
+        L.fe_get_boundary_report_all.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_int32)]
         L.fe_multi_enable_cloud_outputs.argtypes = [C.c_void_p, C.c_int32]
         L.fe_multi_get_cloud_outputs.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_void_p),
                                                  C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_void_p)]

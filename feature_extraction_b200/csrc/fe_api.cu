@@ -45,7 +45,7 @@ struct GraphKey {
   SubBatch sb;
   int by;        // density_blocks_per_scan: K4c's grid
   bool bigScan;  // a scan of more than 65,535 points: launch_surface_grid adds the radix kernel
-  bool bnd;
+  int bnd;       // boundary report: 0 off, 4 radius kinds (k_boundary_*), FE_BOUNDARY_KINDS all kinds
   int epoch;
   bool operator==(const GraphKey& o) const {
     const SubBatch &a = sb, &b = o.sb;
@@ -97,6 +97,8 @@ struct Slot {
   DevCounters* d_ctr = nullptr;
   unsigned long long* d_bnd = nullptr;  // tolerance-boundary report: [scan][4] pair counts
   unsigned long long* h_bnd = nullptr;
+  unsigned long long *d_bndX = nullptr, *h_bndX = nullptr;  // fe_enable_boundary_report_all: [scan][6], kinds 4-9
+  unsigned* d_gate = nullptr;  // kind 6 per (scan, ring) as the K2 kernels leave it (GateCount)
   // pinned host mirrors
   long long* h_scan_off = nullptr;
   int* h_chunk_off = nullptr;
@@ -138,7 +140,9 @@ struct fe_ctx {
   int64_t graphReplays = 0;
   int angleLibm = 0;          // fe_set_angle_libm
   double bndEps = 0.0;        // fe_enable_boundary_report: > 0 = count the pairs within bndEps of every radius
-  std::vector<int64_t> bndCounts;  // [scan][4] of the last batch call
+  bool bndAll = false;        // fe_enable_boundary_report_all: also kinds 4-9
+  std::vector<int64_t> bndCounts;     // [scan][4] of the last batch call
+  std::vector<int64_t> bndCountsAll;  // [scan][FE_BOUNDARY_KINDS] of the last batch call (bndAll)
   // results (host, pinned, grown on demand)
   std::vector<int64_t> kpOffsets;
   fe_point_t* h_kp = nullptr;
@@ -306,9 +310,9 @@ void free_slot(Slot& s) {
   void* dv[] = {s.d_ringPts, s.d_pts, s.d_surf, s.d_crop, s.d_sorted, s.d_full, s.d_cropMeta, s.d_keyA, s.d_keyB, s.d_valA, s.d_valB,
                 s.d_sortedKey, s.d_rho, s.d_scan_off, s.d_chunk_off, s.d_surfCnt, s.d_cropCnt, s.d_rot, s.d_kfBase,
                 s.d_kfCnt, s.d_kcBase, s.d_kcCnt, s.d_kpBase, s.d_kpCnt, s.d_kpOff, s.d_kpScan, s.d_kpNbr, s.d_kpNbrOff, s.d_kpRank, s.d_kpListM, s.d_kpListL, s.d_rowStart,
-                s.d_surfN, s.d_perScan, s.d_outOff, s.d_ovfRings, s.d_ovfRings2, s.d_ovfMerge, s.d_ovfMerge2, s.d_ovfSurf, s.d_slabs, s.d_gridHdr, s.d_tabOk, s.d_kfPool, s.d_kcPool, s.d_kpPool, s.d_kpOut, s.d_gather, s.d_desc, s.d_ctr, s.d_bnd, s.d_ringBase, s.d_ovfRuns, s.d_scanFlag, s.d_perScan2, s.d_outOff2, s.d_gather2, s.d_chunkTab};
+                s.d_surfN, s.d_perScan, s.d_outOff, s.d_ovfRings, s.d_ovfRings2, s.d_ovfMerge, s.d_ovfMerge2, s.d_ovfSurf, s.d_slabs, s.d_gridHdr, s.d_tabOk, s.d_kfPool, s.d_kcPool, s.d_kpPool, s.d_kpOut, s.d_gather, s.d_desc, s.d_ctr, s.d_bnd, s.d_bndX, s.d_gate, s.d_ringBase, s.d_ovfRuns, s.d_scanFlag, s.d_perScan2, s.d_outOff2, s.d_gather2, s.d_chunkTab};
   for (void* p : dv) if (p) cudaFree(p);
-  void* hv[] = {s.h_scan_off, s.h_chunk_off, s.h_rot, s.h_ctr, s.h_kpOff, s.h_perScan, s.h_bnd, s.h_cloudOff, s.h_kcOff};
+  void* hv[] = {s.h_scan_off, s.h_chunk_off, s.h_rot, s.h_ctr, s.h_kpOff, s.h_perScan, s.h_bnd, s.h_bndX, s.h_cloudOff, s.h_kcOff};
   for (void* p : hv) if (p) cudaFreeHost(p);
   for (cudaEvent_t e : s.ev) cudaEventDestroy(e);
   for (GraphEntry& g : s.graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
@@ -500,6 +504,14 @@ int set_kernel_attrs(fe_ctx* ctx) {
                           (int)desc_smem_bytes(DCAP_L, 512)));
   CK(cudaFuncSetAttribute(k_surface_grid_cells<NT_SURF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)surf_cells_smem_bytes(SURF_MAX_CELLS)));
+  // the boundary report's K2 instantiations (kind 6).  Named after every other kernel: the order in which the host
+  // code first names the kernels is the order the compiler meets them, and the kernels above compile as they did
+  // before these existed only in this order.
+  CK(cudaFuncSetAttribute(k_cluster_rings_bnd<ECAP, NTF, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmem));
+  CK(cudaFuncSetAttribute(k_ring_runs_bnd<NW_RR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW>)));
+  CK(cudaFuncSetAttribute(k_ring_runs_bnd<NW_RR_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW, NW_RR_SMALL>)));
+  CK(cudaFuncSetAttribute(k_ring_runs_wide_bnd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(NW_RR * sizeof(RunBufT<RW2>))));
+  CK(cudaFuncSetAttribute(k_cluster_rings_bnd<ECAP_L, NT2, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemL));
   return FE_OK;
 }
 
@@ -608,7 +620,9 @@ void launch_density(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int64_
 
 // K2 + K3 for `nscans` scans: the 2-blocks-per-SM instantiation first, then the large one over
 // whatever scans it deferred (an immediate exit when there are none).
-void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool wantKc, bool merge, bool marks = false, bool lean = false) {
+// gate: count kind 6 of the boundary report (fe_enable_boundary_report_all) with the GateCount instantiations of K2
+void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool wantKc, bool merge, bool marks = false, bool lean = false,
+                       const GateCount* gate = nullptr) {
   // Every stage is a chain of instantiations: the fast one takes all scans and defers those that do
   // not fit its shared memory to a list; the large shared-memory one takes that list; what does not
   // fit there either goes to the instantiation whose per-entry arrays live in global memory.
@@ -625,11 +639,12 @@ void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool w
   const int sr = singleRing ? 1 : 0;
   // inList / inN: the scans the previous instantiation deferred to this one (null: every scan); outList / outN: where
   // this one defers what it cannot take (null: the last of the chain); slabs: per-entry arrays in global memory
+  // `gate...`: nothing, or the GateCount of a *_bnd kernel
   auto k2 = [&](auto kernel, int grid, int nt, size_t smem, const int* inList, const int* inN, int* outList, int* outN,
-                unsigned char* slabs) {
+                unsigned char* slabs, auto... gate) {
     kernel<<<grid, nt, smem, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_kfPool,
                                          s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr, inList, inN, outList,
-                                         outN, slabs);
+                                         outN, slabs, gate...);
     ctx->launches++;
   };
   auto k3 = [&](auto kernel, int grid, int nt, size_t smem, const int* inList, const int* inN, int* outList, int* outN,
@@ -641,30 +656,45 @@ void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool w
   // K2: the run-based kernel takes every scan; what it cannot handle (a ring with more than RW runs — unordered
   // input — or more ring entries than the scan's scratch slot) goes down the chain of grid-based instantiations.
   if (ctx->gridClustering) {
-    k2(k_cluster_rings<ECAP, NTF, 4, false>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr);
+    if (gate) k2(k_cluster_rings_bnd<ECAP, NTF, 4, false>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr, *gate);
+    else k2(k_cluster_rings<ECAP, NTF, 4, false>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr);
   } else {
-    auto rr = [&](auto kernel, int nt, size_t smem) {
+    auto rr = [&](auto kernel, int nt, size_t smem, auto... gate) {
       kernel<<<nscans, nt, smem, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_ringPts,
                                              s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
-                                             s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR);
+                                             s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR, gate...);
       ctx->launches++;
     };
-    if (nscans <= GRAPH_MAX_SCANS)  // a handful of scans: a warp for each of a scan's 16 rings at once (latency, not throughput)
-      rr(k_ring_runs<NW_RR_SMALL>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>));
-    else
-      rr(k_ring_runs<NW_RR>, NT_RR, sizeof(RingRunsSmT<RW>));
+    if (nscans <= GRAPH_MAX_SCANS) {  // a handful of scans: a warp for each of a scan's 16 rings at once (latency, not throughput)
+      if (gate) rr(k_ring_runs_bnd<NW_RR_SMALL>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>), *gate);
+      else rr(k_ring_runs<NW_RR_SMALL>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>));
+    } else {
+      if (gate) rr(k_ring_runs_bnd<NW_RR>, NT_RR, sizeof(RingRunsSmT<RW>), *gate);
+      else rr(k_ring_runs<NW_RR>, NT_RR, sizeof(RingRunsSmT<RW>));
+    }
     if (!lean) {
-      k_ring_runs_wide<<<std::min(nscans * 4, ctx->numSms * 7), NT_RR, NW_RR * sizeof(RunBufT<RW2>), s.stream>>>(
-          s.d_scan_off, P, s.d_ringPts, s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
-          s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR);
-      ctx->launches++;
+      auto wide = [&](auto kernel, auto... gate) {
+        kernel<<<std::min(nscans * 4, ctx->numSms * 7), NT_RR, NW_RR * sizeof(RunBufT<RW2>), s.stream>>>(
+            s.d_scan_off, P, s.d_ringPts, s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
+            s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR, gate...);
+        ctx->launches++;
+      };
+      if (gate) wide(k_ring_runs_wide_bnd, *gate);
+      else wide(k_ring_runs_wide);
     }
   }
   // lean: the fallback instantiations are left out; whatever the first kernel deferred shows in the counters and the
   // caller runs the sub-batch again with the whole chain
   if (!lean) {
-    k2(k_cluster_rings<ECAP_L, NTL, 1, false>, gridL, NTL, kClusterSmemL2, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr);
-    k2(k_cluster_rings<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs);
+    if (gate) {
+      // 512 threads, not NTL: a second caller of the 1024-thread cluster helpers changes how k_cluster_rings<ECAP_L, NTL>
+      // compiles (the capacity is the same, hence the same deferrals and clusters)
+      k2(k_cluster_rings_bnd<ECAP_L, NT2, 1, false>, gridL, NT2, kClusterSmemL, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr, *gate);
+      k2(k_cluster_rings_bnd<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs, *gate);
+    } else {
+      k2(k_cluster_rings<ECAP_L, NTL, 1, false>, gridL, NTL, kClusterSmemL2, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr);
+      k2(k_cluster_rings<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs);
+    }
   }
   if (marks) mark(ctx, s, "K2 ring clusters");
   if (merge) {
@@ -690,10 +720,18 @@ BoundarySpec boundary_spec(const fe_ctx* ctx) {
   return B;
 }
 
+// which kinds the boundary report counts: 0 (off), 4 or FE_BOUNDARY_KINDS
+int bnd_kinds(const fe_ctx* ctx) { return ctx->bndEps > 0.0 ? (ctx->bndAll ? FE_BOUNDARY_KINDS : 4) : 0; }
+
 int ensure_bnd(fe_ctx* ctx, Slot& s) {
   if (!s.d_bnd) {
     CK(dalloc(&s.d_bnd, (size_t)s.capScans * 4));
     CK(halloc(&s.h_bnd, (size_t)s.capScans * 4));
+  }
+  if (ctx->bndAll && !s.d_bndX) {
+    CK(dalloc(&s.d_bndX, (size_t)s.capScans * 6));
+    CK(halloc(&s.h_bndX, (size_t)s.capScans * 6));
+    CK(dalloc(&s.d_gate, (size_t)s.capScans * 16));
   }
   return FE_OK;
 }
@@ -739,6 +777,7 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
   }
   mark(ctx, s, "K1 level+crop+ring");
   const bool bnd = ctx->bndEps > 0.0 && nscans > 0;
+  const bool bndAll = bnd && ctx->bndAll;  // kinds 4-9 too
   if (bnd) {
     int st = ensure_bnd(ctx, s);
     if (st) return st;
@@ -747,14 +786,29 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
                                                    boundary_spec(ctx), s.d_bnd);
     ctx->launches++;
   }
+  const GateCount gate = {ctx->bndEps, s.d_gate};  // (after ensure_bnd: d_gate is allocated on the first call with bndAll)
+  if (bndAll) {
+    CK(cudaMemsetAsync(s.d_bndX, 0, (size_t)nscans * 6 * sizeof(unsigned long long), s.stream));
+    CK(cudaMemsetAsync(s.d_gate, 0, (size_t)nscans * 16 * sizeof(unsigned), s.stream));
+    const int nch = s.h_chunk_off[nscans];  // every chunk of the sub-batch: the matrices of all of them are staged by now
+    if (nch > 0) {
+      if (sb.lay.raw) k_boundary_crop_ring<true><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, ctx->bndEps, s.d_bndX);
+      else k_boundary_crop_ring<false><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, ctx->bndEps, s.d_bndX);
+      ctx->launches++;
+    }
+  }
   if (sb.desc) {
     int st = ensure_rowstart(ctx, s, P, nscans);
     if (st) return st;
   }
-  launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean);
+  launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean, bndAll ? &gate : nullptr);
   mark(ctx, s, "K3 merge keypoints");
   if (bnd) {
     k_boundary_merge<<<nscans, 128, 0, s.stream>>>(s.d_kfPool, s.d_kfBase, s.d_kfCnt, P, boundary_spec(ctx), s.d_bnd);
+    ctx->launches++;
+  }
+  if (bndAll) {
+    k_boundary_gate_sum<<<(nscans + 255) / 256, 256, 0, s.stream>>>(s.d_gate, nscans, s.d_bndX);
     ctx->launches++;
   }
   if (nscans <= GRAPH_MAX_SCANS) {  // a handful of scans: offsets and ordered copy in one launch
@@ -782,6 +836,12 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
                                                          boundary_spec(ctx), s.d_bnd);
       ctx->launches += 2;
     }
+    if (bndAll) {
+      k_boundary_bins<<<ctx->numSms * 4, 256, 0, s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_sorted, surf_index(P, s),
+                                                             s.d_scan_off, P, ctx->d_axes, ctx->axesCap, s.d_kpRank, ctx->bndEps,
+                                                             s.d_bndX);
+      ctx->launches++;
+    }
     launch_density(ctx, s, nscans, P, sb.npts);
     mark(ctx, s, "K4c density");
     launch_desc_hist(ctx, s, nscans, P, gridKp, ctx->recordOutput, sb.lean);
@@ -804,6 +864,7 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
   CK(cudaMemcpyAsync(s.h_ctr, s.d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, s.stream));
   CK(cudaMemcpyAsync(s.h_kpOff, s.d_kpOff, (size_t)(nscans + 1) * sizeof(int), cudaMemcpyDeviceToHost, s.stream));
   if (bnd) CK(cudaMemcpyAsync(s.h_bnd, s.d_bnd, (size_t)nscans * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s.stream));
+  if (bndAll) CK(cudaMemcpyAsync(s.h_bndX, s.d_bndX, (size_t)nscans * 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s.stream));
   if (recordDone) CK(cudaEventRecord(s.evDone, s.stream));
   CK(cudaGetLastError());
   return FE_OK;
@@ -880,7 +941,7 @@ int enqueue_subbatch(fe_ctx* ctx, Slot& s, const SubBatch& sb, const double* lat
   if (ctx->bndEps > 0.0) { st = ensure_bnd(ctx, s); if (st) return st; }
   s.sb.lean = ctx->leanHold == 0;
   if (ctx->leanHold > 0) ctx->leanHold--;
-  const GraphKey key = {s.sb, density_blocks_per_scan(sb.nscans, sb.npts), s.maxScanPts > 65535, ctx->bndEps > 0.0, ctx->epoch};
+  const GraphKey key = {s.sb, density_blocks_per_scan(sb.nscans, sb.npts), s.maxScanPts > 65535, bnd_kinds(ctx), ctx->epoch};
   GraphEntry* ge = nullptr;
   for (GraphEntry& g : s.graphs) if (g.key == key) { ge = &g; break; }
   if (ge && ge->exec) {  // replay
@@ -931,6 +992,12 @@ int complete_subbatch(fe_ctx* ctx, Slot& s, int64_t kpBase) {
   for (int i = 0; i <= ns; i++) ctx->kpOffsets[s.firstScan + i] = kpBase + s.h_kpOff[i];
   if (ctx->bndEps > 0.0 && s.h_bnd)
     for (int i = 0; i < ns * 4; i++) ctx->bndCounts[(size_t)s.firstScan * 4 + i] = (int64_t)s.h_bnd[i];
+  if (ctx->bndAll && s.h_bndX)
+    for (int i = 0; i < ns; i++) {
+      int64_t* row = &ctx->bndCountsAll[((size_t)s.firstScan + i) * FE_BOUNDARY_KINDS];
+      for (int k = 0; k < 4; k++) row[k] = (int64_t)s.h_bnd[i * 4 + k];
+      for (int k = 0; k < 6; k++) row[4 + k] = (int64_t)s.h_bndX[i * 6 + k];
+    }
   return FE_OK;
 }
 
@@ -1161,20 +1228,34 @@ int fe_set_angle_libm(fe_ctx_t* ctx, int32_t mode) {
   return FE_OK;
 }
 
-int fe_enable_boundary_report(fe_ctx_t* ctx, double eps_m) {
+static int enable_boundary_report(fe_ctx_t* ctx, double eps_m, bool all) {
   if (!ctx || !(eps_m == eps_m)) return FE_ERR_INVALID;
   if (int st = sync_slots(ctx)) return st;
   ctx->bndEps = eps_m > 0.0 ? eps_m : 0.0;
+  ctx->bndAll = all && ctx->bndEps > 0.0;
   ctx->bndCounts.clear();
+  ctx->bndCountsAll.clear();
   ctx->epoch++;
   return FE_OK;
 }
+
+int fe_enable_boundary_report(fe_ctx_t* ctx, double eps_m) { return enable_boundary_report(ctx, eps_m, false); }
+
+int fe_enable_boundary_report_all(fe_ctx_t* ctx, double eps_m) { return enable_boundary_report(ctx, eps_m, true); }
 
 int fe_get_boundary_report(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans) {
   if (!ctx || !counts || !n_scans) return FE_ERR_INVALID;
   if (!(ctx->bndEps > 0.0)) return fail(ctx, FE_ERR_INVALID, "boundary report not enabled (fe_enable_boundary_report)");
   *counts = ctx->bndCounts.data();
   *n_scans = (int32_t)(ctx->bndCounts.size() / 4);
+  return FE_OK;
+}
+
+int fe_get_boundary_report_all(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans) {
+  if (!ctx || !counts || !n_scans) return FE_ERR_INVALID;
+  if (!ctx->bndAll) return fail(ctx, FE_ERR_INVALID, "boundary report of all kinds not enabled (fe_enable_boundary_report_all)");
+  *counts = ctx->bndCountsAll.data();
+  *n_scans = (int32_t)(ctx->bndCountsAll.size() / FE_BOUNDARY_KINDS);
   return FE_OK;
 }
 
@@ -1228,6 +1309,7 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
   const int64_t launches0 = ctx->launches;
   ctx->kpOffsets.assign((size_t)n_scans + 1, 0);
   ctx->bndCounts.assign(ctx->bndEps > 0.0 ? (size_t)n_scans * 4 : 0, 0);
+  ctx->bndCountsAll.assign(ctx->bndAll ? (size_t)n_scans * FE_BOUNDARY_KINDS : 0, 0);
   ctx->cloudOff.clear(); ctx->kcOff.clear();
   ctx->cloudRun = ctx->kcRun = 0;
   if (ctx->cloudOutputs) { ctx->cloudOff.assign((size_t)n_scans + 1, 0); ctx->kcOff.assign((size_t)n_scans + 1, 0); }
@@ -1354,6 +1436,7 @@ int fe_process_batch_device(fe_ctx_t* ctx, const fe_point_t* d_points, const int
     st = enqueue_subbatch(ctx, s, sb, lateRp);
     if (st) return st;
     ctx->bndCounts.assign(ctx->bndEps > 0.0 ? (size_t)n_scans * 4 : 0, 0);
+    ctx->bndCountsAll.assign(ctx->bndAll ? (size_t)n_scans * FE_BOUNDARY_KINDS : 0, 0);
     s.firstScan = 0;
     st = complete_subbatch(ctx, s, 0);
     if (st) return st;

@@ -101,6 +101,17 @@ struct DevCounters {
   unsigned long long dens_work[2];  // K4c: distance tests, marked points
 };
 
+// Kind 6 of the tolerance-boundary report (fe_enable_boundary_report_all): ring clusters whose xy diameter lies within
+// eps of the gate 2 * clusterRadiusThreshold (src:316), counted by the K2 kernels where they decide the gate.  The
+// device functions of K2 take it as a trailing parameter pack `gate...`: empty in the kernels that run without that
+// report (their code is what it was without it), one GateCount in the separate *_bnd kernels.
+struct GateCount {
+  double eps;
+  unsigned* cnt;  // [scan][16], zeroed by the first K2 kernel of a scan: the run kernels count ring r in slot r,
+                  // the grid kernels (which redo a whole scan) count every cluster of the scan in slot 0
+  __device__ GateCount at(int slot) const { return GateCount{eps, cnt + slot}; }
+};
+
 // getElevationAngles, src:147-156, literally: double atan2 / cos / sin / atan2.
 __device__ __noinline__ float elevation_deg_literal(float xf, float yf, float zf) {
   const double x = xf, y = yf, z = zf;
@@ -158,6 +169,20 @@ struct RawLayout {  // records of fe_point_layout_t; raw == nullptr: the input i
   const unsigned char* raw;
   int stride, xo, yo, zo;
 };
+
+// pcl::transformPointCloud, PCL 1.8.0 scalar form: left to right, unfused, + translation 0
+__device__ __forceinline__ float3 level_xyz(const float m[9], const float4 p) {
+  float3 q;
+  q.x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], p.x), __fmul_rn(m[1], p.y)), __fmul_rn(m[2], p.z)), 0.0f);
+  q.y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[3], p.x), __fmul_rn(m[4], p.y)), __fmul_rn(m[5], p.z)), 0.0f);
+  q.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[6], p.x), __fmul_rn(m[7], p.y)), __fmul_rn(m[8], p.z)), 0.0f);
+  return q;
+}
+
+// pcl::PassThrough x3 (src:169-183) on a finite point: inclusive float limits
+__device__ __forceinline__ bool crop_keeps(const DevParams& P, const float4 q) {
+  return !(q.z < P.zmin || q.z > P.zmax) && !(q.y < P.ymin || q.y > P.ymax) && !(q.x < P.xmin || q.x > P.xmax);
+}
 
 // K1's chunk table: per chunk {scan, (chunk of the scan << 12) | points, first point lo, hi}.  One warp per scan.
 __global__ void __launch_bounds__(256) k_chunk_table(const long long* __restrict__ scan_off, const int* __restrict__ chunk_off,
@@ -233,19 +258,15 @@ __global__ void __launch_bounds__(256, 6) k_level_crop_ring(
       }
       float el = p.w;
       if (flags & F_ROT) {
-        // pcl::transformPointCloud, PCL 1.8.0 scalar form: left to right, unfused, + translation 0
-        q.x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], p.x), __fmul_rn(m[1], p.y)), __fmul_rn(m[2], p.z)), 0.0f);
-        q.y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[3], p.x), __fmul_rn(m[4], p.y)), __fmul_rn(m[5], p.z)), 0.0f);
-        q.z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[6], p.x), __fmul_rn(m[7], p.y)), __fmul_rn(m[8], p.z)), 0.0f);
+        const float3 l = level_xyz(m, p);
+        q.x = l.x; q.y = l.y; q.z = l.z;
       } else {
         q.x = p.x; q.y = p.y; q.z = p.z;
       }
       const bool fin = finite3(q.x, q.y, q.z);
       // pcl::PassThrough: non-finite dropped, inclusive float limits (src:169-183)
       fc = fin;
-      if (flags & F_CROP)
-        fc = fin && !(q.z < P.zmin || q.z > P.zmax) && !(q.y < P.ymin || q.y > P.ymax) &&
-             !(q.x < P.xmin || q.x > P.xmax);
+      if (flags & F_CROP) fc = fin && crop_keeps(P, q);
       // getElevationAngles, src:147-156.  The angle only travels with the cropped cloud (the
       // descriptor surface never reads it), so it is evaluated for the crop survivors alone.
       if ((flags & F_ELEV) && (fc || (!FUSED && full_out))) el = elevation_deg(p.x, p.y, p.z);
@@ -799,14 +820,14 @@ __device__ __forceinline__ long long piece_pos(const int* pre, int nch, int i, l
 // ============================================================================================
 // K2 — per-ring clustering and getCylinderSegments gating for one scan per block.
 // ============================================================================================
-template <int CAP, int NT>
+template <int CAP, int NT, class... G>
 __device__ void cluster_rings_scan(
     ClusterSm& S, const int s, const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta,
     const int* __restrict__ cropCnt, const long long* __restrict__ scan_off,
     const int* __restrict__ chunk_off, const DevParams& P, int single_ring,
     float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
     float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
-    DevCounters* __restrict__ ctr, int* __restrict__ ovfList, int* __restrict__ ovfCount) {
+    DevCounters* __restrict__ ctr, int* __restrict__ ovfList, int* __restrict__ ovfCount, G... gate) {
   const int tid = threadIdx.x;
   int* pre = S.misc;
   int* sc = S.misc + MAXCHUNK + 1;
@@ -814,6 +835,7 @@ __device__ void cluster_rings_scan(
   const long long base = scan_off[s];
   const int nch = chunk_off[s + 1] - chunk_off[s];
   if (tid < 16) { kfBase[s * 16 + tid] = 0; kfCnt[s * 16 + tid] = 0; if (kcBase) { kcBase[s * 16 + tid] = 0; kcCnt[s * 16 + tid] = 0; } }
+  if constexpr (sizeof...(G) > 0) if (tid < 16) (gate.cnt, ...)[s * 16 + tid] = 0;
   if (nch > MAXCHUNK) { if (tid == 0) atomicOr(&ctr->err, ERR_CHUNKS); return; }
   const int Nc = chunk_prefix<NT>(cropCnt + chunk_off[s], nch, pre, sc);
   if (Nc == 0) return;
@@ -925,6 +947,8 @@ __device__ void cluster_rings_scan(
               }
               const double ddx = maxx - minx, ddy = maxy - miny;
               const double diameter = sqrt(__dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy)));
+              if constexpr (sizeof...(G) > 0)
+                if (pass == 0 && fabs(diameter - P.two_radius_threshold) < (gate.eps, ...)) atomicAdd(&(gate.cnt, ...)[s * 16], 1u);
               if (diameter < P.two_radius_threshold) {
                 ok = 1;
                 cen.x = (float)(sumx / (double)size);
@@ -1001,6 +1025,34 @@ __global__ void __launch_bounds__(NT, MINB) k_cluster_rings(
       __syncthreads();
       cluster_rings_scan<CAP, NT>(S, scanList[i], crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
                               kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount);
+    }
+  }
+}
+
+// k_cluster_rings, also counting the clusters on the diameter gate's boundary (kind 6); a copy for the same reason
+// as k_ring_runs_bnd.
+template <int CAP, int NT, int MINB, bool GLOBAL>
+__global__ void __launch_bounds__(NT, MINB) k_cluster_rings_bnd(
+    const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta,
+    const int* __restrict__ cropCnt, const long long* __restrict__ scan_off,
+    const int* __restrict__ chunk_off, DevParams P, int single_ring,
+    float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
+    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
+    DevCounters* __restrict__ ctr, const int* __restrict__ scanList, const int* __restrict__ nList,
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, unsigned char* __restrict__ slabs, GateCount gate) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  ClusterSm S;
+  if (GLOBAL) cluster_carve_global<CAP, NT>(slabs + (size_t)blockIdx.x * cluster_slab_bytes(CAP), smem_raw, S);
+  else cluster_sm_carve<CAP, NT>(smem_raw, S);
+  if (!scanList) {
+    cluster_rings_scan<CAP, NT>(S, blockIdx.x, crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
+                            kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount, gate);
+  } else {
+    const int n = *nList;
+    for (int i = blockIdx.x; i < n; i += gridDim.x) {
+      __syncthreads();
+      cluster_rings_scan<CAP, NT>(S, scanList[i], crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
+                              kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount, gate);
     }
   }
 }
@@ -1876,18 +1928,14 @@ constexpr size_t desc_smem_bytes(int cap, int nt) {
   return (size_t)cap * 24 + FE_DESC_LEN * 4 + 64 + 0 * nt;
 }
 
-// One neighbour's contribution (3dsc.hpp computePoint, the body of the neighbour loop): bin and
-// weight.  Returns false when PCL skips the neighbour.  o = keypoint, q = surface point,
-// (axx, axy, -0) = normalised x axis, dens = local point density of q.
-__device__ __forceinline__ bool shape_context_contribution(const float4 o, const float4 q, const float d2, const float axx,
-                                                           const float axy, const DevParams& P, const float* __restrict__ lut,
-                                                           const int dens, int& bin, float& wgt) {
-  if (fabsf(d2 - 0.0f) < 1.17549435e-38f) return false;  // pcl::utils::equal(nn_dists, 0)
-  if (dens <= 0) return false;
+// The angles a neighbour is binned by (3dsc.hpp computePoint): azimuth phi and elevation th in degrees.
+// o = keypoint, q = surface point, (axx, axy, -0) = normalised x axis; pox, poy: q - o in x and y.
+__device__ __forceinline__ void shape_context_angles(const float4 o, const float4 q, const float axx, const float axy,
+                                                     const DevParams& P, float& phi, float& th, float& pox, float& poy) {
   const float axz = -0.0f;
-  const float rr = __fsqrt_rn(d2);
   // pcl::geometry::project(neighbour, origin, normal=(0,0,1), proj); proj -= origin
-  const float pox = __fsub_rn(q.x, o.x), poy = __fsub_rn(q.y, o.y), poz = __fsub_rn(q.z, o.z);
+  pox = __fsub_rn(q.x, o.x); poy = __fsub_rn(q.y, o.y);
+  const float poz = __fsub_rn(q.z, o.z);
   const float lambda = eigen_sum3(__fmul_rn(0.0f, pox), __fmul_rn(0.0f, poy), __fmul_rn(1.0f, poz));
   float prx = __fsub_rn(__fsub_rn(q.x, __fmul_rn(lambda, 0.0f)), o.x);
   float pry = __fsub_rn(__fsub_rn(q.y, __fmul_rn(lambda, 0.0f)), o.y);
@@ -1906,7 +1954,7 @@ __device__ __forceinline__ bool shape_context_contribution(const float4 o, const
   // algorithm of glibc <= 2.40, restated operation by operation (glibc_f32.h) — the same last bit as the
   // reference's x86-64 build, so a neighbour on a bin edge lands in the same bin; 1: correctly rounded
   // (evaluated in double, then narrowed), what glibc >= 2.41 (CORE-MATH) returns.
-  float phi = P.angle_libm ? (float)atan2((double)crn, (double)dt) : glibc::atan2f_fdlibm(crn, dt);
+  phi = P.angle_libm ? (float)atan2((double)crn, (double)dt) : glibc::atan2f_fdlibm(crn, dt);
   phi = __fmul_rn(phi, 57.29578f);
   const float cdn = eigen_sum3(__fmul_rn(crx, 0.0f), __fmul_rn(cry, 0.0f), __fmul_rn(crz, 1.0f));
   phi = (cdn < 0.f) ? __fsub_rn(360.0f, phi) : phi;
@@ -1915,10 +1963,23 @@ __device__ __forceinline__ bool shape_context_contribution(const float4 o, const
     const float inv = __fdiv_rn(1.0f, __fsqrt_rn(eigen_sum3(__fmul_rn(nox, nox), __fmul_rn(noy, noy), __fmul_rn(noz, noz))));
     nox = __fmul_rn(nox, inv); noy = __fmul_rn(noy, inv); noz = __fmul_rn(noz, inv);
   }
-  float th = eigen_sum3(__fmul_rn(0.0f, nox), __fmul_rn(0.0f, noy), __fmul_rn(1.0f, noz));
+  th = eigen_sum3(__fmul_rn(0.0f, nox), __fmul_rn(0.0f, noy), __fmul_rn(1.0f, noz));
   const float t1 = (-1.0f < th) ? th : -1.0f;  // std::max(-1.0f, theta)
   const float t2 = (t1 < 1.0f) ? t1 : 1.0f;    // std::min(1.0f, .)
   th = __fmul_rn(P.angle_libm ? (float)acos((double)t2) : glibc::acosf_fdlibm(t2), 57.29578f);
+}
+
+// One neighbour's contribution (3dsc.hpp computePoint, the body of the neighbour loop): bin and
+// weight.  Returns false when PCL skips the neighbour.  o = keypoint, q = surface point,
+// (axx, axy, -0) = normalised x axis, dens = local point density of q.
+__device__ __forceinline__ bool shape_context_contribution(const float4 o, const float4 q, const float d2, const float axx,
+                                                           const float axy, const DevParams& P, const float* __restrict__ lut,
+                                                           const int dens, int& bin, float& wgt) {
+  if (fabsf(d2 - 0.0f) < 1.17549435e-38f) return false;  // pcl::utils::equal(nn_dists, 0)
+  if (dens <= 0) return false;
+  const float rr = __fsqrt_rn(d2);
+  float phi, th, pox, poy;
+  shape_context_angles(o, q, axx, axy, P, phi, th, pox, poy);
   int j = 0, k = 0, l = 0;
 #pragma unroll
   for (int a = 15; a >= 1; a--) if (rr <= P.radii[a]) j = a - 1;
@@ -2666,6 +2727,121 @@ __global__ void __launch_bounds__(256) k_boundary_density(
     }
   }
   if (cnt) atomicAdd(&bnd[4 * s + 3], cnt);
+}
+
+// ---- kinds 4-9 (fe_enable_boundary_report_all): the threshold decisions in metres or degrees that are not radius
+// predicates.  Margins are evaluated in double with + - * / sqrt only (no FMA: -fmad=false), in the order of
+// include/fe_b200.h, so the oracle's counts agree to the last pair.  bndx[6 * scan + k - 4] counts kind k. ----
+constexpr double BND_DEG = 0.017453292519943295;  // pi / 180
+
+// kinds 4 (crop box) and 5 (ring-window ends): one block per K1 chunk, K1's decode, levelling and crop again
+template <bool RAW>
+__global__ void __launch_bounds__(256) k_boundary_crop_ring(const float4* __restrict__ pts, const int4* __restrict__ chunkTab,
+                                                            const float* __restrict__ rot, DevParams P, RawLayout L, double eps,
+                                                            unsigned long long* __restrict__ bndx) {
+  const int4 ct = __ldg(chunkTab + blockIdx.x);
+  const int s = ct.x, nIn = ct.y & 4095;
+  const long long base = (long long)(((unsigned long long)(unsigned)ct.w << 32) | (unsigned)ct.z);
+  float m[9];
+#pragma unroll
+  for (int i = 0; i < 9; i++) m[i] = rot[s * 9 + i];
+  const double lo[3] = {(double)P.xmin, (double)P.ymin, (double)P.zmin}, hi[3] = {(double)P.xmax, (double)P.ymax, (double)P.zmax};
+  unsigned nCrop = 0, nRing = 0;
+  for (int j0 = 0; j0 < nIn; j0 += 256) {  // warp-uniform trip count: the sums below take the full warp
+    const int j = j0 + threadIdx.x;
+    if (j >= nIn) continue;
+    float4 p;
+    if (RAW) {
+      const unsigned char* rec = L.raw + (base + j) * (long long)L.stride;
+      p = make_float4(load_f32_any(rec + L.xo), load_f32_any(rec + L.yo), load_f32_any(rec + L.zo), 0.0f);
+    } else {
+      p = __ldg(pts + base + j);
+    }
+    const float3 l = level_xyz(m, p);
+    const float4 q = make_float4(l.x, l.y, l.z, 0.0f);
+    if (!finite3(q.x, q.y, q.z)) continue;
+    const double v[3] = {(double)q.x, (double)q.y, (double)q.z};
+    bool inside = true, near = false;
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+      inside = inside && v[a] > lo[a] - eps && v[a] < hi[a] + eps;
+      near = near || fabs(v[a] - lo[a]) < eps || fabs(v[a] - hi[a]) < eps;
+    }
+    if (inside && near) nCrop++;
+    if (!crop_keeps(P, q)) continue;
+    const float el = elevation_deg(p.x, p.y, p.z);
+    if (!isfinite(el)) continue;
+    const double range = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(v[0], v[0]), __dmul_rn(v[1], v[1])), __dmul_rn(v[2], v[2])));
+    double dmin = fabs((double)el + 16.0);
+    for (int e = -14; e <= 16; e += 2) dmin = fmin(dmin, fabs((double)el - (double)e));
+    if (__dmul_rn(range, __dmul_rn(dmin, BND_DEG)) < eps) nRing++;
+  }
+  __syncwarp();
+  nCrop = __reduce_add_sync(FE_FULL, nCrop);
+  nRing = __reduce_add_sync(FE_FULL, nRing);
+  if ((threadIdx.x & 31) == 0) {
+    if (nCrop) atomicAdd(&bndx[6 * s + 0], (unsigned long long)nCrop);
+    if (nRing) atomicAdd(&bndx[6 * s + 1], (unsigned long long)nRing);
+  }
+}
+
+// kind 6: the per-ring counts the GateCount instantiations of K2 left, summed per scan
+__global__ void __launch_bounds__(256) k_boundary_gate_sum(const unsigned* __restrict__ gate, int n_scans,
+                                                           unsigned long long* __restrict__ bndx) {
+  const int s = blockIdx.x * 256 + threadIdx.x;
+  if (s >= n_scans) return;
+  unsigned t = 0;
+  for (int r = 0; r < 16; r++) t += gate[s * 16 + r];
+  bndx[6 * s + 2] = t;
+}
+
+// kinds 7-9 (3DSC radial shells, elevation and azimuth edges): the (keypoint, neighbour) pairs K4d bins — the sweep of
+// K4b, the angles of shape_context_angles with the keypoint's x axis
+__global__ void __launch_bounds__(256) k_boundary_bins(
+    const float4* __restrict__ kpOut, const int* __restrict__ kpScan, const int* __restrict__ kpOff, int n_scans,
+    const float4* __restrict__ sorted, SurfIndex X, const long long* __restrict__ scan_off, DevParams P,
+    const float2* __restrict__ axes, int axesCap, const int* __restrict__ kpRank, double eps,
+    unsigned long long* __restrict__ bndx) {
+  const int total = kpOff[n_scans];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  for (int g = blockIdx.x; g < total; g += gridDim.x) {
+    const float4 o = kpOut[g];
+    const int s = kpScan[g];
+    const int rank = kpRank[g];
+    if (!finite3(o.x, o.y, o.z) || rank >= axesCap) continue;  // no bins (K4d reports the axis overflow)
+    const float2 ax = axes[rank];
+    const long long base = scan_off[s];
+    const float4* so = sorted + base;
+    const ScanGrid G = scan_grid(X, s, base, P);
+    const int cx0 = surf_cell(o.x - P.Rpad, P.sx0, P.sg_inv, P.sg_nx), cx1 = surf_cell(o.x + P.Rpad, P.sx0, P.sg_inv, P.sg_nx);
+    const int cy0 = surf_cell(o.y - P.Rpad, P.sy0, P.sg_inv, P.sg_ny), cy1 = surf_cell(o.y + P.Rpad, P.sy0, P.sg_inv, P.sg_ny);
+    unsigned long long nRad = 0, nEl = 0, nAz = 0;
+    for (int r = cy0 + w; r <= cy1; r += 8) {
+      int b, e;
+      G.row_span(r, cx0, cx1, b, e);
+      for (int i = b + lane; i < e; i += 32) {
+        const float4 q = so[i];
+        const float d2 = l2_simple(o.x, o.y, o.z, q.x, q.y, q.z);
+        if (!(d2 < P.R2f) || fabsf(d2 - 0.0f) < 1.17549435e-38f) continue;  // not a neighbour; pcl::utils::equal(d2, 0)
+        const float rr = __fsqrt_rn(d2);
+        float phi, th, pox, poy;
+        shape_context_angles(o, q, ax.x, ax.y, P, phi, th, pox, poy);
+        double dr = fabs((double)rr - (double)P.radii[1]), dt = fabs((double)th - (double)P.theta[1]);
+        double dp = fabs((double)phi - (double)P.phi[0]);
+        for (int a = 2; a <= 14; a++) dr = fmin(dr, fabs((double)rr - (double)P.radii[a]));
+        for (int a = 2; a <= 10; a++) dt = fmin(dt, fabs((double)th - (double)P.theta[a]));
+        for (int a = 1; a <= 12; a++) dp = fmin(dp, fabs((double)phi - (double)P.phi[a]));
+        const double rho = sqrt(__dadd_rn(__dmul_rn((double)pox, (double)pox), __dmul_rn((double)poy, (double)poy)));
+        if (dr < eps) nRad++;
+        if (__dmul_rn((double)rr, __dmul_rn(dt, BND_DEG)) < eps) nEl++;
+        // straight above or below the keypoint (rho = 0, phi NaN): any horizontal move picks the azimuth bin
+        if (rho == 0.0 || __dmul_rn(rho, __dmul_rn(dp, BND_DEG)) < eps) nAz++;
+      }
+    }
+    if (nRad) atomicAdd(&bndx[6 * s + 3], nRad);
+    if (nEl) atomicAdd(&bndx[6 * s + 4], nEl);
+    if (nAz) atomicAdd(&bndx[6 * s + 5], nAz);
+  }
 }
 
 // test hook: the device's fdlibm restatement (glibc_f32.h) element-wise; op 0 atan2f(a,b), 1 acosf(a), 2 atanf(a)

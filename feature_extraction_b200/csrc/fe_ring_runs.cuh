@@ -112,11 +112,12 @@ __device__ bool rr_runs_linked(const RB& B, const float4* P, int a, int b, float
 // (P is the block's own scratch, written in phase A of the same kernel: plain pointers, no read-only path.)
 // One ring: entries P[0, n) in original order.  Returns false when the ring has more runs than the buffer
 // holds (nothing has been written then).  Warp-uniform; all 32 lanes call.
-template <class RB>
+// gate...: nothing, or a GateCount whose cnt is the ring's slot of the kind-6 count.
+template <class RB, class... G>
 __device__ bool rr_cluster_ring(RB& B, const float4* P, const int n, const DevParams& Pm,
                                 float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBaseOut, int* __restrict__ kfCntOut,
                                 float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBaseOut, int* __restrict__ kcCntOut,
-                                DevCounters* __restrict__ ctr) {
+                                DevCounters* __restrict__ ctr, G... gate) {
   const int lane = threadIdx.x & 31;
   const unsigned le = lanemask_lt() | (1u << lane);
   const float r2f = Pm.r2f_cluster;
@@ -246,6 +247,7 @@ __device__ bool rr_cluster_ring(RB& B, const float4* P, const int n, const DevPa
       const double ddx = maxx - minx, ddy = maxy - miny;
       const double diameter = sqrt(__dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy)));  // src:314
       ok = diameter < Pm.two_radius_threshold;
+      if constexpr (sizeof...(G) > 0) if (fabs(diameter - Pm.two_radius_threshold) < (gate.eps, ...)) atomicAdd((gate.cnt, ...), 1u);
     }
     const unsigned om = __ballot_sync(FE_FULL, ok);
     // the flag travels in the sign of csize (sizes are > 0)
@@ -325,11 +327,12 @@ __device__ bool rr_cluster_ring(RB& B, const float4* P, const int n, const DevPa
 // Phase B for one scan whose ring segments [ringBase[r], ringBase[r+1]) are in place at RP: the warps take rings
 // off the block's counter.  A ring with more runs than a warp's buffer holds is listed for the wide kernel (its
 // outputs are untouched); the other rings of the scan are finished here.
-template <int RWT, int NW>
+template <int RWT, int NW, class... G>
 __device__ void rr_scan_rings(RingRunsSmT<RWT, NW>& S, const int s, const float4* RP, const int nRings, const DevParams& P,
                               float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
                               float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
-                              DevCounters* __restrict__ ctr, int* __restrict__ ovfRuns, int* __restrict__ ovfRunsCount) {
+                              DevCounters* __restrict__ ctr, int* __restrict__ ovfRuns, int* __restrict__ ovfRunsCount,
+                              G... gate) {
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   RunBufT<RWT>& B = S.rb[w];
   for (;;) {
@@ -340,7 +343,8 @@ __device__ void rr_scan_rings(RingRunsSmT<RWT, NW>& S, const int s, const float4
     const int r0 = S.ringBase[ring], n = S.ringBase[ring + 1] - r0;
     if (n == 0) continue;
     const bool done = rr_cluster_ring(B, RP + r0, n, P, kfPool, kfCap, &kfBase[s * 16 + ring], &kfCnt[s * 16 + ring], kcPool, kcCap,
-                                      kcBase ? &kcBase[s * 16 + ring] : nullptr, kcBase ? &kcCnt[s * 16 + ring] : nullptr, ctr);
+                                      kcBase ? &kcBase[s * 16 + ring] : nullptr, kcBase ? &kcCnt[s * 16 + ring] : nullptr, ctr,
+                                      gate.at(s * 16 + ring)...);
     if (!done && lane == 0) ovfRuns[atomicAdd(ovfRunsCount, 1)] = s * 16 + ring;
   }
 }
@@ -449,14 +453,122 @@ __global__ void __launch_bounds__(NW * 32, NW == NW_RR ? 12 : 1) k_ring_runs(
   rr_scan_rings<RW, NW>(S, s, RP, nRings, P, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfRuns, ovfRunsCount);
 }
 
+// k_ring_runs, also counting the clusters on the diameter gate's boundary (kind 6).  A copy, not a shared body: with the
+// body moved into a device function the compiler allocates k_ring_runs' registers differently.
+// First kernel: one block per scan, every scan.  A ring of more than RW runs is handed to the second kernel (the
+// ring segments and their offsets stay in global memory, so nothing is bucketed twice); a scan with more ring
+// entries than its scratch slot goes straight to the grid-based kernels.
+template <int NW>
+__global__ void __launch_bounds__(NW * 32, NW == NW_RR ? 12 : 1) k_ring_runs_bnd(
+    const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta, const int* __restrict__ cropCnt,
+    const long long* __restrict__ scan_off, const int* __restrict__ chunk_off, DevParams P, int single_ring,
+    float4* ringPts, int* __restrict__ ringBaseOut, float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
+    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
+    DevCounters* __restrict__ ctr, int* __restrict__ ovfRuns, int* __restrict__ ovfRunsCount, int* __restrict__ scanFlag,
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, GateCount gate) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  RingRunsSmT<RW, NW>& S = *reinterpret_cast<RingRunsSmT<RW, NW>*>(smem_raw);
+  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const long long base = scan_off[s];
+  const int nScan = (int)(scan_off[s + 1] - base);
+  const int nch = chunk_off[s + 1] - chunk_off[s];
+  if (tid < 16) { kfBase[s * 16 + tid] = 0; kfCnt[s * 16 + tid] = 0; if (kcBase) { kcBase[s * 16 + tid] = 0; kcCnt[s * 16 + tid] = 0; } }
+  if (tid == 0) scanFlag[s] = 0;  // the wide kernel sets it when it sends the scan on to the grid-based kernels
+  if (tid < 16) gate.cnt[s * 16 + tid] = 0;
+  if (nch > MAXCHUNK) { if (tid == 0) atomicOr(&ctr->err, ERR_CHUNKS); return; }
+  if (tid < NW * 17) (&S.cnt[0][0])[tid] = 0;
+  if (tid == 0) { S.nextRing = 0; S.defer = 0; }
+  const int Nc = chunk_prefix<NW * 32>(cropCnt + chunk_off[s], nch, S.pre, S.sc);  // ends with a barrier
+  if (Nc == 0) return;
+  const int nRings = single_ring ? 1 : 16;
+  // ---- phase A: stable bucketing of the crop survivors by ring ----
+  // every warp owns a contiguous range of the survivors; (1) per-warp counts, (2) offsets, (3) scatter
+  const int lo = (int)((long long)Nc * w / NW), hi = (int)((long long)Nc * (w + 1) / NW);
+  int* mycnt = S.cnt[w];
+  for (int i0 = lo; i0 < hi; i0 += 32) {
+    const int i = i0 + lane;
+    unsigned m = 0;
+    if (i < hi) m = ring_mask_of(cropMeta[piece_pos(S.pre, nch, i, base)] & 63u, single_ring);
+    const int first = m ? __ffs(m) - 1 : 16;
+    const unsigned peers = __match_any_sync(FE_FULL, first);
+    if (i < hi && lane == __ffs(peers) - 1) mycnt[first] += __popc(peers);
+    __syncwarp();
+    unsigned dual = __ballot_sync(FE_FULL, __popc(m) > 1);  // on a window's end value: also in the next ring (rare)
+    while (dual) {
+      const int src = __ffs(dual) - 1;
+      dual &= dual - 1;
+      const int f2 = __shfl_sync(FE_FULL, first, src) + 1;
+      if (lane == 0) mycnt[f2] += 1;
+      __syncwarp();
+    }
+  }
+  __syncthreads();
+  if (tid < 16) {
+    // S.cnt[w][h] becomes the first slot of warp w's entries of ring h inside the ring's segment
+    int run = 0;
+    for (int ww = 0; ww < NW; ww++) { const int c = S.cnt[ww][tid]; S.cnt[ww][tid] = run; run += c; }
+    S.ringBase[tid + 1] = run;  // totals for now
+  }
+  __syncthreads();
+  if (tid == 0) {
+    int run = 0;
+    S.ringBase[0] = 0;
+    for (int h = 0; h < 16; h++) { const int c = S.ringBase[h + 1]; S.ringBase[h + 1] = run + c; run += c; }
+    if (run > nScan) {  // more ring entries than the scan's slot holds (end-value points count twice): grid path
+      S.defer = 1;
+      ovfList[atomicAdd(ovfCount, 1)] = s;
+    }
+  }
+  __syncthreads();
+  if (S.defer) return;
+  float4* RP = ringPts + base;
+  for (int i0 = lo; i0 < hi; i0 += 32) {
+    const int i = i0 + lane;
+    unsigned m = 0;
+    float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (i < hi) {
+      const long long pp = piece_pos(S.pre, nch, i, base);
+      m = ring_mask_of(cropMeta[pp] & 63u, single_ring);
+      if (m) q = crop[pp];
+    }
+    const int first = m ? __ffs(m) - 1 : 16;
+    const unsigned anyDual = __ballot_sync(FE_FULL, __popc(m) > 1);
+    if (!anyDual) {
+      const unsigned peers = __match_any_sync(FE_FULL, first);
+      const int leader = __ffs(peers) - 1;
+      int old = 0;
+      if (lane == leader) { old = mycnt[first]; mycnt[first] = old + __popc(peers); }
+      old = __shfl_sync(FE_FULL, old, leader);
+      if (m) RP[S.ringBase[first] + old + __popc(peers & lanemask_lt())] = q;
+      __syncwarp();
+    } else {  // a point of this window belongs to two rings: ring by ring, so that every ring keeps the original order
+      for (int h = 0; h < nRings; h++) {
+        const bool in = (m >> h) & 1u;
+        const unsigned bm = __ballot_sync(FE_FULL, in);
+        if (!bm) continue;
+        const int old = mycnt[h];
+        if (in) RP[S.ringBase[h] + old + __popc(bm & lanemask_lt())] = q;
+        __syncwarp();
+        if (lane == 0) mycnt[h] = old + __popc(bm);
+        __syncwarp();
+      }
+    }
+  }
+  __syncthreads();  // the block's global writes are visible to all its threads from here on
+  // ---- phase B: a warp per ring, rings handed out dynamically ----
+  if (tid < 17) ringBaseOut[s * 17 + tid] = S.ringBase[tid];  // for the wide kernel, should a ring of this scan need it
+  rr_scan_rings<RW, NW>(S, s, RP, nRings, P, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfRuns, ovfRunsCount, gate);
+}
+
 // Second kernel: the rings the first one listed (hundreds of poles in one ring), a warp per ring with RW2 runs;
 // what exceeds that — entries in arbitrary order, mostly — sends the ring's whole scan to the grid-based kernels.
-__global__ void __launch_bounds__(NT_RR) k_ring_runs_wide(
-    const long long* __restrict__ scan_off, DevParams P, const float4* ringPts, const int* __restrict__ ringBaseIn,
+template <class... G>
+__device__ __forceinline__ void ring_runs_wide_blocks(
+    const long long* __restrict__ scan_off, const DevParams& P, const float4* ringPts, const int* __restrict__ ringBaseIn,
     float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
     float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
     DevCounters* __restrict__ ctr, const int* __restrict__ ringList, const int* __restrict__ nList, int* __restrict__ scanFlag,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount) {
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, G... gate) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   RunBufT<RW2>* bufs = reinterpret_cast<RunBufT<RW2>*>(smem_raw);
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -466,9 +578,31 @@ __global__ void __launch_bounds__(NT_RR) k_ring_runs_wide(
     const int id = ringList[li], s = id >> 4, ring = id & 15;
     const int r0 = ringBaseIn[s * 17 + ring], n = ringBaseIn[s * 17 + ring + 1] - r0;
     const bool done = rr_cluster_ring(B, ringPts + scan_off[s] + r0, n, P, kfPool, kfCap, &kfBase[s * 16 + ring], &kfCnt[s * 16 + ring],
-                                      kcPool, kcCap, kcBase ? &kcBase[s * 16 + ring] : nullptr, kcBase ? &kcCnt[s * 16 + ring] : nullptr, ctr);
+                                      kcPool, kcCap, kcBase ? &kcBase[s * 16 + ring] : nullptr, kcBase ? &kcCnt[s * 16 + ring] : nullptr, ctr,
+                                      gate.at(s * 16 + ring)...);
     if (!done && lane == 0 && atomicExch(&scanFlag[s], 1) == 0) ovfList[atomicAdd(ovfCount, 1)] = s;
   }
+}
+
+__global__ void __launch_bounds__(NT_RR) k_ring_runs_wide(
+    const long long* __restrict__ scan_off, DevParams P, const float4* ringPts, const int* __restrict__ ringBaseIn,
+    float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
+    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
+    DevCounters* __restrict__ ctr, const int* __restrict__ ringList, const int* __restrict__ nList, int* __restrict__ scanFlag,
+    int* __restrict__ ovfList, int* __restrict__ ovfCount) {
+  ring_runs_wide_blocks(scan_off, P, ringPts, ringBaseIn, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ringList, nList,
+                        scanFlag, ovfList, ovfCount);
+}
+
+// the same, also counting the clusters on the diameter gate's boundary (kind 6)
+__global__ void __launch_bounds__(NT_RR) k_ring_runs_wide_bnd(
+    const long long* __restrict__ scan_off, DevParams P, const float4* ringPts, const int* __restrict__ ringBaseIn,
+    float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
+    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
+    DevCounters* __restrict__ ctr, const int* __restrict__ ringList, const int* __restrict__ nList, int* __restrict__ scanFlag,
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, GateCount gate) {
+  ring_runs_wide_blocks(scan_off, P, ringPts, ringBaseIn, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ringList, nList,
+                        scanFlag, ovfList, ovfCount, gate);
 }
 
 }  // namespace fe

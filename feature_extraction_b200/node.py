@@ -305,6 +305,20 @@ class FeatureExtractionNode:
             return np.zeros((0, 4), np.int64)
         return np.ctypeslib.as_array(p, shape=(n.value, 4)).copy()
 
+    def enableBoundaryReportAll(self, eps_m=1e-6):
+        """fe_enable_boundary_report_all: the four radius kinds plus the crop box, ring-window ends, cluster diameter
+        gate and 3DSC radial, elevation and azimuth bin edges (kinds 4-9 of include/fe_b200.h)."""
+        self._check(N.lib().fe_enable_boundary_report_all(self._ctx, float(eps_m)))
+
+    def boundaryReportAll(self):
+        """-> (n_scans, 10) int64: the counts of kinds 0-9 of the last batch call."""
+        p = C.POINTER(C.c_int64)()
+        n = C.c_int32(0)
+        self._check(N.lib().fe_get_boundary_report_all(self._ctx, C.byref(p), C.byref(n)))
+        if n.value == 0:
+            return np.zeros((0, 10), np.int64)
+        return np.ctypeslib.as_array(p, shape=(n.value, 10)).copy()
+
     def h2dProbe(self, host_array):
         """Bench hook: bare host->device copy of `host_array` through the staging buffer; -> ms (CUDA events)."""
         ms = C.c_float(0)

@@ -202,6 +202,38 @@ int fe_set_angle_libm(fe_ctx_t* ctx, int32_t mode);
 int fe_enable_boundary_report(fe_ctx_t* ctx, double eps_m);
 int fe_get_boundary_report(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans);
 
+/* The same report over every threshold decision of the path in metres or degrees.  After
+ * fe_enable_boundary_report_all(ctx, eps_m > 0) every batch call counts kinds 0-9 and
+ * fe_get_boundary_report_all returns n_scans x FE_BOUNDARY_KINDS counts of the last call (FE_ERR_INVALID unless
+ * the report was enabled with _all); fe_get_boundary_report still returns the n_scans x 4 of kinds 0-3.  A margin
+ * is evaluated in IEEE double with + - * / sqrt only, in the order written here (no FMA), so the CPU oracle gets
+ * the same count to the last pair.  DEG = 0.017453292519943295 (pi/180 as a double); "within eps" is < eps_m.
+ *   [0-3] as above
+ *   [4] crop box, src:169-183: points of the levelled full cloud with finite x, y, z such that, with
+ *       lo_a = (double)(float)min_a, hi_a = (double)(float)max_a and v_a = (double) the levelled coordinate, every
+ *       axis has lo_a - eps < v_a < hi_a + eps and some axis has |v_a - lo_a| < eps or |v_a - hi_a| < eps
+ *   [5] ring-window ends, src:195-202: crop survivors with a finite elevation el (float, degrees);
+ *       range = sqrt(((double)x*x + (double)y*y) + (double)z*z) of the cropped levelled point, counted once when
+ *       range * (min over e = -16, -14, ..., 16 of |(double)el - e| * DEG) < eps
+ *   [6] cluster diameter gate, src:314-316: ring clusters (every ring) that passed the size gate, counted when
+ *       |diameter - 2 * cluster_radius_threshold| < eps, diameter being the double each side computes: sqrt on the
+ *       device, pow(., 0.5) in the oracle.  The two differ by at most an ulp, so at eps >= 1e-9 m the counts agree.
+ *   [7] 3DSC radial shells (3dsc.hpp, called at src:350-353): (keypoint, neighbour) pairs that reach the binning
+ *       (finite keypoint, d2 < (float)R^2, d2 not pcl::utils::equal to 0); r = sqrtf(d2) as binned, counted when
+ *       min over a = 1..14 of |(double)r - (double)radii[a]| < eps (radii[15] is kind 2's sphere)
+ *   [8] 3DSC elevation edges: the same pairs, counted when (double)r * (min over a = 1..10 of
+ *       |(double)theta - (double)theta_div[a]| * DEG) < eps, theta the float angle as binned
+ *   [9] 3DSC azimuth edges: the same pairs; pox, poy = the float differences q - o in x and y,
+ *       rho = sqrt((double)pox*pox + (double)poy*poy); counted when rho == 0 (straight above or below the keypoint)
+ *       or rho * (min over a = 0..12 of |(double)phi - (double)phi_div[a]| * DEG) < eps (0 and 360 deg both: that
+ *       half-plane separates bin 0 from bin 11)
+ * With FE_LIBM_CORRECTLY_ROUNDED, kinds 8 and 9 are counted on the angles the device bins with.  The batch routes
+ * all fill the report (fe_process_batch, fe_process_batch_layout, fe_process_batch_device, any number of
+ * sub-batches); fe_multi_* has none.  eps_m <= 0 disables the report. */
+#define FE_BOUNDARY_KINDS 10
+int fe_enable_boundary_report_all(fe_ctx_t* ctx, double eps_m);
+int fe_get_boundary_report_all(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans);
+
 /* CUDA-event stopwatch on the context's stream (the stream every kernel of
  * fe_process_batch_device is launched on): begin, run any number of calls, end -> elapsed ms. */
 int fe_timer_begin(fe_ctx_t* ctx);
