@@ -27,6 +27,7 @@ EXPORTS = [
     "fe_set_angle_libm", "fe_enable_boundary_report", "fe_get_boundary_report",
     "fe_enable_boundary_report_all", "fe_get_boundary_report_all",
     "fe_multi_enable_cloud_outputs", "fe_multi_get_cloud_outputs",
+    "fe_match_descriptors", "fe_match_descriptors_device",
 ]
 
 
@@ -71,6 +72,17 @@ class BatchResult(C.Structure):
         ("descriptors", C.c_void_p),
         ("on_device", C.c_int32),
         ("gpu_launches", C.c_int64),
+    ]
+
+
+class MatchResult(C.Structure):
+    """fe_match_result_t: per query row, the best reference row and shift, its distance and the second-best row's."""
+    _fields_ = [
+        ("n_queries", C.c_int64),
+        ("best", C.POINTER(C.c_int64)),
+        ("shift", C.POINTER(C.c_int32)),
+        ("dist2", C.POINTER(C.c_float)),
+        ("second_dist2", C.POINTER(C.c_float)),
     ]
 
 
@@ -141,6 +153,9 @@ def lib():
         L.fe_multi_enable_cloud_outputs.argtypes = [C.c_void_p, C.c_int32]
         L.fe_multi_get_cloud_outputs.argtypes = [C.c_void_p, C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_void_p),
                                                  C.POINTER(C.POINTER(C.c_int64)), C.POINTER(C.c_void_p)]
+        for f in (L.fe_match_descriptors, L.fe_match_descriptors_device):
+            f.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32,
+                          C.POINTER(MatchResult)]
         L.fe_debug_enable_graphs.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int64)]
         L.fe_debug_lean_reruns.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         L.fe_debug_density_work.argtypes = [C.c_void_p, C.c_void_p]

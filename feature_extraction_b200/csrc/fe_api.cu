@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "fe_kernels.cuh"
+#include "fe_match.h"
 
 using namespace fe;
 
@@ -156,6 +157,17 @@ struct fe_ctx {
   std::vector<const char*> stName;
   std::vector<float> stMs;
   int64_t launches = 0;
+  // fe_match_descriptors*: buffers of their own, so that a match call leaves the last batch call's results alone
+  float *d_matchQ = nullptr, *d_matchR = nullptr;  // uploaded rows of the host variant
+  int64_t capMatchQ = 0, capMatchR = 0;            // floats
+  fe_match::Item *h_items = nullptr, *d_items = nullptr;
+  int64_t capItemsHost = 0, capItems = 0;
+  fe_match::Partial* d_part = nullptr;
+  int64_t capPart = 0;
+  unsigned char* d_matchRes = nullptr;  // n_queries x {best int64 | dist2 | second_dist2 | shift}, as h_matchRes
+  long long* h_matchRes = nullptr;      // pinned, MATCH_RES_WORDS long longs per query
+  int64_t capMatchRes = 0, capMatchResHost = 0;  // queries
+  bool matchAttrs = false;
   std::string err;
 };
 
@@ -1193,6 +1205,10 @@ void fe_destroy(fe_ctx_t* ctx) {
   if (ctx->h_desc) cudaFreeHost(ctx->h_desc);
   if (ctx->h_cloud) cudaFreeHost(ctx->h_cloud);
   if (ctx->h_kc) cudaFreeHost(ctx->h_kc);
+  void* dm[] = {ctx->d_matchQ, ctx->d_matchR, ctx->d_items, ctx->d_part, ctx->d_matchRes};
+  for (void* p : dm) if (p) cudaFree(p);
+  if (ctx->h_items) cudaFreeHost(ctx->h_items);
+  if (ctx->h_matchRes) cudaFreeHost(ctx->h_matchRes);
   delete ctx;
 }
 
@@ -1507,6 +1523,140 @@ int fe_download(fe_ctx_t* ctx, void* host_dst, const void* device_src, int64_t b
   CK(cudaSetDevice(ctx->device));
   if (bytes > 0) CK(cudaMemcpy(host_dst, device_src, (size_t)bytes, cudaMemcpyDeviceToHost));
   return FE_OK;
+}
+
+}  // extern "C"
+
+// ---- descriptor matching (fe_match.cu) -----------------------------------------------------------------
+
+namespace {
+
+// one query's result in h_matchRes / d_matchRes: best (8 B) | dist2 | second_dist2 | shift, as four arrays
+constexpr int MATCH_RES_WORDS = 3;  // long longs per query, 20 of the 24 bytes used
+
+template <class T>
+int grow_device(fe_ctx* ctx, T** buf, int64_t* cap, int64_t need) {
+  if (need <= *cap) return FE_OK;
+  if (*buf) { CK(cudaFree(*buf)); *buf = nullptr; *cap = 0; }
+  const int64_t ncap = need + need / 2;
+  CK(dalloc(buf, (size_t)ncap));
+  *cap = ncap;
+  return FE_OK;
+}
+
+const char* check_offsets(const int64_t* o, int32_t G) {
+  if (o[0] < 0) return "negative entry";
+  for (int32_t g = 0; g < G; g++)
+    if (o[g + 1] < o[g]) return "decreasing entries";
+  return nullptr;
+}
+
+// both entry points: rows q / r are device memory (onDevice) or host memory to upload
+int match_descriptors(fe_ctx* ctx, const float* q, int64_t qStride, const int64_t* qo, const float* r, int64_t rStride,
+                      const int64_t* ro, int32_t G, fe_match_result_t* out, bool onDevice) {
+  if (!ctx || !out) return FE_ERR_INVALID;
+  ctx->err.clear();
+  if (G < 0) return fail(ctx, FE_ERR_INVALID, "n_groups must not be negative");
+  if (qStride < FE_DESC_LEN || rStride < FE_DESC_LEN) return fail(ctx, FE_ERR_INVALID, "a row stride is below FE_DESC_LEN");
+  if (!qo || !ro) return fail(ctx, FE_ERR_INVALID, "query_offsets and ref_offsets need n_groups + 1 entries");
+  if (const char* e = check_offsets(qo, G)) return fail(ctx, FE_ERR_INVALID, std::string("query_offsets: ") + e);
+  if (const char* e = check_offsets(ro, G)) return fail(ctx, FE_ERR_INVALID, std::string("ref_offsets: ") + e);
+  const int64_t nQ = qo[G] - qo[0], nR = ro[G] - ro[0];
+  if (nQ > 0 && !q) return fail(ctx, FE_ERR_INVALID, "query is NULL but there are query rows");
+  if (nR > 0 && !r) return fail(ctx, FE_ERR_INVALID, "ref is NULL but there are reference rows");
+  if (nQ >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 query rows");
+  CK(cudaSetDevice(ctx->device));
+  int st = ensure_slot(ctx, ctx->slot[0], false);  // for its stream only: the slot's buffers are not touched
+  if (st) return st;
+  cudaStream_t stream = ctx->slot[0].stream;
+
+  // the work items (fe_match.h): per group, reference segment outer and query tile inner, so that the warps running at
+  // one time share a segment of reference rows in L2
+  const int64_t QT = fe_match::ITEM_QUERIES, RS = fe_match::ITEM_REFS;
+  int64_t nItems = 0;
+  for (int32_t g = 0; g < G; g++) {
+    const int64_t nq = qo[g + 1] - qo[g], nr = ro[g + 1] - ro[g];
+    if (nq > 0) nItems += ((nq + QT - 1) / QT) * std::max<int64_t>((nr + RS - 1) / RS, 1);
+  }
+  if (nItems >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "too many query tiles x reference segments");
+  st = grow_pinned(ctx, &ctx->h_matchRes, &ctx->capMatchResHost, nQ, 4096, 0, MATCH_RES_WORDS);
+  if (st) return st;
+  out->n_queries = nQ;
+  long long* h = ctx->h_matchRes;
+  out->best = (const int64_t*)h;
+  out->dist2 = (const float*)(h + nQ);
+  out->second_dist2 = out->dist2 + nQ;
+  out->shift = (const int32_t*)(out->second_dist2 + nQ);
+  if (nQ == 0) return FE_OK;
+
+  st = grow_pinned(ctx, &ctx->h_items, &ctx->capItemsHost, nItems, 4096, 0);
+  if (st) return st;
+  int64_t nPart = 0, k = 0;
+  for (int32_t g = 0; g < G; g++) {
+    const int64_t nq = qo[g + 1] - qo[g], nr = ro[g + 1] - ro[g];
+    if (nq == 0) continue;
+    const int64_t nseg = std::max<int64_t>((nr + RS - 1) / RS, 1);
+    for (int64_t sg = 0; sg < nseg; sg++)
+      for (int64_t t = 0; t < nq; t += QT) {
+        fe_match::Item& I = ctx->h_items[k++];
+        I.q0 = qo[g] + t;
+        I.r0 = ro[g] + sg * RS;
+        I.out = qo[g] + t - qo[0];
+        I.part = nseg > 1 ? nPart + t * nseg : 0;
+        I.nq = (int32_t)std::min(QT, nq - t);
+        I.nr = (int32_t)std::min(RS, nr - sg * RS);
+        I.nseg = (int32_t)nseg;
+        I.seg = (int32_t)sg;
+      }
+    if (nseg > 1) nPart += nq * nseg;
+  }
+
+  if (!ctx->matchAttrs) {
+    CK(fe_match::set_attributes());
+    ctx->matchAttrs = true;
+  }
+  int64_t qBias = 0, rBias = 0;
+  if (!onDevice) {  // rows [qo[0], qo[G]) and [ro[0], ro[G]) only; the last row of a side ends FE_DESC_LEN floats in
+    const int64_t qf = (nQ - 1) * qStride + FE_DESC_LEN, rf = nR > 0 ? (nR - 1) * rStride + FE_DESC_LEN : 0;
+    if ((st = grow_device(ctx, &ctx->d_matchQ, &ctx->capMatchQ, qf))) return st;
+    if ((st = grow_device(ctx, &ctx->d_matchR, &ctx->capMatchR, rf))) return st;
+    CK(cudaMemcpyAsync(ctx->d_matchQ, q + qo[0] * qStride, (size_t)qf * sizeof(float), cudaMemcpyHostToDevice, stream));
+    if (rf > 0) CK(cudaMemcpyAsync(ctx->d_matchR, r + ro[0] * rStride, (size_t)rf * sizeof(float), cudaMemcpyHostToDevice, stream));
+    q = ctx->d_matchQ;
+    r = ctx->d_matchR;
+    qBias = qo[0];
+    rBias = ro[0];
+  }
+  if ((st = grow_device(ctx, &ctx->d_items, &ctx->capItems, nItems))) return st;
+  if ((st = grow_device(ctx, &ctx->d_part, &ctx->capPart, std::max<int64_t>(nPart, 1)))) return st;
+  if ((st = grow_device(ctx, &ctx->d_matchRes, &ctx->capMatchRes, nQ * MATCH_RES_WORDS * 8))) return st;
+  CK(cudaMemcpyAsync(ctx->d_items, ctx->h_items, (size_t)nItems * sizeof(fe_match::Item), cudaMemcpyHostToDevice, stream));
+  fe_match::Result res;
+  res.best = (long long*)ctx->d_matchRes;
+  res.dist2 = (float*)(res.best + nQ);
+  res.second = res.dist2 + nQ;
+  res.shift = (int*)(res.second + nQ);
+  CK(fe_match::launch(q, qStride, qBias, r, rStride, rBias, ctx->d_items, (int)nItems, nPart > 0, ctx->d_part, res, stream));
+  ctx->launches += nPart > 0 ? 2 : 1;
+  CK(cudaMemcpyAsync(ctx->h_matchRes, ctx->d_matchRes, (size_t)nQ * 20, cudaMemcpyDeviceToHost, stream));
+  CK(cudaStreamSynchronize(stream));
+  return FE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fe_match_descriptors(fe_ctx_t* ctx, const float* query, int64_t query_stride, const int64_t* query_offsets,
+                         const float* ref, int64_t ref_stride, const int64_t* ref_offsets, int32_t n_groups,
+                         fe_match_result_t* out) {
+  return match_descriptors(ctx, query, query_stride, query_offsets, ref, ref_stride, ref_offsets, n_groups, out, false);
+}
+
+int fe_match_descriptors_device(fe_ctx_t* ctx, const float* query, int64_t query_stride, const int64_t* query_offsets,
+                                const float* ref, int64_t ref_stride, const int64_t* ref_offsets, int32_t n_groups,
+                                fe_match_result_t* out) {
+  return match_descriptors(ctx, query, query_stride, query_offsets, ref, ref_stride, ref_offsets, n_groups, out, true);
 }
 
 // ---- one entry point per reference function ----------------------------------------------------------

@@ -62,6 +62,41 @@ def _batch_args(n_records, scan_offsets, roll_pitch):
     return offs, rp, B
 
 
+def _descriptor_rows(a):
+    """(K, 1980) bins or (K, 1996) records -> (array kept alive, row stride in floats, pointer to the first bin)."""
+    a = np.ascontiguousarray(a, np.float32)
+    if a.ndim != 2 or a.shape[1] not in (DESC_LEN, RECORD_FLOATS):
+        raise ValueError("descriptors must be (K, %d) bins or (K, %d) records, got %s" % (DESC_LEN, RECORD_FLOATS, a.shape))
+    first = 5 if a.shape[1] == RECORD_FLOATS else 0  # x, y, z, pad, intensity, then the bins
+    return a, a.shape[1], C.c_void_p(a.ctypes.data + 4 * first if len(a) else None)
+
+
+def _match_offsets(query_offsets, ref_offsets, n_query, n_ref):
+    """Validate the groups of a match call before raw pointers cross the C-ABI; None for both = one group of all rows."""
+    if query_offsets is None and ref_offsets is None and n_query is not None:
+        query_offsets, ref_offsets = [0, n_query], [0, n_ref]
+    if query_offsets is None or ref_offsets is None:
+        raise ValueError("query_offsets and ref_offsets go together")
+    qo = np.ascontiguousarray(query_offsets, np.int64).reshape(-1)
+    ro = np.ascontiguousarray(ref_offsets, np.int64).reshape(-1)
+    if len(qo) < 1 or len(qo) != len(ro):
+        raise ValueError("query_offsets and ref_offsets need the same n_groups + 1 entries (got %d and %d)" % (len(qo), len(ro)))
+    for name, o, n in (("query_offsets", qo, n_query), ("ref_offsets", ro, n_ref)):
+        if o[0] < 0 or np.any(np.diff(o) < 0):
+            raise ValueError("%s must start at >= 0 and be non-decreasing" % name)
+        if n is not None and o[-1] > n:
+            raise ValueError("%s[-1] = %d exceeds the %d rows passed" % (name, o[-1], n))
+    return qo, ro, len(qo) - 1
+
+
+def _unpack_match(res):
+    n = int(res.n_queries)
+    if n == 0:
+        return np.zeros(0, np.int64), np.zeros(0, np.int32), np.zeros(0, np.float32), np.zeros(0, np.float32)
+    return (np.ctypeslib.as_array(res.best, shape=(n,)).copy(), np.ctypeslib.as_array(res.shift, shape=(n,)).copy(),
+            np.ctypeslib.as_array(res.dist2, shape=(n,)).copy(), np.ctypeslib.as_array(res.second_dist2, shape=(n,)).copy())
+
+
 class PinnedBuffer:
     """Page-locked host memory from fe_host_alloc, exposed as a numpy array."""
 
@@ -270,6 +305,34 @@ class FeatureExtractionNode:
         self.last_launches = int(res.gpu_launches)
         ko = np.ctypeslib.as_array(res.keypoint_offsets, shape=(B + 1,)).copy()
         return ko, int(res.n_keypoints), res.keypoints, res.descriptors
+
+    def matchDescriptors(self, query, ref, query_offsets=None, ref_offsets=None):
+        """fe_match_descriptors: for every query row, the reference row and azimuth shift of the smallest
+        12-shift distance within its group (include/fe_b200.h).  `query` / `ref` are host arrays of (K, 1980) bins
+        or (K, 1996) pcl::PointDescriptor records; no offsets = one group of all rows.
+        -> best (n,) int64 (absolute reference row, -1 = none), shift (n,) int32, dist2 (n,), second_dist2 (n,) float32
+        """
+        q, qs, qp = _descriptor_rows(query)
+        r, rs, rp = _descriptor_rows(ref)
+        qo, ro, G = _match_offsets(query_offsets, ref_offsets, len(q), len(r))
+        res = N.MatchResult()
+        self._check(N.lib().fe_match_descriptors(self._ctx, qp, qs, _ptr(qo), rp, rs, _ptr(ro), G, C.byref(res)))
+        return _unpack_match(res)
+
+    def matchDescriptorsDevice(self, q_ptr, q_stride, q_offsets, r_ptr, r_stride, r_offsets):
+        """fe_match_descriptors_device: rows already in HBM (raw device pointers, e.g. the descriptors
+        processBatchDevice returns; a record pointer must point at its first bin, record base + 5 floats), queued on the
+        context's stream behind the batch call.  Same results as matchDescriptors."""
+        for st in (q_stride, r_stride):
+            if int(st) < DESC_LEN:
+                raise ValueError("a row stride must be at least %d floats, got %d" % (DESC_LEN, int(st)))
+        qo, ro, G = _match_offsets(q_offsets, r_offsets, None, None)  # the device buffers' sizes are the caller's business
+        if (qo[-1] > qo[0] and not q_ptr) or (ro[-1] > ro[0] and not r_ptr):
+            raise ValueError("a device pointer is NULL while its side has rows")
+        res = N.MatchResult()
+        self._check(N.lib().fe_match_descriptors_device(self._ctx, C.c_void_p(q_ptr), int(q_stride), _ptr(qo), C.c_void_p(r_ptr),
+                                                        int(r_stride), _ptr(ro), G, C.byref(res)))
+        return _unpack_match(res)
 
     def download(self, device_ptr, shape, dtype=np.float32):
         """Copy a device-resident result of processBatchDevice to a new host array."""

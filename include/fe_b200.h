@@ -234,6 +234,60 @@ int fe_get_boundary_report(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_sca
 int fe_enable_boundary_report_all(fe_ctx_t* ctx, double eps_m);
 int fe_get_boundary_report_all(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans);
 
+/* ---- descriptor matching: the step downstream of ~features ---------------------------------- */
+/* 3DSC descriptors of one pole seen from two scans have their 12 azimuth blocks rotated against each other by an
+ * unknown amount: the x axis of a descriptor comes from the mt19937 draws of the keypoint's position in the output
+ * order, and levelling removes roll and pitch but not yaw.  The matcher therefore compares two descriptors by the
+ * minimum over the 12 azimuth rotations (Frome et al., ECCV 2004), evaluated to the last bit as follows.
+ *
+ * Rows.  A descriptor row is FE_DESC_LEN = 1980 floats, bin (l, k, j) at [l*165 + k*15 + j] (l azimuth, k elevation,
+ * j radial), and row i starts i * stride floats after row 0.  stride = FE_DESC_LEN for plain bins; for the records of
+ * fe_enable_record_output, stride = FE_RECORD_FLOATS and the row pointer is the record base + 5 floats.
+ *
+ * Distance.  For a query row a, a reference row b and a shift s in [0, 12):
+ *   P(la, lb) = the chain over m = 0..164 ascending of  acc = 0.0f;  t = a[la*165+m] - b[lb*165+m];  acc = fmaf(t, t, acc)
+ *   d_s(a, b) = 0.0f;  for l = 0..11 ascending:  d_s = d_s + P(l, (l + s) mod 12)        (float adds)
+ * fmaf is the correctly rounded fused multiply-add, every other operation a separate IEEE float operation.  So if
+ * b[((l+s) mod 12)*165 + m] == a[l*165 + m] for every l and m, d_s(a, b) == 0.
+ *
+ * Groups.  query_offsets[0..n_groups] and ref_offsets[0..n_groups] are host arrays of row indices, non-decreasing
+ * and not negative.  Query rows [qo[g], qo[g+1]) are compared with reference rows [ro[g], ro[g+1]) and with nothing
+ * else.  Output row i belongs to query row qo[0] + i: n_queries = qo[G] - qo[0].  One scan against a map is one
+ * group; scan s against scan s-1 of one batch result is qo = keypoint_offsets + 1, ro = keypoint_offsets, G = B - 1.
+ *
+ * Per query, over the candidates (r, s) of its group (r the absolute reference row index):
+ *   best, shift   the candidate with the smallest d_s; a candidate replaces the current best only if its d_s is
+ *                 smaller (the current value starts at +inf), ties go to the lower r, then to the lower s; a NaN
+ *                 distance never wins (so the all-NaN rows of zero-neighbour keypoints never match)
+ *   dist2         d_s of the best candidate
+ *   second_dist2  the smallest per-row minimum over the group's other reference rows (for a ratio test); equal to
+ *                 dist2 when another row ties the best
+ * A query without a winning candidate, e.g. every query of a group without reference rows, gets best = -1,
+ * shift = -1, dist2 = second_dist2 = +inf.
+ *
+ * Results are context-owned pinned host memory, valid until the next match call.  A match call leaves the results of
+ * the last batch call alone, device pointers of fe_process_batch_device included, so one can process, match on the
+ * returned `descriptors` and read both.  FE_ERR_INVALID (the context stays usable) when a stride is below
+ * FE_DESC_LEN, an offsets array decreases or has a negative entry, n_groups < 0, or a row pointer is NULL while its
+ * side has rows.  n_groups = 0 and empty groups are not errors. */
+typedef struct fe_match_result {
+  int64_t n_queries;
+  const int64_t* best;         /* n_queries: absolute reference row index, -1 = none */
+  const int32_t* shift;        /* n_queries: s of the best candidate, -1 = none       */
+  const float* dist2;          /* n_queries */
+  const float* second_dist2;   /* n_queries */
+} fe_match_result_t;
+
+/* Rows in host memory: only rows [qo[0], qo[G]) and [ro[0], ro[G]) are uploaded. */
+int fe_match_descriptors(fe_ctx_t* ctx, const float* query, int64_t query_stride, const int64_t* query_offsets,
+                         const float* ref, int64_t ref_stride, const int64_t* ref_offsets, int32_t n_groups,
+                         fe_match_result_t* out);
+/* Rows already in device memory, e.g. the `descriptors` of fe_process_batch_device.  Runs on the context's stream,
+ * behind whatever a batch call queued there: no synchronisation is needed in between. */
+int fe_match_descriptors_device(fe_ctx_t* ctx, const float* query, int64_t query_stride, const int64_t* query_offsets,
+                                const float* ref, int64_t ref_stride, const int64_t* ref_offsets, int32_t n_groups,
+                                fe_match_result_t* out);
+
 /* CUDA-event stopwatch on the context's stream (the stream every kernel of
  * fe_process_batch_device is launched on): begin, run any number of calls, end -> elapsed ms. */
 int fe_timer_begin(fe_ctx_t* ctx);
