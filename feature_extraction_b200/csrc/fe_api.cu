@@ -96,9 +96,7 @@ struct Slot {
   float4 *d_kfPool = nullptr, *d_kcPool = nullptr, *d_kpPool = nullptr, *d_kpOut = nullptr, *d_gather = nullptr;
   float* d_desc = nullptr;
   DevCounters* d_ctr = nullptr;
-  unsigned long long* d_bnd = nullptr;  // tolerance-boundary report: [scan][4] pair counts
-  unsigned long long* h_bnd = nullptr;
-  unsigned long long *d_bndX = nullptr, *h_bndX = nullptr;  // fe_enable_boundary_report_all: [scan][6], kinds 4-9
+  unsigned long long *d_boundary = nullptr, *h_boundary = nullptr;  // tolerance-boundary report: [scan][FE_BOUNDARY_KINDS] counts
   unsigned* d_gate = nullptr;  // kind 6 per (scan, ring) as the K2 kernels leave it (GateCount)
   // pinned host mirrors
   long long* h_scan_off = nullptr;
@@ -140,10 +138,10 @@ struct fe_ctx {
   bool useGraphs = true;      // fe_debug_enable_graphs
   int64_t graphReplays = 0;
   int angleLibm = 0;          // fe_set_angle_libm
-  double bndEps = 0.0;        // fe_enable_boundary_report: > 0 = count the pairs within bndEps of every radius
-  bool bndAll = false;        // fe_enable_boundary_report_all: also kinds 4-9
+  double bndEps = 0.0;        // boundary report: the decisions within bndEps of their threshold are counted
+  int bndKinds = 0;           // ... of kinds 0-3 (4, fe_enable_boundary_report), 0-9 (FE_BOUNDARY_KINDS, _all) or none (0)
   std::vector<int64_t> bndCounts;     // [scan][4] of the last batch call
-  std::vector<int64_t> bndCountsAll;  // [scan][FE_BOUNDARY_KINDS] of the last batch call (bndAll)
+  std::vector<int64_t> bndCountsAll;  // [scan][FE_BOUNDARY_KINDS] of the last batch call (all kinds enabled)
   // results (host, pinned, grown on demand)
   std::vector<int64_t> kpOffsets;
   fe_point_t* h_kp = nullptr;
@@ -322,9 +320,9 @@ void free_slot(Slot& s) {
   void* dv[] = {s.d_ringPts, s.d_pts, s.d_surf, s.d_crop, s.d_sorted, s.d_full, s.d_cropMeta, s.d_keyA, s.d_keyB, s.d_valA, s.d_valB,
                 s.d_sortedKey, s.d_rho, s.d_scan_off, s.d_chunk_off, s.d_surfCnt, s.d_cropCnt, s.d_rot, s.d_kfBase,
                 s.d_kfCnt, s.d_kcBase, s.d_kcCnt, s.d_kpBase, s.d_kpCnt, s.d_kpOff, s.d_kpScan, s.d_kpNbr, s.d_kpNbrOff, s.d_kpRank, s.d_kpListM, s.d_kpListL, s.d_rowStart,
-                s.d_surfN, s.d_perScan, s.d_outOff, s.d_ovfRings, s.d_ovfRings2, s.d_ovfMerge, s.d_ovfMerge2, s.d_ovfSurf, s.d_slabs, s.d_gridHdr, s.d_tabOk, s.d_kfPool, s.d_kcPool, s.d_kpPool, s.d_kpOut, s.d_gather, s.d_desc, s.d_ctr, s.d_bnd, s.d_bndX, s.d_gate, s.d_ringBase, s.d_ovfRuns, s.d_scanFlag, s.d_perScan2, s.d_outOff2, s.d_gather2, s.d_chunkTab};
+                s.d_surfN, s.d_perScan, s.d_outOff, s.d_ovfRings, s.d_ovfRings2, s.d_ovfMerge, s.d_ovfMerge2, s.d_ovfSurf, s.d_slabs, s.d_gridHdr, s.d_tabOk, s.d_kfPool, s.d_kcPool, s.d_kpPool, s.d_kpOut, s.d_gather, s.d_desc, s.d_ctr, s.d_boundary, s.d_gate, s.d_ringBase, s.d_ovfRuns, s.d_scanFlag, s.d_perScan2, s.d_outOff2, s.d_gather2, s.d_chunkTab};
   for (void* p : dv) if (p) cudaFree(p);
-  void* hv[] = {s.h_scan_off, s.h_chunk_off, s.h_rot, s.h_ctr, s.h_kpOff, s.h_perScan, s.h_bnd, s.h_bndX, s.h_cloudOff, s.h_kcOff};
+  void* hv[] = {s.h_scan_off, s.h_chunk_off, s.h_rot, s.h_ctr, s.h_kpOff, s.h_perScan, s.h_boundary, s.h_cloudOff, s.h_kcOff};
   for (void* p : hv) if (p) cudaFreeHost(p);
   for (cudaEvent_t e : s.ev) cudaEventDestroy(e);
   for (GraphEntry& g : s.graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
@@ -503,7 +501,7 @@ int set_kernel_attrs(fe_ctx* ctx) {
   CK(cudaFuncSetAttribute(k_cluster_rings<ECAP, NTF, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmem));
   CK(cudaFuncSetAttribute(k_ring_runs<NW_RR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW>)));
   CK(cudaFuncSetAttribute(k_ring_runs<NW_RR_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW, NW_RR_SMALL>)));
-  CK(cudaFuncSetAttribute(k_ring_runs_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(NW_RR * sizeof(RunBufT<RW2>))));
+  CK(cudaFuncSetAttribute(k_ring_runs_wide<>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(NW_RR * sizeof(RunBufT<RW2>))));
   CK(cudaFuncSetAttribute(k_cluster_rings<ECAP_L, NTL, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemL2));
   CK(cudaFuncSetAttribute(k_merge_keypoints<ECAP_M, NTM, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemM));
   CK(cudaFuncSetAttribute(k_merge_keypoints<ECAP_L, NT2, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemL));
@@ -519,11 +517,12 @@ int set_kernel_attrs(fe_ctx* ctx) {
   // the boundary report's K2 instantiations (kind 6).  Named after every other kernel: the order in which the host
   // code first names the kernels is the order the compiler meets them, and the kernels above compile as they did
   // before these existed only in this order.
-  CK(cudaFuncSetAttribute(k_cluster_rings_bnd<ECAP, NTF, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmem));
-  CK(cudaFuncSetAttribute(k_ring_runs_bnd<NW_RR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW>)));
-  CK(cudaFuncSetAttribute(k_ring_runs_bnd<NW_RR_SMALL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW, NW_RR_SMALL>)));
-  CK(cudaFuncSetAttribute(k_ring_runs_wide_bnd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(NW_RR * sizeof(RunBufT<RW2>))));
-  CK(cudaFuncSetAttribute(k_cluster_rings_bnd<ECAP_L, NT2, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemL));
+  CK(cudaFuncSetAttribute(k_cluster_rings<ECAP, NTF, 4, false, GateCount>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmem));
+  CK(cudaFuncSetAttribute(k_ring_runs<NW_RR, GateCount>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RingRunsSmT<RW>)));
+  CK(cudaFuncSetAttribute(k_ring_runs<NW_RR_SMALL, GateCount>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)sizeof(RingRunsSmT<RW, NW_RR_SMALL>)));
+  CK(cudaFuncSetAttribute(k_ring_runs_wide<GateCount>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(NW_RR * sizeof(RunBufT<RW2>))));
+  CK(cudaFuncSetAttribute(k_cluster_rings<ECAP_L, NT2, 1, false, GateCount>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kClusterSmemL));
   return FE_OK;
 }
 
@@ -632,15 +631,21 @@ void launch_density(fe_ctx* ctx, Slot& s, int nscans, const DevParams& P, int64_
 
 // K2 + K3 for `nscans` scans: the 2-blocks-per-SM instantiation first, then the large one over
 // whatever scans it deferred (an immediate exit when there are none).
-// gate: count kind 6 of the boundary report (fe_enable_boundary_report_all) with the GateCount instantiations of K2
+// gate...: nothing, or the GateCount with which the K2 instantiations count kind 6 of the boundary report
+// (fe_enable_boundary_report_all)
+template <class... G>
 void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool wantKc, bool merge, bool marks = false, bool lean = false,
-                       const GateCount* gate = nullptr) {
+                       G... gate) {
   // Every stage is a chain of instantiations: the fast one takes all scans and defers those that do
   // not fit its shared memory to a list; the large shared-memory one takes that list; what does not
   // fit there either goes to the instantiation whose per-entry arrays live in global memory.
   const DevParams& P = ctx->dp;
   const int gridL = std::min(nscans, ctx->numSms), gridG = std::min(nscans, NGLOBAL);
   const size_t smemG = cluster_smem_bytes_global(NT2);
+  // K2's large instantiation counting kind 6 runs 512 threads, not NTL: a second caller of the 1024-thread cluster
+  // helpers changes how k_cluster_rings<ECAP_L, NTL> compiles (the capacity is the same, hence the same deferrals
+  // and clusters)
+  constexpr int ntL = sizeof...(G) > 0 ? NT2 : NTL;
   int* ovfR = &s.d_ctr->ovf_rings;
   int* ovfR2 = &s.d_ctr->ovf_rings2;
   int* ovfM = &s.d_ctr->ovf_merge;
@@ -651,9 +656,8 @@ void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool w
   const int sr = singleRing ? 1 : 0;
   // inList / inN: the scans the previous instantiation deferred to this one (null: every scan); outList / outN: where
   // this one defers what it cannot take (null: the last of the chain); slabs: per-entry arrays in global memory
-  // `gate...`: nothing, or the GateCount of a *_bnd kernel
   auto k2 = [&](auto kernel, int grid, int nt, size_t smem, const int* inList, const int* inN, int* outList, int* outN,
-                unsigned char* slabs, auto... gate) {
+                unsigned char* slabs) {
     kernel<<<grid, nt, smem, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_kfPool,
                                          s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr, inList, inN, outList,
                                          outN, slabs, gate...);
@@ -668,45 +672,31 @@ void launch_clustering(fe_ctx* ctx, Slot& s, int nscans, bool singleRing, bool w
   // K2: the run-based kernel takes every scan; what it cannot handle (a ring with more than RW runs — unordered
   // input — or more ring entries than the scan's scratch slot) goes down the chain of grid-based instantiations.
   if (ctx->gridClustering) {
-    if (gate) k2(k_cluster_rings_bnd<ECAP, NTF, 4, false>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr, *gate);
-    else k2(k_cluster_rings<ECAP, NTF, 4, false>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr);
+    k2(k_cluster_rings<ECAP, NTF, 4, false, G...>, nscans, NTF, kClusterSmem, nullptr, nullptr, s.d_ovfRings, ovfR, nullptr);
   } else {
-    auto rr = [&](auto kernel, int nt, size_t smem, auto... gate) {
+    auto rr = [&](auto kernel, int nt, size_t smem) {
       kernel<<<nscans, nt, smem, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, P, sr, s.d_ringPts,
                                              s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
                                              s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR, gate...);
       ctx->launches++;
     };
-    if (nscans <= GRAPH_MAX_SCANS) {  // a handful of scans: a warp for each of a scan's 16 rings at once (latency, not throughput)
-      if (gate) rr(k_ring_runs_bnd<NW_RR_SMALL>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>), *gate);
-      else rr(k_ring_runs<NW_RR_SMALL>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>));
-    } else {
-      if (gate) rr(k_ring_runs_bnd<NW_RR>, NT_RR, sizeof(RingRunsSmT<RW>), *gate);
-      else rr(k_ring_runs<NW_RR>, NT_RR, sizeof(RingRunsSmT<RW>));
-    }
+    if (nscans <= GRAPH_MAX_SCANS)  // a handful of scans: a warp for each of a scan's 16 rings at once (latency, not throughput)
+      rr(k_ring_runs<NW_RR_SMALL, G...>, NW_RR_SMALL * 32, sizeof(RingRunsSmT<RW, NW_RR_SMALL>));
+    else
+      rr(k_ring_runs<NW_RR, G...>, NT_RR, sizeof(RingRunsSmT<RW>));
     if (!lean) {
-      auto wide = [&](auto kernel, auto... gate) {
-        kernel<<<std::min(nscans * 4, ctx->numSms * 7), NT_RR, NW_RR * sizeof(RunBufT<RW2>), s.stream>>>(
-            s.d_scan_off, P, s.d_ringPts, s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
-            s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR, gate...);
-        ctx->launches++;
-      };
-      if (gate) wide(k_ring_runs_wide_bnd, *gate);
-      else wide(k_ring_runs_wide);
+      k_ring_runs_wide<G...><<<std::min(nscans * 4, ctx->numSms * 7), NT_RR, NW_RR * sizeof(RunBufT<RW2>), s.stream>>>(
+          s.d_scan_off, P, s.d_ringPts, s.d_ringBase, s.d_kfPool, s.capKf, s.d_kfBase, s.d_kfCnt, kc, s.capKc, kcB, kcC, s.d_ctr,
+          s.d_ovfRuns, &s.d_ctr->ovf_runs, s.d_scanFlag, s.d_ovfRings, ovfR, gate...);
+      ctx->launches++;
     }
   }
   // lean: the fallback instantiations are left out; whatever the first kernel deferred shows in the counters and the
   // caller runs the sub-batch again with the whole chain
   if (!lean) {
-    if (gate) {
-      // 512 threads, not NTL: a second caller of the 1024-thread cluster helpers changes how k_cluster_rings<ECAP_L, NTL>
-      // compiles (the capacity is the same, hence the same deferrals and clusters)
-      k2(k_cluster_rings_bnd<ECAP_L, NT2, 1, false>, gridL, NT2, kClusterSmemL, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr, *gate);
-      k2(k_cluster_rings_bnd<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs, *gate);
-    } else {
-      k2(k_cluster_rings<ECAP_L, NTL, 1, false>, gridL, NTL, kClusterSmemL2, s.d_ovfRings, ovfR, s.d_ovfRings2, ovfR2, nullptr);
-      k2(k_cluster_rings<ECAP_G, NT2, 1, true>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs);
-    }
+    k2(k_cluster_rings<ECAP_L, ntL, 1, false, G...>, gridL, ntL, cluster_smem_bytes(ECAP_L, ntL), s.d_ovfRings, ovfR, s.d_ovfRings2,
+       ovfR2, nullptr);
+    k2(k_cluster_rings<ECAP_G, NT2, 1, true, G...>, gridG, NT2, smemG, s.d_ovfRings2, ovfR2, nullptr, nullptr, s.d_slabs);
   }
   if (marks) mark(ctx, s, "K2 ring clusters");
   if (merge) {
@@ -732,17 +722,10 @@ BoundarySpec boundary_spec(const fe_ctx* ctx) {
   return B;
 }
 
-// which kinds the boundary report counts: 0 (off), 4 or FE_BOUNDARY_KINDS
-int bnd_kinds(const fe_ctx* ctx) { return ctx->bndEps > 0.0 ? (ctx->bndAll ? FE_BOUNDARY_KINDS : 4) : 0; }
-
 int ensure_bnd(fe_ctx* ctx, Slot& s) {
-  if (!s.d_bnd) {
-    CK(dalloc(&s.d_bnd, (size_t)s.capScans * 4));
-    CK(halloc(&s.h_bnd, (size_t)s.capScans * 4));
-  }
-  if (ctx->bndAll && !s.d_bndX) {
-    CK(dalloc(&s.d_bndX, (size_t)s.capScans * 6));
-    CK(halloc(&s.h_bndX, (size_t)s.capScans * 6));
+  if (!s.d_boundary) {
+    CK(dalloc(&s.d_boundary, (size_t)s.capScans * FE_BOUNDARY_KINDS));
+    CK(halloc(&s.h_boundary, (size_t)s.capScans * FE_BOUNDARY_KINDS));
     CK(dalloc(&s.d_gate, (size_t)s.capScans * 16));
   }
   return FE_OK;
@@ -788,24 +771,22 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
     }
   }
   mark(ctx, s, "K1 level+crop+ring");
-  const bool bnd = ctx->bndEps > 0.0 && nscans > 0;
-  const bool bndAll = bnd && ctx->bndAll;  // kinds 4-9 too
-  if (bnd) {
+  const int kinds = nscans > 0 ? ctx->bndKinds : 0;  // of the boundary report: 0, 4 or FE_BOUNDARY_KINDS
+  const bool allKinds = kinds == FE_BOUNDARY_KINDS;
+  const BoundarySpec B = boundary_spec(ctx);
+  if (kinds) {
     int st = ensure_bnd(ctx, s);
     if (st) return st;
-    CK(cudaMemsetAsync(s.d_bnd, 0, (size_t)nscans * 4 * sizeof(unsigned long long), s.stream));
-    k_boundary_rings<<<nscans, 256, 0, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, 0,
-                                                   boundary_spec(ctx), s.d_bnd);
+    CK(cudaMemsetAsync(s.d_boundary, 0, (size_t)nscans * FE_BOUNDARY_KINDS * sizeof(unsigned long long), s.stream));
+    k_boundary_rings<<<nscans, 256, 0, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, 0, B, s.d_boundary);
     ctx->launches++;
   }
-  const GateCount gate = {ctx->bndEps, s.d_gate};  // (after ensure_bnd: d_gate is allocated on the first call with bndAll)
-  if (bndAll) {
-    CK(cudaMemsetAsync(s.d_bndX, 0, (size_t)nscans * 6 * sizeof(unsigned long long), s.stream));
+  if (allKinds) {
     CK(cudaMemsetAsync(s.d_gate, 0, (size_t)nscans * 16 * sizeof(unsigned), s.stream));
     const int nch = s.h_chunk_off[nscans];  // every chunk of the sub-batch: the matrices of all of them are staged by now
     if (nch > 0) {
-      if (sb.lay.raw) k_boundary_crop_ring<true><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, ctx->bndEps, s.d_bndX);
-      else k_boundary_crop_ring<false><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, ctx->bndEps, s.d_bndX);
+      if (sb.lay.raw) k_boundary_crop_ring<true><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, B.eps, s.d_boundary);
+      else k_boundary_crop_ring<false><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, B.eps, s.d_boundary);
       ctx->launches++;
     }
   }
@@ -813,14 +794,15 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
     int st = ensure_rowstart(ctx, s, P, nscans);
     if (st) return st;
   }
-  launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean, bndAll ? &gate : nullptr);
+  if (allKinds) launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean, GateCount{B.eps, s.d_gate});
+  else launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean);
   mark(ctx, s, "K3 merge keypoints");
-  if (bnd) {
-    k_boundary_merge<<<nscans, 128, 0, s.stream>>>(s.d_kfPool, s.d_kfBase, s.d_kfCnt, P, boundary_spec(ctx), s.d_bnd);
+  if (kinds) {
+    k_boundary_merge<<<nscans, 128, 0, s.stream>>>(s.d_kfPool, s.d_kfBase, s.d_kfCnt, P, B, s.d_boundary);
     ctx->launches++;
   }
-  if (bndAll) {
-    k_boundary_gate_sum<<<(nscans + 255) / 256, 256, 0, s.stream>>>(s.d_gate, nscans, s.d_bndX);
+  if (allKinds) {
+    k_boundary_gate_sum<<<(nscans + 255) / 256, 256, 0, s.stream>>>(s.d_gate, nscans, s.d_boundary);
     ctx->launches++;
   }
   if (nscans <= GRAPH_MAX_SCANS) {  // a handful of scans: offsets and ordered copy in one launch
@@ -840,18 +822,17 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
     const int gridKp = ctx->numSms * 8;
     launch_desc_mark(ctx, s, nscans, P, gridKp);
     mark(ctx, s, "K4b mark neighbours");
-    if (bnd) {  // before K4c turns the marks in rho into densities
+    if (kinds) {  // before K4c turns the marks in rho into densities
       k_boundary_support<<<ctx->numSms * 4, 256, 0, s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_sorted, surf_index(P, s),
-                                                         s.d_scan_off, P, boundary_spec(ctx), s.d_bnd);
+                                                         s.d_scan_off, P, B, s.d_boundary);
       if (sb.npts > 0)
-        k_boundary_density<<<nscans, 256, 0, s.stream>>>(s.d_sorted, surf_index(P, s), s.d_scan_off, P, s.d_surfN, s.d_rho,
-                                                         boundary_spec(ctx), s.d_bnd);
+        k_boundary_density<<<nscans, 256, 0, s.stream>>>(s.d_sorted, surf_index(P, s), s.d_scan_off, P, s.d_surfN, s.d_rho, B,
+                                                         s.d_boundary);
       ctx->launches += 2;
     }
-    if (bndAll) {
+    if (allKinds) {
       k_boundary_bins<<<ctx->numSms * 4, 256, 0, s.stream>>>(s.d_kpOut, s.d_kpScan, s.d_kpOff, nscans, s.d_sorted, surf_index(P, s),
-                                                             s.d_scan_off, P, ctx->d_axes, ctx->axesCap, s.d_kpRank, ctx->bndEps,
-                                                             s.d_bndX);
+                                                             s.d_scan_off, P, ctx->d_axes, ctx->axesCap, s.d_kpRank, B.eps, s.d_boundary);
       ctx->launches++;
     }
     launch_density(ctx, s, nscans, P, sb.npts);
@@ -875,8 +856,9 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
   }
   CK(cudaMemcpyAsync(s.h_ctr, s.d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, s.stream));
   CK(cudaMemcpyAsync(s.h_kpOff, s.d_kpOff, (size_t)(nscans + 1) * sizeof(int), cudaMemcpyDeviceToHost, s.stream));
-  if (bnd) CK(cudaMemcpyAsync(s.h_bnd, s.d_bnd, (size_t)nscans * 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s.stream));
-  if (bndAll) CK(cudaMemcpyAsync(s.h_bndX, s.d_bndX, (size_t)nscans * 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s.stream));
+  if (kinds)
+    CK(cudaMemcpyAsync(s.h_boundary, s.d_boundary, (size_t)nscans * FE_BOUNDARY_KINDS * sizeof(unsigned long long),
+                       cudaMemcpyDeviceToHost, s.stream));
   if (recordDone) CK(cudaEventRecord(s.evDone, s.stream));
   CK(cudaGetLastError());
   return FE_OK;
@@ -950,10 +932,10 @@ int enqueue_subbatch(fe_ctx* ctx, Slot& s, const SubBatch& sb, const double* lat
   if (bytes) CK(cudaMemcpyAsync(s.d_pts, upload, bytes, cudaMemcpyHostToDevice, s.stream));
   // every allocation the pipeline may need happens before a capture starts
   if (sb.desc) { st = ensure_rowstart(ctx, s, ctx->dp, sb.nscans); if (st) return st; }
-  if (ctx->bndEps > 0.0) { st = ensure_bnd(ctx, s); if (st) return st; }
+  if (ctx->bndKinds) { st = ensure_bnd(ctx, s); if (st) return st; }
   s.sb.lean = ctx->leanHold == 0;
   if (ctx->leanHold > 0) ctx->leanHold--;
-  const GraphKey key = {s.sb, density_blocks_per_scan(sb.nscans, sb.npts), s.maxScanPts > 65535, bnd_kinds(ctx), ctx->epoch};
+  const GraphKey key = {s.sb, density_blocks_per_scan(sb.nscans, sb.npts), s.maxScanPts > 65535, ctx->bndKinds, ctx->epoch};
   GraphEntry* ge = nullptr;
   for (GraphEntry& g : s.graphs) if (g.key == key) { ge = &g; break; }
   if (ge && ge->exec) {  // replay
@@ -1002,13 +984,12 @@ int complete_subbatch(fe_ctx* ctx, Slot& s, int64_t kpBase) {
   if (s.h_ctr->err) return fail(ctx, FE_ERR_CAPACITY, err_bits(s.h_ctr->err));
   const int ns = s.sb.nscans;
   for (int i = 0; i <= ns; i++) ctx->kpOffsets[s.firstScan + i] = kpBase + s.h_kpOff[i];
-  if (ctx->bndEps > 0.0 && s.h_bnd)
-    for (int i = 0; i < ns * 4; i++) ctx->bndCounts[(size_t)s.firstScan * 4 + i] = (int64_t)s.h_bnd[i];
-  if (ctx->bndAll && s.h_bndX)
+  if (ctx->bndKinds && s.h_boundary)
     for (int i = 0; i < ns; i++) {
-      int64_t* row = &ctx->bndCountsAll[((size_t)s.firstScan + i) * FE_BOUNDARY_KINDS];
-      for (int k = 0; k < 4; k++) row[k] = (int64_t)s.h_bnd[i * 4 + k];
-      for (int k = 0; k < 6; k++) row[4 + k] = (int64_t)s.h_bndX[i * 6 + k];
+      const unsigned long long* row = s.h_boundary + (size_t)i * FE_BOUNDARY_KINDS;
+      const size_t scan = (size_t)s.firstScan + i;
+      std::copy(row, row + 4, &ctx->bndCounts[scan * 4]);
+      if (ctx->bndKinds == FE_BOUNDARY_KINDS) std::copy(row, row + FE_BOUNDARY_KINDS, &ctx->bndCountsAll[scan * FE_BOUNDARY_KINDS]);
     }
   return FE_OK;
 }
@@ -1248,7 +1229,7 @@ static int enable_boundary_report(fe_ctx_t* ctx, double eps_m, bool all) {
   if (!ctx || !(eps_m == eps_m)) return FE_ERR_INVALID;
   if (int st = sync_slots(ctx)) return st;
   ctx->bndEps = eps_m > 0.0 ? eps_m : 0.0;
-  ctx->bndAll = all && ctx->bndEps > 0.0;
+  ctx->bndKinds = eps_m > 0.0 ? (all ? FE_BOUNDARY_KINDS : 4) : 0;
   ctx->bndCounts.clear();
   ctx->bndCountsAll.clear();
   ctx->epoch++;
@@ -1261,7 +1242,7 @@ int fe_enable_boundary_report_all(fe_ctx_t* ctx, double eps_m) { return enable_b
 
 int fe_get_boundary_report(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans) {
   if (!ctx || !counts || !n_scans) return FE_ERR_INVALID;
-  if (!(ctx->bndEps > 0.0)) return fail(ctx, FE_ERR_INVALID, "boundary report not enabled (fe_enable_boundary_report)");
+  if (!ctx->bndKinds) return fail(ctx, FE_ERR_INVALID, "boundary report not enabled (fe_enable_boundary_report)");
   *counts = ctx->bndCounts.data();
   *n_scans = (int32_t)(ctx->bndCounts.size() / 4);
   return FE_OK;
@@ -1269,7 +1250,8 @@ int fe_get_boundary_report(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_sca
 
 int fe_get_boundary_report_all(fe_ctx_t* ctx, const int64_t** counts, int32_t* n_scans) {
   if (!ctx || !counts || !n_scans) return FE_ERR_INVALID;
-  if (!ctx->bndAll) return fail(ctx, FE_ERR_INVALID, "boundary report of all kinds not enabled (fe_enable_boundary_report_all)");
+  if (ctx->bndKinds != FE_BOUNDARY_KINDS)
+    return fail(ctx, FE_ERR_INVALID, "boundary report of all kinds not enabled (fe_enable_boundary_report_all)");
   *counts = ctx->bndCountsAll.data();
   *n_scans = (int32_t)(ctx->bndCountsAll.size() / FE_BOUNDARY_KINDS);
   return FE_OK;
@@ -1324,8 +1306,8 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
   const bool desc = ctx->params.estimate_descriptors != 0;
   const int64_t launches0 = ctx->launches;
   ctx->kpOffsets.assign((size_t)n_scans + 1, 0);
-  ctx->bndCounts.assign(ctx->bndEps > 0.0 ? (size_t)n_scans * 4 : 0, 0);
-  ctx->bndCountsAll.assign(ctx->bndAll ? (size_t)n_scans * FE_BOUNDARY_KINDS : 0, 0);
+  ctx->bndCounts.assign(ctx->bndKinds ? (size_t)n_scans * 4 : 0, 0);
+  ctx->bndCountsAll.assign(ctx->bndKinds == FE_BOUNDARY_KINDS ? (size_t)n_scans * FE_BOUNDARY_KINDS : 0, 0);
   ctx->cloudOff.clear(); ctx->kcOff.clear();
   ctx->cloudRun = ctx->kcRun = 0;
   if (ctx->cloudOutputs) { ctx->cloudOff.assign((size_t)n_scans + 1, 0); ctx->kcOff.assign((size_t)n_scans + 1, 0); }
@@ -1451,8 +1433,8 @@ int fe_process_batch_device(fe_ctx_t* ctx, const fe_point_t* d_points, const int
     if (st) return st;
     st = enqueue_subbatch(ctx, s, sb, lateRp);
     if (st) return st;
-    ctx->bndCounts.assign(ctx->bndEps > 0.0 ? (size_t)n_scans * 4 : 0, 0);
-    ctx->bndCountsAll.assign(ctx->bndAll ? (size_t)n_scans * FE_BOUNDARY_KINDS : 0, 0);
+    ctx->bndCounts.assign(ctx->bndKinds ? (size_t)n_scans * 4 : 0, 0);
+    ctx->bndCountsAll.assign(ctx->bndKinds == FE_BOUNDARY_KINDS ? (size_t)n_scans * FE_BOUNDARY_KINDS : 0, 0);
     s.firstScan = 0;
     st = complete_subbatch(ctx, s, 0);
     if (st) return st;

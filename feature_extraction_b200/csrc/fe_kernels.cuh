@@ -103,8 +103,9 @@ struct DevCounters {
 
 // Kind 6 of the tolerance-boundary report (fe_enable_boundary_report_all): ring clusters whose xy diameter lies within
 // eps of the gate 2 * clusterRadiusThreshold (src:316), counted by the K2 kernels where they decide the gate.  The
-// device functions of K2 take it as a trailing parameter pack `gate...`: empty in the kernels that run without that
-// report (their code is what it was without it), one GateCount in the separate *_bnd kernels.
+// K2 kernels and their device functions take it as a trailing parameter pack `gate...`: empty in the instantiations
+// that run without that report (their code is what it was without it), one GateCount in the report-on ones
+// (k_ring_runs<NW, GateCount>, k_ring_runs_wide<GateCount>, k_cluster_rings<..., GateCount>).
 struct GateCount {
   double eps;
   unsigned* cnt;  // [scan][16], zeroed by the first K2 kernel of a scan: the run kernels count ring r in slot r,
@@ -1002,8 +1003,8 @@ __device__ void cluster_rings_scan(
 }
 
 // scanList == nullptr: block b handles scan b and defers oversized scans to ovfList;
-// otherwise the blocks loop over scanList[0 .. *nList) (the deferred scans).
-template <int CAP, int NT, int MINB, bool GLOBAL>
+// otherwise the blocks loop over scanList[0 .. *nList) (the deferred scans).  gate...: nothing, or a GateCount.
+template <int CAP, int NT, int MINB, bool GLOBAL, class... G>
 __global__ void __launch_bounds__(NT, MINB) k_cluster_rings(
     const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta,
     const int* __restrict__ cropCnt, const long long* __restrict__ scan_off,
@@ -1011,48 +1012,20 @@ __global__ void __launch_bounds__(NT, MINB) k_cluster_rings(
     float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
     float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
     DevCounters* __restrict__ ctr, const int* __restrict__ scanList, const int* __restrict__ nList,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount, unsigned char* __restrict__ slabs) {
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, unsigned char* __restrict__ slabs, G... gate) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ClusterSm S;
   if (GLOBAL) cluster_carve_global<CAP, NT>(slabs + (size_t)blockIdx.x * cluster_slab_bytes(CAP), smem_raw, S);
   else cluster_sm_carve<CAP, NT>(smem_raw, S);
   if (!scanList) {
     cluster_rings_scan<CAP, NT>(S, blockIdx.x, crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
-                            kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount);
+                            kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount, gate...);
   } else {
     const int n = *nList;
     for (int i = blockIdx.x; i < n; i += gridDim.x) {
       __syncthreads();
       cluster_rings_scan<CAP, NT>(S, scanList[i], crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
-                              kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount);
-    }
-  }
-}
-
-// k_cluster_rings, also counting the clusters on the diameter gate's boundary (kind 6); a copy for the same reason
-// as k_ring_runs_bnd.
-template <int CAP, int NT, int MINB, bool GLOBAL>
-__global__ void __launch_bounds__(NT, MINB) k_cluster_rings_bnd(
-    const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta,
-    const int* __restrict__ cropCnt, const long long* __restrict__ scan_off,
-    const int* __restrict__ chunk_off, DevParams P, int single_ring,
-    float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
-    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
-    DevCounters* __restrict__ ctr, const int* __restrict__ scanList, const int* __restrict__ nList,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount, unsigned char* __restrict__ slabs, GateCount gate) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  ClusterSm S;
-  if (GLOBAL) cluster_carve_global<CAP, NT>(slabs + (size_t)blockIdx.x * cluster_slab_bytes(CAP), smem_raw, S);
-  else cluster_sm_carve<CAP, NT>(smem_raw, S);
-  if (!scanList) {
-    cluster_rings_scan<CAP, NT>(S, blockIdx.x, crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
-                            kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount, gate);
-  } else {
-    const int n = *nList;
-    for (int i = blockIdx.x; i < n; i += gridDim.x) {
-      __syncthreads();
-      cluster_rings_scan<CAP, NT>(S, scanList[i], crop, cropMeta, cropCnt, scan_off, chunk_off, P, single_ring, kfPool, kfCap,
-                              kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount, gate);
+                              kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfList, ovfCount, gate...);
     }
   }
 }
@@ -2568,7 +2541,7 @@ __global__ void __launch_bounds__(256) k_record_frame(const float4* __restrict__
 // Tolerance-boundary report (fe_enable_boundary_report) — audit kernels, not part of the hot path.
 // BASELINE.json north_star: "points lying within 1e-6 m of a tolerance boundary reported
 // separately".  Every radius predicate of the path is d2 < r2f in float; a pair is on the boundary
-// when |sqrt((double)d2) - sqrt((double)r2f)| < eps.  bnd[4*scan + k] counts them per predicate:
+// when |sqrt((double)d2) - sqrt((double)r2f)| < eps.  bnd[FE_BOUNDARY_KINDS * scan + k] counts them per predicate:
 //   0 ring clustering (src:269-276): unordered pairs of crop points sharing a ring
 //   1 cross-ring merge (src:222-229): unordered pairs of ring centroids (pseudo z, src:217)
 //   2 3DSC support radius (src:350): (keypoint, surface point) pairs
@@ -2638,7 +2611,7 @@ __global__ void __launch_bounds__(256) k_boundary_rings(
       }
     }
   }
-  if (cnt) atomicAdd(&bnd[4 * s + 0], cnt);
+  if (cnt) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 0], cnt);
 }
 
 // one block per scan: all pairs of the scan's ring centroids with the pseudo z of src:217
@@ -2669,7 +2642,7 @@ __global__ void __launch_bounds__(128) k_boundary_merge(const float4* __restrict
       if (on_boundary(B, 1, l2_simple(p.x, p.y, p.z, q.x, q.y, q.z))) cnt++;
     }
   }
-  if (cnt) atomicAdd(&bnd[4 * s + 1], cnt);
+  if (cnt) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 1], cnt);
 }
 
 // keypoints against the search surface (slot 2): the sweep of K4b, widened by eps
@@ -2697,7 +2670,7 @@ __global__ void __launch_bounds__(256) k_boundary_support(
         if (on_boundary(B, 2, l2_simple(o.x, o.y, o.z, q.x, q.y, q.z))) cnt++;
       }
     }
-    if (cnt) atomicAdd(&bnd[4 * s + 2], cnt);
+    if (cnt) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 2], cnt);
   }
 }
 
@@ -2726,19 +2699,19 @@ __global__ void __launch_bounds__(256) k_boundary_density(
       }
     }
   }
-  if (cnt) atomicAdd(&bnd[4 * s + 3], cnt);
+  if (cnt) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 3], cnt);
 }
 
 // ---- kinds 4-9 (fe_enable_boundary_report_all): the threshold decisions in metres or degrees that are not radius
 // predicates.  Margins are evaluated in double with + - * / sqrt only (no FMA: -fmad=false), in the order of
-// include/fe_b200.h, so the oracle's counts agree to the last pair.  bndx[6 * scan + k - 4] counts kind k. ----
+// include/fe_b200.h, so the oracle's counts agree to the last pair.  bnd[FE_BOUNDARY_KINDS * scan + k] counts kind k. ----
 constexpr double BND_DEG = 0.017453292519943295;  // pi / 180
 
 // kinds 4 (crop box) and 5 (ring-window ends): one block per K1 chunk, K1's decode, levelling and crop again
 template <bool RAW>
 __global__ void __launch_bounds__(256) k_boundary_crop_ring(const float4* __restrict__ pts, const int4* __restrict__ chunkTab,
                                                             const float* __restrict__ rot, DevParams P, RawLayout L, double eps,
-                                                            unsigned long long* __restrict__ bndx) {
+                                                            unsigned long long* __restrict__ bnd) {
   const int4 ct = __ldg(chunkTab + blockIdx.x);
   const int s = ct.x, nIn = ct.y & 4095;
   const long long base = (long long)(((unsigned long long)(unsigned)ct.w << 32) | (unsigned)ct.z);
@@ -2780,19 +2753,19 @@ __global__ void __launch_bounds__(256) k_boundary_crop_ring(const float4* __rest
   nCrop = __reduce_add_sync(FE_FULL, nCrop);
   nRing = __reduce_add_sync(FE_FULL, nRing);
   if ((threadIdx.x & 31) == 0) {
-    if (nCrop) atomicAdd(&bndx[6 * s + 0], (unsigned long long)nCrop);
-    if (nRing) atomicAdd(&bndx[6 * s + 1], (unsigned long long)nRing);
+    if (nCrop) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 4], (unsigned long long)nCrop);
+    if (nRing) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 5], (unsigned long long)nRing);
   }
 }
 
 // kind 6: the per-ring counts the GateCount instantiations of K2 left, summed per scan
 __global__ void __launch_bounds__(256) k_boundary_gate_sum(const unsigned* __restrict__ gate, int n_scans,
-                                                           unsigned long long* __restrict__ bndx) {
+                                                           unsigned long long* __restrict__ bnd) {
   const int s = blockIdx.x * 256 + threadIdx.x;
   if (s >= n_scans) return;
   unsigned t = 0;
   for (int r = 0; r < 16; r++) t += gate[s * 16 + r];
-  bndx[6 * s + 2] = t;
+  bnd[FE_BOUNDARY_KINDS * s + 6] = t;
 }
 
 // kinds 7-9 (3DSC radial shells, elevation and azimuth edges): the (keypoint, neighbour) pairs K4d bins — the sweep of
@@ -2801,7 +2774,7 @@ __global__ void __launch_bounds__(256) k_boundary_bins(
     const float4* __restrict__ kpOut, const int* __restrict__ kpScan, const int* __restrict__ kpOff, int n_scans,
     const float4* __restrict__ sorted, SurfIndex X, const long long* __restrict__ scan_off, DevParams P,
     const float2* __restrict__ axes, int axesCap, const int* __restrict__ kpRank, double eps,
-    unsigned long long* __restrict__ bndx) {
+    unsigned long long* __restrict__ bnd) {
   const int total = kpOff[n_scans];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   for (int g = blockIdx.x; g < total; g += gridDim.x) {
@@ -2838,9 +2811,9 @@ __global__ void __launch_bounds__(256) k_boundary_bins(
         if (rho == 0.0 || __dmul_rn(rho, __dmul_rn(dp, BND_DEG)) < eps) nAz++;
       }
     }
-    if (nRad) atomicAdd(&bndx[6 * s + 3], nRad);
-    if (nEl) atomicAdd(&bndx[6 * s + 4], nEl);
-    if (nAz) atomicAdd(&bndx[6 * s + 5], nAz);
+    if (nRad) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 7], nRad);
+    if (nEl) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 8], nEl);
+    if (nAz) atomicAdd(&bnd[FE_BOUNDARY_KINDS * s + 9], nAz);
   }
 }
 

@@ -352,14 +352,15 @@ __device__ void rr_scan_rings(RingRunsSmT<RWT, NW>& S, const int s, const float4
 // First kernel: one block per scan, every scan.  A ring of more than RW runs is handed to the second kernel (the
 // ring segments and their offsets stay in global memory, so nothing is bucketed twice); a scan with more ring
 // entries than its scratch slot goes straight to the grid-based kernels.
-template <int NW>
+// gate...: nothing, or the GateCount of the boundary report's kind 6 (zeroed here for the scan's 16 rings).
+template <int NW, class... G>
 __global__ void __launch_bounds__(NW * 32, NW == NW_RR ? 12 : 1) k_ring_runs(
     const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta, const int* __restrict__ cropCnt,
     const long long* __restrict__ scan_off, const int* __restrict__ chunk_off, DevParams P, int single_ring,
     float4* ringPts, int* __restrict__ ringBaseOut, float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
     float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
     DevCounters* __restrict__ ctr, int* __restrict__ ovfRuns, int* __restrict__ ovfRunsCount, int* __restrict__ scanFlag,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount) {
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, G... gate) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   RingRunsSmT<RW, NW>& S = *reinterpret_cast<RingRunsSmT<RW, NW>*>(smem_raw);
   const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
@@ -368,6 +369,7 @@ __global__ void __launch_bounds__(NW * 32, NW == NW_RR ? 12 : 1) k_ring_runs(
   const int nch = chunk_off[s + 1] - chunk_off[s];
   if (tid < 16) { kfBase[s * 16 + tid] = 0; kfCnt[s * 16 + tid] = 0; if (kcBase) { kcBase[s * 16 + tid] = 0; kcCnt[s * 16 + tid] = 0; } }
   if (tid == 0) scanFlag[s] = 0;  // the wide kernel sets it when it sends the scan on to the grid-based kernels
+  if constexpr (sizeof...(G) > 0) if (tid < 16) (gate.cnt, ...)[s * 16 + tid] = 0;
   if (nch > MAXCHUNK) { if (tid == 0) atomicOr(&ctr->err, ERR_CHUNKS); return; }
   if (tid < NW * 17) (&S.cnt[0][0])[tid] = 0;
   if (tid == 0) { S.nextRing = 0; S.defer = 0; }
@@ -450,114 +452,7 @@ __global__ void __launch_bounds__(NW * 32, NW == NW_RR ? 12 : 1) k_ring_runs(
   __syncthreads();  // the block's global writes are visible to all its threads from here on
   // ---- phase B: a warp per ring, rings handed out dynamically ----
   if (tid < 17) ringBaseOut[s * 17 + tid] = S.ringBase[tid];  // for the wide kernel, should a ring of this scan need it
-  rr_scan_rings<RW, NW>(S, s, RP, nRings, P, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfRuns, ovfRunsCount);
-}
-
-// k_ring_runs, also counting the clusters on the diameter gate's boundary (kind 6).  A copy, not a shared body: with the
-// body moved into a device function the compiler allocates k_ring_runs' registers differently.
-// First kernel: one block per scan, every scan.  A ring of more than RW runs is handed to the second kernel (the
-// ring segments and their offsets stay in global memory, so nothing is bucketed twice); a scan with more ring
-// entries than its scratch slot goes straight to the grid-based kernels.
-template <int NW>
-__global__ void __launch_bounds__(NW * 32, NW == NW_RR ? 12 : 1) k_ring_runs_bnd(
-    const float4* __restrict__ crop, const unsigned* __restrict__ cropMeta, const int* __restrict__ cropCnt,
-    const long long* __restrict__ scan_off, const int* __restrict__ chunk_off, DevParams P, int single_ring,
-    float4* ringPts, int* __restrict__ ringBaseOut, float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
-    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
-    DevCounters* __restrict__ ctr, int* __restrict__ ovfRuns, int* __restrict__ ovfRunsCount, int* __restrict__ scanFlag,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount, GateCount gate) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  RingRunsSmT<RW, NW>& S = *reinterpret_cast<RingRunsSmT<RW, NW>*>(smem_raw);
-  const int s = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  const long long base = scan_off[s];
-  const int nScan = (int)(scan_off[s + 1] - base);
-  const int nch = chunk_off[s + 1] - chunk_off[s];
-  if (tid < 16) { kfBase[s * 16 + tid] = 0; kfCnt[s * 16 + tid] = 0; if (kcBase) { kcBase[s * 16 + tid] = 0; kcCnt[s * 16 + tid] = 0; } }
-  if (tid == 0) scanFlag[s] = 0;  // the wide kernel sets it when it sends the scan on to the grid-based kernels
-  if (tid < 16) gate.cnt[s * 16 + tid] = 0;
-  if (nch > MAXCHUNK) { if (tid == 0) atomicOr(&ctr->err, ERR_CHUNKS); return; }
-  if (tid < NW * 17) (&S.cnt[0][0])[tid] = 0;
-  if (tid == 0) { S.nextRing = 0; S.defer = 0; }
-  const int Nc = chunk_prefix<NW * 32>(cropCnt + chunk_off[s], nch, S.pre, S.sc);  // ends with a barrier
-  if (Nc == 0) return;
-  const int nRings = single_ring ? 1 : 16;
-  // ---- phase A: stable bucketing of the crop survivors by ring ----
-  // every warp owns a contiguous range of the survivors; (1) per-warp counts, (2) offsets, (3) scatter
-  const int lo = (int)((long long)Nc * w / NW), hi = (int)((long long)Nc * (w + 1) / NW);
-  int* mycnt = S.cnt[w];
-  for (int i0 = lo; i0 < hi; i0 += 32) {
-    const int i = i0 + lane;
-    unsigned m = 0;
-    if (i < hi) m = ring_mask_of(cropMeta[piece_pos(S.pre, nch, i, base)] & 63u, single_ring);
-    const int first = m ? __ffs(m) - 1 : 16;
-    const unsigned peers = __match_any_sync(FE_FULL, first);
-    if (i < hi && lane == __ffs(peers) - 1) mycnt[first] += __popc(peers);
-    __syncwarp();
-    unsigned dual = __ballot_sync(FE_FULL, __popc(m) > 1);  // on a window's end value: also in the next ring (rare)
-    while (dual) {
-      const int src = __ffs(dual) - 1;
-      dual &= dual - 1;
-      const int f2 = __shfl_sync(FE_FULL, first, src) + 1;
-      if (lane == 0) mycnt[f2] += 1;
-      __syncwarp();
-    }
-  }
-  __syncthreads();
-  if (tid < 16) {
-    // S.cnt[w][h] becomes the first slot of warp w's entries of ring h inside the ring's segment
-    int run = 0;
-    for (int ww = 0; ww < NW; ww++) { const int c = S.cnt[ww][tid]; S.cnt[ww][tid] = run; run += c; }
-    S.ringBase[tid + 1] = run;  // totals for now
-  }
-  __syncthreads();
-  if (tid == 0) {
-    int run = 0;
-    S.ringBase[0] = 0;
-    for (int h = 0; h < 16; h++) { const int c = S.ringBase[h + 1]; S.ringBase[h + 1] = run + c; run += c; }
-    if (run > nScan) {  // more ring entries than the scan's slot holds (end-value points count twice): grid path
-      S.defer = 1;
-      ovfList[atomicAdd(ovfCount, 1)] = s;
-    }
-  }
-  __syncthreads();
-  if (S.defer) return;
-  float4* RP = ringPts + base;
-  for (int i0 = lo; i0 < hi; i0 += 32) {
-    const int i = i0 + lane;
-    unsigned m = 0;
-    float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (i < hi) {
-      const long long pp = piece_pos(S.pre, nch, i, base);
-      m = ring_mask_of(cropMeta[pp] & 63u, single_ring);
-      if (m) q = crop[pp];
-    }
-    const int first = m ? __ffs(m) - 1 : 16;
-    const unsigned anyDual = __ballot_sync(FE_FULL, __popc(m) > 1);
-    if (!anyDual) {
-      const unsigned peers = __match_any_sync(FE_FULL, first);
-      const int leader = __ffs(peers) - 1;
-      int old = 0;
-      if (lane == leader) { old = mycnt[first]; mycnt[first] = old + __popc(peers); }
-      old = __shfl_sync(FE_FULL, old, leader);
-      if (m) RP[S.ringBase[first] + old + __popc(peers & lanemask_lt())] = q;
-      __syncwarp();
-    } else {  // a point of this window belongs to two rings: ring by ring, so that every ring keeps the original order
-      for (int h = 0; h < nRings; h++) {
-        const bool in = (m >> h) & 1u;
-        const unsigned bm = __ballot_sync(FE_FULL, in);
-        if (!bm) continue;
-        const int old = mycnt[h];
-        if (in) RP[S.ringBase[h] + old + __popc(bm & lanemask_lt())] = q;
-        __syncwarp();
-        if (lane == 0) mycnt[h] = old + __popc(bm);
-        __syncwarp();
-      }
-    }
-  }
-  __syncthreads();  // the block's global writes are visible to all its threads from here on
-  // ---- phase B: a warp per ring, rings handed out dynamically ----
-  if (tid < 17) ringBaseOut[s * 17 + tid] = S.ringBase[tid];  // for the wide kernel, should a ring of this scan need it
-  rr_scan_rings<RW, NW>(S, s, RP, nRings, P, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfRuns, ovfRunsCount, gate);
+  rr_scan_rings<RW, NW>(S, s, RP, nRings, P, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ovfRuns, ovfRunsCount, gate...);
 }
 
 // Second kernel: the rings the first one listed (hundreds of poles in one ring), a warp per ring with RW2 runs;
@@ -584,25 +479,15 @@ __device__ __forceinline__ void ring_runs_wide_blocks(
   }
 }
 
+template <class... G>
 __global__ void __launch_bounds__(NT_RR) k_ring_runs_wide(
     const long long* __restrict__ scan_off, DevParams P, const float4* ringPts, const int* __restrict__ ringBaseIn,
     float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
     float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
     DevCounters* __restrict__ ctr, const int* __restrict__ ringList, const int* __restrict__ nList, int* __restrict__ scanFlag,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount) {
+    int* __restrict__ ovfList, int* __restrict__ ovfCount, G... gate) {
   ring_runs_wide_blocks(scan_off, P, ringPts, ringBaseIn, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ringList, nList,
-                        scanFlag, ovfList, ovfCount);
-}
-
-// the same, also counting the clusters on the diameter gate's boundary (kind 6)
-__global__ void __launch_bounds__(NT_RR) k_ring_runs_wide_bnd(
-    const long long* __restrict__ scan_off, DevParams P, const float4* ringPts, const int* __restrict__ ringBaseIn,
-    float4* __restrict__ kfPool, int kfCap, int* __restrict__ kfBase, int* __restrict__ kfCnt,
-    float4* __restrict__ kcPool, int kcCap, int* __restrict__ kcBase, int* __restrict__ kcCnt,
-    DevCounters* __restrict__ ctr, const int* __restrict__ ringList, const int* __restrict__ nList, int* __restrict__ scanFlag,
-    int* __restrict__ ovfList, int* __restrict__ ovfCount, GateCount gate) {
-  ring_runs_wide_blocks(scan_off, P, ringPts, ringBaseIn, kfPool, kfCap, kfBase, kfCnt, kcPool, kcCap, kcBase, kcCnt, ctr, ringList, nList,
-                        scanFlag, ovfList, ovfCount, gate);
+                        scanFlag, ovfList, ovfCount, gate...);
 }
 
 }  // namespace fe
