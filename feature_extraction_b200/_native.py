@@ -28,6 +28,7 @@ EXPORTS = [
     "fe_enable_boundary_report_all", "fe_get_boundary_report_all",
     "fe_multi_enable_cloud_outputs", "fe_multi_get_cloud_outputs",
     "fe_match_descriptors", "fe_match_descriptors_device",
+    "fe_register_params_default", "fe_register_matches", "fe_register_matches_device", "fe_match_device_best",
 ]
 
 
@@ -83,6 +84,32 @@ class MatchResult(C.Structure):
         ("shift", C.POINTER(C.c_int32)),
         ("dist2", C.POINTER(C.c_float)),
         ("second_dist2", C.POINTER(C.c_float)),
+    ]
+
+
+class RegisterParams(C.Structure):
+    """fe_register_params_t: inlier radius and minimum separation (m), hypothesis cap, inliers for status 2, refinement
+    rounds."""
+    _fields_ = [
+        ("inlier_radius", C.c_double),
+        ("min_separation", C.c_double),
+        ("max_hypotheses", C.c_int32),
+        ("min_inliers", C.c_int32),
+        ("refine_iterations", C.c_int32),
+    ]
+
+
+class RegisterResult(C.Structure):
+    """fe_register_result_t: per group the motion {c, s, tx, ty}, rms, counts and status; per query row its inlier."""
+    _fields_ = [
+        ("n_groups", C.c_int32),
+        ("n_queries", C.c_int64),
+        ("pose", C.POINTER(C.c_double)),
+        ("rms", C.POINTER(C.c_double)),
+        ("n_inliers", C.POINTER(C.c_int32)),
+        ("n_hypotheses", C.POINTER(C.c_int32)),
+        ("status", C.POINTER(C.c_int32)),
+        ("assoc", C.POINTER(C.c_int64)),
     ]
 
 
@@ -156,6 +183,12 @@ def lib():
         for f in (L.fe_match_descriptors, L.fe_match_descriptors_device):
             f.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32,
                           C.POINTER(MatchResult)]
+        L.fe_register_params_default.argtypes = [C.POINTER(RegisterParams)]
+        L.fe_register_params_default.restype = None
+        for f in (L.fe_register_matches, L.fe_register_matches_device):
+            f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                          C.POINTER(RegisterParams), C.POINTER(RegisterResult)]
+        L.fe_match_device_best.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
         L.fe_debug_enable_graphs.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int64)]
         L.fe_debug_lean_reruns.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         L.fe_debug_density_work.argtypes = [C.c_void_p, C.c_void_p]

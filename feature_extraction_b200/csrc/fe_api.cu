@@ -13,6 +13,7 @@
 
 #include "fe_kernels.cuh"
 #include "fe_match.h"
+#include "fe_register.h"
 
 using namespace fe;
 
@@ -166,6 +167,15 @@ struct fe_ctx {
   long long* h_matchRes = nullptr;      // pinned, MATCH_RES_WORDS long longs per query
   int64_t capMatchRes = 0, capMatchResHost = 0;  // queries
   bool matchAttrs = false;
+  // fe_register_matches*: buffers of their own, so that a register call leaves the batch and match results alone
+  fe_point_t *d_regQ = nullptr, *d_regR = nullptr;  // uploaded keypoints of the host variant
+  int64_t capRegQ = 0, capRegR = 0;
+  long long* d_regBest = nullptr;                   // uploaded `best` of the host variant
+  int64_t capRegBest = 0;
+  int64_t* h_regOffs = nullptr;                     // pinned: query then reference offsets
+  int64_t *d_regOffs = nullptr, capRegOffsHost = 0, capRegOffs = 0;
+  unsigned char *d_regScratch = nullptr, *d_regRes = nullptr, *h_regRes = nullptr;  // results: reg_layout()
+  int64_t capRegScratch = 0, capRegRes = 0, capRegResHost = 0;  // bytes
   std::string err;
 };
 
@@ -1186,10 +1196,11 @@ void fe_destroy(fe_ctx_t* ctx) {
   if (ctx->h_desc) cudaFreeHost(ctx->h_desc);
   if (ctx->h_cloud) cudaFreeHost(ctx->h_cloud);
   if (ctx->h_kc) cudaFreeHost(ctx->h_kc);
-  void* dm[] = {ctx->d_matchQ, ctx->d_matchR, ctx->d_items, ctx->d_part, ctx->d_matchRes};
+  void* dm[] = {ctx->d_matchQ, ctx->d_matchR, ctx->d_items, ctx->d_part, ctx->d_matchRes,
+                ctx->d_regQ, ctx->d_regR, ctx->d_regBest, ctx->d_regOffs, ctx->d_regScratch, ctx->d_regRes};
   for (void* p : dm) if (p) cudaFree(p);
-  if (ctx->h_items) cudaFreeHost(ctx->h_items);
-  if (ctx->h_matchRes) cudaFreeHost(ctx->h_matchRes);
+  void* hm[] = {ctx->h_items, ctx->h_matchRes, ctx->h_regOffs, ctx->h_regRes};
+  for (void* p : hm) if (p) cudaFreeHost(p);
   delete ctx;
 }
 
@@ -1639,6 +1650,171 @@ int fe_match_descriptors_device(fe_ctx_t* ctx, const float* query, int64_t query
                                 const float* ref, int64_t ref_stride, const int64_t* ref_offsets, int32_t n_groups,
                                 fe_match_result_t* out) {
   return match_descriptors(ctx, query, query_stride, query_offsets, ref, ref_stride, ref_offsets, n_groups, out, true);
+}
+
+int fe_match_device_best(fe_ctx_t* ctx, const int64_t** best) {
+  if (!ctx || !best) return FE_ERR_INVALID;
+  if (!ctx->d_matchRes) return fail(ctx, FE_ERR_INVALID, "no match call has run on this context");
+  *best = (const int64_t*)ctx->d_matchRes;  // the first n_queries words of the match results (MATCH_RES_WORDS)
+  return FE_OK;
+}
+
+void fe_register_params_default(fe_register_params_t* p) {
+  if (!p) return;
+  p->inlier_radius = 0.5;
+  p->min_separation = 1.0;
+  p->max_hypotheses = 512;
+  p->min_inliers = 16;
+  p->refine_iterations = 4;
+}
+
+}  // extern "C"
+
+// ---- registration (fe_register.cu) -----------------------------------------------------------------------
+
+namespace {
+
+// The results of a register call in h_regRes / d_regRes, one copy: pose (G x 4) | rms (G) | assoc (nQ) as 8-byte words,
+// then n_inliers | n_hypotheses | status (G each) | the device's error flag as 4-byte words.
+struct RegLayout {
+  int64_t pose, rms, assoc, nInl, nHyp, status, err, bytes;
+};
+RegLayout reg_layout(int64_t G, int64_t nQ) {
+  RegLayout L;
+  L.pose = 0;
+  L.rms = L.pose + 32 * G;
+  L.assoc = L.rms + 8 * G;
+  L.nInl = L.assoc + 8 * nQ;
+  L.nHyp = L.nInl + 4 * G;
+  L.status = L.nHyp + 4 * G;
+  L.err = L.status + 4 * G;
+  L.bytes = L.err + 4;
+  return L;
+}
+
+// both entry points: keypoints and `best` are device memory (onDevice) or host memory to upload
+int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, const int64_t* best, const int64_t* qo,
+                     const int64_t* ro, int32_t G, const fe_register_params_t* prm, fe_register_result_t* out,
+                     bool onDevice) {
+  if (!ctx || !out) return FE_ERR_INVALID;
+  ctx->err.clear();
+  if (!prm) return fail(ctx, FE_ERR_INVALID, "params is NULL");
+  const fe_register_params_t p = *prm;
+  if (!(std::isfinite(p.inlier_radius) && p.inlier_radius > 0.0))
+    return fail(ctx, FE_ERR_INVALID, "inlier_radius must be finite and > 0");
+  if (!(std::isfinite(p.min_separation) && p.min_separation > 0.0))
+    return fail(ctx, FE_ERR_INVALID, "min_separation must be finite and > 0");
+  if (p.max_hypotheses < 1 || p.max_hypotheses > 65536) return fail(ctx, FE_ERR_INVALID, "max_hypotheses must be in [1, 65536]");
+  if (p.min_inliers < 1) return fail(ctx, FE_ERR_INVALID, "min_inliers must be >= 1");
+  if (p.refine_iterations < 0 || p.refine_iterations > 1000)
+    return fail(ctx, FE_ERR_INVALID, "refine_iterations must be in [0, 1000]");
+  if (G < 0) return fail(ctx, FE_ERR_INVALID, "n_groups must not be negative");
+  if (!qo || !ro) return fail(ctx, FE_ERR_INVALID, "query_offsets and ref_offsets need n_groups + 1 entries");
+  if (const char* e = check_offsets(qo, G)) return fail(ctx, FE_ERR_INVALID, std::string("query_offsets: ") + e);
+  if (const char* e = check_offsets(ro, G)) return fail(ctx, FE_ERR_INVALID, std::string("ref_offsets: ") + e);
+  for (int32_t g = 0; g < G; g++)  // so that h * P of the hypothesis map fits 64 bits (P < 2^47, h < 2^16)
+    if (qo[g + 1] - qo[g] >= (1LL << 24)) return fail(ctx, FE_ERR_INVALID, "a group has 2^24 or more query rows");
+  const int64_t nQ = qo[G] - qo[0], nR = ro[G] - ro[0];
+  if (nQ > 0 && (!q || !best)) return fail(ctx, FE_ERR_INVALID, "query_kp or best is NULL but there are query rows");
+  if (nR > 0 && !r) return fail(ctx, FE_ERR_INVALID, "ref_kp is NULL but there are reference rows");
+  if (nQ >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 query rows");
+  if (!onDevice)
+    for (int32_t g = 0; g < G; g++)
+      for (int64_t k = qo[g]; k < qo[g + 1]; k++) {
+        const int64_t b = best[k - qo[0]];
+        if (b != -1 && (b < ro[g] || b >= ro[g + 1]))
+          return fail(ctx, FE_ERR_INVALID, "best[" + std::to_string(k - qo[0]) + "] is neither -1 nor a reference row of its group");
+      }
+  CK(cudaSetDevice(ctx->device));
+  int st = ensure_slot(ctx, ctx->slot[0], false);  // for its stream only: the slot's buffers are not touched
+  if (st) return st;
+  cudaStream_t stream = ctx->slot[0].stream;
+
+  const RegLayout L = reg_layout(G, nQ);
+  st = grow_pinned(ctx, &ctx->h_regRes, &ctx->capRegResHost, L.bytes, 4096, 0);
+  if (st) return st;
+  unsigned char* h = ctx->h_regRes;
+  out->n_groups = G;
+  out->n_queries = nQ;
+  out->pose = (const double*)(h + L.pose);
+  out->rms = (const double*)(h + L.rms);
+  out->assoc = (const int64_t*)(h + L.assoc);
+  out->n_inliers = (const int32_t*)(h + L.nInl);
+  out->n_hypotheses = (const int32_t*)(h + L.nHyp);
+  out->status = (const int32_t*)(h + L.status);
+  if (G == 0) return FE_OK;
+
+  st = grow_pinned(ctx, &ctx->h_regOffs, &ctx->capRegOffsHost, 2 * (int64_t)(G + 1), 4096, 0);
+  if (st) return st;
+  memcpy(ctx->h_regOffs, qo, (size_t)(G + 1) * sizeof(int64_t));
+  memcpy(ctx->h_regOffs + G + 1, ro, (size_t)(G + 1) * sizeof(int64_t));
+  int64_t qBias = 0, rBias = 0;
+  if (!onDevice) {  // rows [qo[0], qo[G]) and [ro[0], ro[G]) only
+    if ((st = grow_device(ctx, &ctx->d_regQ, &ctx->capRegQ, std::max<int64_t>(nQ, 1)))) return st;
+    if ((st = grow_device(ctx, &ctx->d_regR, &ctx->capRegR, std::max<int64_t>(nR, 1)))) return st;
+    if ((st = grow_device(ctx, &ctx->d_regBest, &ctx->capRegBest, std::max<int64_t>(nQ, 1)))) return st;
+    if (nQ > 0) {
+      CK(cudaMemcpyAsync(ctx->d_regQ, q + qo[0], (size_t)nQ * sizeof(fe_point_t), cudaMemcpyHostToDevice, stream));
+      CK(cudaMemcpyAsync(ctx->d_regBest, best, (size_t)nQ * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
+    }
+    if (nR > 0) CK(cudaMemcpyAsync(ctx->d_regR, r + ro[0], (size_t)nR * sizeof(fe_point_t), cudaMemcpyHostToDevice, stream));
+    q = ctx->d_regQ;
+    r = ctx->d_regR;
+    best = (const int64_t*)ctx->d_regBest;
+    qBias = qo[0];
+    rBias = ro[0];
+  }
+  const int64_t scratchBytes = std::max<int64_t>(nQ, 1) * (4 + 8 + 8 + 8);
+  if ((st = grow_device(ctx, &ctx->d_regOffs, &ctx->capRegOffs, 2 * (int64_t)(G + 1)))) return st;
+  if ((st = grow_device(ctx, &ctx->d_regScratch, &ctx->capRegScratch, scratchBytes))) return st;
+  if ((st = grow_device(ctx, &ctx->d_regRes, &ctx->capRegRes, L.bytes))) return st;
+  CK(cudaMemcpyAsync(ctx->d_regOffs, ctx->h_regOffs, (size_t)(2 * (G + 1)) * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
+  unsigned char* d = ctx->d_regRes;
+  CK(cudaMemsetAsync(d + L.err, 0, 4, stream));
+  fe_register::Out o;
+  o.pose = (double*)(d + L.pose);
+  o.rms = (double*)(d + L.rms);
+  o.assoc = (long long*)(d + L.assoc);
+  o.nInl = (int*)(d + L.nInl);
+  o.nHyp = (int*)(d + L.nHyp);
+  o.status = (int*)(d + L.status);
+  o.err = (int*)(d + L.err);
+  const int64_t n1 = std::max<int64_t>(nQ, 1);
+  fe_register::Scratch sc;  // 8-byte arrays first
+  sc.assocNew = (long long*)ctx->d_regScratch;
+  sc.d2Cur = (double*)(sc.assocNew + n1);
+  sc.d2New = sc.d2Cur + n1;
+  sc.corr = (int*)(sc.d2New + n1);
+  fe_register::Params kp;
+  kp.r2 = p.inlier_radius * p.inlier_radius;
+  kp.sep2 = p.min_separation * p.min_separation;
+  kp.twoR = 2.0 * p.inlier_radius;
+  kp.maxH = p.max_hypotheses;
+  kp.minInliers = p.min_inliers;
+  kp.refine = p.refine_iterations;
+  CK(fe_register::launch(q, qBias, r, rBias, (const long long*)best, ctx->d_regOffs, ctx->d_regOffs + G + 1, G, kp, o, sc,
+                         stream));
+  ctx->launches += 1;
+  CK(cudaMemcpyAsync(h, d, (size_t)L.bytes, cudaMemcpyDeviceToHost, stream));
+  CK(cudaStreamSynchronize(stream));
+  if (*(const int32_t*)(h + L.err)) return fail(ctx, FE_ERR_INVALID, "an entry of best is neither -1 nor a reference row of its group");
+  return FE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fe_register_matches(fe_ctx_t* ctx, const fe_point_t* query_kp, const fe_point_t* ref_kp, const int64_t* best,
+                        const int64_t* query_offsets, const int64_t* ref_offsets, int32_t n_groups,
+                        const fe_register_params_t* params, fe_register_result_t* out) {
+  return register_matches(ctx, query_kp, ref_kp, best, query_offsets, ref_offsets, n_groups, params, out, false);
+}
+
+int fe_register_matches_device(fe_ctx_t* ctx, const fe_point_t* query_kp, const fe_point_t* ref_kp, const int64_t* best,
+                               const int64_t* query_offsets, const int64_t* ref_offsets, int32_t n_groups,
+                               const fe_register_params_t* params, fe_register_result_t* out) {
+  return register_matches(ctx, query_kp, ref_kp, best, query_offsets, ref_offsets, n_groups, params, out, true);
 }
 
 // ---- one entry point per reference function ----------------------------------------------------------

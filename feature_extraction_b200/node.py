@@ -97,6 +97,36 @@ def _unpack_match(res):
             np.ctypeslib.as_array(res.dist2, shape=(n,)).copy(), np.ctypeslib.as_array(res.second_dist2, shape=(n,)).copy())
 
 
+def register_params_default(**overrides):
+    """fe_register_params_default, with any field overridden by keyword."""
+    p = N.RegisterParams()
+    N.lib().fe_register_params_default(C.byref(p))
+    for k, v in overrides.items():
+        if not hasattr(p, k):
+            raise ValueError("fe_register_params_t has no field %r" % k)
+        setattr(p, k, v)
+    return p
+
+
+def _keypoint_rows(a):
+    a = np.ascontiguousarray(a, np.float32)
+    if a.ndim != 2 or a.shape[1] != 4:
+        raise ValueError("keypoints must be (K, 4) float32 {x, y, z, elevation}, got %s" % (a.shape,))
+    return a
+
+
+def _unpack_register(res):
+    G, n = int(res.n_groups), int(res.n_queries)
+
+    def arr(p, shape, dtype):
+        if int(np.prod(shape)) == 0:
+            return np.zeros(shape, dtype)
+        return np.ctypeslib.as_array(p, shape=shape).copy()
+    return {"pose": arr(res.pose, (G, 4), np.float64), "rms": arr(res.rms, (G,), np.float64),
+            "n_inliers": arr(res.n_inliers, (G,), np.int32), "n_hypotheses": arr(res.n_hypotheses, (G,), np.int32),
+            "status": arr(res.status, (G,), np.int32), "assoc": arr(res.assoc, (n,), np.int64)}
+
+
 class PinnedBuffer:
     """Page-locked host memory from fe_host_alloc, exposed as a numpy array."""
 
@@ -333,6 +363,54 @@ class FeatureExtractionNode:
         self._check(N.lib().fe_match_descriptors_device(self._ctx, C.c_void_p(q_ptr), int(q_stride), _ptr(qo), C.c_void_p(r_ptr),
                                                         int(r_stride), _ptr(ro), G, C.byref(res)))
         return _unpack_match(res)
+
+    def matchDeviceBest(self):
+        """fe_match_device_best: device address of the last match call's `best` (int64 per query row), for
+        registerMatchesDevice."""
+        p = C.c_void_p()
+        self._check(N.lib().fe_match_device_best(self._ctx, C.byref(p)))
+        return p.value
+
+    def registerMatches(self, query_kp, ref_kp, best, query_offsets, ref_offsets, params=None):
+        """fe_register_matches: the planar motion of every group from its matched keypoints (include/fe_b200.h,
+        "registration").  Keypoints are (K, 4) host arrays addressed by absolute row; `best` as matchDescriptors returns
+        it for the same offsets.  -> dict of pose (G, 4) float64 {c, s, tx, ty} mapping query xy into the reference
+        frame, rms (G,), n_inliers, n_hypotheses, status (G,) int32 (0 no hypothesis, 1 too few inliers, 2 registered),
+        assoc (n,) int64 (the reference row each query row is an inlier of, -1 = none)."""
+        q = _keypoint_rows(query_kp)
+        r = _keypoint_rows(ref_kp)
+        b = np.ascontiguousarray(best, np.int64).reshape(-1)
+        qo, ro, G = _match_offsets(query_offsets, ref_offsets, len(q), len(r))
+        if len(b) != qo[-1] - qo[0]:
+            raise ValueError("best needs one entry per query row: %d, got %d" % (qo[-1] - qo[0], len(b)))
+        prm = params if params is not None else register_params_default()
+        res = N.RegisterResult()
+        self._check(N.lib().fe_register_matches(self._ctx, _ptr(q) if len(q) else None, _ptr(r) if len(r) else None,
+                                                _ptr(b) if len(b) else None, _ptr(qo), _ptr(ro), G, C.byref(prm),
+                                                C.byref(res)))
+        return _unpack_register(res)
+
+    def registerMatchesDevice(self, q_ptr, r_ptr, best_ptr, q_offsets, r_offsets, params=None):
+        """fe_register_matches_device: keypoints (e.g. processBatchDevice's) and `best` (matchDeviceBest()) already in
+        HBM, queued on the context's stream behind the batch and match calls.  Same results as registerMatches."""
+        qo, ro, G = _match_offsets(q_offsets, r_offsets, None, None)  # the device buffers' sizes are the caller's business
+        if (qo[-1] > qo[0] and not (q_ptr and best_ptr)) or (ro[-1] > ro[0] and not r_ptr):
+            raise ValueError("a device pointer is NULL while its side has rows")
+        prm = params if params is not None else register_params_default()
+        res = N.RegisterResult()
+        self._check(N.lib().fe_register_matches_device(self._ctx, C.c_void_p(q_ptr), C.c_void_p(r_ptr), C.c_void_p(best_ptr),
+                                                       _ptr(qo), _ptr(ro), G, C.byref(prm), C.byref(res)))
+        return _unpack_register(res)
+
+    def scan_to_scan(self, ko, kp, descriptors, params=None):
+        """Scan s against scan s - 1 of one batch result (processBatch's keypoint_offsets, keypoints, descriptors):
+        match, then register.  -> registerMatches' dict for the B - 1 groups plus `best`; pose[s - 1] maps scan s's
+        levelled xy into scan s - 1's."""
+        ko = np.ascontiguousarray(ko, np.int64)
+        best = self.matchDescriptors(descriptors, descriptors, ko[1:], ko[:-1])[0]
+        out = self.registerMatches(kp, kp, best, ko[1:], ko[:-1], params)
+        out["best"] = best
+        return out
 
     def download(self, device_ptr, shape, dtype=np.float32):
         """Copy a device-resident result of processBatchDevice to a new host array."""

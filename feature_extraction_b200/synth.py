@@ -53,3 +53,25 @@ def generate(config, n_scans, scan_index_base=0, azimuth_steps=0, n_threads=0, o
     if st != 0:
         raise RuntimeError("fes_generate: capacity too small")
     return out[: offs[-1]], offs, rp[:n_scans]
+
+
+def generate_poses(config, scene_index, poses, azimuth_steps=0, n_threads=0):
+    """One scene seen from several sensor poses: the scene of generate()'s scan `scene_index`, rendered from each
+    poses[s] = (x, y, yaw) of the scene frame (metres, radians).  Scan 0 at pose (0, 0, 0) is generate()'s scan
+    `scene_index` byte for byte; scans s >= 1 draw roll, pitch and noise from a stream of their own.
+    -> points (N,4) float32, scan_offsets (n_scans+1,) int64, roll_pitch (n_scans,2) float64."""
+    poses = np.ascontiguousarray(poses, np.float64).reshape(-1, 3)
+    n_scans = len(poses)
+    A = azimuth_steps or default_azimuth_steps(config)
+    cap = 16 * A * n_scans
+    out = np.empty((max(cap, 1), 4), np.float32)
+    offs = np.zeros(n_scans + 1, np.int64)
+    rp = np.zeros((max(n_scans, 1), 2), np.float64)
+    if n_threads <= 0:
+        n_threads = len(os.sched_getaffinity(0))
+    st = _lib().fes_generate_poses(C.c_int(config), C.c_int64(scene_index), C.c_int(n_scans), C.c_int(A),
+                                   C.c_int(n_threads), poses.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p),
+                                   C.c_int64(cap), offs.ctypes.data_as(C.c_void_p), rp.ctypes.data_as(C.c_void_p))
+    if st != 0:
+        raise RuntimeError("fes_generate_poses: capacity too small")
+    return out[: offs[-1]], offs, rp[:n_scans]

@@ -128,10 +128,34 @@ inline void add_cols(std::vector<std::vector<int> >& cols, int A, double az_c, d
   for (int a = a0; a <= a1; a++) cols[((a % A) + A) % A].push_back(id);
 }
 
-int64_t generate_scan(int config, uint64_t scan_index, int A, fe_point_t* out, double* roll_pitch) {
-  Rng g((uint64_t)config * 0x100000001B3ull + scan_index * 0x9E3779B97F4A7C15ull + 12345u);
-  Scene sc;
-  build_scene(config, g, sc);
+uint64_t scene_seed(int config, uint64_t scan_index) {
+  return (uint64_t)config * 0x100000001B3ull + scan_index * 0x9E3779B97F4A7C15ull + 12345u;
+}
+
+// The scene `sc` as the sensor at pose = (x, y, yaw) of the scene frame sees it: every object moved by
+// R(-yaw) * (world - (x, y)).  The ground plane does not move.  At the identity pose every coordinate comes out
+// bit for bit as it went in (x*1 + y*0 == x).
+Scene posed(const Scene& sc, const double* pose) {
+  const double c = cos(pose[2]), s = sin(pose[2]);
+  auto move = [&](double& x, double& y) {
+    const double dx = x - pose[0], dy = y - pose[1];
+    x = c * dx + s * dy;
+    y = -s * dx + c * dy;
+  };
+  Scene o = sc;
+  for (Cyl& k : o.cyl) move(k.x, k.y);
+  for (Sph& k : o.sph) move(k.x, k.y);
+  for (Box& k : o.box) {
+    move(k.cx, k.cy);
+    const double yc = k.yaw_c * c + k.yaw_s * s, ys = k.yaw_s * c - k.yaw_c * s;  // yaw - pose yaw
+    k.yaw_c = yc;
+    k.yaw_s = ys;
+  }
+  return o;
+}
+
+// Renders the scene `sc`, given in the sensor's levelled frame: roll, pitch, range noise and dropout are drawn from g.
+int64_t render_scan(int config, const Scene& sc, Rng& g, int A, fe_point_t* out, double* roll_pitch) {
   double roll, pitch;
   if (config == 1) { roll = 0.02; pitch = -0.015; }
   else { roll = g.uni(-0.05, 0.05); pitch = g.uni(-0.05, 0.05); }
@@ -237,19 +261,18 @@ int64_t generate_scan(int config, uint64_t scan_index, int A, fe_point_t* out, d
   return n;
 }
 
-}  // namespace
+int64_t generate_scan(int config, uint64_t scan_index, int A, fe_point_t* out, double* roll_pitch) {
+  Rng g(scene_seed(config, scan_index));
+  Scene sc;
+  build_scene(config, g, sc);
+  return render_scan(config, sc, g, A, out, roll_pitch);
+}
 
-extern "C" {
-
-int fes_default_azimuth_steps(int config) { return config == 3 ? 7200 : 1800; }
-
-// Generates scans [scan_index_base, scan_index_base + n_scans) of `config` (1..5, BASELINE.json
-// configs) into `out` (capacity cap_points; 16*A*n_scans always suffices), CSR offsets into
-// scan_offsets[n_scans+1], roll/pitch into roll_pitch[2*n_scans].  Returns 0, or 3 if cap_points
-// is too small.
-int fes_generate(int config, int64_t scan_index_base, int n_scans, int azimuth_steps, int n_threads,
-                 fe_point_t* out, int64_t cap_points, int64_t* scan_offsets, double* roll_pitch) {
-  const int A = azimuth_steps > 0 ? azimuth_steps : fes_default_azimuth_steps(config);
+// Runs scan(i, out_slot, roll_pitch + 2i) for i in [0, n_scans) on n_threads threads and packs the scans into `out`
+// in order.  Returns 0, or 3 if cap_points is too small.
+template <class F>
+int generate_scans(int n_scans, int A, int n_threads, fe_point_t* out, int64_t cap_points, int64_t* scan_offsets,
+                   double* roll_pitch, const F& scan) {
   const int64_t slot = 16LL * A;
   if (n_threads < 1) n_threads = 1;
   std::vector<int64_t> counts(n_scans, 0);
@@ -266,8 +289,7 @@ int fes_generate(int config, int64_t scan_index_base, int n_scans, int azimuth_s
       for (;;) {
         int i = next.fetch_add(1);
         if (i >= nb) break;
-        counts[b0 + i] = generate_scan(config == 5 ? 2 : config, (uint64_t)(scan_index_base + b0 + i), A,
-                                       tmp.data() + (size_t)i * slot, roll_pitch + 2 * (b0 + i));
+        counts[b0 + i] = scan(b0 + i, tmp.data() + (size_t)i * slot, roll_pitch + 2 * (b0 + i));
       }
     };
     if (n_threads == 1) worker();
@@ -285,6 +307,48 @@ int fes_generate(int config, int64_t scan_index_base, int n_scans, int azimuth_s
     }
   }
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fes_default_azimuth_steps(int config) { return config == 3 ? 7200 : 1800; }
+
+// Generates scans [scan_index_base, scan_index_base + n_scans) of `config` (1..5, BASELINE.json
+// configs) into `out` (capacity cap_points; 16*A*n_scans always suffices), CSR offsets into
+// scan_offsets[n_scans+1], roll/pitch into roll_pitch[2*n_scans].  Returns 0, or 3 if cap_points
+// is too small.
+int fes_generate(int config, int64_t scan_index_base, int n_scans, int azimuth_steps, int n_threads,
+                 fe_point_t* out, int64_t cap_points, int64_t* scan_offsets, double* roll_pitch) {
+  const int A = azimuth_steps > 0 ? azimuth_steps : fes_default_azimuth_steps(config);
+  const int cfg = config == 5 ? 2 : config;
+  return generate_scans(n_scans, A, n_threads, out, cap_points, scan_offsets, roll_pitch,
+                        [&](int i, fe_point_t* o, double* rp) {
+                          return generate_scan(cfg, (uint64_t)(scan_index_base + i), A, o, rp);
+                        });
+}
+
+// One scene seen from n_scans sensor poses: the scene of fes_generate's scan `scene_index` (same seed, same
+// build_scene), rendered from poses[3s .. 3s+2] = (x, y, yaw) of the scene frame, in metres and radians.  Scan 0 draws
+// roll, pitch and noise from the scene's generator where build_scene left it, exactly as fes_generate does, so scan 0
+// at pose (0, 0, 0) is fes_generate's scan `scene_index` byte for byte.  Scan s >= 1 draws them from a generator of its
+// own, seeded by (config, scene_index, s).  Outputs and return value as fes_generate.
+int fes_generate_poses(int config, int64_t scene_index, int n_scans, int azimuth_steps, int n_threads,
+                       const double* poses, fe_point_t* out, int64_t cap_points, int64_t* scan_offsets,
+                       double* roll_pitch) {
+  const int A = azimuth_steps > 0 ? azimuth_steps : fes_default_azimuth_steps(config);
+  const int cfg = config == 5 ? 2 : config;
+  const uint64_t seed = scene_seed(cfg, (uint64_t)scene_index);
+  Rng g0(seed);
+  Scene sc;
+  build_scene(cfg, g0, sc);
+  return generate_scans(n_scans, A, n_threads, out, cap_points, scan_offsets, roll_pitch,
+                        [&](int i, fe_point_t* o, double* rp) {
+                          Rng g = g0;
+                          if (i > 0) g = Rng(seed ^ ((uint64_t)i * 0xD1B54A32D192ED03ull));
+                          return render_scan(cfg, posed(sc, poses + 3 * i), g, A, o, rp);
+                        });
 }
 
 }  // extern "C"

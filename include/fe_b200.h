@@ -288,6 +288,101 @@ int fe_match_descriptors_device(fe_ctx_t* ctx, const float* query, int64_t query
                                 const float* ref, int64_t ref_stride, const int64_t* ref_offsets, int32_t n_groups,
                                 fe_match_result_t* out);
 
+/* ---- registration: the planar motion between two scans from their matched keypoints ----------------------------- */
+/* Levelling removes roll and pitch, so the motion between two scans is planar: a yaw and an xy translation (keypoint z
+ * is the mean height of the visible ring centroids and depends on range; it is not used).  Descriptor matches propose
+ * motions, two at a time; every query keypoint of the group votes on each, descriptor or not.  The motion is evaluated
+ * to the last bit as follows.
+ *
+ * Arithmetic.  IEEE double with + - * / sqrt only, each operation rounded on its own (no FMA), in the order written;
+ * |x| is exact.  Positions are the x, y floats of fe_point_t keypoints widened to double: p_k of query row k, r_j of
+ * reference row j.
+ *
+ * Inputs.  Query and reference keypoints addressed by absolute row index; best[i] for query row qo[0] + i, the
+ * absolute reference row of the group or -1 (fe_match_result_t.best as a match call returns it); query_offsets,
+ * ref_offsets and n_groups as in the match call that produced `best`.
+ *
+ * Correspondences of group g: its query rows k with best >= 0, numbered 0 .. n_c - 1 in ascending row order; q_a is the
+ * position of the reference row best of correspondence a.  Pairs (a, b), a < b, are numbered a*n_c - a*(a+1)/2 +
+ * (b - a - 1); there are P = n_c*(n_c-1)/2.  With H = min(P, max_hypotheses), hypothesis h in [0, H) is pair
+ * floor(h*P / H) (64-bit integers): every pair when P <= H, else H evenly spaced ones.  No random numbers.
+ *
+ * Motion of a hypothesis (a, b): u = p_b - p_a, v = q_b - q_a, lu = ux*ux + uy*uy, lv = vx*vx + vy*vy.  Rejected when
+ * lu < sep2 or lv < sep2 (sep2 = min_separation*min_separation) or |sqrt(lu) - sqrt(lv)| >= 2*inlier_radius (a rigid
+ * motion preserves distances).  Otherwise nn = sqrt(lu*lv), c = (ux*vx + uy*vy)/nn, s = (ux*vy - uy*vx)/nn,
+ * mp = (p_a + p_b)*0.5 and mq = (q_a + q_b)*0.5 per coordinate, tx = mqx - (c*mpx - s*mpy), ty = mqy - (s*mpx + c*mpy).
+ * A motion (c, s, tx, ty) maps a query position to w = ((c*px - s*py) + tx, (s*px + c*py) + ty), in the reference
+ * scan's levelled frame.
+ *
+ * Evaluation of a motion.  Every query row k of the group, best = -1 included, visits the group's reference rows j in
+ * ascending order with d = w - r_j, d2 = dx*dx + dy*dy, and takes j when d2 is below its current value, which starts at
+ * r2 = inlier_radius*inlier_radius.  A row that took one is an inlier: assoc_k = the last j taken, d2_k its d2 (so the
+ * nearest reference row, the lower row on ties, when it lies within the radius); otherwise assoc_k = -1.  Two query rows
+ * may share a reference row.  The score is the number of inliers.  The winning hypothesis has the highest score, then
+ * the lowest h.
+ *
+ * Refinement, at most refine_iterations rounds, from the winner's motion and evaluation.  A round stops the refinement
+ * when there are fewer than 2 inliers.  Otherwise, with the inliers (k, assoc_k) in ascending k and every sum formed
+ * sequentially in that order from 0.0, m their number: mp = (sum p_k) / m, mq = (sum r_assoc_k) / m per coordinate,
+ * A = sum((pkx - mpx)*(qx - mqx) + (pky - mpy)*(qy - mqy)), B = sum((pkx - mpx)*(qy - mqy) - (pky - mpy)*(qx - mqx))
+ * with q = r_assoc_k, n = sqrt(A*A + B*B).  It stops when n == 0; else the new motion is c = A/n, s = B/n and t as
+ * above, and it is evaluated.  A lower score stops the refinement with the old motion kept; otherwise the new motion
+ * and evaluation replace the old, and the refinement stops if no assoc_k changed.
+ *
+ * Outputs per group: pose = (c, s, tx, ty) of the final motion (yaw = atan2(s, c) is the caller's: no libm enters the
+ * contract); n_inliers = its score; n_hypotheses = the hypotheses not rejected; rms = sqrt(sum d2_k / n_inliers) over
+ * the final inliers in ascending k, 0 without inliers; status 0 when no hypothesis survived (pose = (1, 0, 0, 0),
+ * everything else 0, every assoc -1), 1 when n_inliers < min_inliers, 2 = registered.  Per query row: assoc under the
+ * final motion, the absolute reference row or -1.
+ *
+ * Cost: H*n_q*n_r distance tests per group (n_q, n_r its query and reference rows) plus n_q*n_r per refinement round,
+ * each about ten double operations; one warp scores a group, one hypothesis per lane.  A scan against a map of 10^5
+ * rows with 512 hypotheses is 10^9 tests on a single warp: split such a map into tiles near the scan.
+ *
+ * Results are context-owned pinned host memory, valid until the next register call; a register call leaves the results
+ * of the last batch and match calls alone.  FE_ERR_INVALID (the context stays usable) when an offsets array decreases
+ * or has a negative entry, n_groups < 0, a group has 2^24 or more query rows, a keypoint or `best` pointer is NULL
+ * while its side has rows, an entry of `best` is neither -1 nor a reference row of its group, or a parameter is out of
+ * range: inlier_radius and min_separation finite and > 0, max_hypotheses in [1, 65536], min_inliers >= 1,
+ * refine_iterations in [0, 1000].  Empty groups and n_groups = 0 are not errors. */
+typedef struct fe_register_params {
+  double inlier_radius;       /* m: a mapped query keypoint this close to a reference keypoint is an inlier */
+  double min_separation;      /* m: both matches of a hypothesis at least this far apart, in either scan   */
+  int32_t max_hypotheses;     /* H at most this many pairs                                                  */
+  int32_t min_inliers;        /* status 2 from this many inliers                                            */
+  int32_t refine_iterations;  /* least-squares rounds over the inliers                                      */
+} fe_register_params_t;
+
+/* 0.5 m, 1.0 m, 512, 16, 4.  min_inliers = 16 is the least count at which no registered pair of the sequence
+ * evaluation (DESIGN.md §13) is off by more than 0.5 m or 2 deg: a jittered pole lattice turned by 90 deg, or a
+ * symmetric handful of poles turned by 180 deg, scores up to 15 inliers. */
+void fe_register_params_default(fe_register_params_t* p);
+
+typedef struct fe_register_result {
+  int32_t n_groups;
+  int64_t n_queries;
+  const double* pose;           /* n_groups x {c, s, tx, ty}                         */
+  const double* rms;            /* n_groups                                          */
+  const int32_t* n_inliers;     /* n_groups                                          */
+  const int32_t* n_hypotheses;  /* n_groups                                          */
+  const int32_t* status;        /* n_groups: 0 no hypothesis, 1 too few inliers, 2 ok */
+  const int64_t* assoc;         /* n_queries: absolute reference row, -1 = none      */
+} fe_register_result_t;
+
+/* Keypoints and `best` in host memory: only rows [qo[0], qo[G]) and [ro[0], ro[G]) are uploaded. */
+int fe_register_matches(fe_ctx_t* ctx, const fe_point_t* query_kp, const fe_point_t* ref_kp, const int64_t* best,
+                        const int64_t* query_offsets, const int64_t* ref_offsets, int32_t n_groups,
+                        const fe_register_params_t* params, fe_register_result_t* out);
+/* Keypoints (e.g. those of fe_process_batch_device) and `best` (fe_match_device_best) in device memory.  Runs on the
+ * context's stream behind the batch and match calls, with no synchronisation in between.  `best` is checked on the
+ * device: a bad entry makes the call return FE_ERR_INVALID after the kernel. */
+int fe_register_matches_device(fe_ctx_t* ctx, const fe_point_t* query_kp, const fe_point_t* ref_kp, const int64_t* best,
+                               const int64_t* query_offsets, const int64_t* ref_offsets, int32_t n_groups,
+                               const fe_register_params_t* params, fe_register_result_t* out);
+/* Device address of the `best` array of the last match call (n_queries entries, valid until the next match call), for
+ * fe_register_matches_device.  FE_ERR_INVALID before the first match call. */
+int fe_match_device_best(fe_ctx_t* ctx, const int64_t** best);
+
 /* CUDA-event stopwatch on the context's stream (the stream every kernel of
  * fe_process_batch_device is launched on): begin, run any number of calls, end -> elapsed ms. */
 int fe_timer_begin(fe_ctx_t* ctx);

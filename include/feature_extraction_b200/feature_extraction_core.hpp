@@ -139,6 +139,24 @@ class FeatureExtractionCore {
     if (r.descriptors) pt_descriptors.assign(r.descriptors, r.descriptors + r.n_keypoints * FE_RECORD_FLOATS);
   }
 
+  // The planar motion of scan `query` against scan `reference` (fe_register_matches, one group): `best` as the match
+  // call returned it for these keypoints, one entry per query keypoint.  pose = {c, s, tx, ty} maps query xy into the
+  // reference scan's levelled frame; returns the status (0 no hypothesis, 1 too few inliers, 2 registered).
+  int registerMatches(const PointCloud& query, const PointCloud& reference, const std::vector<int64_t>& best,
+                      double pose[4], int* nInliers = nullptr, const fe_register_params_t* params = nullptr) {
+    if (best.size() != query.size()) throw std::runtime_error("registerMatches: best needs one entry per query keypoint");
+    fe_register_params_t p;
+    fe_register_params_default(&p);
+    const int64_t qo[2] = {0, (int64_t)query.size()};
+    const int64_t ro[2] = {0, (int64_t)reference.size()};
+    fe_register_result_t r;
+    check(fe_register_matches(ctx_, query.data(), reference.data(), best.data(), qo, ro, 1, params ? params : &p, &r),
+          "registerMatches");
+    for (int i = 0; i < 4; i++) pose[i] = r.pose[i];
+    if (nInliers) *nInliers = r.n_inliers[0];
+    return r.status[0];
+  }
+
   fe_ctx_t* context() { return ctx_; }
 
  private:

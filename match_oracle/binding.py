@@ -58,3 +58,29 @@ def match_descriptors(query, ref, query_offsets=None, ref_offsets=None, n_thread
                                      _p(best), _p(shift), _p(d), _p(sd))
     assert st == 0, st
     return best[:n], shift[:n], d[:n], sd[:n]
+
+
+def register_matches(query_kp, ref_kp, best, query_offsets, ref_offsets, inlier_radius=0.5, min_separation=1.0,
+                     max_hypotheses=512, min_inliers=16, refine_iterations=4):
+    """feo_register_matches on the CPU.  query_kp / ref_kp: (K, 4) float32 keypoints addressed by absolute row;
+    best: (qo[-1] - qo[0],) int64.  -> dict of pose (G, 4) float64 {c, s, tx, ty}, rms (G,), n_inliers (G,),
+    n_hypotheses (G,), status (G,) int32 and assoc (n,) int64."""
+    q = np.ascontiguousarray(query_kp, np.float32).reshape(-1, 4)
+    r = np.ascontiguousarray(ref_kp, np.float32).reshape(-1, 4)
+    b = np.ascontiguousarray(best, np.int64).reshape(-1)
+    qo = np.ascontiguousarray(query_offsets, np.int64)
+    ro = np.ascontiguousarray(ref_offsets, np.int64)
+    G = len(qo) - 1
+    n = int(qo[-1] - qo[0])
+    assert len(b) == n, (len(b), n)
+    out = {"pose": np.zeros((max(G, 1), 4)), "rms": np.zeros(max(G, 1)), "n_inliers": np.zeros(max(G, 1), np.int32),
+           "n_hypotheses": np.zeros(max(G, 1), np.int32), "status": np.zeros(max(G, 1), np.int32),
+           "assoc": np.zeros(max(n, 1), np.int64)}
+    st = lib().feo_register_matches(
+        _p(q) if len(q) else None, _p(r) if len(r) else None, _p(b) if n else None, _p(qo), _p(ro), C.c_int32(G),
+        C.c_double(inlier_radius), C.c_double(min_separation), C.c_int32(max_hypotheses), C.c_int32(min_inliers),
+        C.c_int32(refine_iterations), _p(out["pose"]), _p(out["rms"]), _p(out["n_inliers"]), _p(out["n_hypotheses"]),
+        _p(out["status"]), _p(out["assoc"]))
+    if st != 0:
+        raise ValueError("feo_register_matches: invalid argument")
+    return {k: (v[:n] if k == "assoc" else v[:G]) for k, v in out.items()}
