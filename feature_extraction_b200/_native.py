@@ -29,7 +29,10 @@ EXPORTS = [
     "fe_multi_enable_cloud_outputs", "fe_multi_get_cloud_outputs",
     "fe_match_descriptors", "fe_match_descriptors_device",
     "fe_register_params_default", "fe_register_matches", "fe_register_matches_device", "fe_match_device_best",
+    "fe_odometry", "fe_odometry_device",
 ]
+
+ODOMETRY_WINDOW = 2  # FE_ODOMETRY_WINDOW_DEFAULT
 
 
 class Params(C.Structure):
@@ -113,6 +116,23 @@ class RegisterResult(C.Structure):
     ]
 
 
+class OdometryResult(C.Structure):
+    """fe_odometry_result_t: per scan pose, motion {c, s, tx, ty}, rms, source, status and counts; per row its inlier."""
+    _fields_ = [
+        ("n_scans", C.c_int32),
+        ("n_rows", C.c_int64),
+        ("pose", C.POINTER(C.c_double)),
+        ("motion", C.POINTER(C.c_double)),
+        ("rms", C.POINTER(C.c_double)),
+        ("source", C.POINTER(C.c_int32)),
+        ("status", C.POINTER(C.c_int32)),
+        ("n_inliers", C.POINTER(C.c_int32)),
+        ("n_hypotheses", C.POINTER(C.c_int32)),
+        ("assoc", C.POINTER(C.c_int64)),
+        ("gpu_launches", C.c_int64),
+    ]
+
+
 def build():
     """Compile libfe_b200.so for sm_100a (nvcc cross-compiles without a GPU)."""
     subprocess.check_call(["make", "-s", "-C", os.path.join(_HERE, "csrc")])
@@ -189,6 +209,9 @@ def lib():
             f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                           C.POINTER(RegisterParams), C.POINTER(RegisterResult)]
         L.fe_match_device_best.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
+        for f in (L.fe_odometry, L.fe_odometry_device):
+            f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                          C.POINTER(RegisterParams), C.POINTER(OdometryResult)]
         L.fe_debug_enable_graphs.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int64)]
         L.fe_debug_lean_reruns.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         L.fe_debug_density_work.argtypes = [C.c_void_p, C.c_void_p]

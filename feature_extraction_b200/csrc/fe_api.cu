@@ -13,6 +13,7 @@
 
 #include "fe_kernels.cuh"
 #include "fe_match.h"
+#include "fe_odometry.h"
 #include "fe_register.h"
 
 using namespace fe;
@@ -176,6 +177,12 @@ struct fe_ctx {
   int64_t *d_regOffs = nullptr, capRegOffsHost = 0, capRegOffs = 0;
   unsigned char *d_regScratch = nullptr, *d_regRes = nullptr, *h_regRes = nullptr;  // results: reg_layout()
   int64_t capRegScratch = 0, capRegRes = 0, capRegResHost = 0;  // bytes
+  // fe_odometry*: buffers of their own, so that an odometry call leaves the batch, match and register results alone
+  unsigned char *d_odoTab = nullptr, *h_odoTab = nullptr;    // ko | so | step offsets | step items of the call
+  unsigned char *d_odoWork = nullptr, *d_odoRes = nullptr, *h_odoRes = nullptr;  // per-step buffers; results: odo_layout()
+  fe_point_t* d_odoKp = nullptr;                             // uploaded keypoints of the host variant
+  long long* d_odoBest = nullptr;                            // uploaded `best` of the host variant
+  int64_t capOdoTab = 0, capOdoTabHost = 0, capOdoWork = 0, capOdoRes = 0, capOdoResHost = 0, capOdoKp = 0, capOdoBest = 0;
   std::string err;
 };
 
@@ -1197,9 +1204,10 @@ void fe_destroy(fe_ctx_t* ctx) {
   if (ctx->h_cloud) cudaFreeHost(ctx->h_cloud);
   if (ctx->h_kc) cudaFreeHost(ctx->h_kc);
   void* dm[] = {ctx->d_matchQ, ctx->d_matchR, ctx->d_items, ctx->d_part, ctx->d_matchRes,
-                ctx->d_regQ, ctx->d_regR, ctx->d_regBest, ctx->d_regOffs, ctx->d_regScratch, ctx->d_regRes};
+                ctx->d_regQ, ctx->d_regR, ctx->d_regBest, ctx->d_regOffs, ctx->d_regScratch, ctx->d_regRes,
+                ctx->d_odoTab, ctx->d_odoWork, ctx->d_odoRes, ctx->d_odoKp, ctx->d_odoBest};
   for (void* p : dm) if (p) cudaFree(p);
-  void* hm[] = {ctx->h_items, ctx->h_matchRes, ctx->h_regOffs, ctx->h_regRes};
+  void* hm[] = {ctx->h_items, ctx->h_matchRes, ctx->h_regOffs, ctx->h_regRes, ctx->h_odoTab, ctx->h_odoRes};
   for (void* p : hm) if (p) cudaFreeHost(p);
   delete ctx;
 }
@@ -1692,12 +1700,8 @@ RegLayout reg_layout(int64_t G, int64_t nQ) {
   return L;
 }
 
-// both entry points: keypoints and `best` are device memory (onDevice) or host memory to upload
-int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, const int64_t* best, const int64_t* qo,
-                     const int64_t* ro, int32_t G, const fe_register_params_t* prm, fe_register_result_t* out,
-                     bool onDevice) {
-  if (!ctx || !out) return FE_ERR_INVALID;
-  ctx->err.clear();
+// the parameter checks of the register and odometry calls, and the kernel's form of the parameters
+int register_params(fe_ctx* ctx, const fe_register_params_t* prm, fe_register::Params* kp) {
   if (!prm) return fail(ctx, FE_ERR_INVALID, "params is NULL");
   const fe_register_params_t p = *prm;
   if (!(std::isfinite(p.inlier_radius) && p.inlier_radius > 0.0))
@@ -1708,6 +1712,23 @@ int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, cons
   if (p.min_inliers < 1) return fail(ctx, FE_ERR_INVALID, "min_inliers must be >= 1");
   if (p.refine_iterations < 0 || p.refine_iterations > 1000)
     return fail(ctx, FE_ERR_INVALID, "refine_iterations must be in [0, 1000]");
+  kp->r2 = p.inlier_radius * p.inlier_radius;
+  kp->sep2 = p.min_separation * p.min_separation;
+  kp->twoR = 2.0 * p.inlier_radius;
+  kp->maxH = p.max_hypotheses;
+  kp->minInliers = p.min_inliers;
+  kp->refine = p.refine_iterations;
+  return FE_OK;
+}
+
+// both entry points: keypoints and `best` are device memory (onDevice) or host memory to upload
+int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, const int64_t* best, const int64_t* qo,
+                     const int64_t* ro, int32_t G, const fe_register_params_t* prm, fe_register_result_t* out,
+                     bool onDevice) {
+  if (!ctx || !out) return FE_ERR_INVALID;
+  ctx->err.clear();
+  fe_register::Params kp;
+  if (int st = register_params(ctx, prm, &kp)) return st;
   if (G < 0) return fail(ctx, FE_ERR_INVALID, "n_groups must not be negative");
   if (!qo || !ro) return fail(ctx, FE_ERR_INVALID, "query_offsets and ref_offsets need n_groups + 1 entries");
   if (const char* e = check_offsets(qo, G)) return fail(ctx, FE_ERR_INVALID, std::string("query_offsets: ") + e);
@@ -1785,13 +1806,6 @@ int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, cons
   sc.d2Cur = (double*)(sc.assocNew + n1);
   sc.d2New = sc.d2Cur + n1;
   sc.corr = (int*)(sc.d2New + n1);
-  fe_register::Params kp;
-  kp.r2 = p.inlier_radius * p.inlier_radius;
-  kp.sep2 = p.min_separation * p.min_separation;
-  kp.twoR = 2.0 * p.inlier_radius;
-  kp.maxH = p.max_hypotheses;
-  kp.minInliers = p.min_inliers;
-  kp.refine = p.refine_iterations;
   CK(fe_register::launch(q, qBias, r, rBias, (const long long*)best, ctx->d_regOffs, ctx->d_regOffs + G + 1, G, kp, o, sc,
                          stream));
   ctx->launches += 1;
@@ -1815,6 +1829,204 @@ int fe_register_matches_device(fe_ctx_t* ctx, const fe_point_t* query_kp, const 
                                const int64_t* query_offsets, const int64_t* ref_offsets, int32_t n_groups,
                                const fe_register_params_t* params, fe_register_result_t* out) {
   return register_matches(ctx, query_kp, ref_kp, best, query_offsets, ref_offsets, n_groups, params, out, true);
+}
+
+}  // extern "C"
+
+// ---- odometry (fe_odometry.cu) -------------------------------------------------------------------------
+
+namespace {
+
+int64_t align16(int64_t b) { return (b + 15) & ~(int64_t)15; }
+
+// The results of an odometry call in h_odoRes / d_odoRes, one copy: pose | motion (B x 4) | rms (B) as doubles, assoc
+// (n_rows) as 8-byte words, then source | status | n_inliers | n_hypotheses (B each) | the device's error flag.
+struct OdoLayout {
+  int64_t pose, motion, rms, assoc, source, status, nInl, nHyp, err, bytes;
+};
+OdoLayout odo_layout(int64_t B, int64_t nRows) {
+  OdoLayout L;
+  L.pose = 0;
+  L.motion = L.pose + 32 * B;
+  L.rms = L.motion + 32 * B;
+  L.assoc = L.rms + 8 * B;
+  L.source = L.assoc + 8 * nRows;
+  L.status = L.source + 4 * B;
+  L.nInl = L.status + 4 * B;
+  L.nHyp = L.nInl + 4 * B;
+  L.err = L.nHyp + 4 * B;
+  L.bytes = L.err + 4;
+  return L;
+}
+
+// both entry points: keypoints and `best` are device memory (onDevice) or host memory to upload
+int odometry(fe_ctx* ctx, const fe_point_t* kp, const int64_t* ko, int32_t B, const int64_t* best, const int64_t* so,
+             int32_t S, int32_t W, const fe_register_params_t* prm, fe_odometry_result_t* out, bool onDevice) {
+  if (!ctx || !out) return FE_ERR_INVALID;
+  ctx->err.clear();
+  fe_register::Params rp;
+  if (int st = register_params(ctx, prm, &rp)) return st;
+  if (B < 0 || S < 0) return fail(ctx, FE_ERR_INVALID, "n_scans and n_sequences must not be negative");
+  if (!ko || !so) return fail(ctx, FE_ERR_INVALID, "keypoint_offsets and sequence_offsets need n_scans + 1 and n_sequences + 1 entries");
+  if (W < 1 || W > 64) return fail(ctx, FE_ERR_INVALID, "window must be in [1, 64]");
+  if (const char* e = check_offsets(ko, B)) return fail(ctx, FE_ERR_INVALID, std::string("keypoint_offsets: ") + e);
+  if (const char* e = check_offsets(so, S)) return fail(ctx, FE_ERR_INVALID, std::string("sequence_offsets: ") + e);
+  if (so[0] != 0 || so[S] != B) return fail(ctx, FE_ERR_INVALID, "sequence_offsets must run from 0 to n_scans");
+  for (int32_t b = 0; b < B; b++)
+    if (ko[b + 1] - ko[b] >= (1LL << 24)) return fail(ctx, FE_ERR_INVALID, "a scan has 2^24 or more keypoints");
+  const int64_t nRows = ko[B] - ko[0];
+  if (nRows >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 keypoint rows");
+
+  // the steps: sequences with a scan t, each with a slot for its largest window
+  std::vector<fe_odo::Step> steps;
+  std::vector<fe_odo::Item> items;
+  std::vector<int64_t> offs;
+  int64_t maxQ = 1, maxR = 1, maxN = 1, bestRows = 0;
+  for (int64_t t = 1;; t++) {
+    fe_odo::Step st;
+    st.item0 = (int64_t)items.size();
+    st.offs0 = (int64_t)offs.size();
+    for (int32_t q = 0; q < S; q++)
+      if (so[q + 1] - so[q] > t) items.push_back({(int)(so[q] + t), (int)so[q]});
+    st.n = (int)((int64_t)items.size() - st.item0);
+    if (st.n == 0) break;
+    offs.resize(offs.size() + 2 * (size_t)(2 * st.n + 1));
+    int64_t* qo = offs.data() + st.offs0;
+    int64_t* ro = qo + 2 * st.n + 1;
+    qo[0] = ro[0] = 0;
+    for (int i = 0; i < st.n; i++) {
+      const int s = items[(size_t)(st.item0 + i)].scan;
+      const int64_t nq = ko[s + 1] - ko[s], slot = ko[s] - ko[s - std::min<int64_t>(W, t)];
+      qo[2 * i + 1] = qo[2 * i + 2] = qo[2 * i] + nq;
+      ro[2 * i + 1] = ro[2 * i + 2] = ro[2 * i] + slot;  // ro[2i + 1] is the device's to write
+      bestRows += nq;
+    }
+    maxQ = std::max(maxQ, qo[2 * st.n]);
+    maxR = std::max(maxR, ro[2 * st.n]);
+    maxN = std::max<int64_t>(maxN, st.n);
+    steps.push_back(st);
+  }
+  if (bestRows > 0 && !best) return fail(ctx, FE_ERR_INVALID, "best is NULL but there are scans to register");
+  if (!steps.empty() && nRows > 0 && !kp) return fail(ctx, FE_ERR_INVALID, "kp is NULL but there are keypoints");
+  if (!onDevice)
+    for (const fe_odo::Item& it : items)
+      for (int64_t k = ko[it.scan]; k < ko[it.scan + 1]; k++) {
+        const int64_t b = best[k - ko[1]];
+        if (b != -1 && (b < ko[it.scan - 1] || b >= ko[it.scan]))
+          return fail(ctx, FE_ERR_INVALID, "best[" + std::to_string(k - ko[1]) + "] is neither -1 nor a row of the previous scan");
+      }
+  CK(cudaSetDevice(ctx->device));
+  int st = ensure_slot(ctx, ctx->slot[0], false);  // for its stream only: the slot's buffers are not touched
+  if (st) return st;
+  cudaStream_t stream = ctx->slot[0].stream;
+
+  const OdoLayout L = odo_layout(B, nRows);
+  if ((st = grow_pinned(ctx, &ctx->h_odoRes, &ctx->capOdoResHost, L.bytes, 4096, 0))) return st;
+  unsigned char* h = ctx->h_odoRes;
+  out->n_scans = B;
+  out->n_rows = nRows;
+  out->pose = (const double*)(h + L.pose);
+  out->motion = (const double*)(h + L.motion);
+  out->rms = (const double*)(h + L.rms);
+  out->assoc = (const int64_t*)(h + L.assoc);
+  out->source = (const int32_t*)(h + L.source);
+  out->status = (const int32_t*)(h + L.status);
+  out->n_inliers = (const int32_t*)(h + L.nInl);
+  out->n_hypotheses = (const int32_t*)(h + L.nHyp);
+  out->gpu_launches = 0;
+  if (B == 0) return FE_OK;
+
+  // tables: ko | so | offsets of every step | items
+  const int64_t tKo = 0, tSo = tKo + 8 * (B + 1), tOffs = tSo + 8 * ((int64_t)S + 1);
+  const int64_t tItems = tOffs + 8 * (int64_t)offs.size(), tBytes = tItems + 8 * (int64_t)items.size();
+  if ((st = grow_pinned(ctx, &ctx->h_odoTab, &ctx->capOdoTabHost, tBytes, 4096, 0))) return st;
+  if ((st = grow_device(ctx, &ctx->d_odoTab, &ctx->capOdoTab, tBytes))) return st;
+  memcpy(ctx->h_odoTab + tKo, ko, 8 * ((size_t)B + 1));
+  memcpy(ctx->h_odoTab + tSo, so, 8 * ((size_t)S + 1));
+  if (!offs.empty()) memcpy(ctx->h_odoTab + tOffs, offs.data(), 8 * offs.size());
+  if (!items.empty()) memcpy(ctx->h_odoTab + tItems, items.data(), 8 * items.size());
+  CK(cudaMemcpyAsync(ctx->d_odoTab, ctx->h_odoTab, (size_t)tBytes, cudaMemcpyHostToDevice, stream));
+  fe_odo::Tables T;
+  T.ko = (const int64_t*)(ctx->d_odoTab + tKo);
+  T.so = (const int64_t*)(ctx->d_odoTab + tSo);
+  T.offs = (int64_t*)(ctx->d_odoTab + tOffs);
+  T.items = (const fe_odo::Item*)(ctx->d_odoTab + tItems);
+
+  // work buffers, sized for the largest step: 16-byte rows first, then 8-byte, then 4-byte arrays
+  const int64_t maxG = 2 * maxN;
+  const int64_t wQ = 0, wR = wQ + 16 * maxQ, wBest = wR + 16 * maxR, wAssoc = wBest + 8 * maxQ;
+  const int64_t wAssocNew = wAssoc + 8 * maxQ, wD2Cur = wAssocNew + 8 * maxQ, wD2New = wD2Cur + 8 * maxQ;
+  const int64_t wWinLo = wD2New + 8 * maxQ, wPose = wWinLo + 8 * maxN, wRms = wPose + 32 * maxG;
+  const int64_t wCorr = wRms + 8 * maxG, wNInl = wCorr + 4 * maxQ, wNHyp = wNInl + 4 * maxG, wStatus = wNHyp + 4 * maxG;
+  const int64_t wBytes = align16(wStatus + 4 * maxG);
+  if ((st = grow_device(ctx, &ctx->d_odoWork, &ctx->capOdoWork, wBytes))) return st;
+  if ((st = grow_device(ctx, &ctx->d_odoRes, &ctx->capOdoRes, L.bytes))) return st;
+  unsigned char* wb = ctx->d_odoWork;
+  unsigned char* d = ctx->d_odoRes;
+  fe_odo::Out o;
+  o.pose = (double*)(d + L.pose);
+  o.motion = (double*)(d + L.motion);
+  o.rms = (double*)(d + L.rms);
+  o.assoc = (long long*)(d + L.assoc);
+  o.source = (int*)(d + L.source);
+  o.status = (int*)(d + L.status);
+  o.nInl = (int*)(d + L.nInl);
+  o.nHyp = (int*)(d + L.nHyp);
+  o.err = (int*)(d + L.err);
+  fe_odo::Work w;
+  w.q = (fe_point_t*)(wb + wQ);
+  w.r = (fe_point_t*)(wb + wR);
+  w.best = (long long*)(wb + wBest);
+  w.winLo = (int64_t*)(wb + wWinLo);
+  w.reg.pose = (double*)(wb + wPose);
+  w.reg.rms = (double*)(wb + wRms);
+  w.reg.assoc = (long long*)(wb + wAssoc);
+  w.reg.nInl = (int*)(wb + wNInl);
+  w.reg.nHyp = (int*)(wb + wNHyp);
+  w.reg.status = (int*)(wb + wStatus);
+  w.reg.err = o.err;
+  w.scratch.corr = (int*)(wb + wCorr);
+  w.scratch.assocNew = (long long*)(wb + wAssocNew);
+  w.scratch.d2Cur = (double*)(wb + wD2Cur);
+  w.scratch.d2New = (double*)(wb + wD2New);
+
+  int64_t kpBias = 0;
+  if (!onDevice) {  // rows [ko[0], ko[B]) and the `best` entries of the scans that are registered
+    if ((st = grow_device(ctx, &ctx->d_odoKp, &ctx->capOdoKp, std::max<int64_t>(nRows, 1)))) return st;
+    if (nRows > 0) CK(cudaMemcpyAsync(ctx->d_odoKp, kp + ko[0], (size_t)nRows * sizeof(fe_point_t), cudaMemcpyHostToDevice, stream));
+    const int64_t nBest = B >= 2 ? ko[B] - ko[1] : 0;
+    if ((st = grow_device(ctx, &ctx->d_odoBest, &ctx->capOdoBest, std::max<int64_t>(nBest, 1)))) return st;
+    if (nBest > 0 && bestRows > 0)
+      CK(cudaMemcpyAsync(ctx->d_odoBest, best, (size_t)nBest * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
+    kp = ctx->d_odoKp;
+    best = (const int64_t*)ctx->d_odoBest;
+    kpBias = ko[0];
+  }
+  CK(cudaMemsetAsync(d + L.err, 0, 4, stream));
+  CK(fe_odo::run(kp, kpBias, (const long long*)best, S, W, steps, T, w, o, rp, stream));
+  const int64_t launches = S > 0 ? 1 + 3 * (int64_t)steps.size() : 0;
+  ctx->launches += launches;
+  out->gpu_launches = launches;
+  CK(cudaMemcpyAsync(h, d, (size_t)L.bytes, cudaMemcpyDeviceToHost, stream));
+  CK(cudaStreamSynchronize(stream));
+  if (*(const int32_t*)(h + L.err)) return fail(ctx, FE_ERR_INVALID, "an entry of best is neither -1 nor a row of the previous scan");
+  return FE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fe_odometry(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypoint_offsets, int32_t n_scans, const int64_t* best,
+                const int64_t* sequence_offsets, int32_t n_sequences, int32_t window, const fe_register_params_t* params,
+                fe_odometry_result_t* out) {
+  return odometry(ctx, kp, keypoint_offsets, n_scans, best, sequence_offsets, n_sequences, window, params, out, false);
+}
+
+int fe_odometry_device(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypoint_offsets, int32_t n_scans,
+                       const int64_t* best, const int64_t* sequence_offsets, int32_t n_sequences, int32_t window,
+                       const fe_register_params_t* params, fe_odometry_result_t* out) {
+  return odometry(ctx, kp, keypoint_offsets, n_scans, best, sequence_offsets, n_sequences, window, params, out, true);
 }
 
 // ---- one entry point per reference function ----------------------------------------------------------

@@ -10,6 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native as N
+from ._native import ODOMETRY_WINDOW
 
 DESC_LEN = N.DESC_LEN
 RECORD_FLOATS = N.RECORD_FLOATS
@@ -125,6 +126,34 @@ def _unpack_register(res):
     return {"pose": arr(res.pose, (G, 4), np.float64), "rms": arr(res.rms, (G,), np.float64),
             "n_inliers": arr(res.n_inliers, (G,), np.int32), "n_hypotheses": arr(res.n_hypotheses, (G,), np.int32),
             "status": arr(res.status, (G,), np.int32), "assoc": arr(res.assoc, (n,), np.int64)}
+
+
+def _unpack_odometry(res):
+    B, n = int(res.n_scans), int(res.n_rows)
+
+    def arr(p, shape, dtype):
+        if int(np.prod(shape)) == 0:
+            return np.zeros(shape, dtype)
+        return np.ctypeslib.as_array(p, shape=shape).copy()
+    return {"pose": arr(res.pose, (B, 4), np.float64), "motion": arr(res.motion, (B, 4), np.float64),
+            "rms": arr(res.rms, (B,), np.float64), "source": arr(res.source, (B,), np.int32),
+            "status": arr(res.status, (B,), np.int32), "n_inliers": arr(res.n_inliers, (B,), np.int32),
+            "n_hypotheses": arr(res.n_hypotheses, (B,), np.int32), "assoc": arr(res.assoc, (n,), np.int64)}
+
+
+def _odometry_offsets(keypoint_offsets, sequence_offsets, n_rows):
+    """Validate the scans and sequences of an odometry call before raw pointers cross the C-ABI."""
+    ko = np.ascontiguousarray(keypoint_offsets, np.int64).reshape(-1)
+    so = np.ascontiguousarray(sequence_offsets, np.int64).reshape(-1)
+    if len(ko) < 1 or len(so) < 1:
+        raise ValueError("keypoint_offsets and sequence_offsets need n_scans + 1 and n_sequences + 1 entries")
+    if ko[0] < 0 or np.any(np.diff(ko) < 0):
+        raise ValueError("keypoint_offsets must start at >= 0 and be non-decreasing")
+    if so[0] != 0 or so[-1] != len(ko) - 1 or np.any(np.diff(so) < 0):
+        raise ValueError("sequence_offsets must run from 0 to n_scans and be non-decreasing")
+    if n_rows is not None and ko[-1] > n_rows:
+        raise ValueError("keypoint_offsets[-1] = %d exceeds the %d keypoints passed" % (ko[-1], n_rows))
+    return ko, so, len(ko) - 1, len(so) - 1
 
 
 class PinnedBuffer:
@@ -409,6 +438,50 @@ class FeatureExtractionNode:
         ko = np.ascontiguousarray(ko, np.int64)
         best = self.matchDescriptors(descriptors, descriptors, ko[1:], ko[:-1])[0]
         out = self.registerMatches(kp, kp, best, ko[1:], ko[:-1], params)
+        out["best"] = best
+        return out
+
+    def odometry(self, kp, keypoint_offsets, best, sequence_offsets, window=ODOMETRY_WINDOW, params=None):
+        """fe_odometry: register every scan of every sequence against a window of its predecessors and chain the motions
+        into poses (include/fe_b200.h, "odometry").  kp: (K, 4) host keypoints addressed by absolute row; `best` as
+        matchDescriptors returns it for scan s against s - 1 (ko[B] - ko[1] entries); sequence_offsets in scans.
+        -> dict of pose (B, 4) {c, s, tx, ty} (scan xy -> its sequence's first scan), motion (B, 4) (scan xy -> the
+        previous scan), rms (B,), source (B,) int32 (0 first scan, 1 registered, 2 predicted), status, n_inliers,
+        n_hypotheses (B,) int32 (status -1 for first scans), assoc (ko[B] - ko[0],) int64."""
+        k = _keypoint_rows(kp)
+        ko, so, B, S = _odometry_offsets(keypoint_offsets, sequence_offsets, len(k))
+        b = np.ascontiguousarray(best, np.int64).reshape(-1)
+        nb = int(ko[-1] - ko[1]) if B >= 2 else 0
+        if len(b) != nb:
+            raise ValueError("best needs one entry per row from keypoint_offsets[1]: %d, got %d" % (nb, len(b)))
+        prm = params if params is not None else register_params_default()
+        res = N.OdometryResult()
+        self._check(N.lib().fe_odometry(self._ctx, _ptr(k) if len(k) else None, _ptr(ko), B, _ptr(b) if len(b) else None,
+                                        _ptr(so), S, int(window), C.byref(prm), C.byref(res)))
+        self.last_launches = int(res.gpu_launches)
+        return _unpack_odometry(res)
+
+    def odometryDevice(self, kp_ptr, keypoint_offsets, best_ptr, sequence_offsets, window=ODOMETRY_WINDOW, params=None):
+        """fe_odometry_device: keypoints (processBatchDevice's) and `best` (matchDeviceBest() after matching scan s
+        against s - 1) already in HBM, queued on the context's stream behind the batch and match calls.  Same results as
+        odometry."""
+        ko, so, B, S = _odometry_offsets(keypoint_offsets, sequence_offsets, None)  # the device buffers' sizes are the caller's
+        if ko[-1] > ko[0] and not kp_ptr:
+            raise ValueError("kp_ptr is NULL while there are keypoints")
+        prm = params if params is not None else register_params_default()
+        res = N.OdometryResult()
+        self._check(N.lib().fe_odometry_device(self._ctx, C.c_void_p(kp_ptr), _ptr(ko), B, C.c_void_p(best_ptr), _ptr(so), S,
+                                               int(window), C.byref(prm), C.byref(res)))
+        self.last_launches = int(res.gpu_launches)
+        return _unpack_odometry(res)
+
+    def sequence_odometry(self, ko, kp, descriptors, sequence_offsets, window=ODOMETRY_WINDOW, params=None):
+        """Poses of the scans of one batch result (processBatch's keypoint_offsets, keypoints, descriptors), cut into
+        sequences by sequence_offsets (in scans): match scan s against scan s - 1, then odometry.  -> odometry's dict
+        plus `best`."""
+        ko = np.ascontiguousarray(ko, np.int64)
+        best = self.matchDescriptors(descriptors, descriptors, ko[1:], ko[:-1])[0] if len(ko) > 2 else np.zeros(0, np.int64)
+        out = self.odometry(kp, ko, best, sequence_offsets, window, params)
         out["best"] = best
         return out
 

@@ -383,6 +383,88 @@ int fe_register_matches_device(fe_ctx_t* ctx, const fe_point_t* query_kp, const 
  * fe_register_matches_device.  FE_ERR_INVALID before the first match call. */
 int fe_match_device_best(fe_ctx_t* ctx, const int64_t** best);
 
+/* ---- odometry: a pose for every scan of a sequence ------------------------------------------------------------- */
+/* Each scan is registered against a window of its predecessors, placed by the motions already estimated, and the
+ * motions are chained into poses.  Evaluated to the last bit as follows: IEEE double with + - * / only, each operation
+ * rounded on its own (no FMA), in the order written, plus registration's own arithmetic.
+ *
+ * Inputs.  Keypoints `kp` addressed by absolute row with the batch's keypoint_offsets ko[0..B] (scan b owns rows
+ * [ko[b], ko[b+1])); sequence_offsets so[0..S] in scans, non-decreasing, so[0] = 0, so[S] = B: sequence q is scans
+ * [so[q], so[q+1]), consecutive scans of one sensor; empty sequences are allowed.  `best`: the matcher's output for
+ * query_offsets = ko + 1, ref_offsets = ko, n_groups = B - 1, i.e. best[i] for row ko[1] + i, ko[B] - ko[1] entries
+ * (none when B < 2).  Entries of rows in the first scan of a sequence are ignored (they point into another
+ * sequence); every other entry is -1 or a row of the previous scan.  `window` W in [1, 64].  Registration parameters as
+ * fe_register_matches takes them.
+ *
+ * Motions.  For local scan t >= 1 of a sequence, motion_t maps scan t's levelled xy into scan t-1's, as
+ * fe_register_matches defines a pose.  For t = 0, motion_0 = (1, 0, 0, 0).
+ *
+ * Step t (one registration group per sequence that has a scan t, steps t = 1, 2, ... in order):
+ *   query       the rows of scan t, with their `best` entries: hypotheses come only from matches into scan t-1.
+ *   window      scan t-1, then t-2, t-3, ... down to max(0, t-W); it stops before the first scan j whose link
+ *               motion_{j+1} was predicted rather than registered.  Scan t-1 is always in it.
+ *   reference   the window's scans in ascending scan order, each scan's rows in ascending order: a contiguous range of
+ *               absolute rows.
+ *   placement   into scan t-1's frame.  Scan t-1's rows are copied unchanged.  Scan j < t-1 is placed by P_j, with
+ *               P_{t-2} = inv(motion_{t-1}) and P_j = compose(P_{j+1}, inv(motion_{j+1})), composed from the local chain
+ *               (never from the poses below, so long sequences lose no precision far from their origin):
+ *                 inv(A)        = (A.c, -A.s, -(A.c*A.tx + A.s*A.ty), A.s*A.tx - A.c*A.ty)
+ *                 compose(A, B) = (A.c*B.c - A.s*B.s, A.s*B.c + A.c*B.s, (A.c*B.tx - A.s*B.ty) + A.tx,
+ *                                  (A.s*B.tx + A.c*B.ty) + A.ty)
+ *               A placed row is the registration contract's w under P_j, x and y rounded to float; z and intensity are
+ *               copied.
+ *   registration  the group (query, placed reference, `best` entries as the rows of scan t-1 within it) is registered
+ *               exactly as fe_register_matches specifies.  Status 2: motion_t is the registered pose (source 1).
+ *               Otherwise motion_t is predicted (source 2): motion_{t-1} (constant velocity), or (1, 0, 0, 0) for t = 1.
+ *
+ * Poses.  pose_0 = (1, 0, 0, 0); pose_t = compose(pose_{t-1}, motion_t): scan t's xy into its sequence's first scan.
+ *
+ * With W = 1 every link's registration outputs (status, n_inliers, n_hypotheses, rms, its pose as motion_t when
+ * registered, assoc) are those of fe_register_matches on scan s against scan s-1, bit for bit.
+ *
+ * Outputs (context-owned pinned memory, valid until the next odometry call; an odometry call leaves the results of
+ * batch, match and register calls alone, and they leave its results alone).  Per scan: pose, motion, source (0 first
+ * scan of its sequence, 1 registered, 2 predicted), and the registration's status, n_inliers, n_hypotheses, rms (status
+ * -1 and everything else 0 for first scans).  Per keypoint row of [ko[0], ko[B]): assoc, the absolute row of the window
+ * keypoint it is an inlier of, or -1 (every row of a first scan).
+ *
+ * Cost: steps run one after the other, three launches each (placement, registration, update), one warp per sequence
+ * in each; a batch of many short sequences is as cheap as registering its pairs, one long sequence is launch-bound.
+ *
+ * FE_ERR_INVALID (the context stays usable) on the argument errors of fe_register_matches' parameters, when an offsets
+ * array is NULL, decreases or has a negative entry, sequence_offsets does not run from 0 to B, B or S is negative, W
+ * is outside [1, 64], a scan has 2^24 or more rows, `kp` or `best` is NULL while there are rows to read, or an entry of
+ * `best` that is read is neither -1 nor a row of the previous scan.  B = 0, S = 0, empty scans and empty sequences are
+ * not errors. */
+/* The window of the sequence evaluation (DESIGN.md §14): the largest registered fraction with no wrong link, the
+ * smallest such window on ties. */
+#define FE_ODOMETRY_WINDOW_DEFAULT 2
+
+typedef struct fe_odometry_result {
+  int32_t n_scans;
+  int64_t n_rows;                /* ko[B] - ko[0]                                                        */
+  const double* pose;            /* n_scans x {c, s, tx, ty}: scan xy -> its sequence's first scan       */
+  const double* motion;          /* n_scans x {c, s, tx, ty}: scan xy -> previous scan                   */
+  const double* rms;             /* n_scans                                                              */
+  const int32_t* source;         /* n_scans: 0 first scan, 1 registered, 2 predicted                     */
+  const int32_t* status;         /* n_scans: registration status, -1 for first scans                     */
+  const int32_t* n_inliers;      /* n_scans                                                              */
+  const int32_t* n_hypotheses;   /* n_scans                                                              */
+  const int64_t* assoc;          /* n_rows: absolute row of the window keypoint, -1 = none               */
+  int64_t gpu_launches;          /* kernels the call launched: 1 + 3 * (longest sequence - 1), or 0     */
+} fe_odometry_result_t;
+
+/* Keypoints and `best` in host memory: only rows [ko[0], ko[B]) and the `best` entries are uploaded. */
+int fe_odometry(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypoint_offsets, int32_t n_scans, const int64_t* best,
+                const int64_t* sequence_offsets, int32_t n_sequences, int32_t window, const fe_register_params_t* params,
+                fe_odometry_result_t* out);
+/* `kp` from fe_process_batch_device and `best` from fe_match_device_best (after a match call of scan s against s-1 on
+ * the same offsets), in device memory.  Runs on the context's stream behind them with no synchronisation in between;
+ * a bad `best` entry is found on the device and makes the call return FE_ERR_INVALID. */
+int fe_odometry_device(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypoint_offsets, int32_t n_scans,
+                       const int64_t* best, const int64_t* sequence_offsets, int32_t n_sequences, int32_t window,
+                       const fe_register_params_t* params, fe_odometry_result_t* out);
+
 /* CUDA-event stopwatch on the context's stream (the stream every kernel of
  * fe_process_batch_device is launched on): begin, run any number of calls, end -> elapsed ms. */
 int fe_timer_begin(fe_ctx_t* ctx);

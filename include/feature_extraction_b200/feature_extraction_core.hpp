@@ -157,6 +157,28 @@ class FeatureExtractionCore {
     return r.status[0];
   }
 
+  // Poses of one sequence of scans (fe_odometry, one sequence): `keypoints` concatenated in scan order with
+  // keypointOffsets (n_scans + 1 entries), `best` as the match call returned it for scan s against s - 1 (one entry per
+  // keypoint from keypointOffsets[1]).  poses gets n_scans x {c, s, tx, ty}, scan xy into the first scan's frame;
+  // sources (if given) 0 first scan, 1 registered, 2 predicted.
+  void odometry(const PointCloud& keypoints, const std::vector<int64_t>& keypointOffsets, const std::vector<int64_t>& best,
+                std::vector<double>& poses, std::vector<int32_t>* sources = nullptr, int window = FE_ODOMETRY_WINDOW_DEFAULT,
+                const fe_register_params_t* params = nullptr) {
+    if (keypointOffsets.empty()) throw std::runtime_error("odometry: keypointOffsets needs n_scans + 1 entries");
+    const int32_t B = (int32_t)keypointOffsets.size() - 1;
+    if (keypointOffsets[B] > (int64_t)keypoints.size()) throw std::runtime_error("odometry: keypointOffsets exceed the keypoints");
+    if ((int64_t)best.size() != (B >= 2 ? keypointOffsets[B] - keypointOffsets[1] : 0))
+      throw std::runtime_error("odometry: best needs one entry per keypoint from keypointOffsets[1]");
+    fe_register_params_t p;
+    fe_register_params_default(&p);
+    const int64_t so[2] = {0, B};
+    fe_odometry_result_t r;
+    check(fe_odometry(ctx_, keypoints.data(), keypointOffsets.data(), B, best.data(), so, 1, window, params ? params : &p, &r),
+          "odometry");
+    poses.assign(r.pose, r.pose + 4 * (int64_t)B);
+    if (sources) sources->assign(r.source, r.source + B);
+  }
+
   fe_ctx_t* context() { return ctx_; }
 
  private:

@@ -1,5 +1,5 @@
-"""ctypes binding of match_oracle/libfe_match_oracle.so: the CPU restatement of fe_match_descriptors
-(include/fe_b200.h, "descriptor matching").
+"""ctypes binding of match_oracle/libfe_match_oracle.so: the CPU restatements of fe_match_descriptors,
+fe_register_matches and fe_odometry (include/fe_b200.h, "descriptor matching", "registration", "odometry").
 
 TEST INFRASTRUCTURE ONLY, like oracle/oracle_binding.py: never imported by the feature_extraction_b200 package.
 """
@@ -84,3 +84,31 @@ def register_matches(query_kp, ref_kp, best, query_offsets, ref_offsets, inlier_
     if st != 0:
         raise ValueError("feo_register_matches: invalid argument")
     return {k: (v[:n] if k == "assoc" else v[:G]) for k, v in out.items()}
+
+
+def odometry(kp, keypoint_offsets, best, sequence_offsets, window=1, inlier_radius=0.5, min_separation=1.0,
+             max_hypotheses=512, min_inliers=16, refine_iterations=4):
+    """feo_odometry on the CPU.  kp: (K, 4) float32 keypoints addressed by absolute row; keypoint_offsets (B + 1,);
+    best: (ko[B] - ko[1],) int64 (scan s against s - 1); sequence_offsets (S + 1,) in scans.  -> dict of pose, motion
+    (B, 4) float64 {c, s, tx, ty}, rms (B,), source, status, n_inliers, n_hypotheses (B,) int32, assoc (ko[B] - ko[0],)
+    int64."""
+    k = np.ascontiguousarray(kp, np.float32).reshape(-1, 4)
+    ko = np.ascontiguousarray(keypoint_offsets, np.int64)
+    so = np.ascontiguousarray(sequence_offsets, np.int64)
+    B, S = len(ko) - 1, len(so) - 1
+    nb = int(ko[-1] - ko[1]) if B >= 2 else 0
+    b = np.ascontiguousarray(best, np.int64).reshape(-1)
+    assert len(b) == nb, (len(b), nb)
+    n = int(ko[-1] - ko[0])
+    m = max(B, 1)
+    out = {"pose": np.zeros((m, 4)), "motion": np.zeros((m, 4)), "rms": np.zeros(m), "source": np.zeros(m, np.int32),
+           "status": np.zeros(m, np.int32), "n_inliers": np.zeros(m, np.int32), "n_hypotheses": np.zeros(m, np.int32),
+           "assoc": np.zeros(max(n, 1), np.int64)}
+    st = lib().feo_odometry(
+        _p(k) if len(k) else None, _p(ko), C.c_int32(B), _p(b) if nb else None, _p(so), C.c_int32(S), C.c_int32(window),
+        C.c_double(inlier_radius), C.c_double(min_separation), C.c_int32(max_hypotheses), C.c_int32(min_inliers),
+        C.c_int32(refine_iterations), _p(out["pose"]), _p(out["motion"]), _p(out["rms"]), _p(out["source"]),
+        _p(out["status"]), _p(out["n_inliers"]), _p(out["n_hypotheses"]), _p(out["assoc"]))
+    if st != 0:
+        raise ValueError("feo_odometry: invalid argument")
+    return {key: (v[:n] if key == "assoc" else v[:B]) for key, v in out.items()}
