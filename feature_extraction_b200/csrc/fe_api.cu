@@ -118,6 +118,34 @@ struct Slot {
   int nev = 0;
 };
 
+// The device and pinned buffers of a match, register or odometry call, carved by one layout (Carve): the results come
+// first at the same offsets in both, so that one copy brings them back; the pinned buffer ends with the tables the call
+// uploads, at their device offsets too.
+struct Workspace {
+  unsigned char* d = nullptr;
+  int64_t dCap = 0;  // bytes
+  unsigned char* h = nullptr;
+  int64_t hCap = 0;
+};
+
+// A typed array at a byte offset of a Workspace buffer.
+template <class T>
+struct Span {
+  int64_t off;
+  T* in(unsigned char* base) const { return (T*)(base + off); }
+};
+
+// Hands out consecutive 16-byte-aligned Spans; `bytes` is the running total.
+struct Carve {
+  int64_t bytes = 0;
+  template <class T>
+  Span<T> take(int64_t n) {
+    const Span<T> s{bytes};
+    bytes = (bytes + n * (int64_t)sizeof(T) + 15) & ~(int64_t)15;
+    return s;
+  }
+};
+
 }  // namespace
 
 struct fe_ctx {
@@ -157,32 +185,11 @@ struct fe_ctx {
   std::vector<const char*> stName;
   std::vector<float> stMs;
   int64_t launches = 0;
-  // fe_match_descriptors*: buffers of their own, so that a match call leaves the last batch call's results alone
-  float *d_matchQ = nullptr, *d_matchR = nullptr;  // uploaded rows of the host variant
-  int64_t capMatchQ = 0, capMatchR = 0;            // floats
-  fe_match::Item *h_items = nullptr, *d_items = nullptr;
-  int64_t capItemsHost = 0, capItems = 0;
-  fe_match::Partial* d_part = nullptr;
-  int64_t capPart = 0;
-  unsigned char* d_matchRes = nullptr;  // n_queries x {best int64 | dist2 | second_dist2 | shift}, as h_matchRes
-  long long* h_matchRes = nullptr;      // pinned, MATCH_RES_WORDS long longs per query
-  int64_t capMatchRes = 0, capMatchResHost = 0;  // queries
+  // fe_match_descriptors*, fe_register_matches* and fe_odometry*: a workspace per family, so that a call leaves the
+  // last batch call's results and the other families' results alone (fe_register_matches_device and
+  // fe_odometry_device may read `best` straight out of matchWs)
+  Workspace matchWs, regWs, odoWs;
   bool matchAttrs = false;
-  // fe_register_matches*: buffers of their own, so that a register call leaves the batch and match results alone
-  fe_point_t *d_regQ = nullptr, *d_regR = nullptr;  // uploaded keypoints of the host variant
-  int64_t capRegQ = 0, capRegR = 0;
-  long long* d_regBest = nullptr;                   // uploaded `best` of the host variant
-  int64_t capRegBest = 0;
-  int64_t* h_regOffs = nullptr;                     // pinned: query then reference offsets
-  int64_t *d_regOffs = nullptr, capRegOffsHost = 0, capRegOffs = 0;
-  unsigned char *d_regScratch = nullptr, *d_regRes = nullptr, *h_regRes = nullptr;  // results: reg_layout()
-  int64_t capRegScratch = 0, capRegRes = 0, capRegResHost = 0;  // bytes
-  // fe_odometry*: buffers of their own, so that an odometry call leaves the batch, match and register results alone
-  unsigned char *d_odoTab = nullptr, *h_odoTab = nullptr;    // ko | so | step offsets | step items of the call
-  unsigned char *d_odoWork = nullptr, *d_odoRes = nullptr, *h_odoRes = nullptr;  // per-step buffers; results: odo_layout()
-  fe_point_t* d_odoKp = nullptr;                             // uploaded keypoints of the host variant
-  long long* d_odoBest = nullptr;                            // uploaded `best` of the host variant
-  int64_t capOdoTab = 0, capOdoTabHost = 0, capOdoWork = 0, capOdoRes = 0, capOdoResHost = 0, capOdoKp = 0, capOdoBest = 0;
   std::string err;
 };
 
@@ -1203,12 +1210,10 @@ void fe_destroy(fe_ctx_t* ctx) {
   if (ctx->h_desc) cudaFreeHost(ctx->h_desc);
   if (ctx->h_cloud) cudaFreeHost(ctx->h_cloud);
   if (ctx->h_kc) cudaFreeHost(ctx->h_kc);
-  void* dm[] = {ctx->d_matchQ, ctx->d_matchR, ctx->d_items, ctx->d_part, ctx->d_matchRes,
-                ctx->d_regQ, ctx->d_regR, ctx->d_regBest, ctx->d_regOffs, ctx->d_regScratch, ctx->d_regRes,
-                ctx->d_odoTab, ctx->d_odoWork, ctx->d_odoRes, ctx->d_odoKp, ctx->d_odoBest};
-  for (void* p : dm) if (p) cudaFree(p);
-  void* hm[] = {ctx->h_items, ctx->h_matchRes, ctx->h_regOffs, ctx->h_regRes, ctx->h_odoTab, ctx->h_odoRes};
-  for (void* p : hm) if (p) cudaFreeHost(p);
+  for (Workspace* w : {&ctx->matchWs, &ctx->regWs, &ctx->odoWs}) {
+    if (w->d) cudaFree(w->d);
+    if (w->h) cudaFreeHost(w->h);
+  }
   delete ctx;
 }
 
@@ -1532,9 +1537,6 @@ int fe_download(fe_ctx_t* ctx, void* host_dst, const void* device_src, int64_t b
 
 namespace {
 
-// one query's result in h_matchRes / d_matchRes: best (8 B) | dist2 | second_dist2 | shift, as four arrays
-constexpr int MATCH_RES_WORDS = 3;  // long longs per query, 20 of the 24 bytes used
-
 template <class T>
 int grow_device(fe_ctx* ctx, T** buf, int64_t* cap, int64_t need) {
   if (need <= *cap) return FE_OK;
@@ -1545,6 +1547,25 @@ int grow_device(fe_ctx* ctx, T** buf, int64_t* cap, int64_t need) {
   return FE_OK;
 }
 
+// What a match, register or odometry call does once its arguments have passed: clear the last error, select the
+// context's device and hand out slot 0's stream (the stream only: the slot's buffers are not touched).
+int begin_call(fe_ctx* ctx, cudaStream_t* stream) {
+  ctx->err.clear();
+  CK(cudaSetDevice(ctx->device));
+  int st = ensure_slot(ctx, ctx->slot[0], false);
+  if (st) return st;
+  *stream = ctx->slot[0].stream;
+  return FE_OK;
+}
+
+// The host variant's upload: elements [first, first + n) of the caller's array p to dst, which p then points at.
+template <class T>
+int upload(fe_ctx* ctx, const T*& p, T* dst, int64_t first, int64_t n, cudaStream_t stream) {
+  if (n > 0) CK(cudaMemcpyAsync(dst, p + first, (size_t)n * sizeof(T), cudaMemcpyHostToDevice, stream));
+  p = dst;
+  return FE_OK;
+}
+
 const char* check_offsets(const int64_t* o, int32_t G) {
   if (o[0] < 0) return "negative entry";
   for (int32_t g = 0; g < G; g++)
@@ -1552,24 +1573,31 @@ const char* check_offsets(const int64_t* o, int32_t G) {
   return nullptr;
 }
 
+// The group checks of the match and register calls: n_groups, both offset arrays, rows on a side whose arrays are
+// missing (haveQ / haveR false; qName / rName name them) and the 2^31 query rows.  Sets the row counts *nQ and *nR.
+int check_groups(fe_ctx* ctx, int32_t G, const int64_t* qo, const int64_t* ro, bool haveQ, const char* qName, bool haveR,
+                 const char* rName, int64_t* nQ, int64_t* nR) {
+  if (G < 0) return fail(ctx, FE_ERR_INVALID, "n_groups must not be negative");
+  if (!qo || !ro) return fail(ctx, FE_ERR_INVALID, "query_offsets and ref_offsets need n_groups + 1 entries");
+  if (const char* e = check_offsets(qo, G)) return fail(ctx, FE_ERR_INVALID, std::string("query_offsets: ") + e);
+  if (const char* e = check_offsets(ro, G)) return fail(ctx, FE_ERR_INVALID, std::string("ref_offsets: ") + e);
+  *nQ = qo[G] - qo[0];
+  *nR = ro[G] - ro[0];
+  if (*nQ > 0 && !haveQ) return fail(ctx, FE_ERR_INVALID, std::string(qName) + " is NULL but there are query rows");
+  if (*nR > 0 && !haveR) return fail(ctx, FE_ERR_INVALID, std::string(rName) + " is NULL but there are reference rows");
+  if (*nQ >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 query rows");
+  return FE_OK;
+}
+
 // both entry points: rows q / r are device memory (onDevice) or host memory to upload
 int match_descriptors(fe_ctx* ctx, const float* q, int64_t qStride, const int64_t* qo, const float* r, int64_t rStride,
                       const int64_t* ro, int32_t G, fe_match_result_t* out, bool onDevice) {
   if (!ctx || !out) return FE_ERR_INVALID;
-  ctx->err.clear();
-  if (G < 0) return fail(ctx, FE_ERR_INVALID, "n_groups must not be negative");
   if (qStride < FE_DESC_LEN || rStride < FE_DESC_LEN) return fail(ctx, FE_ERR_INVALID, "a row stride is below FE_DESC_LEN");
-  if (!qo || !ro) return fail(ctx, FE_ERR_INVALID, "query_offsets and ref_offsets need n_groups + 1 entries");
-  if (const char* e = check_offsets(qo, G)) return fail(ctx, FE_ERR_INVALID, std::string("query_offsets: ") + e);
-  if (const char* e = check_offsets(ro, G)) return fail(ctx, FE_ERR_INVALID, std::string("ref_offsets: ") + e);
-  const int64_t nQ = qo[G] - qo[0], nR = ro[G] - ro[0];
-  if (nQ > 0 && !q) return fail(ctx, FE_ERR_INVALID, "query is NULL but there are query rows");
-  if (nR > 0 && !r) return fail(ctx, FE_ERR_INVALID, "ref is NULL but there are reference rows");
-  if (nQ >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 query rows");
-  CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], false);  // for its stream only: the slot's buffers are not touched
-  if (st) return st;
-  cudaStream_t stream = ctx->slot[0].stream;
+  int64_t nQ, nR;
+  if (int st = check_groups(ctx, G, qo, ro, q, "query", r, "ref", &nQ, &nR)) return st;
+  cudaStream_t stream;
+  if (int st = begin_call(ctx, &stream)) return st;
 
   // the work items (fe_match.h): per group, reference segment outer and query tile inner, so that the warps running at
   // one time share a segment of reference rows in L2
@@ -1580,26 +1608,32 @@ int match_descriptors(fe_ctx* ctx, const float* q, int64_t qStride, const int64_
     if (nq > 0) nItems += ((nq + QT - 1) / QT) * std::max<int64_t>((nr + RS - 1) / RS, 1);
   }
   if (nItems >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "too many query tiles x reference segments");
-  st = grow_pinned(ctx, &ctx->h_matchRes, &ctx->capMatchResHost, nQ, 4096, 0, MATCH_RES_WORDS);
+  Workspace& ws = ctx->matchWs;
+  Carve c;  // results (best at 0: fe_match_device_best) | items (uploaded) | partials and rows (device only)
+  const Span<int64_t> best = c.take<int64_t>(nQ);
+  const Span<float> dist2 = c.take<float>(nQ), second = c.take<float>(nQ);
+  const Span<int32_t> shift = c.take<int32_t>(nQ);
+  const int64_t resBytes = c.bytes;
+  const Span<fe_match::Item> items = c.take<fe_match::Item>(nItems);
+  const int64_t hostBytes = c.bytes;
+  int st = grow_pinned(ctx, &ws.h, &ws.hCap, hostBytes, 4096, 0);
   if (st) return st;
   out->n_queries = nQ;
-  long long* h = ctx->h_matchRes;
-  out->best = (const int64_t*)h;
-  out->dist2 = (const float*)(h + nQ);
-  out->second_dist2 = out->dist2 + nQ;
-  out->shift = (const int32_t*)(out->second_dist2 + nQ);
+  out->best = best.in(ws.h);
+  out->dist2 = dist2.in(ws.h);
+  out->second_dist2 = second.in(ws.h);
+  out->shift = shift.in(ws.h);
   if (nQ == 0) return FE_OK;
 
-  st = grow_pinned(ctx, &ctx->h_items, &ctx->capItemsHost, nItems, 4096, 0);
-  if (st) return st;
   int64_t nPart = 0, k = 0;
+  fe_match::Item* hItems = items.in(ws.h);
   for (int32_t g = 0; g < G; g++) {
     const int64_t nq = qo[g + 1] - qo[g], nr = ro[g + 1] - ro[g];
     if (nq == 0) continue;
     const int64_t nseg = std::max<int64_t>((nr + RS - 1) / RS, 1);
     for (int64_t sg = 0; sg < nseg; sg++)
       for (int64_t t = 0; t < nq; t += QT) {
-        fe_match::Item& I = ctx->h_items[k++];
+        fe_match::Item& I = hItems[k++];
         I.q0 = qo[g] + t;
         I.r0 = ro[g] + sg * RS;
         I.out = qo[g] + t - qo[0];
@@ -1611,35 +1645,33 @@ int match_descriptors(fe_ctx* ctx, const float* q, int64_t qStride, const int64_
       }
     if (nseg > 1) nPart += nq * nseg;
   }
+  const Span<fe_match::Partial> part = c.take<fe_match::Partial>(nPart);
+  // the host variant's rows [qo[0], qo[G]) and [ro[0], ro[G]); the last row of a side ends FE_DESC_LEN floats in
+  const int64_t qf = onDevice ? 0 : (nQ - 1) * qStride + FE_DESC_LEN, rf = onDevice || nR == 0 ? 0 : (nR - 1) * rStride + FE_DESC_LEN;
+  const Span<float> qRows = c.take<float>(qf), rRows = c.take<float>(rf);
+  if ((st = grow_device(ctx, &ws.d, &ws.dCap, c.bytes))) return st;
 
   if (!ctx->matchAttrs) {
     CK(fe_match::set_attributes());
     ctx->matchAttrs = true;
   }
   int64_t qBias = 0, rBias = 0;
-  if (!onDevice) {  // rows [qo[0], qo[G]) and [ro[0], ro[G]) only; the last row of a side ends FE_DESC_LEN floats in
-    const int64_t qf = (nQ - 1) * qStride + FE_DESC_LEN, rf = nR > 0 ? (nR - 1) * rStride + FE_DESC_LEN : 0;
-    if ((st = grow_device(ctx, &ctx->d_matchQ, &ctx->capMatchQ, qf))) return st;
-    if ((st = grow_device(ctx, &ctx->d_matchR, &ctx->capMatchR, rf))) return st;
-    CK(cudaMemcpyAsync(ctx->d_matchQ, q + qo[0] * qStride, (size_t)qf * sizeof(float), cudaMemcpyHostToDevice, stream));
-    if (rf > 0) CK(cudaMemcpyAsync(ctx->d_matchR, r + ro[0] * rStride, (size_t)rf * sizeof(float), cudaMemcpyHostToDevice, stream));
-    q = ctx->d_matchQ;
-    r = ctx->d_matchR;
+  if (!onDevice) {
+    if ((st = upload(ctx, q, qRows.in(ws.d), qo[0] * qStride, qf, stream))) return st;
+    if ((st = upload(ctx, r, rRows.in(ws.d), ro[0] * rStride, rf, stream))) return st;
     qBias = qo[0];
     rBias = ro[0];
   }
-  if ((st = grow_device(ctx, &ctx->d_items, &ctx->capItems, nItems))) return st;
-  if ((st = grow_device(ctx, &ctx->d_part, &ctx->capPart, std::max<int64_t>(nPart, 1)))) return st;
-  if ((st = grow_device(ctx, &ctx->d_matchRes, &ctx->capMatchRes, nQ * MATCH_RES_WORDS * 8))) return st;
-  CK(cudaMemcpyAsync(ctx->d_items, ctx->h_items, (size_t)nItems * sizeof(fe_match::Item), cudaMemcpyHostToDevice, stream));
+  CK(cudaMemcpyAsync(ws.d + resBytes, ws.h + resBytes, (size_t)(hostBytes - resBytes), cudaMemcpyHostToDevice, stream));
   fe_match::Result res;
-  res.best = (long long*)ctx->d_matchRes;
-  res.dist2 = (float*)(res.best + nQ);
-  res.second = res.dist2 + nQ;
-  res.shift = (int*)(res.second + nQ);
-  CK(fe_match::launch(q, qStride, qBias, r, rStride, rBias, ctx->d_items, (int)nItems, nPart > 0, ctx->d_part, res, stream));
+  res.best = (long long*)best.in(ws.d);
+  res.dist2 = dist2.in(ws.d);
+  res.second = second.in(ws.d);
+  res.shift = shift.in(ws.d);
+  CK(fe_match::launch(q, qStride, qBias, r, rStride, rBias, items.in(ws.d), (int)nItems, nPart > 0, part.in(ws.d), res,
+                      stream));
   ctx->launches += nPart > 0 ? 2 : 1;
-  CK(cudaMemcpyAsync(ctx->h_matchRes, ctx->d_matchRes, (size_t)nQ * 20, cudaMemcpyDeviceToHost, stream));
+  CK(cudaMemcpyAsync(ws.h, ws.d, (size_t)resBytes, cudaMemcpyDeviceToHost, stream));
   CK(cudaStreamSynchronize(stream));
   return FE_OK;
 }
@@ -1662,8 +1694,8 @@ int fe_match_descriptors_device(fe_ctx_t* ctx, const float* query, int64_t query
 
 int fe_match_device_best(fe_ctx_t* ctx, const int64_t** best) {
   if (!ctx || !best) return FE_ERR_INVALID;
-  if (!ctx->d_matchRes) return fail(ctx, FE_ERR_INVALID, "no match call has run on this context");
-  *best = (const int64_t*)ctx->d_matchRes;  // the first n_queries words of the match results (MATCH_RES_WORDS)
+  if (!ctx->matchWs.d) return fail(ctx, FE_ERR_INVALID, "no match call has run on this context");
+  *best = (const int64_t*)ctx->matchWs.d;  // match_descriptors carves `best` at offset 0
   return FE_OK;
 }
 
@@ -1681,24 +1713,6 @@ void fe_register_params_default(fe_register_params_t* p) {
 // ---- registration (fe_register.cu) -----------------------------------------------------------------------
 
 namespace {
-
-// The results of a register call in h_regRes / d_regRes, one copy: pose (G x 4) | rms (G) | assoc (nQ) as 8-byte words,
-// then n_inliers | n_hypotheses | status (G each) | the device's error flag as 4-byte words.
-struct RegLayout {
-  int64_t pose, rms, assoc, nInl, nHyp, status, err, bytes;
-};
-RegLayout reg_layout(int64_t G, int64_t nQ) {
-  RegLayout L;
-  L.pose = 0;
-  L.rms = L.pose + 32 * G;
-  L.assoc = L.rms + 8 * G;
-  L.nInl = L.assoc + 8 * nQ;
-  L.nHyp = L.nInl + 4 * G;
-  L.status = L.nHyp + 4 * G;
-  L.err = L.status + 4 * G;
-  L.bytes = L.err + 4;
-  return L;
-}
 
 // the parameter checks of the register and odometry calls, and the kernel's form of the parameters
 int register_params(fe_ctx* ctx, const fe_register_params_t* prm, fe_register::Params* kp) {
@@ -1726,19 +1740,12 @@ int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, cons
                      const int64_t* ro, int32_t G, const fe_register_params_t* prm, fe_register_result_t* out,
                      bool onDevice) {
   if (!ctx || !out) return FE_ERR_INVALID;
-  ctx->err.clear();
   fe_register::Params kp;
   if (int st = register_params(ctx, prm, &kp)) return st;
-  if (G < 0) return fail(ctx, FE_ERR_INVALID, "n_groups must not be negative");
-  if (!qo || !ro) return fail(ctx, FE_ERR_INVALID, "query_offsets and ref_offsets need n_groups + 1 entries");
-  if (const char* e = check_offsets(qo, G)) return fail(ctx, FE_ERR_INVALID, std::string("query_offsets: ") + e);
-  if (const char* e = check_offsets(ro, G)) return fail(ctx, FE_ERR_INVALID, std::string("ref_offsets: ") + e);
+  int64_t nQ, nR;
+  if (int st = check_groups(ctx, G, qo, ro, q && best, "query_kp or best", r, "ref_kp", &nQ, &nR)) return st;
   for (int32_t g = 0; g < G; g++)  // so that h * P of the hypothesis map fits 64 bits (P < 2^47, h < 2^16)
     if (qo[g + 1] - qo[g] >= (1LL << 24)) return fail(ctx, FE_ERR_INVALID, "a group has 2^24 or more query rows");
-  const int64_t nQ = qo[G] - qo[0], nR = ro[G] - ro[0];
-  if (nQ > 0 && (!q || !best)) return fail(ctx, FE_ERR_INVALID, "query_kp or best is NULL but there are query rows");
-  if (nR > 0 && !r) return fail(ctx, FE_ERR_INVALID, "ref_kp is NULL but there are reference rows");
-  if (nQ >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 query rows");
   if (!onDevice)
     for (int32_t g = 0; g < G; g++)
       for (int64_t k = qo[g]; k < qo[g + 1]; k++) {
@@ -1746,72 +1753,68 @@ int register_matches(fe_ctx* ctx, const fe_point_t* q, const fe_point_t* r, cons
         if (b != -1 && (b < ro[g] || b >= ro[g + 1]))
           return fail(ctx, FE_ERR_INVALID, "best[" + std::to_string(k - qo[0]) + "] is neither -1 nor a reference row of its group");
       }
-  CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], false);  // for its stream only: the slot's buffers are not touched
-  if (st) return st;
-  cudaStream_t stream = ctx->slot[0].stream;
+  cudaStream_t stream;
+  if (int st = begin_call(ctx, &stream)) return st;
 
-  const RegLayout L = reg_layout(G, nQ);
-  st = grow_pinned(ctx, &ctx->h_regRes, &ctx->capRegResHost, L.bytes, 4096, 0);
+  Workspace& ws = ctx->regWs;
+  Carve c;  // results | query then reference offsets (uploaded) | scratch and the host variant's rows (device only)
+  const Span<double> pose = c.take<double>(4 * (int64_t)G), rms = c.take<double>(G);
+  const Span<int64_t> assoc = c.take<int64_t>(nQ);
+  const Span<int32_t> nInl = c.take<int32_t>(G), nHyp = c.take<int32_t>(G), status = c.take<int32_t>(G);
+  const Span<int32_t> err = c.take<int32_t>(1);  // the device's error flag
+  const int64_t resBytes = c.bytes;
+  const Span<int64_t> offs = c.take<int64_t>(2 * ((int64_t)G + 1));
+  const int64_t hostBytes = c.bytes;
+  const Span<long long> assocNew = c.take<long long>(nQ);
+  const Span<double> d2Cur = c.take<double>(nQ), d2New = c.take<double>(nQ);
+  const Span<int32_t> corr = c.take<int32_t>(nQ);
+  const int64_t nUp = onDevice ? 0 : 1;  // the host variant's rows [qo[0], qo[G]) and [ro[0], ro[G]), and `best`
+  const Span<fe_point_t> qRows = c.take<fe_point_t>(nUp * nQ), rRows = c.take<fe_point_t>(nUp * nR);
+  const Span<int64_t> bestRows = c.take<int64_t>(nUp * nQ);
+  int st = grow_pinned(ctx, &ws.h, &ws.hCap, hostBytes, 4096, 0);
   if (st) return st;
-  unsigned char* h = ctx->h_regRes;
   out->n_groups = G;
   out->n_queries = nQ;
-  out->pose = (const double*)(h + L.pose);
-  out->rms = (const double*)(h + L.rms);
-  out->assoc = (const int64_t*)(h + L.assoc);
-  out->n_inliers = (const int32_t*)(h + L.nInl);
-  out->n_hypotheses = (const int32_t*)(h + L.nHyp);
-  out->status = (const int32_t*)(h + L.status);
+  out->pose = pose.in(ws.h);
+  out->rms = rms.in(ws.h);
+  out->assoc = assoc.in(ws.h);
+  out->n_inliers = nInl.in(ws.h);
+  out->n_hypotheses = nHyp.in(ws.h);
+  out->status = status.in(ws.h);
   if (G == 0) return FE_OK;
 
-  st = grow_pinned(ctx, &ctx->h_regOffs, &ctx->capRegOffsHost, 2 * (int64_t)(G + 1), 4096, 0);
-  if (st) return st;
-  memcpy(ctx->h_regOffs, qo, (size_t)(G + 1) * sizeof(int64_t));
-  memcpy(ctx->h_regOffs + G + 1, ro, (size_t)(G + 1) * sizeof(int64_t));
+  if ((st = grow_device(ctx, &ws.d, &ws.dCap, c.bytes))) return st;
+  memcpy(offs.in(ws.h), qo, (size_t)(G + 1) * sizeof(int64_t));
+  memcpy(offs.in(ws.h) + G + 1, ro, (size_t)(G + 1) * sizeof(int64_t));
   int64_t qBias = 0, rBias = 0;
-  if (!onDevice) {  // rows [qo[0], qo[G]) and [ro[0], ro[G]) only
-    if ((st = grow_device(ctx, &ctx->d_regQ, &ctx->capRegQ, std::max<int64_t>(nQ, 1)))) return st;
-    if ((st = grow_device(ctx, &ctx->d_regR, &ctx->capRegR, std::max<int64_t>(nR, 1)))) return st;
-    if ((st = grow_device(ctx, &ctx->d_regBest, &ctx->capRegBest, std::max<int64_t>(nQ, 1)))) return st;
-    if (nQ > 0) {
-      CK(cudaMemcpyAsync(ctx->d_regQ, q + qo[0], (size_t)nQ * sizeof(fe_point_t), cudaMemcpyHostToDevice, stream));
-      CK(cudaMemcpyAsync(ctx->d_regBest, best, (size_t)nQ * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
-    }
-    if (nR > 0) CK(cudaMemcpyAsync(ctx->d_regR, r + ro[0], (size_t)nR * sizeof(fe_point_t), cudaMemcpyHostToDevice, stream));
-    q = ctx->d_regQ;
-    r = ctx->d_regR;
-    best = (const int64_t*)ctx->d_regBest;
+  if (!onDevice) {
+    if ((st = upload(ctx, q, qRows.in(ws.d), qo[0], nQ, stream))) return st;
+    if ((st = upload(ctx, best, bestRows.in(ws.d), 0, nQ, stream))) return st;
+    if ((st = upload(ctx, r, rRows.in(ws.d), ro[0], nR, stream))) return st;
     qBias = qo[0];
     rBias = ro[0];
   }
-  const int64_t scratchBytes = std::max<int64_t>(nQ, 1) * (4 + 8 + 8 + 8);
-  if ((st = grow_device(ctx, &ctx->d_regOffs, &ctx->capRegOffs, 2 * (int64_t)(G + 1)))) return st;
-  if ((st = grow_device(ctx, &ctx->d_regScratch, &ctx->capRegScratch, scratchBytes))) return st;
-  if ((st = grow_device(ctx, &ctx->d_regRes, &ctx->capRegRes, L.bytes))) return st;
-  CK(cudaMemcpyAsync(ctx->d_regOffs, ctx->h_regOffs, (size_t)(2 * (G + 1)) * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
-  unsigned char* d = ctx->d_regRes;
-  CK(cudaMemsetAsync(d + L.err, 0, 4, stream));
+  CK(cudaMemcpyAsync(ws.d + resBytes, ws.h + resBytes, (size_t)(hostBytes - resBytes), cudaMemcpyHostToDevice, stream));
+  CK(cudaMemsetAsync(err.in(ws.d), 0, sizeof(int32_t), stream));
   fe_register::Out o;
-  o.pose = (double*)(d + L.pose);
-  o.rms = (double*)(d + L.rms);
-  o.assoc = (long long*)(d + L.assoc);
-  o.nInl = (int*)(d + L.nInl);
-  o.nHyp = (int*)(d + L.nHyp);
-  o.status = (int*)(d + L.status);
-  o.err = (int*)(d + L.err);
-  const int64_t n1 = std::max<int64_t>(nQ, 1);
-  fe_register::Scratch sc;  // 8-byte arrays first
-  sc.assocNew = (long long*)ctx->d_regScratch;
-  sc.d2Cur = (double*)(sc.assocNew + n1);
-  sc.d2New = sc.d2Cur + n1;
-  sc.corr = (int*)(sc.d2New + n1);
-  CK(fe_register::launch(q, qBias, r, rBias, (const long long*)best, ctx->d_regOffs, ctx->d_regOffs + G + 1, G, kp, o, sc,
+  o.pose = pose.in(ws.d);
+  o.rms = rms.in(ws.d);
+  o.assoc = (long long*)assoc.in(ws.d);
+  o.nInl = nInl.in(ws.d);
+  o.nHyp = nHyp.in(ws.d);
+  o.status = status.in(ws.d);
+  o.err = err.in(ws.d);
+  fe_register::Scratch sc;
+  sc.assocNew = assocNew.in(ws.d);
+  sc.d2Cur = d2Cur.in(ws.d);
+  sc.d2New = d2New.in(ws.d);
+  sc.corr = corr.in(ws.d);
+  CK(fe_register::launch(q, qBias, r, rBias, (const long long*)best, offs.in(ws.d), offs.in(ws.d) + G + 1, G, kp, o, sc,
                          stream));
   ctx->launches += 1;
-  CK(cudaMemcpyAsync(h, d, (size_t)L.bytes, cudaMemcpyDeviceToHost, stream));
+  CK(cudaMemcpyAsync(ws.h, ws.d, (size_t)resBytes, cudaMemcpyDeviceToHost, stream));
   CK(cudaStreamSynchronize(stream));
-  if (*(const int32_t*)(h + L.err)) return fail(ctx, FE_ERR_INVALID, "an entry of best is neither -1 nor a reference row of its group");
+  if (*err.in(ws.h)) return fail(ctx, FE_ERR_INVALID, "an entry of best is neither -1 nor a reference row of its group");
   return FE_OK;
 }
 
@@ -1837,33 +1840,10 @@ int fe_register_matches_device(fe_ctx_t* ctx, const fe_point_t* query_kp, const 
 
 namespace {
 
-int64_t align16(int64_t b) { return (b + 15) & ~(int64_t)15; }
-
-// The results of an odometry call in h_odoRes / d_odoRes, one copy: pose | motion (B x 4) | rms (B) as doubles, assoc
-// (n_rows) as 8-byte words, then source | status | n_inliers | n_hypotheses (B each) | the device's error flag.
-struct OdoLayout {
-  int64_t pose, motion, rms, assoc, source, status, nInl, nHyp, err, bytes;
-};
-OdoLayout odo_layout(int64_t B, int64_t nRows) {
-  OdoLayout L;
-  L.pose = 0;
-  L.motion = L.pose + 32 * B;
-  L.rms = L.motion + 32 * B;
-  L.assoc = L.rms + 8 * B;
-  L.source = L.assoc + 8 * nRows;
-  L.status = L.source + 4 * B;
-  L.nInl = L.status + 4 * B;
-  L.nHyp = L.nInl + 4 * B;
-  L.err = L.nHyp + 4 * B;
-  L.bytes = L.err + 4;
-  return L;
-}
-
 // both entry points: keypoints and `best` are device memory (onDevice) or host memory to upload
 int odometry(fe_ctx* ctx, const fe_point_t* kp, const int64_t* ko, int32_t B, const int64_t* best, const int64_t* so,
              int32_t S, int32_t W, const fe_register_params_t* prm, fe_odometry_result_t* out, bool onDevice) {
   if (!ctx || !out) return FE_ERR_INVALID;
-  ctx->err.clear();
   fe_register::Params rp;
   if (int st = register_params(ctx, prm, &rp)) return st;
   if (B < 0 || S < 0) return fail(ctx, FE_ERR_INVALID, "n_scans and n_sequences must not be negative");
@@ -1915,101 +1895,101 @@ int odometry(fe_ctx* ctx, const fe_point_t* kp, const int64_t* ko, int32_t B, co
         if (b != -1 && (b < ko[it.scan - 1] || b >= ko[it.scan]))
           return fail(ctx, FE_ERR_INVALID, "best[" + std::to_string(k - ko[1]) + "] is neither -1 nor a row of the previous scan");
       }
-  CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], false);  // for its stream only: the slot's buffers are not touched
-  if (st) return st;
-  cudaStream_t stream = ctx->slot[0].stream;
+  cudaStream_t stream;
+  if (int st = begin_call(ctx, &stream)) return st;
 
-  const OdoLayout L = odo_layout(B, nRows);
-  if ((st = grow_pinned(ctx, &ctx->h_odoRes, &ctx->capOdoResHost, L.bytes, 4096, 0))) return st;
-  unsigned char* h = ctx->h_odoRes;
+  Workspace& ws = ctx->odoWs;
+  Carve c;  // results | tables (uploaded) | the steps' work buffers and the host variant's rows (device only)
+  const Span<double> pose = c.take<double>(4 * (int64_t)B), motion = c.take<double>(4 * (int64_t)B), rms = c.take<double>(B);
+  const Span<int64_t> assoc = c.take<int64_t>(nRows);
+  const Span<int32_t> source = c.take<int32_t>(B), status = c.take<int32_t>(B), nInl = c.take<int32_t>(B);
+  const Span<int32_t> nHyp = c.take<int32_t>(B), err = c.take<int32_t>(1);  // err: the device's error flag
+  const int64_t resBytes = c.bytes;
+  const Span<int64_t> tKo = c.take<int64_t>((int64_t)B + 1), tSo = c.take<int64_t>((int64_t)S + 1);
+  const Span<int64_t> tOffs = c.take<int64_t>((int64_t)offs.size());
+  const Span<fe_odo::Item> tItems = c.take<fe_odo::Item>((int64_t)items.size());
+  const int64_t hostBytes = c.bytes;
+  // sized for the largest step
+  const int64_t maxG = 2 * maxN;
+  const Span<fe_point_t> wQ = c.take<fe_point_t>(maxQ), wR = c.take<fe_point_t>(maxR);
+  const Span<long long> wBest = c.take<long long>(maxQ), wAssoc = c.take<long long>(maxQ);
+  const Span<long long> wAssocNew = c.take<long long>(maxQ);
+  const Span<double> wD2Cur = c.take<double>(maxQ), wD2New = c.take<double>(maxQ);
+  const Span<int64_t> wWinLo = c.take<int64_t>(maxN);
+  const Span<double> wPose = c.take<double>(4 * maxG), wRms = c.take<double>(maxG);
+  const Span<int32_t> wCorr = c.take<int32_t>(maxQ), wNInl = c.take<int32_t>(maxG), wNHyp = c.take<int32_t>(maxG);
+  const Span<int32_t> wStatus = c.take<int32_t>(maxG);
+  // the host variant's rows [ko[0], ko[B]) and the `best` entries of the scans that are registered
+  const int64_t nBest = onDevice || bestRows == 0 || B < 2 ? 0 : ko[B] - ko[1];
+  const Span<fe_point_t> kpRows = c.take<fe_point_t>(onDevice ? 0 : nRows);
+  const Span<int64_t> bestUp = c.take<int64_t>(nBest);
+  int st = grow_pinned(ctx, &ws.h, &ws.hCap, hostBytes, 4096, 0);
+  if (st) return st;
   out->n_scans = B;
   out->n_rows = nRows;
-  out->pose = (const double*)(h + L.pose);
-  out->motion = (const double*)(h + L.motion);
-  out->rms = (const double*)(h + L.rms);
-  out->assoc = (const int64_t*)(h + L.assoc);
-  out->source = (const int32_t*)(h + L.source);
-  out->status = (const int32_t*)(h + L.status);
-  out->n_inliers = (const int32_t*)(h + L.nInl);
-  out->n_hypotheses = (const int32_t*)(h + L.nHyp);
+  out->pose = pose.in(ws.h);
+  out->motion = motion.in(ws.h);
+  out->rms = rms.in(ws.h);
+  out->assoc = assoc.in(ws.h);
+  out->source = source.in(ws.h);
+  out->status = status.in(ws.h);
+  out->n_inliers = nInl.in(ws.h);
+  out->n_hypotheses = nHyp.in(ws.h);
   out->gpu_launches = 0;
   if (B == 0) return FE_OK;
 
-  // tables: ko | so | offsets of every step | items
-  const int64_t tKo = 0, tSo = tKo + 8 * (B + 1), tOffs = tSo + 8 * ((int64_t)S + 1);
-  const int64_t tItems = tOffs + 8 * (int64_t)offs.size(), tBytes = tItems + 8 * (int64_t)items.size();
-  if ((st = grow_pinned(ctx, &ctx->h_odoTab, &ctx->capOdoTabHost, tBytes, 4096, 0))) return st;
-  if ((st = grow_device(ctx, &ctx->d_odoTab, &ctx->capOdoTab, tBytes))) return st;
-  memcpy(ctx->h_odoTab + tKo, ko, 8 * ((size_t)B + 1));
-  memcpy(ctx->h_odoTab + tSo, so, 8 * ((size_t)S + 1));
-  if (!offs.empty()) memcpy(ctx->h_odoTab + tOffs, offs.data(), 8 * offs.size());
-  if (!items.empty()) memcpy(ctx->h_odoTab + tItems, items.data(), 8 * items.size());
-  CK(cudaMemcpyAsync(ctx->d_odoTab, ctx->h_odoTab, (size_t)tBytes, cudaMemcpyHostToDevice, stream));
+  if ((st = grow_device(ctx, &ws.d, &ws.dCap, c.bytes))) return st;
+  memcpy(tKo.in(ws.h), ko, 8 * ((size_t)B + 1));
+  memcpy(tSo.in(ws.h), so, 8 * ((size_t)S + 1));
+  if (!offs.empty()) memcpy(tOffs.in(ws.h), offs.data(), 8 * offs.size());
+  if (!items.empty()) memcpy(tItems.in(ws.h), items.data(), sizeof(fe_odo::Item) * items.size());
+  CK(cudaMemcpyAsync(ws.d + resBytes, ws.h + resBytes, (size_t)(hostBytes - resBytes), cudaMemcpyHostToDevice, stream));
   fe_odo::Tables T;
-  T.ko = (const int64_t*)(ctx->d_odoTab + tKo);
-  T.so = (const int64_t*)(ctx->d_odoTab + tSo);
-  T.offs = (int64_t*)(ctx->d_odoTab + tOffs);
-  T.items = (const fe_odo::Item*)(ctx->d_odoTab + tItems);
-
-  // work buffers, sized for the largest step: 16-byte rows first, then 8-byte, then 4-byte arrays
-  const int64_t maxG = 2 * maxN;
-  const int64_t wQ = 0, wR = wQ + 16 * maxQ, wBest = wR + 16 * maxR, wAssoc = wBest + 8 * maxQ;
-  const int64_t wAssocNew = wAssoc + 8 * maxQ, wD2Cur = wAssocNew + 8 * maxQ, wD2New = wD2Cur + 8 * maxQ;
-  const int64_t wWinLo = wD2New + 8 * maxQ, wPose = wWinLo + 8 * maxN, wRms = wPose + 32 * maxG;
-  const int64_t wCorr = wRms + 8 * maxG, wNInl = wCorr + 4 * maxQ, wNHyp = wNInl + 4 * maxG, wStatus = wNHyp + 4 * maxG;
-  const int64_t wBytes = align16(wStatus + 4 * maxG);
-  if ((st = grow_device(ctx, &ctx->d_odoWork, &ctx->capOdoWork, wBytes))) return st;
-  if ((st = grow_device(ctx, &ctx->d_odoRes, &ctx->capOdoRes, L.bytes))) return st;
-  unsigned char* wb = ctx->d_odoWork;
-  unsigned char* d = ctx->d_odoRes;
+  T.ko = tKo.in(ws.d);
+  T.so = tSo.in(ws.d);
+  T.offs = tOffs.in(ws.d);
+  T.items = tItems.in(ws.d);
   fe_odo::Out o;
-  o.pose = (double*)(d + L.pose);
-  o.motion = (double*)(d + L.motion);
-  o.rms = (double*)(d + L.rms);
-  o.assoc = (long long*)(d + L.assoc);
-  o.source = (int*)(d + L.source);
-  o.status = (int*)(d + L.status);
-  o.nInl = (int*)(d + L.nInl);
-  o.nHyp = (int*)(d + L.nHyp);
-  o.err = (int*)(d + L.err);
+  o.pose = pose.in(ws.d);
+  o.motion = motion.in(ws.d);
+  o.rms = rms.in(ws.d);
+  o.assoc = (long long*)assoc.in(ws.d);
+  o.source = source.in(ws.d);
+  o.status = status.in(ws.d);
+  o.nInl = nInl.in(ws.d);
+  o.nHyp = nHyp.in(ws.d);
+  o.err = err.in(ws.d);
   fe_odo::Work w;
-  w.q = (fe_point_t*)(wb + wQ);
-  w.r = (fe_point_t*)(wb + wR);
-  w.best = (long long*)(wb + wBest);
-  w.winLo = (int64_t*)(wb + wWinLo);
-  w.reg.pose = (double*)(wb + wPose);
-  w.reg.rms = (double*)(wb + wRms);
-  w.reg.assoc = (long long*)(wb + wAssoc);
-  w.reg.nInl = (int*)(wb + wNInl);
-  w.reg.nHyp = (int*)(wb + wNHyp);
-  w.reg.status = (int*)(wb + wStatus);
+  w.q = wQ.in(ws.d);
+  w.r = wR.in(ws.d);
+  w.best = wBest.in(ws.d);
+  w.winLo = wWinLo.in(ws.d);
+  w.reg.pose = wPose.in(ws.d);
+  w.reg.rms = wRms.in(ws.d);
+  w.reg.assoc = wAssoc.in(ws.d);
+  w.reg.nInl = wNInl.in(ws.d);
+  w.reg.nHyp = wNHyp.in(ws.d);
+  w.reg.status = wStatus.in(ws.d);
   w.reg.err = o.err;
-  w.scratch.corr = (int*)(wb + wCorr);
-  w.scratch.assocNew = (long long*)(wb + wAssocNew);
-  w.scratch.d2Cur = (double*)(wb + wD2Cur);
-  w.scratch.d2New = (double*)(wb + wD2New);
+  w.scratch.corr = wCorr.in(ws.d);
+  w.scratch.assocNew = wAssocNew.in(ws.d);
+  w.scratch.d2Cur = wD2Cur.in(ws.d);
+  w.scratch.d2New = wD2New.in(ws.d);
 
   int64_t kpBias = 0;
-  if (!onDevice) {  // rows [ko[0], ko[B]) and the `best` entries of the scans that are registered
-    if ((st = grow_device(ctx, &ctx->d_odoKp, &ctx->capOdoKp, std::max<int64_t>(nRows, 1)))) return st;
-    if (nRows > 0) CK(cudaMemcpyAsync(ctx->d_odoKp, kp + ko[0], (size_t)nRows * sizeof(fe_point_t), cudaMemcpyHostToDevice, stream));
-    const int64_t nBest = B >= 2 ? ko[B] - ko[1] : 0;
-    if ((st = grow_device(ctx, &ctx->d_odoBest, &ctx->capOdoBest, std::max<int64_t>(nBest, 1)))) return st;
-    if (nBest > 0 && bestRows > 0)
-      CK(cudaMemcpyAsync(ctx->d_odoBest, best, (size_t)nBest * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
-    kp = ctx->d_odoKp;
-    best = (const int64_t*)ctx->d_odoBest;
+  if (!onDevice) {
+    if ((st = upload(ctx, kp, kpRows.in(ws.d), ko[0], nRows, stream))) return st;
+    if ((st = upload(ctx, best, bestUp.in(ws.d), 0, nBest, stream))) return st;
     kpBias = ko[0];
   }
-  CK(cudaMemsetAsync(d + L.err, 0, 4, stream));
+  CK(cudaMemsetAsync(o.err, 0, sizeof(int32_t), stream));
   CK(fe_odo::run(kp, kpBias, (const long long*)best, S, W, steps, T, w, o, rp, stream));
   const int64_t launches = S > 0 ? 1 + 3 * (int64_t)steps.size() : 0;
   ctx->launches += launches;
   out->gpu_launches = launches;
-  CK(cudaMemcpyAsync(h, d, (size_t)L.bytes, cudaMemcpyDeviceToHost, stream));
+  CK(cudaMemcpyAsync(ws.h, ws.d, (size_t)resBytes, cudaMemcpyDeviceToHost, stream));
   CK(cudaStreamSynchronize(stream));
-  if (*(const int32_t*)(h + L.err)) return fail(ctx, FE_ERR_INVALID, "an entry of best is neither -1 nor a row of the previous scan");
+  if (*err.in(ws.h)) return fail(ctx, FE_ERR_INVALID, "an entry of best is neither -1 nor a row of the previous scan");
   return FE_OK;
 }
 

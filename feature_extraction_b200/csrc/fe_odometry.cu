@@ -21,9 +21,7 @@ namespace fe_odo {
 
 constexpr int WARPS = 4;  // warps per block, each on its own sequence
 
-struct Motion {
-  double c, s, tx, ty;
-};
+using fe_register::Motion;
 
 __device__ __forceinline__ Motion load(const double* m) { return Motion{m[0], m[1], m[2], m[3]}; }
 

@@ -21,10 +21,6 @@ namespace fe_register {
 constexpr int WARPS = 4;  // warps per block (independent: each runs its own group)
 constexpr unsigned FULL = 0xffffffffu;
 
-struct Motion {
-  double c, s, tx, ty;
-};
-
 // row i of an array whose first element is row `bias`
 __device__ __forceinline__ void xy(const fe_point_t* p, int64_t bias, int64_t i, double& x, double& y) {
   x = (double)__ldg(&p[i - bias].x);

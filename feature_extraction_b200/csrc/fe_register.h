@@ -8,6 +8,11 @@
 
 namespace fe_register {
 
+// A planar motion (x, y) -> (c x - s y + tx, s x + c y + ty), as the kernels of fe_register.cu and fe_odometry.cu use it.
+struct Motion {
+  double c, s, tx, ty;
+};
+
 struct Params {
   double r2, sep2, twoR;  // inlier_radius^2, min_separation^2, 2 * inlier_radius
   int maxH, minInliers, refine;

@@ -90,12 +90,17 @@ def _match_offsets(query_offsets, ref_offsets, n_query, n_ref):
     return qo, ro, len(qo) - 1
 
 
+def _copy_out(p, shape, dtype):
+    """A copy of a result array at p: the context reuses that memory in its next call of the same kind."""
+    if int(np.prod(shape)) == 0:
+        return np.zeros(shape, dtype)
+    return np.ctypeslib.as_array(p, shape=shape).copy()
+
+
 def _unpack_match(res):
-    n = int(res.n_queries)
-    if n == 0:
-        return np.zeros(0, np.int64), np.zeros(0, np.int32), np.zeros(0, np.float32), np.zeros(0, np.float32)
-    return (np.ctypeslib.as_array(res.best, shape=(n,)).copy(), np.ctypeslib.as_array(res.shift, shape=(n,)).copy(),
-            np.ctypeslib.as_array(res.dist2, shape=(n,)).copy(), np.ctypeslib.as_array(res.second_dist2, shape=(n,)).copy())
+    n = (int(res.n_queries),)
+    return (_copy_out(res.best, n, np.int64), _copy_out(res.shift, n, np.int32), _copy_out(res.dist2, n, np.float32),
+            _copy_out(res.second_dist2, n, np.float32))
 
 
 def register_params_default(**overrides):
@@ -118,27 +123,17 @@ def _keypoint_rows(a):
 
 def _unpack_register(res):
     G, n = int(res.n_groups), int(res.n_queries)
-
-    def arr(p, shape, dtype):
-        if int(np.prod(shape)) == 0:
-            return np.zeros(shape, dtype)
-        return np.ctypeslib.as_array(p, shape=shape).copy()
-    return {"pose": arr(res.pose, (G, 4), np.float64), "rms": arr(res.rms, (G,), np.float64),
-            "n_inliers": arr(res.n_inliers, (G,), np.int32), "n_hypotheses": arr(res.n_hypotheses, (G,), np.int32),
-            "status": arr(res.status, (G,), np.int32), "assoc": arr(res.assoc, (n,), np.int64)}
+    return {"pose": _copy_out(res.pose, (G, 4), np.float64), "rms": _copy_out(res.rms, (G,), np.float64),
+            "n_inliers": _copy_out(res.n_inliers, (G,), np.int32), "n_hypotheses": _copy_out(res.n_hypotheses, (G,), np.int32),
+            "status": _copy_out(res.status, (G,), np.int32), "assoc": _copy_out(res.assoc, (n,), np.int64)}
 
 
 def _unpack_odometry(res):
     B, n = int(res.n_scans), int(res.n_rows)
-
-    def arr(p, shape, dtype):
-        if int(np.prod(shape)) == 0:
-            return np.zeros(shape, dtype)
-        return np.ctypeslib.as_array(p, shape=shape).copy()
-    return {"pose": arr(res.pose, (B, 4), np.float64), "motion": arr(res.motion, (B, 4), np.float64),
-            "rms": arr(res.rms, (B,), np.float64), "source": arr(res.source, (B,), np.int32),
-            "status": arr(res.status, (B,), np.int32), "n_inliers": arr(res.n_inliers, (B,), np.int32),
-            "n_hypotheses": arr(res.n_hypotheses, (B,), np.int32), "assoc": arr(res.assoc, (n,), np.int64)}
+    return {"pose": _copy_out(res.pose, (B, 4), np.float64), "motion": _copy_out(res.motion, (B, 4), np.float64),
+            "rms": _copy_out(res.rms, (B,), np.float64), "source": _copy_out(res.source, (B,), np.int32),
+            "status": _copy_out(res.status, (B,), np.int32), "n_inliers": _copy_out(res.n_inliers, (B,), np.int32),
+            "n_hypotheses": _copy_out(res.n_hypotheses, (B,), np.int32), "assoc": _copy_out(res.assoc, (n,), np.int64)}
 
 
 def _odometry_offsets(keypoint_offsets, sequence_offsets, n_rows):

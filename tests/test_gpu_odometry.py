@@ -9,7 +9,7 @@ import pytest
 from match_oracle import binding as mo
 from odometry_cases import constructed, oracle_chain, scan_pairs_best
 from register_cases import oracle_params, sequence
-from util import to_fe_params
+from util import bits_equal, to_fe_params
 
 pytestmark = pytest.mark.gpu
 
@@ -134,7 +134,18 @@ def test_device_chain_equals_the_host_entry_point(ob, synth):
 
 
 def test_register_and_odometry_results_leave_each_other_alone(node):
+    """The host results of a match, a register and an odometry call each survive the other two kinds of call."""
     from feature_extraction_b200 import _native as N
+    from match_cases import constructed as match_case, random_rows
+    rng = np.random.default_rng(25)
+    mq, mr, mqo, mro = match_case(rng)
+    m_res = N.MatchResult()
+    assert N.lib().fe_match_descriptors(node._ctx, mq.ctypes.data_as(C.c_void_p), mq.shape[1], mqo.ctypes.data_as(C.c_void_p),
+                                        mr.ctypes.data_as(C.c_void_p), mr.shape[1], mro.ctypes.data_as(C.c_void_p),
+                                        len(mqo) - 1, C.byref(m_res)) == N.FE_OK
+    from feature_extraction_b200.node import _unpack_match, _unpack_odometry, _unpack_register
+    match_before = _unpack_match(m_res)
+    same_match = lambda a, b_: all(np.array_equal(x.view(np.uint8), y.view(np.uint8)) for x, y in zip(a, b_))  # noqa: E731
     kp, ko, best, so, _, _ = constructed()
     b = scan_pairs_best(ko, best, so)
     res = N.RegisterResult()
@@ -143,8 +154,8 @@ def test_register_and_odometry_results_leave_each_other_alone(node):
     assert N.lib().fe_register_matches(node._ctx, kp.ctypes.data_as(C.c_void_p), kp.ctypes.data_as(C.c_void_p),
                                        b.ctypes.data_as(C.c_void_p), qo.ctypes.data_as(C.c_void_p),
                                        ro.ctypes.data_as(C.c_void_p), len(qo) - 1, C.byref(prm), C.byref(res)) == N.FE_OK
-    from feature_extraction_b200.node import _unpack_odometry, _unpack_register
     reg_before = _unpack_register(res)
+    assert same_match(_unpack_match(m_res), match_before)  # the match results survive a register call
     odo_res = N.OdometryResult()
     so_ = so.copy()
     assert N.lib().fe_odometry(node._ctx, kp.ctypes.data_as(C.c_void_p), ko.ctypes.data_as(C.c_void_p), len(ko) - 1,
@@ -153,10 +164,18 @@ def test_register_and_odometry_results_leave_each_other_alone(node):
     odo_before = _unpack_odometry(odo_res)
     assert_reg = lambda a, b_: all(np.array_equal(a[k], b_[k]) for k in a)  # noqa: E731
     assert assert_reg(_unpack_register(res), reg_before)  # the register results survive an odometry call
+    assert same_match(_unpack_match(m_res), match_before)  # and so do the match results
     node.registerMatches(kp, kp, b, qo, ro)
     assert_same(_unpack_odometry(odo_res), odo_before)  # and the odometry results a register call
+    # a larger match call, which grows the match buffers: the register and odometry results survive it
+    node.matchDescriptors(random_rows(rng, 300), random_rows(rng, 2000))
+    assert assert_reg(_unpack_register(res), reg_before)
+    assert_same(_unpack_odometry(odo_res), odo_before)
     assert_same(odo_before, mo.odometry(kp, ko, best, so, 2))
     assert assert_reg(reg_before, mo.register_matches(kp, kp, b, qo, ro))
+    m_ora = mo.match_descriptors(mq, mr, mqo, mro)
+    assert all(np.array_equal(x, y) for x, y in zip(match_before[:2], m_ora[:2]))
+    assert all(bits_equal(x, y) for x, y in zip(match_before[2:], m_ora[2:]))
 
 
 def test_invalid_arguments_leave_the_context_usable(node):
