@@ -64,10 +64,47 @@ struct GraphEntry {
   int64_t launches = 0;
 };
 
+// A device buffer and a pinned buffer carved by one layout (Carve).  A slot has one per group of its arrays.  A match,
+// register or odometry call has one of its own, whose results come first at the same offsets in both, so that one copy
+// brings them back; the pinned buffer ends with the tables the call uploads, at their device offsets too.
+struct Workspace {
+  unsigned char* d = nullptr;
+  int64_t dCap = 0;  // bytes
+  unsigned char* h = nullptr;
+  int64_t hCap = 0;
+};
+
+// A typed array at a byte offset of a Workspace buffer.
+template <class T>
+struct Span {
+  int64_t off;
+  T* in(unsigned char* base) const { return (T*)(base + off); }
+};
+
+// Hands out consecutive `align`-byte-aligned Spans; `bytes` is the running total.
+struct Carve {
+  int64_t align = 16;
+  int64_t bytes = 0;
+  template <class T>
+  Span<T> take(int64_t n) {
+    const Span<T> s{bytes};
+    bytes = (bytes + n * (int64_t)sizeof(T) + align - 1) & ~(align - 1);
+    return s;
+  }
+};
+
+// The groups of a slot's arrays, one per lifetime (slot_arrays lists each group's arrays).  Opening a slot (open_slot)
+// makes its stream and events only; ensure_group allocates a group in full when a call first needs it.
+enum Group { CORE, POINTS, FULL, CLOUDS, REPORT, GRID, NGROUPS };
+
+// Rule: no array that a captured graph can name is moved or freed before the slot is destroyed (free_slot).  A group
+// is allocated once, in full, and never grown.  GraphKey depends on this: a replay finds every array where the
+// capture saw it.  The context's pinned result buffers may grow (grow_pinned): they are copied into outside any graph.
 struct Slot {
   cudaStream_t stream = nullptr;
   SubBatch sb;  // the sub-batch in flight (or the last one)
   std::vector<GraphEntry> graphs;
+  Workspace group[NGROUPS];
   int64_t capPts = 0;
   int capScans = 0, capChunks = 0;
   int64_t capKp = 0;
@@ -90,11 +127,9 @@ struct Slot {
   int *h_cloudOff = nullptr, *h_kcOff = nullptr;     // pinned: per-scan offsets of the two cloud outputs of the sub-batch
   unsigned char* d_gridHdr = nullptr;  // per-scan index of the halo cell grid (bit map, word prefix, slot table)
   int* d_tabOk = nullptr;
-  int64_t capGridHdr = 0;
   int *d_ringBase = nullptr, *d_ovfRuns = nullptr, *d_scanFlag = nullptr;  // K2: ring segment offsets per scan, rings for the wide run kernel
   int *d_ovfRings = nullptr, *d_ovfRings2 = nullptr, *d_ovfMerge = nullptr, *d_ovfMerge2 = nullptr, *d_ovfSurf = nullptr;
   unsigned char* d_slabs = nullptr;
-  int64_t capRowStart = 0;
   float4 *d_kfPool = nullptr, *d_kcPool = nullptr, *d_kpPool = nullptr, *d_kpOut = nullptr, *d_gather = nullptr;
   float* d_desc = nullptr;
   DevCounters* d_ctr = nullptr;
@@ -116,34 +151,6 @@ struct Slot {
   std::vector<cudaEvent_t> ev;
   std::vector<const char*> evName;
   int nev = 0;
-};
-
-// The device and pinned buffers of a match, register or odometry call, carved by one layout (Carve): the results come
-// first at the same offsets in both, so that one copy brings them back; the pinned buffer ends with the tables the call
-// uploads, at their device offsets too.
-struct Workspace {
-  unsigned char* d = nullptr;
-  int64_t dCap = 0;  // bytes
-  unsigned char* h = nullptr;
-  int64_t hCap = 0;
-};
-
-// A typed array at a byte offset of a Workspace buffer.
-template <class T>
-struct Span {
-  int64_t off;
-  T* in(unsigned char* base) const { return (T*)(base + off); }
-};
-
-// Hands out consecutive 16-byte-aligned Spans; `bytes` is the running total.
-struct Carve {
-  int64_t bytes = 0;
-  template <class T>
-  Span<T> take(int64_t n) {
-    const Span<T> s{bytes};
-    bytes = (bytes + n * (int64_t)sizeof(T) + 15) & ~(int64_t)15;
-    return s;
-  }
 };
 
 }  // namespace
@@ -280,6 +287,10 @@ void leveling_matrix(double roll, double pitch, float m[9]) {
 
 int bits_for_host(int v) { int b = 0; while (v > 0) { b++; v >>= 1; } return b; }
 
+// cells of the descriptor grid along x and along y at most: surface_grid clamps to it, and the GRID group's row starts
+// are sized by it
+constexpr int SURF_GRID_MAX = 2048;
+
 // surface keep-box and 2-D grid for keypoints known to lie inside [x0,x1]x[y0,y1]x[z0,z1]
 void surface_grid(DevParams& dp, double R, float x0, float x1, float y0, float y1, float z0, float z1) {
   const double rrho = R / 5.0;
@@ -290,12 +301,12 @@ void surface_grid(DevParams& dp, double R, float x0, float x1, float y0, float y
   float cell = (float)(rrho * 1.001);
   if (!(cell > 1e-6f)) cell = 1e-6f;
   const float ex = dp.sx1 - dp.sx0, ey = dp.sy1 - dp.sy0;
-  const float maxdim = 2047.0f;
+  const float maxdim = (float)(SURF_GRID_MAX - 1);
   if (ex / cell > maxdim) cell = ex / maxdim;
   if (ey / cell > maxdim) cell = ey / maxdim;
   dp.sg_inv = 1.0f / cell;
-  dp.sg_nx = std::max(1, std::min(2048, (int)floorf(ex * dp.sg_inv) + 1));
-  dp.sg_ny = std::max(1, std::min(2048, (int)floorf(ey * dp.sg_inv) + 1));
+  dp.sg_nx = std::max(1, std::min(SURF_GRID_MAX, (int)floorf(ex * dp.sg_inv) + 1));
+  dp.sg_ny = std::max(1, std::min(SURF_GRID_MAX, (int)floorf(ey * dp.sg_inv) + 1));
   dp.sg_bx = std::max(1, bits_for_host(dp.sg_nx - 1));
   dp.Rpad = (float)(R * 1.0001 + 1e-6);
   dp.rhopad = (float)(rrho * 1.0001 + 1e-6);
@@ -340,15 +351,15 @@ cudaError_t dalloc(T** p, size_t n) { return cudaMalloc((void**)p, std::max<size
 template <class T>
 cudaError_t halloc(T** p, size_t n) { return cudaHostAlloc((void**)p, std::max<size_t>(n, 1) * sizeof(T), cudaHostAllocDefault); }
 
+void free_ws(Workspace& w) {
+  if (w.d) cudaFree(w.d);
+  if (w.h) cudaFreeHost(w.h);
+  w = Workspace();
+}
+
 void free_slot(Slot& s) {
-  void* dv[] = {s.d_ringPts, s.d_pts, s.d_surf, s.d_crop, s.d_sorted, s.d_full, s.d_cropMeta, s.d_keyA, s.d_keyB, s.d_valA, s.d_valB,
-                s.d_sortedKey, s.d_rho, s.d_scan_off, s.d_chunk_off, s.d_surfCnt, s.d_cropCnt, s.d_rot, s.d_kfBase,
-                s.d_kfCnt, s.d_kcBase, s.d_kcCnt, s.d_kpBase, s.d_kpCnt, s.d_kpOff, s.d_kpScan, s.d_kpNbr, s.d_kpNbrOff, s.d_kpRank, s.d_kpListM, s.d_kpListL, s.d_rowStart,
-                s.d_surfN, s.d_perScan, s.d_outOff, s.d_ovfRings, s.d_ovfRings2, s.d_ovfMerge, s.d_ovfMerge2, s.d_ovfSurf, s.d_slabs, s.d_gridHdr, s.d_tabOk, s.d_kfPool, s.d_kcPool, s.d_kpPool, s.d_kpOut, s.d_gather, s.d_desc, s.d_ctr, s.d_boundary, s.d_gate, s.d_ringBase, s.d_ovfRuns, s.d_scanFlag, s.d_perScan2, s.d_outOff2, s.d_gather2, s.d_chunkTab};
-  for (void* p : dv) if (p) cudaFree(p);
-  void* hv[] = {s.h_scan_off, s.h_chunk_off, s.h_rot, s.h_ctr, s.h_kpOff, s.h_perScan, s.h_boundary, s.h_cloudOff, s.h_kcOff};
-  for (void* p : hv) if (p) cudaFreeHost(p);
-  for (cudaEvent_t e : s.ev) cudaEventDestroy(e);
+  for (Workspace& w : s.group) free_ws(w);
+  for (cudaEvent_t e : s.ev) if (e) cudaEventDestroy(e);
   for (GraphEntry& g : s.graphs) if (g.exec) cudaGraphExecDestroy(g.exec);
   if (s.evDone) cudaEventDestroy(s.evDone);
   if (s.evT0) cudaEventDestroy(s.evT0);
@@ -357,52 +368,130 @@ void free_slot(Slot& s) {
   s = Slot();
 }
 
-int ensure_slot(fe_ctx* ctx, Slot& s, bool ownPoints) {
-  if (s.stream) {
-    if (ownPoints && !s.d_pts) CK(dalloc(&s.d_pts, (size_t)s.capPts));
-    return FE_OK;
-  }
+// A slot's stream, its events and its capacities, nothing else.  The stream is made last: a slot with a stream is open.
+int open_slot(fe_ctx* ctx, Slot& s) {
+  if (s.stream) return FE_OK;
   const fe_limits_t& L = ctx->lim;
   s.capPts = L.max_points_per_call;
   s.capScans = L.max_scans_per_call;
   s.capChunks = (int)(s.capPts / CH) + s.capScans + 1;
   s.capKp = L.max_keypoints_per_call;
   s.capKf = (int)L.max_ring_clusters_per_call;
-  s.capKc = 0;
-  CK(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-  CK(cudaEventCreateWithFlags(&s.evDone, cudaEventDisableTiming));
-  CK(cudaEventCreate(&s.evT0));
-  CK(cudaEventCreate(&s.evT1));
-  const size_t np = (size_t)s.capPts, ns = (size_t)s.capScans;
-  if (ownPoints) CK(dalloc(&s.d_pts, np));
-  CK(dalloc(&s.d_surf, np)); CK(dalloc(&s.d_crop, np)); CK(dalloc(&s.d_sorted, np)); CK(dalloc(&s.d_ringPts, np));
-  CK(dalloc(&s.d_cropMeta, np)); CK(dalloc(&s.d_keyA, np)); CK(dalloc(&s.d_keyB, np));
-  CK(dalloc(&s.d_valA, np)); CK(dalloc(&s.d_valB, np)); CK(dalloc(&s.d_sortedKey, np));
-  CK(dalloc(&s.d_rho, np));
-  CK(dalloc(&s.d_scan_off, ns + 1)); CK(dalloc(&s.d_chunk_off, ns + 1));
-  CK(dalloc(&s.d_surfCnt, (size_t)s.capChunks)); CK(dalloc(&s.d_cropCnt, (size_t)s.capChunks));
-  CK(dalloc(&s.d_chunkTab, (size_t)s.capChunks));
-  CK(dalloc(&s.d_rot, ns * 9));
-  CK(dalloc(&s.d_kfBase, ns * 16)); CK(dalloc(&s.d_kfCnt, ns * 16));
-  CK(dalloc(&s.d_kcBase, ns * 16)); CK(dalloc(&s.d_kcCnt, ns * 16));
-  CK(dalloc(&s.d_kpBase, ns)); CK(dalloc(&s.d_kpCnt, ns)); CK(dalloc(&s.d_kpOff, ns + 1));
-  CK(dalloc(&s.d_kpScan, (size_t)s.capKp)); CK(dalloc(&s.d_kpNbr, (size_t)s.capKp));
-  CK(dalloc(&s.d_kpNbrOff, (size_t)s.capKp)); CK(dalloc(&s.d_kpRank, (size_t)s.capKp));
-  CK(dalloc(&s.d_kpListM, (size_t)s.capKp)); CK(dalloc(&s.d_kpListL, (size_t)s.capKp));
-  CK(dalloc(&s.d_surfN, ns)); CK(dalloc(&s.d_perScan, ns)); CK(dalloc(&s.d_outOff, ns + 1)); CK(dalloc(&s.d_tabOk, ns));
-  CK(dalloc(&s.d_ringBase, ns * 17)); CK(dalloc(&s.d_ovfRuns, ns * 16)); CK(dalloc(&s.d_scanFlag, ns));
-  CK(dalloc(&s.d_ovfRings, ns)); CK(dalloc(&s.d_ovfRings2, ns)); CK(dalloc(&s.d_ovfMerge, ns)); CK(dalloc(&s.d_ovfMerge2, ns));
-  CK(dalloc(&s.d_ovfSurf, ns));
-  CK(dalloc(&s.d_slabs, (size_t)NGLOBAL * cluster_slab_bytes(ECAP_G)));
-  CK(dalloc(&s.d_kfPool, (size_t)s.capKf)); CK(dalloc(&s.d_kpPool, (size_t)s.capKp)); CK(dalloc(&s.d_kpOut, (size_t)s.capKp));
-  CK(dalloc(&s.d_desc, (size_t)s.capKp * FE_RECORD_FLOATS));  // room for either output layout
-  CK(dalloc(&s.d_ctr, 1));
-  CK(halloc(&s.h_scan_off, ns + 1)); CK(halloc(&s.h_chunk_off, ns + 1)); CK(halloc(&s.h_rot, ns * 9));
-  CK(halloc(&s.h_ctr, 1)); CK(halloc(&s.h_kpOff, ns + 1)); CK(halloc(&s.h_perScan, ns + 1));
-  s.ev.resize(24);
-  for (auto& e : s.ev) CK(cudaEventCreate(&e));
+  s.capKc = (int)std::min<int64_t>(s.capPts, 1 << 26);
+  s.ev.assign(24, nullptr);
   s.evName.assign(24, "");
+  cudaError_t e = cudaEventCreateWithFlags(&s.evDone, cudaEventDisableTiming);
+  for (cudaEvent_t* t : {&s.evT0, &s.evT1}) if (e == cudaSuccess) e = cudaEventCreate(t);
+  for (cudaEvent_t& t : s.ev) if (e == cudaSuccess) e = cudaEventCreate(&t);
+  cudaStream_t stream = nullptr;
+  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking);
+  if (e != cudaSuccess) {
+    free_slot(s);
+    cudaGetLastError();
+    return fail(ctx, FE_ERR_CUDA, std::string("opening a slot: ") + cudaGetErrorString(e));
+  }
+  s.stream = stream;
   return FE_OK;
+}
+
+// Lays out one group of a slot's arrays at 256 bytes, the alignment cudaMalloc gives: without bases it only adds up
+// the bytes of the device and the pinned buffer; with them it also points the slot's arrays into the buffers.
+struct GroupCarve {
+  Carve d{256}, h{256};
+  unsigned char *dBase = nullptr, *hBase = nullptr;
+  template <class T>
+  void dev(T*& p, int64_t n) { const Span<T> a = d.take<T>(n); if (dBase) p = a.in(dBase); }
+  template <class T>
+  void pin(T*& p, int64_t n) { const Span<T> a = h.take<T>(n); if (hBase) p = a.in(hBase); }
+};
+
+// Every array of the slot's group g, with its element count: the one list that sizes the group and sets its pointers.
+void slot_arrays(Slot& s, Group g, GroupCarve& c) {
+  const int64_t np = s.capPts, ns = s.capScans, nkp = s.capKp;
+  switch (g) {
+    case CORE:  // everything the pipeline sizes from the limits
+      c.dev(s.d_surf, np); c.dev(s.d_crop, np); c.dev(s.d_sorted, np); c.dev(s.d_ringPts, np);
+      c.dev(s.d_cropMeta, np); c.dev(s.d_keyA, np); c.dev(s.d_keyB, np);
+      c.dev(s.d_valA, np); c.dev(s.d_valB, np); c.dev(s.d_sortedKey, np);
+      c.dev(s.d_rho, np);
+      c.dev(s.d_scan_off, ns + 1); c.dev(s.d_chunk_off, ns + 1);
+      c.dev(s.d_surfCnt, s.capChunks); c.dev(s.d_cropCnt, s.capChunks);
+      c.dev(s.d_chunkTab, s.capChunks);
+      c.dev(s.d_rot, ns * 9);
+      c.dev(s.d_kfBase, ns * 16); c.dev(s.d_kfCnt, ns * 16);
+      c.dev(s.d_kcBase, ns * 16); c.dev(s.d_kcCnt, ns * 16);
+      c.dev(s.d_kpBase, ns); c.dev(s.d_kpCnt, ns); c.dev(s.d_kpOff, ns + 1);
+      c.dev(s.d_kpScan, nkp); c.dev(s.d_kpNbr, nkp);
+      c.dev(s.d_kpNbrOff, nkp); c.dev(s.d_kpRank, nkp);
+      c.dev(s.d_kpListM, nkp); c.dev(s.d_kpListL, nkp);
+      c.dev(s.d_surfN, ns); c.dev(s.d_perScan, ns); c.dev(s.d_outOff, ns + 1); c.dev(s.d_tabOk, ns);
+      c.dev(s.d_ringBase, ns * 17); c.dev(s.d_ovfRuns, ns * 16); c.dev(s.d_scanFlag, ns);
+      c.dev(s.d_ovfRings, ns); c.dev(s.d_ovfRings2, ns); c.dev(s.d_ovfMerge, ns); c.dev(s.d_ovfMerge2, ns);
+      c.dev(s.d_ovfSurf, ns);
+      c.dev(s.d_slabs, (int64_t)NGLOBAL * cluster_slab_bytes(ECAP_G));
+      c.dev(s.d_kfPool, s.capKf); c.dev(s.d_kpPool, nkp); c.dev(s.d_kpOut, nkp);
+      c.dev(s.d_desc, nkp * FE_RECORD_FLOATS);  // room for either output layout
+      c.dev(s.d_ctr, 1);
+      c.pin(s.h_scan_off, ns + 1); c.pin(s.h_chunk_off, ns + 1); c.pin(s.h_rot, ns * 9);
+      c.pin(s.h_ctr, 1); c.pin(s.h_kpOff, ns + 1); c.pin(s.h_perScan, ns + 1);
+      break;
+    case POINTS:  // host points staged for the pipeline (fe_process_batch_device reads the caller's array instead)
+      c.dev(s.d_pts, np);
+      break;
+    case FULL:  // fe_get_elevation_angles, fe_rotate_cloud
+      c.dev(s.d_full, np);
+      break;
+    case CLOUDS:  // the two cloud outputs and the keypoint_cloud pool
+      c.dev(s.d_kcPool, s.capKc); c.dev(s.d_gather, np); c.dev(s.d_gather2, s.capKc);
+      c.dev(s.d_perScan2, ns); c.dev(s.d_outOff2, ns + 1);
+      c.pin(s.h_cloudOff, ns + 1); c.pin(s.h_kcOff, ns + 1);
+      break;
+    case REPORT:  // the boundary report
+      c.dev(s.d_boundary, ns * FE_BOUNDARY_KINDS); c.dev(s.d_gate, ns * 16);
+      c.pin(s.h_boundary, ns * FE_BOUNDARY_KINDS);
+      break;
+    case GRID:  // rows of every grid surface_grid can make; headers of every grid the counting sort takes
+      c.dev(s.d_rowStart, ns * (SURF_GRID_MAX + 1)); c.dev(s.d_gridHdr, ns * grid_hdr_bytes(SURF_MAX_CELLS));
+      break;
+    case NGROUPS: break;
+  }
+}
+
+// Allocates group g of an open slot, once and in full.  Its arrays are set only when both of its buffers exist; on a
+// failure nothing is held, the CUDA error is cleared (a later launch check must not report it) and the next call tries
+// again.
+int ensure_group(fe_ctx* ctx, Slot& s, Group g) {
+  Workspace& w = s.group[g];
+  if (w.d) return FE_OK;  // every group has device arrays
+  GroupCarve c;
+  slot_arrays(s, g, c);
+  unsigned char *d = nullptr, *h = nullptr;
+  cudaError_t e = cudaMalloc((void**)&d, (size_t)c.d.bytes);
+  if (e == cudaSuccess && c.h.bytes > 0) {
+    e = cudaHostAlloc((void**)&h, (size_t)c.h.bytes, cudaHostAllocDefault);
+    if (e != cudaSuccess) cudaFree(d);
+  }
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    char b[160];
+    snprintf(b, sizeof b, "slot arrays of %lld device and %lld pinned bytes: %s", (long long)c.d.bytes, (long long)c.h.bytes,
+             cudaGetErrorString(e));
+    return fail(ctx, FE_ERR_CUDA, b);
+  }
+  w = Workspace{d, c.d.bytes, h, c.h.bytes};
+  GroupCarve set;
+  set.dBase = d;
+  set.hBase = h;
+  slot_arrays(s, g, set);
+  return FE_OK;
+}
+
+// Opens the slot and allocates `groups` in the order given.
+int ensure_slot(fe_ctx* ctx, Slot& s, std::initializer_list<Group> groups) {
+  int st = open_slot(ctx, s);
+  for (Group g : groups)
+    if (st == FE_OK) st = ensure_group(ctx, s, g);
+  return st;
 }
 
 void mark(fe_ctx* ctx, Slot& s, const char* name) {
@@ -471,26 +560,6 @@ int stage_scans(fe_ctx* ctx, Slot& s, const int64_t* offs, const double* rp, int
   return FE_OK;
 }
 
-// P: the parameters whose descriptor grid the surface index of the launches will use
-int ensure_rowstart(fe_ctx* ctx, Slot& s, const DevParams& P, int nscans) {
-  const int64_t need = (int64_t)std::max(nscans, s.capScans) * (P.sg_ny + 1);
-  if (need > s.capRowStart) {
-    if (s.d_rowStart) { CK(cudaStreamSynchronize(s.stream)); CK(cudaFree(s.d_rowStart)); s.d_rowStart = nullptr; }
-    CK(dalloc(&s.d_rowStart, (size_t)need));
-    s.capRowStart = need;
-  }
-  const int64_t ncells = (int64_t)P.sg_nx * P.sg_ny;
-  if (ncells <= SURF_MAX_CELLS) {
-    const int64_t needT = (int64_t)std::max(nscans, s.capScans) * grid_hdr_bytes((int)ncells);
-    if (needT > s.capGridHdr) {
-      if (s.d_gridHdr) { CK(cudaStreamSynchronize(s.stream)); CK(cudaFree(s.d_gridHdr)); s.d_gridHdr = nullptr; }
-      CK(dalloc(&s.d_gridHdr, (size_t)needT));
-      s.capGridHdr = needT;
-    }
-  }
-  return FE_OK;
-}
-
 SurfIndex surf_index(const DevParams& P, const Slot& s) {
   const int64_t ncells = (int64_t)P.sg_nx * P.sg_ny;
   SurfIndex X;
@@ -500,20 +569,6 @@ SurfIndex surf_index(const DevParams& P, const Slot& s) {
   X.gridStride = grid_hdr_bytes((int)ncells);
   X.tabOk = s.d_tabOk;
   return X;
-}
-
-int ensure_kc(fe_ctx* ctx, Slot& s) {
-  if (s.capKc == 0) {
-    s.capKc = (int)std::min<int64_t>(s.capPts, 1 << 26);
-    CK(dalloc(&s.d_kcPool, (size_t)s.capKc));
-    CK(dalloc(&s.d_gather, (size_t)s.capPts));
-    CK(dalloc(&s.d_gather2, (size_t)s.capKc));
-    CK(dalloc(&s.d_perScan2, (size_t)s.capScans));
-    CK(dalloc(&s.d_outOff2, (size_t)s.capScans + 1));
-    CK(halloc(&s.h_cloudOff, (size_t)s.capScans + 1));
-    CK(halloc(&s.h_kcOff, (size_t)s.capScans + 1));
-  }
-  return FE_OK;
 }
 
 const size_t kClusterSmem = cluster_smem_bytes(ECAP, NTF);
@@ -746,15 +801,6 @@ BoundarySpec boundary_spec(const fe_ctx* ctx) {
   return B;
 }
 
-int ensure_bnd(fe_ctx* ctx, Slot& s) {
-  if (!s.d_boundary) {
-    CK(dalloc(&s.d_boundary, (size_t)s.capScans * FE_BOUNDARY_KINDS));
-    CK(halloc(&s.h_boundary, (size_t)s.capScans * FE_BOUNDARY_KINDS));
-    CK(dalloc(&s.d_gate, (size_t)s.capScans * 16));
-  }
-  return FE_OK;
-}
-
 // Enqueue the kernels of the slot's sub-batch s.sb, K1 to K4d, and the copies of its counters, keypoint offsets and
 // boundary counts to the pinned mirrors; its scan offsets must be on the device already (stage_scans_copy).  With
 // `lateRp` the levelling matrices are computed here, interleaved with K1.  recordDone: record the slot's evDone.
@@ -799,8 +845,6 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
   const bool allKinds = kinds == FE_BOUNDARY_KINDS;
   const BoundarySpec B = boundary_spec(ctx);
   if (kinds) {
-    int st = ensure_bnd(ctx, s);
-    if (st) return st;
     CK(cudaMemsetAsync(s.d_boundary, 0, (size_t)nscans * FE_BOUNDARY_KINDS * sizeof(unsigned long long), s.stream));
     k_boundary_rings<<<nscans, 256, 0, s.stream>>>(s.d_crop, s.d_cropMeta, s.d_cropCnt, s.d_scan_off, s.d_chunk_off, 0, B, s.d_boundary);
     ctx->launches++;
@@ -813,10 +857,6 @@ int enqueue_pipeline(fe_ctx* ctx, Slot& s, const double* lateRp, bool recordDone
       else k_boundary_crop_ring<false><<<nch, 256, 0, s.stream>>>(sb.pts, s.d_chunkTab, s.d_rot, P, sb.lay, B.eps, s.d_boundary);
       ctx->launches++;
     }
-  }
-  if (sb.desc) {
-    int st = ensure_rowstart(ctx, s, P, nscans);
-    if (st) return st;
   }
   if (allKinds) launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean, GateCount{B.eps, s.d_gate});
   else launch_clustering(ctx, s, nscans, false, sb.wantKc, true, true, sb.lean);
@@ -942,9 +982,13 @@ int lean_rerun_if_deferred(fe_ctx* ctx, Slot& s) {
 // lean_rerun_if_deferred repairs the rare miss.
 int enqueue_subbatch(fe_ctx* ctx, Slot& s, const SubBatch& sb, const double* lateRp, const void* upload = nullptr,
                      size_t bytes = 0) {
+  // every group the pipeline may need is allocated before it is enqueued, so never while a capture runs
+  int st = sb.desc ? ensure_group(ctx, s, GRID) : FE_OK;
+  if (st == FE_OK && ctx->bndKinds) st = ensure_group(ctx, s, REPORT);
+  if (st == FE_OK && sb.wantKc) st = ensure_group(ctx, s, CLOUDS);
+  if (st) return st;
   s.sb = sb;
   s.sb.lean = false;
-  int st;
   if (lateRp || !ctx->useGraphs || ctx->stageTiming || sb.nscans > GRAPH_MAX_SCANS) {
     // offsets and chunk table ahead of the points: with the points first, 10k scans through fe_process_batch took
     // 49 instead of 43 ms on a B200 (1,000 W)
@@ -954,9 +998,6 @@ int enqueue_subbatch(fe_ctx* ctx, Slot& s, const SubBatch& sb, const double* lat
     return enqueue_pipeline(ctx, s, lateRp, true);
   }
   if (bytes) CK(cudaMemcpyAsync(s.d_pts, upload, bytes, cudaMemcpyHostToDevice, s.stream));
-  // every allocation the pipeline may need happens before a capture starts
-  if (sb.desc) { st = ensure_rowstart(ctx, s, ctx->dp, sb.nscans); if (st) return st; }
-  if (ctx->bndKinds) { st = ensure_bnd(ctx, s); if (st) return st; }
   s.sb.lean = ctx->leanHold == 0;
   if (ctx->leanHold > 0) ctx->leanHold--;
   const GraphKey key = {s.sb, density_blocks_per_scan(sb.nscans, sb.npts), s.maxScanPts > 65535, ctx->bndKinds, ctx->epoch};
@@ -1210,10 +1251,7 @@ void fe_destroy(fe_ctx_t* ctx) {
   if (ctx->h_desc) cudaFreeHost(ctx->h_desc);
   if (ctx->h_cloud) cudaFreeHost(ctx->h_cloud);
   if (ctx->h_kc) cudaFreeHost(ctx->h_kc);
-  for (Workspace* w : {&ctx->matchWs, &ctx->regWs, &ctx->odoWs}) {
-    if (w->d) cudaFree(w->d);
-    if (w->h) cudaFreeHost(w->h);
-  }
+  for (Workspace* w : {&ctx->matchWs, &ctx->regWs, &ctx->odoWs}) free_ws(*w);
   delete ctx;
 }
 
@@ -1340,7 +1378,7 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
   int nsub = 0;
   while (first < n_scans) {
     Slot& s = ctx->slot[cur];
-    int st = ensure_slot(ctx, s, true);
+    int st = ensure_slot(ctx, s, {CORE, POINTS});
     if (st) return st;
     // previous sub-batch of this slot must have been finalised (its device buffers are reused)
     st = finalize_subbatch(ctx, s, kpRun);
@@ -1361,7 +1399,6 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
     sb.lay = RawLayout{isFloat4 ? nullptr : (const unsigned char*)s.d_pts, stride, xo, yo, zo};
     st = stage_scans(ctx, s, scan_offsets + first, roll_pitch + 2 * first, sb.nscans, &sb.npts, &sb.nch);
     if (st) return st;
-    if (sb.wantKc) { st = ensure_kc(ctx, s); if (st) return st; }
     st = enqueue_subbatch(ctx, s, sb, nullptr, points + scan_offsets[first] * (int64_t)stride, (size_t)npts * (size_t)stride);
     if (st) return st;
     s.busy = true; s.firstScan = first;
@@ -1445,7 +1482,7 @@ int fe_process_batch_device(fe_ctx_t* ctx, const fe_point_t* d_points, const int
   const bool desc = ctx->params.estimate_descriptors != 0;
   const int64_t launches0 = ctx->launches;
   Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, false);
+  int st = ensure_slot(ctx, s, {CORE});
   if (st) return st;
   ctx->kpOffsets.assign((size_t)n_scans + 1, 0);
   if (n_scans > 0) {
@@ -1477,7 +1514,7 @@ int fe_process_batch_device(fe_ctx_t* ctx, const fe_point_t* d_points, const int
 int fe_timer_begin(fe_ctx_t* ctx) {
   if (!ctx) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], false);
+  int st = open_slot(ctx, ctx->slot[0]);
   if (st) return st;
   CK(cudaEventRecord(ctx->slot[0].evT0, ctx->slot[0].stream));
   return FE_OK;
@@ -1493,7 +1530,7 @@ int fe_timer_end(fe_ctx_t* ctx, float* elapsed_ms) {
 }
 
 int fe_get_batch_stats(fe_ctx_t* ctx, int64_t out[10]) {
-  if (!ctx || !out || !ctx->slot[0].stream) return FE_ERR_INVALID;
+  if (!ctx || !out || !ctx->slot[0].h_ctr) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
   Slot& s = ctx->slot[0];
   CK(cudaStreamSynchronize(s.stream));
@@ -1548,11 +1585,11 @@ int grow_device(fe_ctx* ctx, T** buf, int64_t* cap, int64_t need) {
 }
 
 // What a match, register or odometry call does once its arguments have passed: clear the last error, select the
-// context's device and hand out slot 0's stream (the stream only: the slot's buffers are not touched).
+// context's device and hand out slot 0's stream (the slot is opened; none of its arrays are allocated).
 int begin_call(fe_ctx* ctx, cudaStream_t* stream) {
   ctx->err.clear();
   CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], false);
+  int st = open_slot(ctx, ctx->slot[0]);
   if (st) return st;
   *stream = ctx->slot[0].stream;
   return FE_OK;
@@ -2013,10 +2050,9 @@ int fe_odometry_device(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypo
 
 // Upload a one-scan cloud and run K1 on it with `flags` and the parameters P, levelled by rp = {roll, pitch} (null:
 // the identity).  K1 compacts its survivors into the chunk pieces; with fullOut it also writes every point, transformed
-// in place, to s.d_full, which is copied to fullOut before this returns.
+// in place, to s.d_full (group FULL), which is copied to fullOut before this returns.
 static int scan_k1(fe_ctx* ctx, Slot& s, const DevParams& P, const fe_point_t* in, int64_t n, int flags,
                    const double* rp = nullptr, fe_point_t* fullOut = nullptr) {
-  if (fullOut && !s.d_full) CK(dalloc(&s.d_full, (size_t)s.capPts));
   int64_t offs[2] = {0, n};
   int64_t npts; int nch;
   int st = stage_scans(ctx, s, offs, rp, 1, &npts, &nch);
@@ -2040,7 +2076,7 @@ static int scan_k1(fe_ctx* ctx, Slot& s, const DevParams& P, const fe_point_t* i
 int fe_get_elevation_angles(fe_ctx_t* ctx, fe_point_t* cloud, int64_t n) {
   if (!ctx || (n > 0 && !cloud) || n < 0) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], true);
+  int st = ensure_slot(ctx, ctx->slot[0], {CORE, POINTS, FULL});
   if (st || n == 0) return st;
   const double rp[2] = {0.0, 0.0};
   return scan_k1(ctx, ctx->slot[0], ctx->dp, cloud, n, F_ELEV, rp, cloud);
@@ -2049,7 +2085,7 @@ int fe_get_elevation_angles(fe_ctx_t* ctx, fe_point_t* cloud, int64_t n) {
 int fe_rotate_cloud(fe_ctx_t* ctx, fe_point_t* cloud, int64_t n, double roll, double pitch) {
   if (!ctx || (n > 0 && !cloud) || n < 0) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
-  int st = ensure_slot(ctx, ctx->slot[0], true);
+  int st = ensure_slot(ctx, ctx->slot[0], {CORE, POINTS, FULL});
   if (st || n == 0) return st;
   const double rp[2] = {roll, pitch};
   return scan_k1(ctx, ctx->slot[0], ctx->dp, cloud, n, F_ROT, rp, cloud);
@@ -2075,9 +2111,7 @@ int fe_filter_cloud(fe_ctx_t* ctx, const fe_point_t* in, int64_t n, fe_point_t* 
   if (n_out) *n_out = 0;
   if (n == 0) return FE_OK;
   Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, true);
-  if (st) return st;
-  st = ensure_kc(ctx, s);
+  int st = ensure_slot(ctx, s, {CORE, POINTS, CLOUDS});
   if (st) return st;
   st = scan_k1(ctx, s, ctx->dp, in, n, F_CROP);
   if (st) return st;
@@ -2099,7 +2133,7 @@ int fe_extract_clusters(fe_ctx_t* ctx, const fe_point_t* cloud, int64_t n, doubl
   if (n > ECAP_G) return fail(ctx, FE_ERR_CAPACITY, "fe_extract_clusters: more than 65535 points");
   if (!(tolerance > 0.0)) return fail(ctx, FE_ERR_INVALID, "tolerance must be > 0");
   Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, true);
+  int st = ensure_slot(ctx, s, {CORE, POINTS});
   if (st) return st;
   if (n > s.capPts) return fail(ctx, FE_ERR_CAPACITY, "fe_extract_clusters: more points than max_points_per_call");
   CK(cudaMemcpyAsync(s.d_pts, cloud, (size_t)n * sizeof(float4), cudaMemcpyHostToDevice, s.stream));
@@ -2135,9 +2169,7 @@ static int stage_keypoints(fe_ctx* ctx, const fe_point_t* cloud, int64_t n, bool
   if (nKc) *nKc = 0;
   if (n == 0) return FE_OK;
   Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, true);
-  if (st) return st;
-  st = ensure_kc(ctx, s);
+  int st = ensure_slot(ctx, s, {CORE, POINTS, CLOUDS});
   if (st) return st;
   st = scan_k1(ctx, s, ctx->dp, cloud, n, singleRing ? 0 : F_RING);
   if (st) return st;
@@ -2188,7 +2220,7 @@ int fe_estimate_descriptors(fe_ctx_t* ctx, const fe_point_t* cloud_full, int64_t
   CK(cudaSetDevice(ctx->device));
   if (k == 0) return FE_OK;  // src:331-332
   Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, true);
+  int st = ensure_slot(ctx, s, {CORE, POINTS, GRID});
   if (st) return st;
   if (k > s.capKp) return fail(ctx, FE_ERR_CAPACITY, "more keypoints than max_keypoints_per_call");
   // the search surface only matters around the keypoints: grid over their bounding box
@@ -2202,8 +2234,6 @@ int fe_estimate_descriptors(fe_ctx_t* ctx, const fe_point_t* cloud_full, int64_t
   DevParams P = ctx->dp;
   surface_grid(P, ctx->params.descriptor_radius, lo[0], hi[0], lo[1], hi[1], lo[2], hi[2]);
   st = scan_k1(ctx, s, P, cloud_full, n, F_SURF);  // n == 0: one empty scan
-  if (st) return st;
-  st = ensure_rowstart(ctx, s, P, 1);
   if (st) return st;
   cudaStream_t q = s.stream;
   std::vector<int> kpOff = {0, (int)k};
@@ -2393,7 +2423,7 @@ int fe_multi_process_batch(fe_multi_t* m, const fe_point_t* points, const int64_
 // bench hook: work of the 3DSC density stage of the last device call: out = {distance tests, marked surface points
 // (distinct points inside some keypoint's support sphere), halo points kept by the cell grid}
 int fe_debug_density_work(fe_ctx_t* ctx, int64_t out[3]) {
-  if (!ctx || !out || !ctx->slot[0].stream) return FE_ERR_INVALID;
+  if (!ctx || !out || !ctx->slot[0].h_ctr) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
   Slot& s = ctx->slot[0];
   CK(cudaStreamSynchronize(s.stream));
@@ -2414,7 +2444,7 @@ int fe_debug_h2d_probe(fe_ctx_t* ctx, const void* host, int64_t bytes, float* ms
   if (!ctx || !host || bytes < 0 || !ms) return FE_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
   Slot& s = ctx->slot[0];
-  int st = ensure_slot(ctx, s, true);
+  int st = ensure_slot(ctx, s, {POINTS});
   if (st) return st;
   const int64_t chunk = s.capPts * (int64_t)sizeof(float4);
   CK(cudaStreamSynchronize(s.stream));
