@@ -30,6 +30,7 @@ EXPORTS = [
     "fe_match_descriptors", "fe_match_descriptors_device",
     "fe_register_params_default", "fe_register_matches", "fe_register_matches_device", "fe_match_device_best",
     "fe_odometry", "fe_odometry_device",
+    "fe_loop_params_default", "fe_loop_closures", "fe_loop_closures_device",
 ]
 
 ODOMETRY_WINDOW = 2  # FE_ODOMETRY_WINDOW_DEFAULT
@@ -113,6 +114,36 @@ class RegisterResult(C.Structure):
         ("n_hypotheses", C.POINTER(C.c_int32)),
         ("status", C.POINTER(C.c_int32)),
         ("assoc", C.POINTER(C.c_int64)),
+    ]
+
+
+class LoopParams(C.Structure):
+    """fe_loop_params_t: a scan's database ends min_gap scans before it; candidates verified per scan, in [1, 16]."""
+    _fields_ = [("min_gap", C.c_int32), ("candidates", C.c_int32)]
+
+
+class LoopResult(C.Structure):
+    """fe_loop_result_t: per scan its loop (rank, scan, motion, rms, counts), per scan x candidate the retrieval and
+    verification outputs, per row its inlier in the loop scan."""
+    _fields_ = [
+        ("n_scans", C.c_int32),
+        ("candidates", C.c_int32),
+        ("n_rows", C.c_int64),
+        ("loop", C.POINTER(C.c_int32)),
+        ("loop_scan", C.POINTER(C.c_int32)),
+        ("pose", C.POINTER(C.c_double)),
+        ("rms", C.POINTER(C.c_double)),
+        ("n_inliers", C.POINTER(C.c_int32)),
+        ("n_hypotheses", C.POINTER(C.c_int32)),
+        ("cand_scan", C.POINTER(C.c_int32)),
+        ("cand_votes", C.POINTER(C.c_int32)),
+        ("cand_status", C.POINTER(C.c_int32)),
+        ("cand_inliers", C.POINTER(C.c_int32)),
+        ("cand_hypotheses", C.POINTER(C.c_int32)),
+        ("cand_rms", C.POINTER(C.c_double)),
+        ("cand_pose", C.POINTER(C.c_double)),
+        ("assoc", C.POINTER(C.c_int64)),
+        ("gpu_launches", C.c_int64),
     ]
 
 
@@ -212,6 +243,11 @@ def lib():
         for f in (L.fe_odometry, L.fe_odometry_device):
             f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                           C.POINTER(RegisterParams), C.POINTER(OdometryResult)]
+        L.fe_loop_params_default.argtypes = [C.POINTER(LoopParams)]
+        L.fe_loop_params_default.restype = None
+        for f in (L.fe_loop_closures, L.fe_loop_closures_device):
+            f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32,
+                          C.POINTER(LoopParams), C.POINTER(RegisterParams), C.POINTER(LoopResult)]
         L.fe_debug_enable_graphs.argtypes = [C.c_void_p, C.c_int32, C.POINTER(C.c_int64)]
         L.fe_debug_lean_reruns.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
         L.fe_debug_density_work.argtypes = [C.c_void_p, C.c_void_p]

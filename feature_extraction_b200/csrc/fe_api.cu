@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "fe_kernels.cuh"
+#include "fe_loop.h"
 #include "fe_match.h"
 #include "fe_odometry.h"
 #include "fe_register.h"
@@ -65,7 +66,7 @@ struct GraphEntry {
 };
 
 // A device buffer and a pinned buffer carved by one layout (Carve).  A slot has one per group of its arrays.  A match,
-// register or odometry call has one of its own, whose results come first at the same offsets in both, so that one copy
+// register, odometry or loop-closure call has one of its own, whose results come first at the same offsets in both, so that one copy
 // brings them back; the pinned buffer ends with the tables the call uploads, at their device offsets too.
 struct Workspace {
   unsigned char* d = nullptr;
@@ -192,10 +193,10 @@ struct fe_ctx {
   std::vector<const char*> stName;
   std::vector<float> stMs;
   int64_t launches = 0;
-  // fe_match_descriptors*, fe_register_matches* and fe_odometry*: a workspace per family, so that a call leaves the
-  // last batch call's results and the other families' results alone (fe_register_matches_device and
+  // fe_match_descriptors*, fe_register_matches*, fe_odometry* and fe_loop_closures*: a workspace per family, so that a
+  // call leaves the last batch call's results and the other families' results alone (fe_register_matches_device and
   // fe_odometry_device may read `best` straight out of matchWs)
-  Workspace matchWs, regWs, odoWs;
+  Workspace matchWs, regWs, odoWs, loopWs;
   bool matchAttrs = false;
   std::string err;
 };
@@ -1251,7 +1252,7 @@ void fe_destroy(fe_ctx_t* ctx) {
   if (ctx->h_desc) cudaFreeHost(ctx->h_desc);
   if (ctx->h_cloud) cudaFreeHost(ctx->h_cloud);
   if (ctx->h_kc) cudaFreeHost(ctx->h_kc);
-  for (Workspace* w : {&ctx->matchWs, &ctx->regWs, &ctx->odoWs}) free_ws(*w);
+  for (Workspace* w : {&ctx->matchWs, &ctx->regWs, &ctx->odoWs, &ctx->loopWs}) free_ws(*w);
   delete ctx;
 }
 
@@ -1584,7 +1585,7 @@ int grow_device(fe_ctx* ctx, T** buf, int64_t* cap, int64_t need) {
   return FE_OK;
 }
 
-// What a match, register or odometry call does once its arguments have passed: clear the last error, select the
+// What a match, register, odometry or loop-closure call does once its arguments have passed: clear the last error, select the
 // context's device and hand out slot 0's stream (the slot is opened; none of its arrays are allocated).
 int begin_call(fe_ctx* ctx, cudaStream_t* stream) {
   ctx->err.clear();
@@ -2044,6 +2045,274 @@ int fe_odometry_device(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypo
                        const int64_t* best, const int64_t* sequence_offsets, int32_t n_sequences, int32_t window,
                        const fe_register_params_t* params, fe_odometry_result_t* out) {
   return odometry(ctx, kp, keypoint_offsets, n_scans, best, sequence_offsets, n_sequences, window, params, out, true);
+}
+
+}  // extern "C"
+
+// ---- loop closures (fe_loop.cu) ------------------------------------------------------------------------------
+
+namespace {
+
+// both entry points: keypoints and descriptor rows are device memory (onDevice) or host memory to upload
+int loop_closures(fe_ctx* ctx, const fe_point_t* kp, const float* desc, int64_t stride, const int64_t* ko, int32_t B,
+                  const int64_t* so, int32_t S, const fe_loop_params_t* lp, const fe_register_params_t* prm,
+                  fe_loop_result_t* out, bool onDevice) {
+  if (!ctx || !out) return FE_ERR_INVALID;
+  fe_register::Params rp;
+  if (int st = register_params(ctx, prm, &rp)) return st;
+  if (!lp) return fail(ctx, FE_ERR_INVALID, "loop_params is NULL");
+  const int K = lp->candidates, gap = lp->min_gap;
+  if (K < 1 || K > fe_loop::MAX_CANDIDATES) return fail(ctx, FE_ERR_INVALID, "candidates must be in [1, 16]");
+  if (gap < 1) return fail(ctx, FE_ERR_INVALID, "min_gap must be >= 1");
+  if (stride < FE_DESC_LEN) return fail(ctx, FE_ERR_INVALID, "the descriptor row stride is below FE_DESC_LEN");
+  if (B < 0 || S < 0) return fail(ctx, FE_ERR_INVALID, "n_scans and n_sequences must not be negative");
+  if (!ko || !so) return fail(ctx, FE_ERR_INVALID, "keypoint_offsets and sequence_offsets need n_scans + 1 and n_sequences + 1 entries");
+  if (const char* e = check_offsets(ko, B)) return fail(ctx, FE_ERR_INVALID, std::string("keypoint_offsets: ") + e);
+  if (const char* e = check_offsets(so, S)) return fail(ctx, FE_ERR_INVALID, std::string("sequence_offsets: ") + e);
+  if (so[0] != 0 || so[S] != B) return fail(ctx, FE_ERR_INVALID, "sequence_offsets must run from 0 to n_scans");
+  for (int32_t b = 0; b < B; b++)
+    if (ko[b + 1] - ko[b] >= (1LL << 24)) return fail(ctx, FE_ERR_INVALID, "a scan has 2^24 or more keypoints");
+  const int64_t nRows = ko[B] - ko[0];
+  if (nRows >= (1LL << 31)) return fail(ctx, FE_ERR_INVALID, "more than 2^31 - 1 keypoint rows");
+  if (nRows > 0 && (!kp || !desc)) return fail(ctx, FE_ERR_INVALID, "kp or desc is NULL but there are keypoints");
+
+  // the tables: eligible scans, retrieval items (scan t against its database, segment outer as match_descriptors lays
+  // them out), and K verification slots per eligible scan, sized for the largest scan of its sequence
+  const int64_t QT = fe_match::ITEM_QUERIES, RS = fe_match::ITEM_REFS;
+  std::vector<int> elig((size_t)B, -1);
+  std::vector<fe_loop::Scan> scans;
+  std::vector<fe_loop::Slot> slots;
+  std::vector<fe_match::Item> items1, items2;
+  std::vector<int64_t> qo{0}, ro{0};
+  int64_t nPart1 = 0, nPart2 = 0, nQ = 0, nR = 0;
+  auto tile_items = [&](std::vector<fe_match::Item>& items, int64_t q0, int64_t nq, int64_t r0, int64_t nr, int64_t nseg,
+                        int64_t out0, int64_t* nPart) {
+    for (int64_t sg = 0; sg < nseg; sg++)
+      for (int64_t t = 0; t < nq; t += QT) {
+        fe_match::Item I;
+        I.q0 = q0 + t;
+        I.r0 = r0 + sg * RS;
+        I.out = out0 + t;
+        I.part = nseg > 1 ? *nPart + t * nseg : 0;
+        I.nq = (int32_t)std::min(QT, nq - t);
+        I.nr = (int32_t)std::max<int64_t>(0, std::min(RS, nr - sg * RS));
+        I.nseg = (int32_t)nseg;
+        I.seg = (int32_t)sg;
+        items.push_back(I);
+      }
+    if (nseg > 1) *nPart += nq * nseg;
+  };
+  for (int32_t q = 0; q < S; q++) {
+    int64_t cap = 0;
+    for (int64_t s = so[q]; s < so[q + 1]; s++) cap = std::max(cap, ko[s + 1] - ko[s]);
+    const int64_t nseg2 = std::max<int64_t>((cap + RS - 1) / RS, 1);
+    for (int64_t s = so[q] + gap; s < so[q + 1]; s++) {
+      elig[(size_t)s] = (int)scans.size();
+      scans.push_back({(int)s, (int)so[q]});
+      const int64_t nq = ko[s + 1] - ko[s], nr = ko[s - gap + 1] - ko[so[q]];
+      tile_items(items1, ko[s], nq, ko[so[q]], nr, std::max<int64_t>((nr + RS - 1) / RS, 1), ko[s] - ko[0], &nPart1);
+      for (int k = 0; k < K; k++) {
+        fe_loop::Slot sl;
+        sl.q0 = nQ;
+        sl.r0 = nR;
+        sl.cap = cap;
+        sl.item0 = (int64_t)items2.size();
+        sl.tiles = (int32_t)((nq + QT - 1) / QT);
+        sl.nseg = (int32_t)nseg2;
+        slots.push_back(sl);
+        tile_items(items2, ko[s], nq, 0, 0, nseg2, nQ, &nPart2);  // r0 and nr are k_loop_place's to write
+        nQ += nq;
+        qo.push_back(nQ);
+        qo.push_back(nQ);
+        ro.push_back(nR);  // the start of the slot's unused tail: k_loop_place writes it
+        nR += cap;
+        ro.push_back(nR);
+      }
+    }
+  }
+  const int E = (int)scans.size(), nSlots = (int)slots.size();
+  if ((int64_t)items1.size() >= (1LL << 31) || (int64_t)items2.size() >= (1LL << 31))
+    return fail(ctx, FE_ERR_INVALID, "too many query tiles x reference segments");
+  cudaStream_t stream;
+  if (int st = begin_call(ctx, &stream)) return st;
+
+  Workspace& ws = ctx->loopWs;
+  const int64_t BK = (int64_t)B * K, G = 2 * (int64_t)nSlots;
+  Carve c;  // results | tables (uploaded) | retrieval, slots, registration and the host variant's rows (device only)
+  const Span<double> pose = c.take<double>(4 * (int64_t)B), rms = c.take<double>(B);
+  const Span<double> cPose = c.take<double>(4 * BK), cRms = c.take<double>(BK);
+  const Span<int64_t> assoc = c.take<int64_t>(nRows);
+  const Span<int32_t> loop = c.take<int32_t>(B), loopScan = c.take<int32_t>(B), nInl = c.take<int32_t>(B);
+  const Span<int32_t> nHyp = c.take<int32_t>(B), cScan = c.take<int32_t>(BK), cVotes = c.take<int32_t>(BK);
+  const Span<int32_t> cStatus = c.take<int32_t>(BK), cInl = c.take<int32_t>(BK), cHyp = c.take<int32_t>(BK);
+  const int64_t resBytes = c.bytes;
+  const Span<int64_t> tKo = c.take<int64_t>((int64_t)B + 1);
+  const Span<int32_t> tElig = c.take<int32_t>(B);
+  const Span<fe_loop::Scan> tScans = c.take<fe_loop::Scan>(E);
+  const Span<fe_loop::Slot> tSlots = c.take<fe_loop::Slot>(nSlots);
+  const Span<fe_match::Item> tItems1 = c.take<fe_match::Item>((int64_t)items1.size());
+  const Span<fe_match::Item> tItems2 = c.take<fe_match::Item>((int64_t)items2.size());
+  const Span<int64_t> tQo = c.take<int64_t>((int64_t)qo.size()), tRo = c.take<int64_t>((int64_t)ro.size());
+  const int64_t hostBytes = c.bytes;
+  const Span<int64_t> best1 = c.take<int64_t>(nRows);
+  const Span<int32_t> shift1 = c.take<int32_t>(nRows), voteScan = c.take<int32_t>(nRows);
+  const Span<float> dist1 = c.take<float>(nRows), second1 = c.take<float>(nRows);
+  const Span<uint64_t> voteKey = c.take<uint64_t>(nRows);
+  const Span<fe_match::Partial> part1 = c.take<fe_match::Partial>(nPart1), part2 = c.take<fe_match::Partial>(nPart2);
+  const Span<fe_point_t> wQ = c.take<fe_point_t>(nQ), wR = c.take<fe_point_t>(nR);
+  const Span<int64_t> best2 = c.take<int64_t>(nQ), slotBest = c.take<int64_t>(nQ);
+  const Span<int32_t> shift2 = c.take<int32_t>(nQ);
+  const Span<float> dist2 = c.take<float>(nQ), second2 = c.take<float>(nQ);
+  const Span<double> gPose = c.take<double>(4 * G), gRms = c.take<double>(G);
+  const Span<int64_t> gAssoc = c.take<int64_t>(nQ), gAssocNew = c.take<int64_t>(nQ);
+  const Span<double> gD2Cur = c.take<double>(nQ), gD2New = c.take<double>(nQ);
+  const Span<int32_t> gNInl = c.take<int32_t>(G), gNHyp = c.take<int32_t>(G), gStatus = c.take<int32_t>(G);
+  const Span<int32_t> gCorr = c.take<int32_t>(nQ), gErr = c.take<int32_t>(1);
+  // the host variant's rows [ko[0], ko[B]); the last descriptor row ends FE_DESC_LEN floats in
+  const int64_t df = onDevice || nRows == 0 ? 0 : (nRows - 1) * stride + FE_DESC_LEN;
+  const Span<fe_point_t> kpRows = c.take<fe_point_t>(onDevice ? 0 : nRows);
+  const Span<float> descRows = c.take<float>(df);
+  int st = grow_pinned(ctx, &ws.h, &ws.hCap, hostBytes, 4096, 0);
+  if (st) return st;
+  out->n_scans = B;
+  out->candidates = K;
+  out->n_rows = nRows;
+  out->loop = loop.in(ws.h);
+  out->loop_scan = loopScan.in(ws.h);
+  out->pose = pose.in(ws.h);
+  out->rms = rms.in(ws.h);
+  out->n_inliers = nInl.in(ws.h);
+  out->n_hypotheses = nHyp.in(ws.h);
+  out->cand_scan = cScan.in(ws.h);
+  out->cand_votes = cVotes.in(ws.h);
+  out->cand_status = cStatus.in(ws.h);
+  out->cand_inliers = cInl.in(ws.h);
+  out->cand_hypotheses = cHyp.in(ws.h);
+  out->cand_rms = cRms.in(ws.h);
+  out->cand_pose = cPose.in(ws.h);
+  out->assoc = assoc.in(ws.h);
+  out->gpu_launches = 0;
+  if (B == 0) return FE_OK;
+
+  if ((st = grow_device(ctx, &ws.d, &ws.dCap, c.bytes))) return st;
+  memcpy(tKo.in(ws.h), ko, 8 * ((size_t)B + 1));
+  memcpy(tElig.in(ws.h), elig.data(), 4 * (size_t)B);
+  if (E) memcpy(tScans.in(ws.h), scans.data(), sizeof(fe_loop::Scan) * scans.size());
+  if (nSlots) memcpy(tSlots.in(ws.h), slots.data(), sizeof(fe_loop::Slot) * slots.size());
+  if (!items1.empty()) memcpy(tItems1.in(ws.h), items1.data(), sizeof(fe_match::Item) * items1.size());
+  if (!items2.empty()) memcpy(tItems2.in(ws.h), items2.data(), sizeof(fe_match::Item) * items2.size());
+  memcpy(tQo.in(ws.h), qo.data(), 8 * qo.size());
+  memcpy(tRo.in(ws.h), ro.data(), 8 * ro.size());
+  CK(cudaMemcpyAsync(ws.d + resBytes, ws.h + resBytes, (size_t)(hostBytes - resBytes), cudaMemcpyHostToDevice, stream));
+  int64_t bias = 0;
+  if (!onDevice) {
+    if ((st = upload(ctx, kp, kpRows.in(ws.d), ko[0], nRows, stream))) return st;
+    if ((st = upload(ctx, desc, descRows.in(ws.d), ko[0] * stride, df, stream))) return st;
+    bias = ko[0];
+  }
+  if (!ctx->matchAttrs) {
+    CK(fe_match::set_attributes());
+    ctx->matchAttrs = true;
+  }
+  fe_loop::Tables T;
+  T.ko = tKo.in(ws.d);
+  T.elig = tElig.in(ws.d);
+  T.scans = tScans.in(ws.d);
+  T.slots = tSlots.in(ws.d);
+  T.items = tItems2.in(ws.d);
+  T.qo = tQo.in(ws.d);
+  T.ro = tRo.in(ws.d);
+  fe_loop::Out o;
+  o.loop = loop.in(ws.d);
+  o.loopScan = loopScan.in(ws.d);
+  o.nInl = nInl.in(ws.d);
+  o.nHyp = nHyp.in(ws.d);
+  o.pose = pose.in(ws.d);
+  o.rms = rms.in(ws.d);
+  o.cScan = cScan.in(ws.d);
+  o.cVotes = cVotes.in(ws.d);
+  o.cStatus = cStatus.in(ws.d);
+  o.cInl = cInl.in(ws.d);
+  o.cHyp = cHyp.in(ws.d);
+  o.cRms = cRms.in(ws.d);
+  o.cPose = cPose.in(ws.d);
+  o.assoc = (long long*)assoc.in(ws.d);
+  fe_loop::Work w;
+  w.best1 = (const long long*)best1.in(ws.d);
+  w.voteScan = voteScan.in(ws.d);
+  w.voteKey = (unsigned long long*)voteKey.in(ws.d);
+  w.q = wQ.in(ws.d);
+  w.r = wR.in(ws.d);
+  w.best2 = (long long*)best2.in(ws.d);
+  w.slotBest = (long long*)slotBest.in(ws.d);
+  w.reg.pose = gPose.in(ws.d);
+  w.reg.rms = gRms.in(ws.d);
+  w.reg.assoc = (long long*)gAssoc.in(ws.d);
+  w.reg.nInl = gNInl.in(ws.d);
+  w.reg.nHyp = gNHyp.in(ws.d);
+  w.reg.status = gStatus.in(ws.d);
+  w.reg.err = gErr.in(ws.d);
+  w.scratch.corr = gCorr.in(ws.d);
+  w.scratch.assocNew = (long long*)gAssocNew.in(ws.d);
+  w.scratch.d2Cur = gD2Cur.in(ws.d);
+  w.scratch.d2New = gD2New.in(ws.d);
+  fe_match::Result r1, r2;
+  r1.best = (long long*)best1.in(ws.d);
+  r1.shift = shift1.in(ws.d);
+  r1.dist2 = dist1.in(ws.d);
+  r1.second = second1.in(ws.d);
+  r2.best = w.best2;
+  r2.shift = shift2.in(ws.d);
+  r2.dist2 = dist2.in(ws.d);
+  r2.second = second2.in(ws.d);
+
+  // retrieval, votes, slots, verification matching, remap, registration, choice: one stream, no round trip
+  int64_t launches = 0;
+  const int n1 = (int)items1.size(), n2 = (int)items2.size();
+  CK(fe_match::launch(desc, stride, bias, desc, stride, bias, tItems1.in(ws.d), n1, nPart1 > 0, part1.in(ws.d), r1, stream));
+  launches += n1 ? (nPart1 > 0 ? 2 : 1) : 0;
+  CK(fe_loop::vote(E, K, gap, T, w, o, stream));
+  CK(fe_loop::place(kp, bias, nSlots, K, T, w, o, stream));
+  CK(fe_match::launch(desc, stride, bias, desc, stride, bias, T.items, n2, nPart2 > 0, part2.in(ws.d), r2, stream));
+  launches += n2 ? (nPart2 > 0 ? 2 : 1) : 0;
+  CK(fe_loop::remap(nSlots, K, T, w, o, stream));
+  if (nSlots > 0) {
+    CK(cudaMemsetAsync(w.reg.err, 0, sizeof(int32_t), stream));
+    CK(fe_register::launch(w.q, 0, w.r, 0, w.slotBest, T.qo, T.ro, (int)G, rp, w.reg, w.scratch, stream));
+  }
+  CK(fe_loop::select(B, K, T, w, o, stream));
+  launches += (E > 0) + 3 * (nSlots > 0) + 1;
+  ctx->launches += launches;
+  out->gpu_launches = launches;
+  CK(cudaMemcpyAsync(ws.h, ws.d, (size_t)resBytes, cudaMemcpyDeviceToHost, stream));
+  CK(cudaStreamSynchronize(stream));
+  return FE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+void fe_loop_params_default(fe_loop_params_t* p) {
+  if (!p) return;
+  p->min_gap = FE_LOOP_MIN_GAP_DEFAULT;
+  p->candidates = FE_LOOP_CANDIDATES_DEFAULT;
+}
+
+int fe_loop_closures(fe_ctx_t* ctx, const fe_point_t* kp, const float* desc, int64_t desc_stride,
+                     const int64_t* keypoint_offsets, int32_t n_scans, const int64_t* sequence_offsets,
+                     int32_t n_sequences, const fe_loop_params_t* loop_params, const fe_register_params_t* params,
+                     fe_loop_result_t* out) {
+  return loop_closures(ctx, kp, desc, desc_stride, keypoint_offsets, n_scans, sequence_offsets, n_sequences, loop_params,
+                       params, out, false);
+}
+
+int fe_loop_closures_device(fe_ctx_t* ctx, const fe_point_t* kp, const float* desc, int64_t desc_stride,
+                            const int64_t* keypoint_offsets, int32_t n_scans, const int64_t* sequence_offsets,
+                            int32_t n_sequences, const fe_loop_params_t* loop_params,
+                            const fe_register_params_t* params, fe_loop_result_t* out) {
+  return loop_closures(ctx, kp, desc, desc_stride, keypoint_offsets, n_scans, sequence_offsets, n_sequences, loop_params,
+                       params, out, true);
 }
 
 // ---- one entry point per reference function ----------------------------------------------------------

@@ -136,6 +136,30 @@ def _unpack_odometry(res):
             "n_hypotheses": _copy_out(res.n_hypotheses, (B,), np.int32), "assoc": _copy_out(res.assoc, (n,), np.int64)}
 
 
+def loop_params_default(**overrides):
+    """fe_loop_params_default, with any field overridden by keyword."""
+    p = N.LoopParams()
+    N.lib().fe_loop_params_default(C.byref(p))
+    for k, v in overrides.items():
+        if not hasattr(p, k):
+            raise ValueError("fe_loop_params_t has no field %r" % k)
+        setattr(p, k, v)
+    return p
+
+
+def _unpack_loop(res):
+    B, K, n = int(res.n_scans), int(res.candidates), int(res.n_rows)
+    return {"loop": _copy_out(res.loop, (B,), np.int32), "loop_scan": _copy_out(res.loop_scan, (B,), np.int32),
+            "pose": _copy_out(res.pose, (B, 4), np.float64), "rms": _copy_out(res.rms, (B,), np.float64),
+            "n_inliers": _copy_out(res.n_inliers, (B,), np.int32), "n_hypotheses": _copy_out(res.n_hypotheses, (B,), np.int32),
+            "cand_scan": _copy_out(res.cand_scan, (B, K), np.int32), "cand_votes": _copy_out(res.cand_votes, (B, K), np.int32),
+            "cand_status": _copy_out(res.cand_status, (B, K), np.int32),
+            "cand_inliers": _copy_out(res.cand_inliers, (B, K), np.int32),
+            "cand_hypotheses": _copy_out(res.cand_hypotheses, (B, K), np.int32),
+            "cand_rms": _copy_out(res.cand_rms, (B, K), np.float64), "cand_pose": _copy_out(res.cand_pose, (B, K, 4), np.float64),
+            "assoc": _copy_out(res.assoc, (n,), np.int64)}
+
+
 def _odometry_offsets(keypoint_offsets, sequence_offsets, n_rows):
     """Validate the scans and sequences of an odometry call before raw pointers cross the C-ABI."""
     ko = np.ascontiguousarray(keypoint_offsets, np.int64).reshape(-1)
@@ -479,6 +503,48 @@ class FeatureExtractionNode:
         out = self.odometry(kp, ko, best, sequence_offsets, window, params)
         out["best"] = best
         return out
+
+    def loopClosures(self, kp, descriptors, keypoint_offsets, sequence_offsets, loop_params=None, params=None):
+        """fe_loop_closures: for every scan, the earlier scan of its sequence it sees again, retrieved by descriptor votes
+        and verified by matching and registration (include/fe_b200.h, "loop closures").  kp: (K, 4) host keypoints and
+        descriptors (K, 1980) bins or (K, 1996) records, both addressed by absolute row; sequence_offsets in scans.
+        -> dict of loop (B,) int32 (rank of the loop among the candidates, -1 none), loop_scan (B,) int32, pose (B, 4)
+        {c, s, tx, ty} (scan xy -> loop scan xy), rms (B,), n_inliers, n_hypotheses (B,) int32; cand_scan, cand_votes,
+        cand_status, cand_inliers, cand_hypotheses (B, candidates) int32, cand_rms (B, candidates), cand_pose
+        (B, candidates, 4); assoc (ko[B] - ko[0],) int64 (the loop scan's row each row is an inlier of, -1 none)."""
+        k = _keypoint_rows(kp)
+        d, stride, dp = _descriptor_rows(descriptors)
+        ko, so, B, S = _odometry_offsets(keypoint_offsets, sequence_offsets, min(len(k), len(d)))
+        lp = loop_params if loop_params is not None else loop_params_default()
+        prm = params if params is not None else register_params_default()
+        res = N.LoopResult()
+        self._check(N.lib().fe_loop_closures(self._ctx, _ptr(k) if len(k) else None, dp, stride, _ptr(ko), B, _ptr(so), S,
+                                             C.byref(lp), C.byref(prm), C.byref(res)))
+        self.last_launches = int(res.gpu_launches)
+        return _unpack_loop(res)
+
+    def loopClosuresDevice(self, kp_ptr, desc_ptr, desc_stride, keypoint_offsets, sequence_offsets, loop_params=None,
+                           params=None):
+        """fe_loop_closures_device: keypoints and descriptor rows already in HBM (e.g. processBatchDevice's; a record
+        pointer must point at its first bin, record base + 5 floats), queued on the context's stream behind the batch
+        call.  Same results as loopClosures."""
+        if int(desc_stride) < DESC_LEN:
+            raise ValueError("the descriptor row stride must be at least %d floats, got %d" % (DESC_LEN, int(desc_stride)))
+        ko, so, B, S = _odometry_offsets(keypoint_offsets, sequence_offsets, None)  # the device buffers' sizes are the caller's
+        if ko[-1] > ko[0] and not (kp_ptr and desc_ptr):
+            raise ValueError("a device pointer is NULL while there are keypoints")
+        lp = loop_params if loop_params is not None else loop_params_default()
+        prm = params if params is not None else register_params_default()
+        res = N.LoopResult()
+        self._check(N.lib().fe_loop_closures_device(self._ctx, C.c_void_p(kp_ptr), C.c_void_p(desc_ptr), int(desc_stride),
+                                                    _ptr(ko), B, _ptr(so), S, C.byref(lp), C.byref(prm), C.byref(res)))
+        self.last_launches = int(res.gpu_launches)
+        return _unpack_loop(res)
+
+    def sequence_loop_closures(self, ko, kp, descriptors, sequence_offsets, loop_params=None, params=None):
+        """Loop closures of the scans of one batch result (processBatch's keypoint_offsets, keypoints, descriptors), cut
+        into sequences by sequence_offsets (in scans), beside sequence_odometry.  -> loopClosures' dict."""
+        return self.loopClosures(kp, descriptors, ko, sequence_offsets, loop_params, params)
 
     def download(self, device_ptr, shape, dtype=np.float32):
         """Copy a device-resident result of processBatchDevice to a new host array."""

@@ -465,6 +465,102 @@ int fe_odometry_device(fe_ctx_t* ctx, const fe_point_t* kp, const int64_t* keypo
                        const int64_t* best, const int64_t* sequence_offsets, int32_t n_sequences, int32_t window,
                        const fe_register_params_t* params, fe_odometry_result_t* out);
 
+/* ---- loop closures: which earlier scan of its sequence a scan sees again, and the motion to it ------------------ */
+/* Every scan is compared with the earlier scans of its own sequence: descriptor votes retrieve candidate scans, and
+ * matching plus registration verify each candidate.  The best verified candidate is the scan's loop constraint, a
+ * measured motion that a pose-graph back end can use against odometry's drift.  Evaluated to the last bit as follows.
+ *
+ * Inputs.  Keypoints `kp` and descriptor rows `desc` (row stride >= FE_DESC_LEN floats, as the matcher takes them),
+ * addressed by absolute row with the batch's keypoint_offsets ko[0..B] (scan b owns rows [ko[b], ko[b+1])).
+ * sequence_offsets so[0..S] exactly as odometry defines them.  fe_loop_params_t, and registration parameters as
+ * fe_register_matches takes them.
+ *
+ * Eligible scans.  Local scan t of sequence q (absolute scan s = so[q] + t) is eligible when t >= min_gap.  Its
+ * database is the rows of scans so[q] .. s - min_gap: the absolute rows [ko[so[q]], ko[s - min_gap + 1]).  Other
+ * sequences are never in it.
+ *
+ * Retrieval.  Every row of an eligible scan gets the matcher's `best` over its database: the group (the scan's rows,
+ * the database's rows) exactly as fe_match_descriptors specifies, the minimum over the 12 shifts ordered by (d, r, s).
+ * A row with best = -1 casts no vote; every other row casts one vote for the scan j that holds its best row.  There is
+ * no ratio test: the same pole seen from neighbouring earlier scans gives near-identical rows, so second_dist2 over a
+ * database carries no information.  The candidates are the scans with at least one vote, ordered by votes descending,
+ * then scan index ascending; at most `candidates` of them are kept, and their order is the candidate rank k.
+ *
+ * Verification of candidate k = scan j.  The group (scan t's rows, scan j's rows) is matched exactly as
+ * fe_match_descriptors specifies, which gives a fresh `best` into scan j, and that group is registered exactly as
+ * fe_register_matches specifies: a motion mapping scan t's levelled xy into scan j's, with its status, counts and rms.
+ * No placement and no odometry input: the library's own motion estimate is not trusted across a loop.
+ *
+ * Choice.  The loop of scan t is the candidate with status 2 that has the most inliers, the lower rank on ties; a scan
+ * without such a candidate has no loop.
+ *
+ * Outputs (context-owned pinned memory, valid until the next loop-closure call; a loop-closure call leaves the results
+ * of batch, match, register and odometry calls alone, and they leave its results alone).  Per scan: loop (rank k or
+ * -1), loop_scan (absolute scan j or -1), and the winner's pose, rms, n_inliers and n_hypotheses ((1, 0, 0, 0) and 0
+ * without a loop).  Per scan x candidates, rank k at [s * candidates + k]: cand_scan (absolute scan, -1 where there are
+ * fewer voted scans), cand_votes, and the candidate's registration status, n_inliers, n_hypotheses, rms and pose;
+ * where cand_scan is -1 the votes are 0, the status -1, the pose (1, 0, 0, 0) and everything else 0.  A scan that is
+ * not eligible has loop -1 and every candidate -1.  Per keypoint row of [ko[0], ko[B]): assoc under the winner's
+ * registration, an absolute row of scan j, or -1 (every row of a scan without a loop).
+ *
+ * Cost.  Retrieval compares sum over eligible scans of n_t * |database_t| descriptor pairs, quadratic in the length of
+ * a sequence: a caller bounds it by how they cut sequences.  Verification is `candidates` scan-pair matches and
+ * registrations per eligible scan.  A call is a fixed chain of at most 9 launches whatever the sequence length
+ * (retrieval match and merge, votes, slot placement, verification match and merge, remap, registration, choice), with
+ * no host round trip in between.
+ *
+ * FE_ERR_INVALID (the context stays usable) on the argument errors of fe_register_matches' parameters, when params or
+ * loop_params is NULL, candidates is outside [1, 16], min_gap < 1, the descriptor stride is below FE_DESC_LEN, an
+ * offsets array is NULL, decreases or has a negative entry, sequence_offsets does not run from 0 to B, B or S is
+ * negative, a scan has 2^24 or more rows, or `kp` or `desc` is NULL while [ko[0], ko[B]) holds rows.  B = 0, S = 0,
+ * empty scans and empty sequences are not errors. */
+typedef struct fe_loop_params {
+  int32_t min_gap;     /* a scan's database ends this many scans before it */
+  int32_t candidates;  /* scans verified per eligible scan, in [1, 16]     */
+} fe_loop_params_t;
+
+/* The setting of the loop evaluation (DESIGN.md §15): the largest found fraction with no wrong loop, the smallest
+ * `candidates` on ties.  min_gap 3 with 4 or more candidates lets one 90 deg lattice alias through. */
+#define FE_LOOP_MIN_GAP_DEFAULT 10
+#define FE_LOOP_CANDIDATES_DEFAULT 8
+
+/* FE_LOOP_MIN_GAP_DEFAULT, FE_LOOP_CANDIDATES_DEFAULT. */
+void fe_loop_params_default(fe_loop_params_t* p);
+
+typedef struct fe_loop_result {
+  int32_t n_scans;
+  int32_t candidates;
+  int64_t n_rows;                   /* ko[B] - ko[0]                                                  */
+  const int32_t* loop;              /* n_scans: rank of the loop among the candidates, -1 = none      */
+  const int32_t* loop_scan;         /* n_scans: absolute scan of the loop, -1 = none                  */
+  const double* pose;               /* n_scans x {c, s, tx, ty}: scan xy -> loop scan xy              */
+  const double* rms;                /* n_scans                                                        */
+  const int32_t* n_inliers;         /* n_scans                                                        */
+  const int32_t* n_hypotheses;      /* n_scans                                                        */
+  const int32_t* cand_scan;         /* n_scans x candidates: absolute scan, -1 = none                 */
+  const int32_t* cand_votes;        /* n_scans x candidates                                           */
+  const int32_t* cand_status;       /* n_scans x candidates: registration status, -1 = no candidate   */
+  const int32_t* cand_inliers;      /* n_scans x candidates                                           */
+  const int32_t* cand_hypotheses;   /* n_scans x candidates                                           */
+  const double* cand_rms;           /* n_scans x candidates                                           */
+  const double* cand_pose;          /* n_scans x candidates x {c, s, tx, ty}                          */
+  const int64_t* assoc;             /* n_rows: absolute row of the loop scan's keypoint, -1 = none    */
+  int64_t gpu_launches;             /* kernels the call launched                                      */
+} fe_loop_result_t;
+
+/* Keypoints and descriptors in host memory: only rows [ko[0], ko[B]) are uploaded. */
+int fe_loop_closures(fe_ctx_t* ctx, const fe_point_t* kp, const float* desc, int64_t desc_stride,
+                     const int64_t* keypoint_offsets, int32_t n_scans, const int64_t* sequence_offsets,
+                     int32_t n_sequences, const fe_loop_params_t* loop_params, const fe_register_params_t* params,
+                     fe_loop_result_t* out);
+/* `kp` and `desc` in device memory, e.g. the `keypoints` and `descriptors` of fe_process_batch_device (a record pointer
+ * must point at its first bin).  Runs on the context's stream behind the batch call, with no synchronisation in
+ * between. */
+int fe_loop_closures_device(fe_ctx_t* ctx, const fe_point_t* kp, const float* desc, int64_t desc_stride,
+                            const int64_t* keypoint_offsets, int32_t n_scans, const int64_t* sequence_offsets,
+                            int32_t n_sequences, const fe_loop_params_t* loop_params,
+                            const fe_register_params_t* params, fe_loop_result_t* out);
+
 /* CUDA-event stopwatch on the context's stream (the stream every kernel of
  * fe_process_batch_device is launched on): begin, run any number of calls, end -> elapsed ms. */
 int fe_timer_begin(fe_ctx_t* ctx);

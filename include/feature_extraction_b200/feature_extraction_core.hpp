@@ -179,6 +179,30 @@ class FeatureExtractionCore {
     if (sources) sources->assign(r.source, r.source + B);
   }
 
+  // Loop closures of one sequence of scans (fe_loop_closures, one sequence): `keypoints` and `descriptors`
+  // (FE_DESC_LEN floats a keypoint) concatenated in scan order with keypointOffsets (n_scans + 1 entries).  loopScans
+  // gets, per scan, the earlier scan it sees again or -1; poses n_scans x {c, s, tx, ty}, scan xy into that scan's
+  // frame ((1, 0, 0, 0) without a loop).
+  void loopClosures(const PointCloud& keypoints, const std::vector<float>& descriptors,
+                    const std::vector<int64_t>& keypointOffsets, std::vector<int32_t>& loopScans, std::vector<double>& poses,
+                    const fe_loop_params_t* loopParams = nullptr, const fe_register_params_t* params = nullptr) {
+    if (keypointOffsets.empty()) throw std::runtime_error("loopClosures: keypointOffsets needs n_scans + 1 entries");
+    const int32_t B = (int32_t)keypointOffsets.size() - 1;
+    if (keypointOffsets[B] > (int64_t)keypoints.size() || keypointOffsets[B] * FE_DESC_LEN > (int64_t)descriptors.size())
+      throw std::runtime_error("loopClosures: keypointOffsets exceed the keypoints or descriptors");
+    fe_register_params_t p;
+    fe_register_params_default(&p);
+    fe_loop_params_t lp;
+    fe_loop_params_default(&lp);
+    const int64_t so[2] = {0, B};
+    fe_loop_result_t r;
+    check(fe_loop_closures(ctx_, keypoints.data(), descriptors.data(), FE_DESC_LEN, keypointOffsets.data(), B, so, 1,
+                           loopParams ? loopParams : &lp, params ? params : &p, &r),
+          "loopClosures");
+    loopScans.assign(r.loop_scan, r.loop_scan + B);
+    poses.assign(r.pose, r.pose + 4 * (int64_t)B);
+  }
+
   fe_ctx_t* context() { return ctx_; }
 
  private:

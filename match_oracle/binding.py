@@ -1,5 +1,6 @@
 """ctypes binding of match_oracle/libfe_match_oracle.so: the CPU restatements of fe_match_descriptors,
-fe_register_matches and fe_odometry (include/fe_b200.h, "descriptor matching", "registration", "odometry").
+fe_register_matches, fe_odometry and fe_loop_closures (include/fe_b200.h, "descriptor matching", "registration",
+"odometry", "loop closures").
 
 TEST INFRASTRUCTURE ONLY, like oracle/oracle_binding.py: never imported by the feature_extraction_b200 package.
 """
@@ -111,4 +112,37 @@ def odometry(kp, keypoint_offsets, best, sequence_offsets, window=1, inlier_radi
         _p(out["status"]), _p(out["n_inliers"]), _p(out["n_hypotheses"]), _p(out["assoc"]))
     if st != 0:
         raise ValueError("feo_odometry: invalid argument")
+    return {key: (v[:n] if key == "assoc" else v[:B]) for key, v in out.items()}
+
+
+def loop_closures(kp, descriptors, keypoint_offsets, sequence_offsets, min_gap, candidates, inlier_radius=0.5,
+                  min_separation=1.0, max_hypotheses=512, min_inliers=16, refine_iterations=4, n_threads=1):
+    """feo_loop_closures on the CPU.  kp: (K, 4) float32 keypoints and descriptors (K, 1980) bins or (K, 1996) records,
+    both addressed by absolute row; keypoint_offsets (B + 1,); sequence_offsets (S + 1,) in scans.  -> dict of loop,
+    loop_scan (B,) int32, pose (B, 4), rms (B,), n_inliers, n_hypotheses (B,) int32; cand_scan, cand_votes, cand_status,
+    cand_inliers, cand_hypotheses (B, candidates) int32, cand_rms (B, candidates), cand_pose (B, candidates, 4); assoc
+    (ko[B] - ko[0],) int64."""
+    k = np.ascontiguousarray(kp, np.float32).reshape(-1, 4)
+    d = np.ascontiguousarray(descriptors, np.float32)
+    assert d.ndim == 2 and d.shape[1] in (DESC_LEN, RECORD_FLOATS), d.shape
+    first = 5 if d.shape[1] == RECORD_FLOATS else 0
+    ko = np.ascontiguousarray(keypoint_offsets, np.int64)
+    so = np.ascontiguousarray(sequence_offsets, np.int64)
+    B, S = len(ko) - 1, len(so) - 1
+    n = int(ko[-1] - ko[0])
+    m, K = max(B, 1), max(int(candidates), 1)
+    i32 = lambda *sh: np.zeros(sh, np.int32)  # noqa: E731
+    out = {"loop": i32(m), "loop_scan": i32(m), "pose": np.zeros((m, 4)), "rms": np.zeros(m), "n_inliers": i32(m),
+           "n_hypotheses": i32(m), "cand_scan": i32(m, K), "cand_votes": i32(m, K), "cand_status": i32(m, K),
+           "cand_inliers": i32(m, K), "cand_hypotheses": i32(m, K), "cand_rms": np.zeros((m, K)),
+           "cand_pose": np.zeros((m, K, 4)), "assoc": np.zeros(max(n, 1), np.int64)}
+    st = lib().feo_loop_closures(
+        _p(k) if len(k) else None, C.c_void_p(d.ctypes.data + 4 * first if len(d) else None), C.c_int64(d.shape[1]), _p(ko),
+        C.c_int32(B), _p(so), C.c_int32(S), C.c_int32(min_gap), C.c_int32(candidates), C.c_double(inlier_radius),
+        C.c_double(min_separation), C.c_int32(max_hypotheses), C.c_int32(min_inliers), C.c_int32(refine_iterations),
+        C.c_int32(n_threads), *[_p(out[f]) for f in ("loop", "loop_scan", "pose", "rms", "n_inliers", "n_hypotheses",
+                                                      "cand_scan", "cand_votes", "cand_status", "cand_inliers",
+                                                      "cand_hypotheses", "cand_rms", "cand_pose", "assoc")])
+    if st != 0:
+        raise ValueError("feo_loop_closures: invalid argument")
     return {key: (v[:n] if key == "assoc" else v[:B]) for key, v in out.items()}
