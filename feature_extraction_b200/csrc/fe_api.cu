@@ -1390,6 +1390,7 @@ static int process_batch_host(fe_ctx_t* ctx, const unsigned char* points, int st
     while (last < n_scans && (last - first) < s.capScans) {
       const int64_t n = scan_offsets[last + 1] - scan_offsets[last];
       if (n < 0) return fail(ctx, FE_ERR_INVALID, "scan_offsets must be non-decreasing");
+      if (n > FE_MAX_SCAN_POINTS) return fail(ctx, FE_ERR_CAPACITY, "a scan of more than 2^20 points");
       if (n > s.capPts || n * stride > s.capPts * 16) return fail(ctx, FE_ERR_CAPACITY, "a single scan exceeds max_points_per_call");
       if (npts + n > s.capPts || (npts + n) * stride > s.capPts * 16) break;
       npts += n;
@@ -1485,6 +1486,8 @@ int fe_process_batch_device(fe_ctx_t* ctx, const fe_point_t* d_points, const int
   Slot& s = ctx->slot[0];
   int st = ensure_slot(ctx, s, {CORE});
   if (st) return st;
+  for (int i = 0; i < n_scans; i++)
+    if (scan_offsets[i + 1] - scan_offsets[i] > FE_MAX_SCAN_POINTS) return fail(ctx, FE_ERR_CAPACITY, "a scan of more than 2^20 points");
   ctx->kpOffsets.assign((size_t)n_scans + 1, 0);
   if (n_scans > 0) {
     // 2048 scans and more: the levelling matrices are computed while K1 runs (enqueue_pipeline)
@@ -2492,6 +2495,8 @@ int fe_estimate_descriptors(fe_ctx_t* ctx, const fe_point_t* cloud_full, int64_t
   int st = ensure_slot(ctx, s, {CORE, POINTS, GRID});
   if (st) return st;
   if (k > s.capKp) return fail(ctx, FE_ERR_CAPACITY, "more keypoints than max_keypoints_per_call");
+  // the 3DSC order key holds a point's index in 20 bits (include/fe_b200.h, per-scan limits)
+  if (n > FE_MAX_SCAN_POINTS) return fail(ctx, FE_ERR_CAPACITY, "a cloud of more than 2^20 points");
   // the search surface only matters around the keypoints: grid over their bounding box
   float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
   for (int64_t i = 0; i < k; i++) {

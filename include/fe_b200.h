@@ -35,10 +35,23 @@ typedef enum fe_status {
   FE_OK = 0,
   FE_ERR_INVALID = 1,       /* bad argument                                              */
   FE_ERR_CUDA = 2,          /* CUDA runtime error (see fe_last_error)                    */
-  FE_ERR_CAPACITY = 3,      /* an output or workspace capacity would be exceeded         */
+  FE_ERR_CAPACITY = 3,      /* an output or workspace capacity would be exceeded; also  */
+                            /* the two per-scan limits below                             */
   FE_ERR_NO_DEVICE = 4,     /* no usable CUDA device: there is no CPU fallback           */
   FE_ERR_UNSUPPORTED = 5
 } fe_status;
+
+/* Per-scan limits, whatever the context's limits are (a call that exceeds one returns FE_ERR_CAPACITY and the
+ * context stays usable):
+ *   - 2^20 points per scan of fe_process_batch and its variants, and 2^20 points in the cloud of
+ *     fe_estimate_descriptors, finite or not; both are checked on the host.  (The single-function entry points such
+ *     as fe_get_elevation_angles take clouds of any size.)
+ *     The per-scan kernels index at most 512 chunks of 2048 points, and the 3DSC summation order key
+ *     (bin << 52 | float bits of d2 << 20 | point index) holds the point's index in its scan in 20 bits.
+ *   - 65,536 keypoints with at least one 3DSC neighbour per scan, or per fe_estimate_descriptors call: the mt19937
+ *     x axes are a precomputed table of that many entries.  Keypoints without a neighbour (NaN rows) do not count. */
+#define FE_MAX_SCAN_POINTS (1 << 20)
+#define FE_MAX_SCAN_DESCRIBED_KEYPOINTS (1 << 16)
 
 /* pcl::PointXYZI as the reference uses it (feature_extraction_node.h:66) minus PCL's padding:
  * 16 bytes, `intensity` carries the elevation angle in degrees after getElevationAngles. */
